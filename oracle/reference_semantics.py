@@ -152,6 +152,119 @@ def rollout_stats_numpy(d, alpha, beta, dt, params, noise, policy_opt=None, h_st
     return dict(ep_rets=ep_rets, ep_lens=ep_lens, l2=l2_fht if policy_opt is not None else None, all_hit=bool(seen.all()))
 
 
+# --------------------------------------------------------------------------------------------------
+# high-precision replay: the same rollout in float64 (or any dtype), batched, on any device
+# --------------------------------------------------------------------------------------------------
+HIT_ALL_GE_LB, HIT_X0_IN_LB_RB = "all_ge_lb", "x0_in_lb_rb"
+
+
+def rollout_reference(d, alpha, beta, dt, params, noise, *, hit_rule=HIT_ALL_GE_LB, lb=1.0, rb=2.0, x0=-1.0,
+                      n_steps_lim=None, hit_index=None, f32_policy_input=False, policy_opt=None, grid=None,
+                      keep_path=False, keep_margin=False, grad_modes=(), dtype=torch.float64, device="cpu"):
+    """The rollout the kernels compute, evaluated in ``dtype`` (float64 by default) from the float32 policy parameters and
+    the float32 increments ``noise[n_pass, K, d]`` (cast to ``dtype``).  Unlike the float32 replays above, which
+    reproduce the reference's own rounding, this one is the yardstick for the size of the kernels' rounding.
+
+    Per pass k (0-based), on the CURRENT state x_k: the hit test (``hit_rule`` all(x >= lb), or lb <= x_0 <= rb);
+    u_k = policy(x_k) (with ``f32_policy_input`` the policy sees x_k cast to float32, as in the NumPy path); then
+    x_{k+1} = x_k + (-grad V(x_k) + sigma u_k) dt + sigma dB_k.  On the first hit pass k*:
+        T = k*,   G = -sum_{j<k*} (1 + |u_j|^2 / 2) dt,   S_exact = sum_{j<k*} u_j . dB_j,
+        S_ref = S_exact + u_k* . dB_k*,   l2 = sum_{j<=k*} |u_j - policy_opt[idx(x_j)]|^2 dt,   logw = G - S_exact.
+    No hit within lim = min(n_steps_lim, n_pass) passes: T = -1, G and S (both modes) over all lim passes, logw = G - S.
+
+    ``hit_index`` (int[K], -1 = never) teacher-forces the pass on which each trajectory stops, so that outputs can be
+    compared with a kernel's along the kernel's own hit passes.  Whatever stops a trajectory, the function returns its own
+    decisions.  The margin of a state is its signed distance to the target boundary (>= 0 means "in the target set");
+    ``T_own`` is the first pass with margin >= 0 among the passes a trajectory ran (-1 = none), and ``margin_first`` the
+    margin at the first pass where the own decision and the forced stop disagree (pass min(T_own, T); NaN where they never
+    do), i.e. how close the reference's state was to deciding the other way.  ``keep_margin``: also return the margin of
+    every decision pass, ``margin[n_run, K]`` (NaN after a trajectory stopped).
+    ``grid = (lo, hi, h)`` with ``policy_opt[n_grid, d]``: idx(x) = floor((clip(x_0, lo, hi) - lo) / h) (clamped).
+    ``keep_path``: also return ``path[K, n_run, d]``, the states x_0 .. x_{n_run - 1}.
+    ``grad_modes`` (any of 'reference', 'exact'): autograd of mean_i(-G_i - sg(G_i) S_i) over all K trajectories
+    (unfinished ones contribute 0), with S = S_ref or S_exact, w.r.t. the parameters: ``grads[mode][key]`` float64 arrays.
+
+    Returns a dict of ``dtype`` tensors on ``device`` (T, T_own int64)."""
+    dev = torch.device(device)
+    noise = torch.as_tensor(np.asarray(noise, dtype=np.float32) if not torch.is_tensor(noise) else noise)
+    noise = noise.to(device=dev, dtype=dtype)
+    n_pass, K, dd = noise.shape
+    assert dd == d
+    lim = n_pass if n_steps_lim is None else min(int(n_steps_lim), n_pass)
+    p = {k: torch.as_tensor(np.asarray(v.detach().cpu().numpy() if torch.is_tensor(v) else v, dtype=np.float32))
+         .to(device=dev, dtype=dtype).requires_grad_(bool(grad_modes)) for k, v in params.items()}
+    sigma, dt_ = float(np.sqrt(2.0 / beta)), float(dt)
+    c4a = torch.as_tensor(np.broadcast_to(4.0 * np.asarray(alpha, dtype=np.float64), (d,)).copy(), device=dev, dtype=dtype)
+    forced = None
+    if hit_index is not None:
+        forced = torch.as_tensor(np.asarray(hit_index.cpu() if torch.is_tensor(hit_index) else hit_index, dtype=np.int64),
+                                 device=dev)
+    pol = None
+    if policy_opt is not None:
+        pol = torch.as_tensor(np.asarray(policy_opt, dtype=np.float64).reshape(-1, d), device=dev, dtype=dtype)
+        g_lo, g_hi, g_h = (float(v) for v in grid)
+    x = torch.as_tensor(np.broadcast_to(np.asarray(x0, dtype=np.float64), (d,)).copy(), device=dev, dtype=dtype).expand(K, d)
+    zero = torch.zeros(K, device=dev, dtype=dtype)
+    G, S, L2 = zero, zero, zero
+    G_out, Sx_out, Sr_out, L2_out = zero, zero, zero, zero
+    alive = torch.ones(K, dtype=torch.bool, device=dev)
+    T = torch.full((K,), -1, dtype=torch.int64, device=dev)
+    T_own = torch.full((K,), -1, dtype=torch.int64, device=dev)
+    margin = torch.full((lim, K), float("nan"), device=dev, dtype=dtype) if keep_margin else None
+    margin_first = torch.full((K,), float("nan"), device=dev, dtype=dtype)
+    path = torch.full((K, lim, d), float("nan"), device=dev, dtype=dtype) if keep_path else None
+    n_run = 0
+    with torch.set_grad_enabled(bool(grad_modes)):
+        for k in range(lim):
+            if not bool(alive.any()):
+                break
+            n_run = k + 1
+            xd = x.detach()
+            if keep_path:
+                path[:, k] = xd
+            m = xd.min(dim=1).values - lb if hit_rule == HIT_ALL_GE_LB else torch.minimum(xd[:, 0] - lb, rb - xd[:, 0])
+            if keep_margin:
+                margin[k] = torch.where(alive, m, margin[k])
+            own = alive & (m >= 0)
+            T_own = torch.where(own & (T_own < 0), torch.full_like(T_own, k), T_own)
+            stop = alive & ((forced == k) if forced is not None else own)
+            margin_first = torch.where((own != stop) & torch.isnan(margin_first), m, margin_first)
+            xin = x.float().to(dtype) if f32_policy_input else x
+            u = policy_torch(p, xin)
+            dB = noise[k]
+            udB = (u * dB).sum(dim=1)
+            r = -(1.0 + 0.5 * (u * u).sum(dim=1)) * dt_
+            if pol is not None:
+                gi = torch.floor((xd[:, 0].clamp(g_lo, g_hi) - g_lo) / g_h).long().clamp(0, pol.shape[0] - 1)
+                L2 = L2 + torch.where(alive, ((u - pol[gi]) ** 2).sum(dim=1) * dt_, zero)
+            G_out = torch.where(stop, G, G_out)
+            Sx_out = torch.where(stop, S, Sx_out)
+            Sr_out = torch.where(stop, S + udB, Sr_out)
+            L2_out = torch.where(stop, L2, L2_out)
+            T = torch.where(stop, torch.full_like(T, k), T)
+            alive = alive & ~stop
+            G = G + torch.where(alive, r, zero)
+            S = S + torch.where(alive, udB, zero)
+            x_next = x + (-(c4a * x * (x * x - 1.0)) + sigma * u) * dt_ + sigma * dB
+            x = torch.where(alive[:, None], x_next, x)
+        done = T >= 0
+        G_out = torch.where(done, G_out, G)
+        Sx_out = torch.where(done, Sx_out, S)
+        Sr_out = torch.where(done, Sr_out, S)
+        L2_out = torch.where(done, L2_out, L2)
+        out = dict(T=T, T_own=T_own, G=G_out.detach(), S_exact=Sx_out.detach(), S_ref=Sr_out.detach(),
+                   logw=(G_out - Sx_out).detach(), l2=L2_out.detach() if pol is not None else None,
+                   margin_first=margin_first, margin=margin[:n_run] if keep_margin else None,
+                   path=path[:, :n_run] if keep_path else None)
+        out["grads"] = {}
+        for i, mode in enumerate(grad_modes):
+            Ssel = {"reference": Sr_out, "exact": Sx_out}[mode]
+            loss = torch.where(done, -G_out - G_out.detach() * Ssel, zero).sum() / K
+            gs = torch.autograd.grad(loss, [p[k] for k in PARAM_KEYS], retain_graph=i + 1 < len(grad_modes))
+            out["grads"][mode] = {k: g.detach().cpu().numpy().astype(np.float64) for k, g in zip(PARAM_KEYS, gs)}
+    return out
+
+
 def transitions_numpy(d, alpha, beta, dt, params, noise, n_max, lb=1.0, rb=2.0, x0=-1.0):
     """Replay of ``sample_trajectories_buffer_vectorized`` (approximate_methods.py:513-545) on recorded increments:
     what ``ReplayBuffer.store_vectorized`` (replay_buffers.py:56-68) has received when the sampler returns.
