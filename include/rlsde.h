@@ -129,6 +129,10 @@ typedef struct rlsde_rollout_cfg {
   int32_t wide_kernel;          /* forward rollout (hidden width 64 / 128 / 256) and reverse pass (128 / 256): 0 = automatic (tcgen05
                                    kernels for batches of at least 512 trajectories at width 256, 64 x SMs below; the reverse pass also needs a
                                    workspace of rlsde_workspace_bytes_bwd), 1 = tcgen05 kernels, 2 = CUDA-core tile kernels */
+  int32_t fwd_policy;           /* policy evaluation of the thread-per-trajectory forward kernel and of the kernel that
+                                   continues its tail: 0 = automatic (tensor cores at d = 1, hidden width 32), 1 = 32 x 32
+                                   layer on the tensor cores (mma.sync, float16 x 3 split; d = 1, hidden width 32 only),
+                                   2 = CUDA cores (FFMA2).  Results differ between 1 and 2 by rounding. */
 } rlsde_rollout_cfg;
 
 /* layout of a statistics record (double[RLSDE_NSTATS]); sums are over the K local trajectories,

@@ -64,7 +64,7 @@ class RlsdeRolloutCfg(C.Structure):
         ("grid_lo", C.c_double), ("grid_hi", C.c_double), ("grid_h", C.c_double),
         # scheduling knobs, 0 = automatic (include/rlsde.h)
         ("fwd_quantum", C.c_int32), ("fwd_blocks_per_sm", C.c_int32), ("fwd_handoff", C.c_int64), ("bwd_warp_share", C.c_int64),
-        ("bwd_kernel", C.c_int32), ("wide_kernel", C.c_int32),
+        ("bwd_kernel", C.c_int32), ("wide_kernel", C.c_int32), ("fwd_policy", C.c_int32),
     ]
 
 
@@ -130,8 +130,9 @@ def load():
 def apply_tuning(cfg, tuning=None):
     """Scheduling knobs of a rollout cfg (include/rlsde.h: they change the schedule, never a result).  ``tuning`` is a dict
     with any of ``fwd_quantum`` (passes per time slice, 0 = run to completion), ``fwd_handoff``, ``bwd_warp_share``,
-    ``fwd_blocks_per_sm``, ``bwd_kernel`` ('mma' | 'ffma'), ``wide_kernel`` ('umma' | 'ffma'); keys that are absent fall back to the environment variables
-    RLSDE_FWD_QUANTUM, RLSDE_FWD_HANDOFF, RLSDE_BWD_WARP_SHARE, RLSDE_FWD_BLOCKS_PER_SM, RLSDE_BWD_KERNEL (read HERE, in
+    ``fwd_blocks_per_sm``, ``bwd_kernel`` ('mma' | 'ffma'), ``wide_kernel`` ('umma' | 'ffma'), ``fwd_policy`` ('mma' | 'ffma');
+    keys that are absent fall back to the environment variables RLSDE_FWD_QUANTUM, RLSDE_FWD_HANDOFF, RLSDE_BWD_WARP_SHARE,
+    RLSDE_FWD_BLOCKS_PER_SM, RLSDE_BWD_KERNEL, RLSDE_WIDE_KERNEL, RLSDE_FWD_POLICY (read HERE, in
     Python -- the library reads none), and to "automatic" if those are unset too."""
     tuning = tuning or {}
 
@@ -153,6 +154,8 @@ def apply_tuning(cfg, tuning=None):
     cfg.bwd_kernel = {"auto": 0, "mma": 1, "ffma": 2}[str(bk).lower()]
     wk = tuning.get("wide_kernel") or os.environ.get("RLSDE_WIDE_KERNEL") or "auto"
     cfg.wide_kernel = {"auto": 0, "umma": 1, "tcgen05": 1, "ffma": 2}[str(wk).lower()]
+    fp = tuning.get("fwd_policy") or os.environ.get("RLSDE_FWD_POLICY") or "auto"
+    cfg.fwd_policy = {"auto": 0, "mma": 1, "ffma": 2}[str(fp).lower()]
     return cfg
 
 

@@ -147,6 +147,7 @@ static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A) {
     if (A.ckpt_every == (1 << b)) A.ckpt_log2 = b;
   A.n_grid = cfg->n_grid; A.grid_lo = cfg->grid_lo; A.grid_hi = cfg->grid_hi; A.grid_h = cfg->grid_h;
   A.blocks_per_sm_cap = cfg->fwd_blocks_per_sm > 0 ? cfg->fwd_blocks_per_sm : 0;
+  if (cfg->fwd_policy < 0 || cfg->fwd_policy > 2) return RLSDE_ERR_INVALID_ARG;
   return RLSDE_OK;
 }
 
@@ -322,20 +323,27 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
     return RLSDE_OK;
   }
   const bool warp_path = use_warp_kernels(A, mlp->d_hidden, sm, (A.flags & RLSDE_F_STORE_PATH) != 0);
+  // ---- policy arithmetic of the thread-per-trajectory kernel and of the kernel that continues its tail (mlp_mma.cuh or
+  // FFMA2).  A function of (d, H, cfg.fwd_policy) only: the replay sampler launches it twice, with and without the
+  // transition stream, and needs the same hit passes from both launches.
+  if (cfg->fwd_policy == 1 && !fwd_mma_shape(env->d, mlp->d_hidden)) return RLSDE_ERR_UNSUPPORTED;
+  A.policy_mma = fwd_mma_shape(env->d, mlp->d_hidden) && cfg->fwd_policy != 2 ? 1 : 0;
   // ---- hidden width 32 on the tensor cores (rollout_umma.cuh with resident weights: tiles of 128 trajectories, one thread
   // per trajectory, lane refill).  The per-pass work of a warp drops from ~1 290 to ~860 instructions; like K1 it ends up
   // bound by the MUFU pipe (71 % busy with the two-MUFU tanh: profiles/r02/ncu_rollout_fwd_umma_h32_v1.txt).  Measured at
   // 1e6 trajectories, budget 1 000 passes (tools/bench_fwd_kernels.py): d = 1 precise tanh 27.5 ms against K1's 25.1 ms,
   // fast tanh 20.6 against 21.5; d = 2: 54.5 % of the FP32 roofline against 52 %; d = 4: 58.1 % against 53.4 %; d = 10:
   // 50.9 % against 44.9 %.  It has no breadth-first schedule, so its launch ends with a tail of (longest trajectory) x
-  // (~1 us per pass).  Automatic where it wins: d >= 2 or the fast tanh, large batches, a bounded pass budget -- and never
-  // when the caller pins a kernel family or a schedule of the thread-per-trajectory kernel.
+  // (~1 us per pass).  At d = 1 the thread-per-trajectory kernel with its 32 x 32 layer on mma.sync (mlp_mma.cuh) beats it
+  // in both tanh modes: 21.1 / 15.4 ms against 27.4 / 20.6 ms (profiles/r03).  Automatic where it wins: d >= 2, large
+  // batches, a bounded pass budget -- and never when the caller pins a kernel family, a schedule or the policy arithmetic
+  // of the thread-per-trajectory kernel.
   {
     const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
     const bool forced = (A.flags & RLSDE_F_KERNEL_TENSOR) != 0;
-    const bool pinned = (A.flags & (RLSDE_F_KERNEL_THREAD | RLSDE_F_KERNEL_WARP)) != 0 || cfg->fwd_quantum != 0 || cfg->fwd_handoff != 0;
-    const bool automatic = !pinned && !warp_path && A.K >= (long long)sm * UMMA_M * 2 && lim_eff <= 4096 &&
-                           (env->d >= 2 || (A.flags & RLSDE_F_TANH_FAST) != 0);
+    const bool pinned = (A.flags & (RLSDE_F_KERNEL_THREAD | RLSDE_F_KERNEL_WARP)) != 0 || cfg->fwd_quantum != 0 ||
+                        cfg->fwd_handoff != 0 || cfg->fwd_policy != 0;
+    const bool automatic = !pinned && !warp_path && A.K >= (long long)sm * UMMA_M * 2 && lim_eff <= 4096 && env->d >= 2;
     if (mlp->d_hidden == 32 && !tr.base && (forced || automatic)) {
       if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
 #define X(D_, H_)                                                                                                          \

@@ -49,49 +49,6 @@ struct alignas(16) BwdMmaWeights {
   float pad[3];
 };
 
-inline uint16_t f32_to_f16_bits(float f) {      // round to nearest even, host side
-  uint32_t x;
-  memcpy(&x, &f, 4);
-  const uint32_t sign = (x >> 16) & 0x8000u;
-  const int32_t exp = (int32_t)((x >> 23) & 0xff) - 127 + 15;
-  uint32_t man = x & 0x7fffffu;
-  if (((x >> 23) & 0xff) == 0xff) return (uint16_t)(sign | 0x7c00u | (man ? 0x200u : 0));
-  if (exp >= 31) return (uint16_t)(sign | 0x7c00u);
-  if (exp <= 0) {
-    if (exp < -10) return (uint16_t)sign;
-    man |= 0x800000u;
-    const int shift = 14 - exp;
-    uint32_t h = man >> shift;
-    const uint32_t rem = man & ((1u << shift) - 1u), half = 1u << (shift - 1);
-    if (rem > half || (rem == half && (h & 1u))) ++h;
-    return (uint16_t)(sign | h);
-  }
-  uint32_t h = ((uint32_t)exp << 10) | (man >> 13);
-  const uint32_t rem = man & 0x1fffu;
-  if (rem > 0x1000u || (rem == 0x1000u && (h & 1u))) ++h;
-  return (uint16_t)(sign | h);
-}
-inline float f16_bits_to_f32(uint16_t h) {
-  const uint32_t sign = (uint32_t)(h & 0x8000u) << 16;
-  uint32_t exp = (h >> 10) & 0x1f, man = h & 0x3ffu;
-  uint32_t x;
-  if (exp == 0) {
-    if (man == 0) { x = sign; }
-    else {
-      int e = -1;
-      do { ++e; man <<= 1; } while (!(man & 0x400u));
-      x = sign | ((uint32_t)(127 - 15 - e) << 23) | ((man & 0x3ffu) << 13);
-    }
-  } else if (exp == 31) {
-    x = sign | 0x7f800000u | (man << 13);
-  } else {
-    x = sign | ((exp - 15 + 127) << 23) | (man << 13);
-  }
-  float f;
-  memcpy(&f, &x, 4);
-  return f;
-}
-
 template <int D>
 inline void pack_bwd_mma_weights(const MlpConst<D, MMA_H>& W, BwdMmaWeights& out) {
   constexpr int H = MMA_H;
@@ -103,30 +60,7 @@ inline void pack_bwd_mma_weights(const MlpConst<D, MMA_H>& W, BwdMmaWeights& out
   (void)wmax;
   out.w3_max = w3max > 0.f ? w3max : 1.0f;
   out.pad[0] = out.pad[1] = out.pad[2] = 0.f;
-  auto w = [&](int o, int i) { return W.W2t[i][o]; };            // W2[out][in] (with the tanh pre-scale)
-  auto split = [&](float a, float b, uint32_t& hi, uint32_t& lo) {
-    const uint16_t ah = f32_to_f16_bits(a), bh = f32_to_f16_bits(b);
-    const uint16_t al = f32_to_f16_bits(a - f16_bits_to_f32(ah)), bl = f32_to_f16_bits(b - f16_bits_to_f32(bh));
-    hi = (uint32_t)ah | ((uint32_t)bh << 16);
-    lo = (uint32_t)al | ((uint32_t)bl << 16);
-  };
-  for (int p = 0; p < 2; ++p)
-    for (int kk = 0; kk < 2; ++kk)
-      for (int jp = 0; jp < 2; ++jp)
-        for (int lane = 0; lane < 32; ++lane) {
-          const int g = lane >> 2, q = lane & 3;
-          for (int jj = 0; jj < 2; ++jj) {
-            const int n = 8 * (2 * jp + jj) + g, k0 = 16 * kk + 2 * q;
-            for (int b = 0; b < 2; ++b) {
-              const int k = k0 + 8 * b;
-              const float e0 = p == 0 ? w(n, k) : w(k, n), e1 = p == 0 ? w(n, k + 1) : w(k + 1, n);
-              uint32_t hi, lo;
-              split(e0, e1, hi, lo);
-              out.frag[p][0][kk][jp][lane][2 * jj + b] = hi;
-              out.frag[p][1][kk][jp][lane][2 * jj + b] = lo;
-            }
-          }
-        }
+  pack_w2_frags<D, H>(W, 2, out.frag);
 }
 
 // d > 4: the d-sized products run on the tensor cores too, with d padded to one k-chunk / two n-tiles of 16:
@@ -152,12 +86,6 @@ template <int D>
 inline void pack_bwd_mma_small(const MlpConst<D, MMA_H>& W, bool fast, BwdMmaSmall& out) {
   constexpr int H = MMA_H;
   static_assert(D <= MMA_DP, "state dimension beyond one padded tile");
-  auto split = [&](float a, float b, uint32_t& hi, uint32_t& lo) {
-    const uint16_t ah = f32_to_f16_bits(a), bh = f32_to_f16_bits(b);
-    const uint16_t al = f32_to_f16_bits(a - f16_bits_to_f32(ah)), bl = f32_to_f16_bits(b - f16_bits_to_f32(bh));
-    hi = (uint32_t)ah | ((uint32_t)bh << 16);
-    lo = (uint32_t)al | ((uint32_t)bl << 16);
-  };
   // element (k, n) of the B operand of product q
   auto elem = [&](int q, int k, int n) -> float {
     switch (q) {
@@ -177,7 +105,7 @@ inline void pack_bwd_mma_small(const MlpConst<D, MMA_H>& W, bool fast, BwdMmaSma
             const int n = k_small ? 8 * (2 * c + jj) + g : 8 * jj + g;
             const int k = (k_small ? 0 : 16 * c) + 2 * t + 8 * b;
             uint32_t hi, lo;
-            split(elem(q, k, n), elem(q, k + 1, n), hi, lo);
+            split_pair_host(elem(q, k, n), elem(q, k + 1, n), hi, lo);
             out.frag[q][0][c][lane][2 * jj + b] = hi;
             out.frag[q][1][c][lane][2 * jj + b] = lo;
           }
@@ -199,23 +127,10 @@ inline void pack_bwd_mma_small(const MlpConst<D, MMA_H>& W, bool fast, BwdMmaSma
 }
 
 // ------------------------------------------------------------------ device helpers
-__device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
 __device__ __forceinline__ uint32_t movm_trans(uint32_t a) {
   uint32_t d;
   asm volatile("movmatrix.sync.aligned.m8n8.trans.b16 %0, %1;" : "=r"(d) : "r"(a));
   return d;
-}
-// x0, x1 -> float16 pairs hi, lo with x ~ hi + lo  (x0 in the low half)
-__device__ __forceinline__ void split_pair(float x0, float x1, uint32_t& hi, uint32_t& lo) {
-  const __half2 h = __floats2half2_rn(x0, x1);
-  const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(x0 - hf.x, x1 - hf.y);
-  hi = *reinterpret_cast<const uint32_t*>(&h);
-  lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 // One m16 row tile in accumulator layout v[j][r] (row = g + 8 (r >> 1), column = 8 j + 2 q + (r & 1)), times `scale`,
 // as the A operand (hi / lo) of a product whose K dimension is the column index: a[kk][4]
@@ -230,25 +145,6 @@ __device__ __forceinline__ void acc_to_a_frags(const float (&v)[4][4], float sca
       else split_pair(v[j][r], v[j][r + 1], ah[kk][r4], al[kk][r4]);
     }
 }
-// acc[j] += A (hi + lo) x B (hi + lo from the shared-memory fragment table of product p), dropping lo x lo.
-// Issue order: the four accumulators take turns, so consecutive HMMAs are independent (dependent ones are 4 apart).
-__device__ __forceinline__ void mma_product_w(float (&acc)[4][4], const uint32_t (&ah)[2][4], const uint32_t (&al)[2][4],
-                                              const uint4* __restrict__ wfrag, int p, int lane) {
-#pragma unroll
-  for (int kk = 0; kk < 2; ++kk) {
-    const uint4 bh0 = wfrag[(((p * 2 + 0) * 2 + kk) * 2 + 0) * 32 + lane];
-    const uint4 bh1 = wfrag[(((p * 2 + 0) * 2 + kk) * 2 + 1) * 32 + lane];
-    const uint4 bl0 = wfrag[(((p * 2 + 1) * 2 + kk) * 2 + 0) * 32 + lane];
-    const uint4 bl1 = wfrag[(((p * 2 + 1) * 2 + kk) * 2 + 1) * 32 + lane];
-    mma16816(acc[0], ah[kk], bh0.x, bh0.y); mma16816(acc[1], ah[kk], bh0.z, bh0.w);
-    mma16816(acc[2], ah[kk], bh1.x, bh1.y); mma16816(acc[3], ah[kk], bh1.z, bh1.w);
-    mma16816(acc[0], al[kk], bh0.x, bh0.y); mma16816(acc[1], al[kk], bh0.z, bh0.w);
-    mma16816(acc[2], al[kk], bh1.x, bh1.y); mma16816(acc[3], al[kk], bh1.z, bh1.w);
-    mma16816(acc[0], ah[kk], bl0.x, bl0.y); mma16816(acc[1], ah[kk], bl0.z, bl0.w);
-    mma16816(acc[2], ah[kk], bl1.x, bl1.y); mma16816(acc[3], ah[kk], bl1.z, bl1.w);
-  }
-}
-
 __device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], const void* smem_ptr) {
   const unsigned addr = (unsigned)__cvta_generic_to_shared(smem_ptr);
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));

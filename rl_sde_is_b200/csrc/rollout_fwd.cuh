@@ -32,7 +32,9 @@
 // slot between passes, never blocking the warp's other lanes); the launch ends when every trajectory has
 // reported completion.  Per-trajectory arithmetic does not depend on the slicing: results are bit-identical.
 #pragma once
+#include <type_traits>
 #include "common.cuh"
+#include "mlp_mma.cuh"
 #include "../../include/rlsde.h"
 
 namespace rlsde {
@@ -73,6 +75,8 @@ struct FwdArgs {
   const long long* order;        // reverse pass: processing order of the trajectories (or nullptr = identity)
   int grad_accumulate;           // reverse pass: add this launch's gradient to grad instead of overwriting it
   int blocks_per_sm_cap;         // > 0: cap on resident blocks per SM of the thread-per-trajectory forward kernel (tuning)
+  int policy_mma;                // 1: the thread-per-trajectory forward kernel evaluates the policy with mlp_forward_mma (and
+                                 // the kernel that continues its handed-over trajectories does the same), 0: with FFMA2
   // ---- transition stream (replay-buffer sampler, approximate_methods.py:513-545): trajectory `t` writes the tuple of
   //      its pass k at slot tr_base[t] + k of the five arrays below.  nullptr = no stream.
   const long long* tr_base;
@@ -142,18 +146,38 @@ struct NoisePlan {
   static constexpr int NZ = 4 * BPP;
 };
 
+// policy evaluation of the thread-per-trajectory forward kernel: mlp_forward_mma (mlp_mma.cuh) is compiled where it has
+// been measured to win, hidden width 32 at d = 1
+constexpr bool fwd_mma_shape(int D, int H) { return D == 1 && H == 32; }
+struct MlpMmaNone { int unused; };
+template <int D, bool MMA> struct FwdMmaSel { typedef typename std::conditional<MMA, MlpMma<D>, MlpMmaNone>::type type; };
+
 // Register budgets.  Left alone, ptxas settles at 67 registers for d = 1 and at ~250 for the wider shapes (2 blocks per
 // SM: two warps per scheduler, every FFMA2 waiting for its LDCU.128), although spill-free allocations exist at 64
 // (d = 1: 8 blocks per SM), <= 102 (d = 2..4: 5 blocks) and <= 128 (d = 10: 4 blocks) -- it finds them when asked.
-template <int D, int H, bool F64, bool FAST>
-__global__ void __launch_bounds__(128, (D == 1 ? 8 : (D <= 4 ? 5 : 4))) rollout_fwd_kernel(const __grid_constant__ MlpConst<D, H> W,
-                                                          const __grid_constant__ FwdArgs A) {
+// The tensor-core policy holds a half-tile of fragments (A hi / lo, accumulators, B operands) on top of the pass state:
+// 80 registers at 6 blocks per SM, measured best (d = 1, 1e6 trajectories: 21.1 ms against 21.8 / 22.2 ms at 5 / 4).
+#ifndef RLSDE_FWD_MMA_MIN_BLOCKS
+#define RLSDE_FWD_MMA_MIN_BLOCKS 6
+#endif
+template <int D, bool MMA>
+constexpr int fwd_min_blocks() { return MMA ? RLSDE_FWD_MMA_MIN_BLOCKS : (D == 1 ? 8 : (D <= 4 ? 5 : 4)); }
+template <int D, int H, bool F64, bool FAST, bool MMA>
+__global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_kernel(const __grid_constant__ MlpConst<D, H> W,
+                                                          const __grid_constant__ FwdArgs A,
+                                                          const __grid_constant__ typename FwdMmaSel<D, MMA>::type M) {
   typedef typename RealT<F64>::type real;
   constexpr int SPB = NoisePlan<D>::SPB;
   constexpr int BPP = NoisePlan<D>::BPP;
   constexpr int NZ = NoisePlan<D>::NZ;
   constexpr unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31;
+  // MMA: the block's copy of the fragment and column tables (mlp_mma.cuh)
+  __shared__ uint4 s_mma[MMA ? mlp_mma_smem_words<D>() : 1];
+  if constexpr (MMA) {
+    for (int i = threadIdx.x; i < mlp_mma_smem_words<D>(); i += blockDim.x) s_mma[i] = reinterpret_cast<const uint4*>(&M)[i];
+    __syncthreads();
+  }
   const bool inject = (A.flags & RLSDE_F_NOISE_INJECTED) != 0;
   const bool s_exact = (A.flags & RLSDE_F_STOCH_INT_EXACT) != 0;
   const bool store_path = (A.flags & RLSDE_F_STORE_PATH) != 0 && A.path != nullptr;
@@ -333,7 +357,8 @@ __global__ void __launch_bounds__(128, (D == 1 ? 8 : (D <= 4 ? 5 : 4))) rollout_
     float xf[D], u[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) xf[i] = (float)x[i];
-    if constexpr (!FAST && RLSDE_FWD_FOLDED) mlp_forward_folded<D, H>(W, xf, u);      // W is a pack_mlp_const_folded image
+    if constexpr (MMA) mlp_forward_mma<D, FAST>(s_mma, reinterpret_cast<const float4*>(s_mma + MLP_MMA_FRAG_WORDS), M.b3, lane, xf, u);
+    else if constexpr (!FAST && RLSDE_FWD_FOLDED) mlp_forward_folded<D, H>(W, xf, u);   // W is a pack_mlp_const_folded image
     else mlp_forward<D, H, FAST>(W, xf, u);
 
     // ---- this pass's Brownian increments

@@ -4,12 +4,15 @@
 
 namespace rlsde {
 
-template <int D, int H, bool F64, bool FAST>
+template <int D, int H, bool F64, bool FAST, bool MMA>
 static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, H> W;
   if (!FAST && RLSDE_FWD_FOLDED) pack_mlp_const_folded<D, H>(params_host, W);
   else pack_mlp_const<D, H>(params_host, FAST, W);
-  auto kern = rollout_fwd_kernel<D, H, F64, FAST>;
+  typename FwdMmaSel<D, MMA>::type M;
+  if constexpr (MMA) pack_mlp_mma<D>(W, M);
+  else M.unused = 0;
+  auto kern = rollout_fwd_kernel<D, H, F64, FAST, MMA>;
   // Small batches: one warp per block so the warps spread over SMs (latency-bound regime);
   // large batches: persistent grid of 128-thread blocks, as many as are co-resident.
   int block = 128;
@@ -46,21 +49,30 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
   } else {
     a.q_ring = nullptr; a.q_cap = 0; a.q_cap_log2 = 0; a.q_quantum = 0; a.q_handoff = 0;
   }
-  kern<<<(unsigned)grid, block, 0, stream>>>(W, a);
+  kern<<<(unsigned)grid, block, 0, stream>>>(W, a, M);
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
-template <int D, int H>
-int launch_rollout_fwd(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+template <int D, int H, bool MMA>
+static int launch_fwd_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0;
   const bool fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
   if (f64) {
-    return fast ? launch_fwd_variant<D, H, true, true>(params_host, args, sm_count, stream)
-                : launch_fwd_variant<D, H, true, false>(params_host, args, sm_count, stream);
+    return fast ? launch_fwd_variant<D, H, true, true, MMA>(params_host, args, sm_count, stream)
+                : launch_fwd_variant<D, H, true, false, MMA>(params_host, args, sm_count, stream);
   }
-  return fast ? launch_fwd_variant<D, H, false, true>(params_host, args, sm_count, stream)
-              : launch_fwd_variant<D, H, false, false>(params_host, args, sm_count, stream);
+  return fast ? launch_fwd_variant<D, H, false, true, MMA>(params_host, args, sm_count, stream)
+              : launch_fwd_variant<D, H, false, false, MMA>(params_host, args, sm_count, stream);
+}
+
+// args.policy_mma selects the policy arithmetic; the caller checks fwd_mma_shape(D, H) before it sets it
+template <int D, int H>
+int launch_rollout_fwd(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+  if constexpr (fwd_mma_shape(D, H)) {
+    if (args.policy_mma) return launch_fwd_policy<D, H, true>(params_host, args, sm_count, stream);
+  }
+  return launch_fwd_policy<D, H, false>(params_host, args, sm_count, stream);
 }
 
 }  // namespace rlsde

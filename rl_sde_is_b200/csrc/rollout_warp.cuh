@@ -151,17 +151,26 @@ __device__ __forceinline__ void warp_policy_exact(const LaneParams<D>& P, const 
 
 // ------------------------------------------------------------------------------------------------ forward
 // RESUME = true: the work items are the continuation records K1 left in the ring when it handed the last live
-// trajectories of its launch over (rollout_fwd.cuh); they are continued with K1's arithmetic (warp_policy_exact).
-template <int D, bool F64, bool FAST, bool RESUME>
+// trajectories of its launch over (rollout_fwd.cuh); they are continued with K1's arithmetic: warp_policy_exact, or with
+// MMA (K1 evaluated its policy with mlp_forward_mma) the same tensor-core sequence with the trajectory's state in all
+// 32 rows of the tile.
+template <int D, bool F64, bool FAST, bool RESUME, bool MMA = false>
 __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel(const __grid_constant__ MlpConst<D, WARP_H> W_param,
                                                                const MlpConst<D, WARP_H>* __restrict__ W_dev,
-                                                               const __grid_constant__ FwdArgs A) {
+                                                               const __grid_constant__ FwdArgs A,
+                                                               const __grid_constant__ typename FwdMmaSel<D, MMA>::type M) {
+  static_assert(!MMA || RESUME, "the tensor-core policy continues K1's trajectories");
   // the policy comes by value (host parameters) or, for the device-resident training loop, from device memory
   const MlpConst<D, WARP_H>& W = W_dev != nullptr ? *W_dev : W_param;
   typedef typename RealT<F64>::type real;
   constexpr int SPB = NoisePlan<D>::SPB;
   constexpr int BPP = NoisePlan<D>::BPP;
   __shared__ __align__(16) float slots[4][WARP_H];
+  __shared__ uint4 s_mma[MMA ? mlp_mma_smem_words<D>() : 1];
+  if constexpr (MMA) {
+    for (int i = threadIdx.x; i < mlp_mma_smem_words<D>(); i += blockDim.x) s_mma[i] = reinterpret_cast<const uint4*>(&M)[i];
+    __syncthreads();
+  }
   const int lane = threadIdx.x & 31;
   float* slot = slots[threadIdx.x >> 5];
   const long long n_warps = (long long)gridDim.x * (blockDim.x >> 5);
@@ -224,7 +233,9 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
       float xf[D], u[D], dB[D];
 #pragma unroll
       for (int i = 0; i < D; ++i) xf[i] = (float)x[i];
-      if constexpr (RESUME) {
+      if constexpr (MMA) {
+        mlp_forward_mma<D, FAST, true>(s_mma, reinterpret_cast<const float4*>(s_mma + MLP_MMA_FRAG_WORDS), M.b3, lane, xf, u);
+      } else if constexpr (RESUME) {
         warp_policy_exact<D, FAST>(P, W, slot, lane, xf, u);
       } else {
         float h1, h2, h1_all[WARP_H];

@@ -47,7 +47,7 @@ static int launch_fwd_warp_variant(const float* params_host, const void* W_dev, 
   if (params_host != nullptr) pack_mlp_const<D, WARP_H>(params_host, FAST, W);
   else memset(&W, 0, sizeof(W));
   rollout_fwd_warp_kernel<D, F64, FAST, false><<<(unsigned)warp_grid(args.K, sm_count), 128, 0, stream>>>(
-      W, params_host != nullptr ? nullptr : reinterpret_cast<const MlpConst<D, WARP_H>*>(W_dev), args);
+      W, params_host != nullptr ? nullptr : reinterpret_cast<const MlpConst<D, WARP_H>*>(W_dev), args, MlpMmaNone{0});
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
@@ -61,24 +61,36 @@ int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const F
               : launch_fwd_warp_variant<D, false, false>(params_host, W_dev, args, sm_count, stream);
 }
 
-template <int D, bool F64, bool FAST>
+template <int D, bool F64, bool FAST, bool MMA>
 static int launch_fwd_warp_resume_variant(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, WARP_H> W;
   if (!FAST && RLSDE_FWD_FOLDED) pack_mlp_const_folded<D, WARP_H>(params_host, W);      // the image K1 itself was launched with
   else pack_mlp_const<D, WARP_H>(params_host, FAST, W);
+  typename FwdMmaSel<D, MMA>::type M;
+  if constexpr (MMA) pack_mlp_mma<D>(W, M);
+  else M.unused = 0;
   // the number of records is only known on the device: a full grid (16 warps per SM), warps without a record leave at once
-  rollout_fwd_warp_kernel<D, F64, FAST, true><<<(unsigned)(sm_count * 4), 128, 0, stream>>>(W, nullptr, args);
+  rollout_fwd_warp_kernel<D, F64, FAST, true, MMA><<<(unsigned)(sm_count * 4), 128, 0, stream>>>(W, nullptr, args, M);
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
+template <int D, bool MMA>
+static int launch_fwd_warp_resume_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
+  if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true, MMA>(params_host, args, sm_count, stream)
+                       : launch_fwd_warp_resume_variant<D, true, false, MMA>(params_host, args, sm_count, stream);
+  return fast ? launch_fwd_warp_resume_variant<D, false, true, MMA>(params_host, args, sm_count, stream)
+              : launch_fwd_warp_resume_variant<D, false, false, MMA>(params_host, args, sm_count, stream);
+}
+
+// continues with the policy arithmetic K1 was launched with (args.policy_mma)
 template <int D>
 int launch_rollout_fwd_warp_resume(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true>(params_host, args, sm_count, stream)
-                       : launch_fwd_warp_resume_variant<D, true, false>(params_host, args, sm_count, stream);
-  return fast ? launch_fwd_warp_resume_variant<D, false, true>(params_host, args, sm_count, stream)
-              : launch_fwd_warp_resume_variant<D, false, false>(params_host, args, sm_count, stream);
+  if constexpr (fwd_mma_shape(D, WARP_H)) {
+    if (args.policy_mma) return launch_fwd_warp_resume_policy<D, true>(params_host, args, sm_count, stream);
+  }
+  return launch_fwd_warp_resume_policy<D, false>(params_host, args, sm_count, stream);
 }
 
 template <int D, bool FAST>
