@@ -99,6 +99,53 @@ __device__ __forceinline__ void rsig_pair(u64 acc, float& r0, float& r1) {
       : "=f"(r0), "=f"(r1) : "l"(acc), "l"(0x3f8000003f800000ull));
 }
 
+// rsig_pair of two packed pairs za = {z0, z1}, zb = {z2, z3} with one MUFU.RCP per G activations instead of one each
+// (G = RLSDE_FWD_RCP_GROUP; the tensor-core forward policy, mlp_mma.cuh):
+//   G = 2:  p = da db (packed),  R = {1 / p.x, 1 / p.y},  ra = R db,  rb = R da
+//   G = 4:  p = da db,  R = 1 / (p.x p.y),  Q = {R p.y, R p.x} = {1 / p.x, 1 / p.y},  ra = Q db,  rb = Q da
+// with d = 2^z + 1 >= 1, so no product can become subnormal.  A product can overflow, which makes the reciprocal 0 and the
+// smaller members' r 0 (or NaN): z is clamped to 63 (G = 2) / 31 (G = 4) first, so that the product of G of them stays
+// below 2^126.  The clamp moves r by at most 2^-31 (r < 2^-31 on both sides of it).
+// Error: the group adds 2 (G = 2) / 4 (G = 4) float32 roundings to each r.  With correctly rounded EX2 and RCP, over
+// z in [-200, 200], |r - 1 / (2^z + 1)| <= k 2^-24 (r + 2^-31) + 2^-31 with k = 3.5 (G = 2) / 4.5 (G = 4), against 2.5
+// ungrouped (tests/test_fwd_grouped_rcp.py restates the arithmetic); MUFU.EX2 / RCP add their own few ulp as before.  So
+// tanh = 1 - 2 r moves by at most ~2 ulp of 1 (~2.4e-7) more than with G = 1.
+#ifndef RLSDE_FWD_RCP_GROUP
+#define RLSDE_FWD_RCP_GROUP 4
+#endif
+template <int G>
+struct RcpGroup {
+  static_assert(G == 1 || G == 2 || G == 4, "RLSDE_FWD_RCP_GROUP is 1, 2 or 4");
+  static constexpr float ZMAX = G == 4 ? 31.0f : 63.0f;   // the clamp on z (unused for G = 1)
+};
+template <int G>
+__device__ __forceinline__ void rsig_group(u64 za, u64 zb, float& r0, float& r1, float& r2, float& r3) {
+  if constexpr (G == 1) {
+    rsig_pair(za, r0, r1);
+    rsig_pair(zb, r2, r3);
+  } else {
+    float z[4];
+    unpack2(za, z[0], z[1]);
+    unpack2(zb, z[2], z[3]);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) asm("min.NaN.f32 %0, %0, %1;" : "+f"(z[i]) : "f"(RcpGroup<G>::ZMAX));   // NaN stays NaN
+    const u64 one = 0x3f8000003f800000ull;
+    const u64 da = add2(pack2(mufu_ex2(z[0]), mufu_ex2(z[1])), one);
+    const u64 db = add2(pack2(mufu_ex2(z[2]), mufu_ex2(z[3])), one);
+    float px, py;
+    unpack2(mul2(da, db), px, py);
+    u64 q;
+    if constexpr (G == 2) {
+      q = pack2(mufu_rcp(px), mufu_rcp(py));
+    } else {
+      const float R = mufu_rcp(__fmul_rn(px, py));
+      q = pack2(__fmul_rn(R, py), __fmul_rn(R, px));
+    }
+    unpack2(mul2(q, db), r0, r1);
+    unpack2(mul2(q, da), r2, r3);
+  }
+}
+
 // acc[o .. o+7] (8 packed accumulators = 16 outputs) += h * w[2o .. 2o+15]
 #define RLSDE_FMA2X8(acc, o, h, w)                                                                                  \
   asm("{\n\t.reg .b64 hh, w0, w1, w2, w3, w4, w5, w6, w7;\n\t"                                                       \

@@ -166,11 +166,18 @@ constexpr int MLP_MMA_FRAG_WORDS = 2 * 2 * 2 * 32;
 template <int D>
 constexpr int mlp_mma_smem_words() { return (int)(offsetof(MlpMma<D>, b3) / 16); }
 
-// activation of a packed pair of pre-activations: r = 1 / (2^z + 1) on a pack_mlp_const_folded image, tanh otherwise
+// activations of two packed pairs of pre-activations of one row: r = 1 / (2^z + 1) on a pack_mlp_const_folded image, with
+// one reciprocal per RLSDE_FWD_RCP_GROUP of them (rsig_group), tanh otherwise.  Which activations share a reciprocal
+// depends only on the layer and the hidden units, never on the lane or the row: the REPL continuation below computes the
+// same groups as the full tile.
 template <bool FAST>
-__device__ __forceinline__ void act_pair_mma(u64 z, float& a0, float& a1) {
-  if constexpr (FAST) tanh_pair<true>(z, a0, a1);
-  else rsig_pair(z, a0, a1);
+__device__ __forceinline__ void act_group_mma(u64 za, u64 zb, float& a0, float& a1, float& a2, float& a3) {
+  if constexpr (FAST) {
+    tanh_pair<true>(za, a0, a1);
+    tanh_pair<true>(zb, a2, a3);
+  } else {
+    rsig_group<RLSDE_FWD_RCP_GROUP>(za, zb, a0, a1, a2, a3);
+  }
 }
 
 // u = policy(x) of the trajectory of this lane; all 32 lanes of the warp must take part (x and u of the other lanes'
@@ -196,7 +203,8 @@ __device__ __forceinline__ void mlp_forward_mma(const uint4* __restrict__ s_frag
     for (int h = 0; h < 2; ++h)
 #pragma unroll
       for (int i = 0; i < D; ++i) xr[h][i] = __shfl_sync(FULL, x[i], quad | (2 * mt + h));
-    // layer 1 straight into the A-fragment layout: a[kk][r4] holds row h = r4 & 1, columns of j = 2 kk + (r4 >> 1)
+    // layer 1 straight into the A-fragment layout: a[kk][r4] holds row h = r4 & 1, columns of j = 2 kk + (r4 >> 1); the
+    // four columns of one (t, h) are one activation group
     uint32_t ah[2][4], al[2][4];
 #pragma unroll
     for (int t = 0; t < 2; ++t) {                  // t = kk: j = 2 t, 2 t + 1
@@ -205,17 +213,22 @@ __device__ __forceinline__ void mlp_forward_mma(const uint4* __restrict__ s_frag
 #pragma unroll
       for (int i = 0; i < D; ++i) ww[i] = col[i * 2 + t];
 #pragma unroll
-      for (int jj = 0; jj < 2; ++jj)
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          if (REPL && h == 1) { ah[t][2 * jj + 1] = ah[t][2 * jj]; al[t][2 * jj + 1] = al[t][2 * jj]; continue; }
-          u64 z = jj ? pack2(bb.z, bb.w) : pack2(bb.x, bb.y);
-#pragma unroll
-          for (int i = 0; i < D; ++i) fma2(z, pack2(xr[h][i], xr[h][i]), jj ? pack2(ww[i].z, ww[i].w) : pack2(ww[i].x, ww[i].y));
-          float a0, a1;
-          act_pair_mma<FAST>(z, a0, a1);
-          split_pair(a0, a1, ah[t][2 * jj + h], al[t][2 * jj + h]);
+      for (int h = 0; h < 2; ++h) {
+        if (REPL && h == 1) {
+          ah[t][1] = ah[t][0]; al[t][1] = al[t][0]; ah[t][3] = ah[t][2]; al[t][3] = al[t][2];
+          continue;
         }
+        u64 z0 = pack2(bb.x, bb.y), z1 = pack2(bb.z, bb.w);
+#pragma unroll
+        for (int i = 0; i < D; ++i) {
+          fma2(z0, pack2(xr[h][i], xr[h][i]), pack2(ww[i].x, ww[i].y));
+          fma2(z1, pack2(xr[h][i], xr[h][i]), pack2(ww[i].z, ww[i].w));
+        }
+        float a[4];
+        act_group_mma<FAST>(z0, z1, a[0], a[1], a[2], a[3]);
+        split_pair(a[0], a[1], ah[t][h], al[t][h]);
+        split_pair(a[2], a[3], ah[t][2 + h], al[t][2 + h]);
+      }
     }
     // layer 2 on the tensor cores, accumulators initialised to the bias
     float acc[4][4];
@@ -226,11 +239,17 @@ __device__ __forceinline__ void mlp_forward_mma(const uint4* __restrict__ s_frag
       acc[2 * t + 1][0] = bb.z; acc[2 * t + 1][1] = bb.w; acc[2 * t + 1][2] = bb.z; acc[2 * t + 1][3] = bb.w;
     }
     mma_product_w(acc, ah, al, s_frag, 0, lane);
+    // activation groups: the columns of n-tiles j and j + 1 (j = 0, 2) of one row
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      act_pair_mma<FAST>(pack2(acc[j][0], acc[j][1]), acc[j][0], acc[j][1]);
-      if constexpr (REPL) { acc[j][2] = acc[j][0]; acc[j][3] = acc[j][1]; }
-      else act_pair_mma<FAST>(pack2(acc[j][2], acc[j][3]), acc[j][2], acc[j][3]);
+    for (int j = 0; j < 4; j += 2) {
+      act_group_mma<FAST>(pack2(acc[j][0], acc[j][1]), pack2(acc[j + 1][0], acc[j + 1][1]),
+                          acc[j][0], acc[j][1], acc[j + 1][0], acc[j + 1][1]);
+      if constexpr (REPL) {
+        acc[j][2] = acc[j][0]; acc[j][3] = acc[j][1]; acc[j + 1][2] = acc[j + 1][0]; acc[j + 1][3] = acc[j + 1][1];
+      } else {
+        act_group_mma<FAST>(pack2(acc[j][2], acc[j][3]), pack2(acc[j + 1][2], acc[j + 1][3]),
+                            acc[j][2], acc[j][3], acc[j + 1][2], acc[j + 1][3]);
+      }
     }
     // head partials: sum over this lane's 8 columns, as one packed accumulator per row (even / odd columns)
 #pragma unroll
