@@ -325,6 +325,12 @@ int rlsde_env_step(const rlsde_env* env, int64_t K, const void* state_dev, const
 int rlsde_noise_fill(uint64_t seed, int64_t traj_offset, int64_t K, int32_t d, int64_t pass_begin, int64_t n_pass,
                      double dt, float* out_dev, void* stream);
 
+/* host only: the bounds behind the clamp-free precise tanh of the d = 1, hidden width 32 tensor-core forward policy, from
+   its folded, pre-scaled image (params_host: state_dict order).  out[0]: an upper bound on every layer-2 pre-activation
+   (the clamp-free layer 2 is used when it is <= 30); out[1]: every layer-1 pre-activation is <= 30 while |x| <= out[1]
+   (negative: for no x) */
+int rlsde_fwd_mma_clamp_bounds(const float* params_host, double* out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -722,4 +722,12 @@ int rlsde_noise_fill(uint64_t seed, int64_t traj_offset, int64_t K, int32_t d, i
   return RLSDE_OK;
 }
 
+int rlsde_fwd_mma_clamp_bounds(const float* params_host, double* out) {
+  if (!params_host || !out) return RLSDE_ERR_INVALID_ARG;
+  MlpConst<1, 32> W;
+  pack_mlp_const_folded<1, 32>(params_host, W);
+  fwd_mma_clamp_bounds<1, 32>(W, out[0], out[1]);
+  return RLSDE_OK;
+}
+
 }  // extern "C"

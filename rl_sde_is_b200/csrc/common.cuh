@@ -43,6 +43,11 @@ __device__ __forceinline__ u64 add2(u64 a, u64 b) {
   asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
   return d;
 }
+__device__ __forceinline__ u64 sub2(u64 a, u64 b) {
+  u64 d;
+  asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+  return d;
+}
 __device__ __forceinline__ u64 mul2(u64 a, u64 b) {
   u64 d;
   asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
@@ -110,6 +115,8 @@ __device__ __forceinline__ void rsig_pair(u64 acc, float& r0, float& r1) {
 // z in [-200, 200], |r - 1 / (2^z + 1)| <= k 2^-24 (r + 2^-31) + 2^-31 with k = 3.5 (G = 2) / 4.5 (G = 4), against 2.5
 // ungrouped (tests/test_fwd_grouped_rcp.py restates the arithmetic); MUFU.EX2 / RCP add their own few ulp as before.  So
 // tanh = 1 - 2 r moves by at most ~2 ulp of 1 (~2.4e-7) more than with G = 1.
+// CLAMP = false leaves the clamp out.  Only for inputs known to stay <= RCP_GROUP_SAFE_Z (fwd_mma_clamp_bounds): there
+// the clamp is the identity, so both forms give the same bits.
 #ifndef RLSDE_FWD_RCP_GROUP
 #define RLSDE_FWD_RCP_GROUP 4
 #endif
@@ -118,7 +125,10 @@ struct RcpGroup {
   static_assert(G == 1 || G == 2 || G == 4, "RLSDE_FWD_RCP_GROUP is 1, 2 or 4");
   static constexpr float ZMAX = G == 4 ? 31.0f : 63.0f;   // the clamp on z (unused for G = 1)
 };
-template <int G>
+// the bound a host-side proof must establish before CLAMP = false: one below the smallest clamp, which leaves room for
+// the float32 / tensor-core rounding of z against its bound computed in double
+constexpr double RCP_GROUP_SAFE_Z = 30.0;
+template <int G, bool CLAMP = true>
 __device__ __forceinline__ void rsig_group(u64 za, u64 zb, float& r0, float& r1, float& r2, float& r3) {
   if constexpr (G == 1) {
     rsig_pair(za, r0, r1);
@@ -127,8 +137,10 @@ __device__ __forceinline__ void rsig_group(u64 za, u64 zb, float& r0, float& r1,
     float z[4];
     unpack2(za, z[0], z[1]);
     unpack2(zb, z[2], z[3]);
+    if constexpr (CLAMP) {
 #pragma unroll
-    for (int i = 0; i < 4; ++i) asm("min.NaN.f32 %0, %0, %1;" : "+f"(z[i]) : "f"(RcpGroup<G>::ZMAX));   // NaN stays NaN
+      for (int i = 0; i < 4; ++i) asm("min.NaN.f32 %0, %0, %1;" : "+f"(z[i]) : "f"(RcpGroup<G>::ZMAX));   // NaN stays NaN
+    }
     const u64 one = 0x3f8000003f800000ull;
     const u64 da = add2(pack2(mufu_ex2(z[0]), mufu_ex2(z[1])), one);
     const u64 db = add2(pack2(mufu_ex2(z[2]), mufu_ex2(z[3])), one);

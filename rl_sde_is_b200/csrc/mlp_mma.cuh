@@ -19,6 +19,7 @@
 // handed-over trajectory by putting its state in all 32 rows (rollout_warp.cuh, RESUME): it gets K1's action bit for bit
 // (and evaluates only what differs, REPL below).
 #pragma once
+#include <cmath>
 #include <cstring>
 #include <cuda_fp16.h>
 #include "common.cuh"
@@ -105,11 +106,14 @@ __device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], 
                : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
                : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
-// x0, x1 -> float16 pairs hi, lo with x ~ hi + lo  (x0 in the low half)
+// x0, x1 -> float16 pairs hi, lo with x ~ hi + lo  (x0 in the low half).  The residual x - hi is one packed subtraction
+// (FADD2; it rounds like the two scalar ones): F2FP, 2 HADD2.F32, FADD2, F2FP per pair.
 __device__ __forceinline__ void split_pair(float x0, float x1, uint32_t& hi, uint32_t& lo) {
   const __half2 h = __floats2half2_rn(x0, x1);
   const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(x0 - hf.x, x1 - hf.y);
+  float l0, l1;
+  unpack2(sub2(pack2(x0, x1), pack2(hf.x, hf.y)), l0, l1);
+  const __half2 l = __floats2half2_rn(l0, l1);
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
@@ -161,22 +165,77 @@ inline void pack_mlp_mma(const MlpConst<D, 32>& W, MlpMma<D>& out) {
       }
   for (int k = 0; k < ((D + 3) & ~3); ++k) out.b3[k] = W.b3[k];
 }
+// Where the clamp of rsig_group cannot bind, proven on the host (in double) from the folded image the kernel is launched
+// with, so that the kernel may leave it out (rsig_group<G, false>) and compute the same bits:
+//   layer 2: its inputs are r in [0, 1], so z2_n <= b2_n + sum_k max(W2_nk, 0) =: z2_max.  The launcher takes the
+//            clamp-free kernel when z2_max <= RCP_GROUP_SAFE_Z;
+//   layer 1: z1_j = b1_j + sum_i W1_ji x_i <= b1_j + (sum_i |W1_ji|) max_i |x_i|, which stays <= RCP_GROUP_SAFE_Z while
+//            max_i |x_i| <= x1_max (negative: for no x).  A warp whose 32 states all satisfy it skips the clamp in layer 1.
+template <int D, int H>
+inline void fwd_mma_clamp_bounds(const MlpConst<D, H>& W, double& z2_max, double& x1_max) {
+  z2_max = -HUGE_VAL;
+  for (int n = 0; n < H; ++n) {
+    double z = (double)W.b2[n];
+    for (int k = 0; k < H; ++k) z += W.W2t[k][n] > 0.0f ? (double)W.W2t[k][n] : 0.0;
+    z2_max = z > z2_max ? z : z2_max;
+  }
+  x1_max = HUGE_VAL;
+  for (int j = 0; j < H; ++j) {
+    double a = 0.0;
+    for (int i = 0; i < D; ++i) a += fabs((double)W.W1t[i][j]);
+    const double room = RCP_GROUP_SAFE_Z - (double)W.b1[j];
+    if (room < 0.0) x1_max = -1.0;
+    else if (a > 0.0 && room / a < x1_max) x1_max = room / a;
+  }
+}
+
 // what a block copies to shared memory at its start (16-byte words): the fragment table, then the column table
 constexpr int MLP_MMA_FRAG_WORDS = 2 * 2 * 2 * 32;
 template <int D>
 constexpr int mlp_mma_smem_words() { return (int)(offsetof(MlpMma<D>, b3) / 16); }
 
 // activations of two packed pairs of pre-activations of one row: r = 1 / (2^z + 1) on a pack_mlp_const_folded image, with
-// one reciprocal per RLSDE_FWD_RCP_GROUP of them (rsig_group), tanh otherwise.  Which activations share a reciprocal
-// depends only on the layer and the hidden units, never on the lane or the row: the REPL continuation below computes the
-// same groups as the full tile.
-template <bool FAST>
+// one reciprocal per RLSDE_FWD_RCP_GROUP of them (rsig_group; CLAMP = false only where fwd_mma_clamp_bounds proves the
+// clamp cannot bind), tanh otherwise.  Which activations share a reciprocal depends only on the layer and the hidden
+// units, never on the lane or the row: the REPL continuation below computes the same groups as the full tile.
+template <bool FAST, bool CLAMP = true>
 __device__ __forceinline__ void act_group_mma(u64 za, u64 zb, float& a0, float& a1, float& a2, float& a3) {
   if constexpr (FAST) {
     tanh_pair<true>(za, a0, a1);
     tanh_pair<true>(zb, a2, a3);
   } else {
-    rsig_group<RLSDE_FWD_RCP_GROUP>(za, zb, a0, a1, a2, a3);
+    rsig_group<RLSDE_FWD_RCP_GROUP, CLAMP>(za, zb, a0, a1, a2, a3);
+  }
+}
+
+// layer 1 of rows g + 8 (2 mt + h), h = 0, 1 (inputs xr[h]) straight into the A-fragment layout of layer 2: a[kk][r4] holds
+// row h = r4 & 1, columns of j = 2 kk + (r4 >> 1); the four columns of one (t, h) are one activation group
+template <int D, bool FAST, bool REPL, bool CLAMP>
+__device__ __forceinline__ void layer1_mma(const float4* col, const float (&xr)[2][D], uint32_t (&ah)[2][4],
+                                           uint32_t (&al)[2][4]) {
+#pragma unroll
+  for (int t = 0; t < 2; ++t) {                  // t = kk: j = 2 t, 2 t + 1
+    const float4 bb = col[D * 2 + t];
+    float4 ww[D];
+#pragma unroll
+    for (int i = 0; i < D; ++i) ww[i] = col[i * 2 + t];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      if (REPL && h == 1) {
+        ah[t][1] = ah[t][0]; al[t][1] = al[t][0]; ah[t][3] = ah[t][2]; al[t][3] = al[t][2];
+        continue;
+      }
+      u64 z0 = pack2(bb.x, bb.y), z1 = pack2(bb.z, bb.w);
+#pragma unroll
+      for (int i = 0; i < D; ++i) {
+        fma2(z0, pack2(xr[h][i], xr[h][i]), pack2(ww[i].x, ww[i].y));
+        fma2(z1, pack2(xr[h][i], xr[h][i]), pack2(ww[i].z, ww[i].w));
+      }
+      float a[4];
+      act_group_mma<FAST, CLAMP>(z0, z1, a[0], a[1], a[2], a[3]);
+      split_pair(a[0], a[1], ah[t][h], al[t][h]);
+      split_pair(a[2], a[3], ah[t][2 + h], al[t][2 + h]);
+    }
   }
 }
 
@@ -185,10 +244,12 @@ __device__ __forceinline__ void act_group_mma(u64 za, u64 zb, float& a0, float& 
 // REPL: every lane holds the same trajectory (the warp-per-trajectory continuation), so all 32 rows are equal: one m16
 // tile and one row per lane are evaluated and copied to the others -- the values the full tile would hold, at a quarter of
 // the MUFU and half of the HMMA work on the latency path of a lone trajectory.
-template <int D, bool FAST, bool REPL = false>
+// CLAMP2 = false: layer 2 without the clamp of rsig_group (the host has proven z2_max <= RCP_GROUP_SAFE_Z);
+// clamp1 = false: layer 1 without it (warp-uniform: every lane's state is within x1_max).  Precise tanh only.
+template <int D, bool FAST, bool REPL = false, bool CLAMP2 = true>
 __device__ __forceinline__ void mlp_forward_mma(const uint4* __restrict__ s_frag, const float4* __restrict__ s_col,
                                                 const float (&b3)[(D + 3) & ~3], int lane, const float (&x)[D],
-                                                float (&u)[D]) {
+                                                float (&u)[D], bool clamp1 = true) {
   static_assert(FAST || RLSDE_FWD_FOLDED, "the precise tanh is evaluated on the folded image");
   constexpr unsigned FULL = 0xffffffffu;
   constexpr int NF = MlpMma<D>::NF;
@@ -203,33 +264,9 @@ __device__ __forceinline__ void mlp_forward_mma(const uint4* __restrict__ s_frag
     for (int h = 0; h < 2; ++h)
 #pragma unroll
       for (int i = 0; i < D; ++i) xr[h][i] = __shfl_sync(FULL, x[i], quad | (2 * mt + h));
-    // layer 1 straight into the A-fragment layout: a[kk][r4] holds row h = r4 & 1, columns of j = 2 kk + (r4 >> 1); the
-    // four columns of one (t, h) are one activation group
     uint32_t ah[2][4], al[2][4];
-#pragma unroll
-    for (int t = 0; t < 2; ++t) {                  // t = kk: j = 2 t, 2 t + 1
-      const float4 bb = col[D * 2 + t];
-      float4 ww[D];
-#pragma unroll
-      for (int i = 0; i < D; ++i) ww[i] = col[i * 2 + t];
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        if (REPL && h == 1) {
-          ah[t][1] = ah[t][0]; al[t][1] = al[t][0]; ah[t][3] = ah[t][2]; al[t][3] = al[t][2];
-          continue;
-        }
-        u64 z0 = pack2(bb.x, bb.y), z1 = pack2(bb.z, bb.w);
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-          fma2(z0, pack2(xr[h][i], xr[h][i]), pack2(ww[i].x, ww[i].y));
-          fma2(z1, pack2(xr[h][i], xr[h][i]), pack2(ww[i].z, ww[i].w));
-        }
-        float a[4];
-        act_group_mma<FAST>(z0, z1, a[0], a[1], a[2], a[3]);
-        split_pair(a[0], a[1], ah[t][h], al[t][h]);
-        split_pair(a[2], a[3], ah[t][2 + h], al[t][2 + h]);
-      }
-    }
+    if (!FAST && !clamp1) layer1_mma<D, FAST, REPL, false>(col, xr, ah, al);
+    else layer1_mma<D, FAST, REPL, true>(col, xr, ah, al);
     // layer 2 on the tensor cores, accumulators initialised to the bias
     float acc[4][4];
 #pragma unroll
@@ -242,13 +279,13 @@ __device__ __forceinline__ void mlp_forward_mma(const uint4* __restrict__ s_frag
     // activation groups: the columns of n-tiles j and j + 1 (j = 0, 2) of one row
 #pragma unroll
     for (int j = 0; j < 4; j += 2) {
-      act_group_mma<FAST>(pack2(acc[j][0], acc[j][1]), pack2(acc[j + 1][0], acc[j + 1][1]),
-                          acc[j][0], acc[j][1], acc[j + 1][0], acc[j + 1][1]);
+      act_group_mma<FAST, CLAMP2>(pack2(acc[j][0], acc[j][1]), pack2(acc[j + 1][0], acc[j + 1][1]),
+                                  acc[j][0], acc[j][1], acc[j + 1][0], acc[j + 1][1]);
       if constexpr (REPL) {
         acc[j][2] = acc[j][0]; acc[j][3] = acc[j][1]; acc[j + 1][2] = acc[j + 1][0]; acc[j + 1][3] = acc[j + 1][1];
       } else {
-        act_group_mma<FAST>(pack2(acc[j][2], acc[j][3]), pack2(acc[j + 1][2], acc[j + 1][3]),
-                            acc[j][2], acc[j][3], acc[j + 1][2], acc[j + 1][3]);
+        act_group_mma<FAST, CLAMP2>(pack2(acc[j][2], acc[j][3]), pack2(acc[j + 1][2], acc[j + 1][3]),
+                                    acc[j][2], acc[j][3], acc[j + 1][2], acc[j + 1][3]);
       }
     }
     // head partials: sum over this lane's 8 columns, as one packed accumulator per row (even / odd columns)

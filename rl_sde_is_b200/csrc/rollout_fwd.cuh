@@ -77,6 +77,8 @@ struct FwdArgs {
   int blocks_per_sm_cap;         // > 0: cap on resident blocks per SM of the thread-per-trajectory forward kernel (tuning)
   int policy_mma;                // 1: the thread-per-trajectory forward kernel evaluates the policy with mlp_forward_mma (and
                                  // the kernel that continues its handed-over trajectories does the same), 0: with FFMA2
+  float mma_x1_max;              // set by the launcher: mlp_forward_mma skips the layer-1 clamp of a warp whose states all
+                                 // have max_i |x_i| <= this (fwd_mma_clamp_bounds)
   // ---- transition stream (replay-buffer sampler, approximate_methods.py:513-545): trajectory `t` writes the tuple of
   //      its pass k at slot tr_base[t] + k of the five arrays below.  nullptr = no stream.
   const long long* tr_base;
@@ -157,12 +159,15 @@ template <int D, bool MMA> struct FwdMmaSel { typedef typename std::conditional<
 // (d = 1: 8 blocks per SM), <= 102 (d = 2..4: 5 blocks) and <= 128 (d = 10: 4 blocks) -- it finds them when asked.
 // The tensor-core policy holds a half-tile of fragments (A hi / lo, accumulators, B operands) on top of the pass state:
 // 80 registers at 6 blocks per SM, measured best (d = 1, 1e6 trajectories: 21.1 ms against 21.8 / 22.2 ms at 5 / 4).
+// At 7 blocks (72 registers) ptxas spills 104 B (float32 state) even with the noise in shared memory.
 #ifndef RLSDE_FWD_MMA_MIN_BLOCKS
 #define RLSDE_FWD_MMA_MIN_BLOCKS 6
 #endif
 template <int D, bool MMA>
 constexpr int fwd_min_blocks() { return MMA ? RLSDE_FWD_MMA_MIN_BLOCKS : (D == 1 ? 8 : (D <= 4 ? 5 : 4)); }
-template <int D, int H, bool F64, bool FAST, bool MMA>
+// CLAMP2 = false (MMA, precise tanh): layer 2 of the policy without the clamp of rsig_group, launched where the host has
+// proven it cannot bind (fwd_mma_clamp_bounds)
+template <int D, int H, bool F64, bool FAST, bool MMA, bool CLAMP2 = true>
 __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_kernel(const __grid_constant__ MlpConst<D, H> W,
                                                           const __grid_constant__ FwdArgs A,
                                                           const __grid_constant__ typename FwdMmaSel<D, MMA>::type M) {
@@ -171,7 +176,11 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
   constexpr int BPP = NoisePlan<D>::BPP;
   constexpr int NZ = NoisePlan<D>::NZ;
   constexpr unsigned FULL = 0xffffffffu;
+  // MMA: the normals of the current noise block wait in shared memory, one column per thread, instead of in registers,
+  // where they cost the tensor-core kernel spills and a select chain per pass
+  constexpr bool NOISE_SMEM = MMA && SPB > 1;
   const int lane = threadIdx.x & 31;
+  __shared__ float s_noise[NOISE_SMEM ? NZ : 1][128];
   // MMA: the block's copy of the fragment and column tables (mlp_mma.cuh)
   __shared__ uint4 s_mma[MMA ? mlp_mma_smem_words<D>() : 1];
   if constexpr (MMA) {
@@ -198,11 +207,11 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
   int k = 0, ck = 0;
   real x[D];
   real G = 0, S = 0, L2 = 0;
-  float z[NZ];
+  float z[NOISE_SMEM ? 1 : NZ];
 #pragma unroll
   for (int i = 0; i < D; ++i) x[i] = F64 ? (real)A.x0_d[i] : (real)A.x0_f[i];
 #pragma unroll
-  for (int i = 0; i < NZ; ++i) z[i] = 0.f;
+  for (int i = 0; i < (NOISE_SMEM ? 1 : NZ); ++i) z[i] = 0.f;
 
   for (unsigned it = 0;; ++it) {
     if ((it & (SPB - 1)) == 0) {
@@ -348,7 +357,10 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
           float zz[4];
           noise_block(A.seed, gt, (unsigned)(k / SPB) * BPP + q, A.noise_scale2, zz);
 #pragma unroll
-          for (int s = 0; s < 4; ++s) z[4 * q + s] = zz[s];
+          for (int s = 0; s < 4; ++s) {
+            if constexpr (NOISE_SMEM) s_noise[4 * q + s][threadIdx.x] = zz[s];
+            else z[4 * q + s] = zz[s];
+          }
         }
       }
     }
@@ -357,7 +369,20 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
     float xf[D], u[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) xf[i] = (float)x[i];
-    if constexpr (MMA) mlp_forward_mma<D, FAST>(s_mma, reinterpret_cast<const float4*>(s_mma + MLP_MMA_FRAG_WORDS), M.b3, lane, xf, u);
+    if constexpr (MMA) {
+      bool clamp1 = true;
+      if constexpr (!FAST) {
+        bool in_x1 = true;
+#pragma unroll
+        for (int i = 0; i < D; ++i) in_x1 = in_x1 && fabsf(xf[i]) <= A.mma_x1_max;
+        clamp1 = !__all_sync(FULL, in_x1);
+      }
+      // two inlined copies of the whole policy, one per value of clamp1: with the branch around layer 1 alone ptxas
+      // spilled ~200 B, with the branch here the float32-state kernel has no spill at all
+      const float4* s_col = reinterpret_cast<const float4*>(s_mma + MLP_MMA_FRAG_WORDS);
+      if (clamp1) mlp_forward_mma<D, FAST, false, CLAMP2>(s_mma, s_col, M.b3, lane, xf, u, true);
+      else mlp_forward_mma<D, FAST, false, CLAMP2>(s_mma, s_col, M.b3, lane, xf, u, false);
+    }
     else if constexpr (!FAST && RLSDE_FWD_FOLDED) mlp_forward_folded<D, H>(W, xf, u);   // W is a pack_mlp_const_folded image
     else mlp_forward<D, H, FAST>(W, xf, u);
 
@@ -371,7 +396,9 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
       const int sub = (int)(it & (SPB - 1));
 #pragma unroll
       for (int i = 0; i < D; ++i) {
-        if constexpr (SPB == 1) {
+        if constexpr (NOISE_SMEM) {
+          dB[i] = s_noise[sub * D + i][threadIdx.x];
+        } else if constexpr (SPB == 1) {
           dB[i] = z[i];
         } else {
           float v = z[i];

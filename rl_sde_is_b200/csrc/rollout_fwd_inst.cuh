@@ -12,7 +12,16 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
   typename FwdMmaSel<D, MMA>::type M;
   if constexpr (MMA) pack_mlp_mma<D>(W, M);
   else M.unused = 0;
+  FwdArgs a = args;
   auto kern = rollout_fwd_kernel<D, H, F64, FAST, MMA>;
+  a.mma_x1_max = -1.0f;
+  if constexpr (MMA && !FAST) {
+    // leave the clamp of the grouped reciprocal out where it provably cannot bind (same bits, fewer instructions)
+    double z2_max, x1_max;
+    fwd_mma_clamp_bounds<D, H>(W, z2_max, x1_max);
+    a.mma_x1_max = (float)x1_max;
+    if (z2_max <= RCP_GROUP_SAFE_Z) kern = rollout_fwd_kernel<D, H, F64, FAST, MMA, false>;
+  }
   // Small batches: one warp per block so the warps spread over SMs (latency-bound regime);
   // large batches: persistent grid of 128-thread blocks, as many as are co-resident.
   int block = 128;
@@ -32,7 +41,6 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
   // Schedule (rollout_fwd.cuh; chosen by the C ABI layer: args.q_quantum passes per slice, or run to completion with
   // the tail handed over to the warp-per-trajectory kernel at args.q_handoff live trajectories): large batches only, and
   // only if the caller's workspace holds a ring with one record per trajectory plus one per lane.
-  FwdArgs a = args;
   const long long lanes = grid * block;
   long long need_cap = 1;
   int cap_log2 = 0;
