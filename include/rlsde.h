@@ -13,6 +13,7 @@
  *                       estimate_fht_vectorized     approximate_methods.py:650-695
  *                       (which call env.step_torch / env.step once per pass:
  *                        environments.py:139-162,201-226; environments_2d.py:134-153,184-205)
+ *   rlsde_rollout_fwd_table  the same rollout at d = 1 under a tabulated control (DP greedy policy, HJB u*)
  *   rlsde_rollout_bwd   eff_loss.backward()         reinforce_deterministic_core.py:240
  *                       (BPTT through every pass; states are never detached, :88)
  *   rlsde_tables        compute_r_table / compute_p_tensor_batch   dynamic_programming.py:3-36
@@ -191,6 +192,21 @@ int rlsde_rollout_fwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
                       void* G_dev, void* S_dev, int32_t* T_dev, void* l2_dev, void* logw_dev,
                       float* path_dev, double* stats_dev, void* workspace_dev, size_t workspace_bytes,
                       void* stream);
+
+/*
+ * Forward rollout at d = 1 under a tabulated control instead of an MLP:  u_j = u_table[idx(X_j)],
+ *   idx(x) = floor((clip(x, grid_lo, grid_hi) - grid_lo) / grid_h), clamped to [0, n_grid - 1],
+ * evaluated on the state in state precision (float32, or float64 with RLSDE_F_STATE_F64) -- the lookup of the l2 error.
+ * u_table_dev: float[cfg->n_grid]; policy_opt_dev (optional, for l2) lives on the same grid.  Everything else is
+ * rlsde_rollout_fwd's: outputs, statistics record, RLSDE_F_NOISE_INJECTED / STOCH_INT_EXACT / STATE_F64 and the hit
+ * rule; tanh and kernel-family flags do not apply, RLSDE_F_STORE_PATH is refused (a table has no gradient).
+ * Errors: env->d != 1 -> RLSDE_ERR_UNSUPPORTED; u_table_dev NULL, n_grid < 1 or grid_h <= 0 -> RLSDE_ERR_INVALID_ARG;
+ * a workspace smaller than rlsde_workspace_bytes(0) -> RLSDE_ERR_WORKSPACE.
+ */
+int rlsde_rollout_fwd_table(const rlsde_env* env, const float* u_table_dev, const rlsde_rollout_cfg* cfg,
+                            const float* noise_dev, const float* policy_opt_dev, void* G_dev, void* S_dev, int32_t* T_dev,
+                            void* l2_dev, void* logw_dev, double* stats_dev, void* workspace_dev, size_t workspace_bytes,
+                            void* stream);
 
 /*
  * Forward rollout that also streams every transition out (replay-buffer sampler, SURVEY 8f-4):

@@ -39,7 +39,7 @@ EXPORTED_SYMBOLS = [
     "rlsde_param_count", "rlsde_workspace_bytes", "rlsde_workspace_bytes_bwd", "rlsde_rollout_fwd", "rlsde_rollout_bwd", "rlsde_reduce_stats",
     "rlsde_tables", "rlsde_tables_colsum", "rlsde_env_step", "rlsde_noise_fill",
     "rlsde_dp_scratch_bytes", "rlsde_dp_sweep", "rlsde_dp_rowmax", "rlsde_rollout_transitions", "rlsde_launch_count", "rlsde_reinforce_step",
-    "rlsde_reinforce_rollout", "rlsde_reinforce_apply", "rlsde_fwd_mma_clamp_bounds",
+    "rlsde_reinforce_rollout", "rlsde_reinforce_apply", "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table",
 ]
 
 
@@ -101,6 +101,8 @@ def load():
     lib.rlsde_workspace_bytes_bwd.argtypes = [i64, C.c_int32, C.c_int32]
     lib.rlsde_rollout_fwd.argtypes = [C.POINTER(RlsdeEnv), C.POINTER(RlsdeMlp), vp, C.POINTER(RlsdeRolloutCfg),
                                       vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
+    lib.rlsde_rollout_fwd_table.argtypes = [C.POINTER(RlsdeEnv), vp, C.POINTER(RlsdeRolloutCfg), vp, vp, vp, vp, vp, vp, vp, vp,
+                                            vp, C.c_size_t, vp]
     lib.rlsde_rollout_transitions.argtypes = [C.POINTER(RlsdeEnv), C.POINTER(RlsdeMlp), vp, C.POINTER(RlsdeRolloutCfg),
                                               vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
     lib.rlsde_reinforce_step.argtypes = [C.POINTER(RlsdeEnv), C.POINTER(RlsdeMlp), vp, vp, vp, C.POINTER(RlsdeRolloutCfg), vp,
@@ -123,7 +125,7 @@ def load():
     for name in ("rlsde_device_info", "rlsde_supported", "rlsde_rollout_fwd", "rlsde_rollout_bwd", "rlsde_reduce_stats",
                  "rlsde_tables", "rlsde_tables_colsum", "rlsde_env_step", "rlsde_noise_fill", "rlsde_dp_sweep", "rlsde_dp_rowmax",
                  "rlsde_rollout_transitions", "rlsde_reinforce_step", "rlsde_reinforce_rollout", "rlsde_reinforce_apply",
-                 "rlsde_fwd_mma_clamp_bounds"):
+                 "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table"):
         getattr(lib, name).restype = C.c_int
     _lib = lib
     return lib

@@ -17,19 +17,25 @@ import torch
 
 from . import _lib as L
 from . import rollout as R
+from .models import TabularPolicy
 from .reinforce_deterministic_core import _next_seed
 
 
 def _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, *, noise, seed, tanh, state_f64, device, dist, kernel="auto",
                         stoch_int="reference", want_logw=False):
-    d, H = R.policy_shape(model)
-    if d != env.d:
-        raise L.RlsdeError(f"policy dimension {d} != env.d {env.d}")
+    """An MLP policy runs on the fused MLP kernels; a ``TabularPolicy`` on ``rlsde_rollout_fwd_table`` (``tanh`` and
+    ``kernel`` do not apply to it)."""
+    table = isinstance(model, TabularPolicy)
+    if table:
+        if env.d != 1:
+            raise L.RlsdeError(f"a TabularPolicy is a 1-D control; env.d = {env.d}")
+    else:
+        d, H = R.policy_shape(model)
+        if d != env.d:
+            raise L.RlsdeError(f"policy dimension {d} != env.d {env.d}")
     rule = L.HIT_X0_IN_LB_RB if env.d == 1 else L.HIT_ALL_GE_LB      # environments.py:48-49 / environments_2d.py:56-57
     env_c = R.env_struct(env, rule)
-    mlp_c = L.make_mlp(d, H)
     dev = R._cuda_device(device)
-    params_host = R.flat_parameters(model).detach().to("cpu", torch.float32).contiguous().numpy()
     if noise is not None:
         noise = torch.as_tensor(np.ascontiguousarray(noise, dtype=np.float32)) if not torch.is_tensor(noise) else noise
         noise = noise.to(device=dev, dtype=torch.float32).contiguous()
@@ -38,11 +44,18 @@ def _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, *, noise, see
         if env.d != 1:
             raise L.RlsdeError("the policy l2 error lookup is defined for the 1-D state grid only (environments.py:318-321)")
         grid = (env.state_space_low, env.state_space_high, env.h_state)
-    opts = dict(seed=_next_seed(seed), n_steps_lim=int(k_max), noise=noise, tanh=tanh, state_f64=state_f64, kernel=kernel,
-                policy_opt=policy_opt, grid=grid, want_logw=want_logw, stoch_int=stoch_int, device=dev)
+    opts = dict(seed=_next_seed(seed), n_steps_lim=int(k_max), noise=noise, state_f64=state_f64, policy_opt=policy_opt,
+                want_logw=want_logw, stoch_int=stoch_int, device=dev)
     if dist is not None:
         opts.update(traj_offset=dist.traj_offset, K_global=dist.K_global)
-    out = R.rollout_forward(env_c, mlp_c, params_host, int(batch_size), **opts)
+    if table:
+        if grid is not None and tuple(float(v) for v in grid) != model.grid:
+            raise L.RlsdeError(f"policy_opt lives on grid {grid}, the TabularPolicy on {model.grid}: they must share one")
+        out = R.rollout_forward_table(env_c, model.table, int(batch_size), grid=model.grid, **opts)
+    else:
+        params_host = R.flat_parameters(model).detach().to("cpu", torch.float32).contiguous().numpy()
+        out = R.rollout_forward(env_c, L.make_mlp(d, H), params_host, int(batch_size), tanh=tanh, kernel=kernel, grid=grid,
+                                **opts)
     stats = out.stats_dev
     if dist is not None:
         stats = dist.all_reduce_stats(stats.clone())

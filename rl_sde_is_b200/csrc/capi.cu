@@ -426,6 +426,46 @@ int rlsde_rollout_fwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
                           path_dev, stats_dev, none, workspace_dev, workspace_bytes, stream_);
 }
 
+int rlsde_rollout_fwd_table(const rlsde_env* env, const float* u_table_dev, const rlsde_rollout_cfg* cfg,
+                            const float* noise_dev, const float* policy_opt_dev, void* G_dev, void* S_dev, int32_t* T_dev,
+                            void* l2_dev, void* logw_dev, double* stats_dev, void* workspace_dev, size_t workspace_bytes,
+                            void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  if (!env || !cfg) return RLSDE_ERR_INVALID_ARG;
+  if (env->d != 1) return RLSDE_ERR_UNSUPPORTED;                 // tables, DP sweeps and the HJB solution are 1-D
+  if (!(env->dt > 0) || !(env->sigma > 0)) return RLSDE_ERR_INVALID_ARG;
+  if (env->hit_rule != RLSDE_HIT_ALL_GE_LB && env->hit_rule != RLSDE_HIT_X0_IN_LB_RB) return RLSDE_ERR_INVALID_ARG;
+  if (!u_table_dev || cfg->n_grid < 1 || !(cfg->grid_h > 0)) return RLSDE_ERR_INVALID_ARG;
+  if (!G_dev || !S_dev || !T_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
+  if (workspace_bytes < WS_COUNTER_BYTES + WS_STATS_BYTES) return RLSDE_ERR_WORKSPACE;
+  FwdArgs A;
+  memset(&A, 0, sizeof(A));
+  fill_env(env, A);
+  int rc = fill_cfg(cfg, A);
+  if (rc != RLSDE_OK) return rc;
+  if (A.flags & RLSDE_F_STORE_PATH) return RLSDE_ERR_INVALID_ARG;                 // no reverse pass through a table
+  if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
+  A.flags &= RLSDE_F_NOISE_INJECTED | RLSDE_F_STOCH_INT_EXACT | RLSDE_F_STATE_F64;   // kernel-family and tanh flags do not apply
+  A.noise = noise_dev; A.policy_opt = policy_opt_dev;
+  A.G = G_dev; A.S = S_dev; A.T = T_dev; A.l2 = l2_dev; A.logw = logw_dev;
+  A.counter = (unsigned long long*)workspace_dev;
+  if (A.K == 0) return RLSDE_OK;
+  int sm = 0;
+  if ((rc = device_sm_count(&sm)) != RLSDE_OK) return rc;
+  cudaError_t e = cudaMemsetAsync(workspace_dev, 0, WS_COUNTER_BYTES, stream);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+  int lrc = launch_rollout_fwd_table(u_table_dev, A, sm, stream);
+  if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd_table launch");
+  if (stats_dev) {
+    double* partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
+    const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
+    lrc = launch_reduce_stats(A.K, lim_eff, (A.flags & RLSDE_F_STATE_F64) != 0, G_dev, S_dev, T_dev, l2_dev, logw_dev,
+                              stats_dev, partial, stream);
+    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reduce_stats launch");
+  }
+  return RLSDE_OK;
+}
+
 int rlsde_rollout_transitions(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
                               const rlsde_rollout_cfg* cfg, const float* noise_dev, const int64_t* slot_base_dev,
                               float* states_dev, float* actions_dev, float* rewards_dev, float* next_states_dev,

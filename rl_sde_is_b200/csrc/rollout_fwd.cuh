@@ -548,4 +548,9 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
 template <int D, int H>
 int launch_rollout_fwd(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream);
 
+// d = 1 rollout under the control table_dev[grid_index(x)] (fwd_tab_d1.cu).  Tables of up to FWD_TAB_SMEM_MAX entries
+// (32 KB) are copied to shared memory when a block starts, larger ones are read through the read-only cache.
+constexpr long long FWD_TAB_SMEM_MAX = 8192;
+int launch_rollout_fwd_table(const float* table_dev, const FwdArgs& args, int sm_count, cudaStream_t stream);
+
 }  // namespace rlsde

@@ -10,6 +10,15 @@
 
 namespace rlsde {
 
+// Cell of the 1-D state grid of cfg.n_grid / grid_lo / grid_hi / grid_h that holds x (state precision, widened to double):
+// idx = floor((clip(x, lo, hi) - lo) / h), clamped to [0, n_grid - 1]   (environments.py:318-321).  The l2 error of
+// TrajOwner::pass and the tabulated control of rollout_fwd_tab_kernel (fwd_tab_d1.cu) both index with it.
+__device__ __forceinline__ long long grid_index(const FwdArgs& A, double x) {
+  const double xc = x < A.grid_lo ? A.grid_lo : (x > A.grid_hi ? A.grid_hi : x);
+  const long long gi = (long long)floor((xc - A.grid_lo) / A.grid_h);
+  return gi < 0 ? 0 : (gi >= A.n_grid ? A.n_grid - 1 : gi);
+}
+
 template <int D, bool F64>
 struct TrajOwner {
   typedef typename RealT<F64>::type real;
@@ -96,10 +105,7 @@ struct TrajOwner {
     const real S_prev = S;
     S = add_rn(S, su);
     if (want_l2) {
-      double xc = (double)x[0];
-      xc = xc < A.grid_lo ? A.grid_lo : (xc > A.grid_hi ? A.grid_hi : xc);
-      long long gi = (long long)floor((xc - A.grid_lo) / A.grid_h);
-      gi = gi < 0 ? 0 : (gi >= A.n_grid ? A.n_grid - 1 : gi);
+      const long long gi = grid_index(A, (double)x[0]);
       const float du = __fsub_rn(u[0], __ldg(A.policy_opt + gi));
       L2 = F64 ? (real)__dadd_rn((double)L2, __dmul_rn((double)__fmul_rn(du, du), A.dt_d))
                : (real)__fadd_rn((float)L2, __fmul_rn(__fmul_rn(du, du), A.dt_f));

@@ -5,7 +5,12 @@ Reference: rl_sde_is/models.py:4-18 (``mlp``) and reinforce_deterministic_core.p
 host-side use (plots, tests); the rollouts evaluate the policy inside the fused CUDA kernels, reading
 the parameters in state_dict order: ``policy.0.weight (H,d)``, ``policy.0.bias (H)``,
 ``policy.2.weight (H,H)``, ``policy.2.bias (H)``, ``policy.4.weight (d,H)``, ``policy.4.bias (d)``.
+
+``TabularPolicy`` is a 1-D control tabulated on ``env.state_space_h`` (the DP greedy policy, the HJB solution u*): the
+rollouts of ``approximate_methods`` evaluate it inside their own kernel (``rlsde_rollout_fwd_table``).
 """
+import numpy as np
+import torch
 import torch.nn as nn
 
 
@@ -36,3 +41,37 @@ class DeterministicPolicy(nn.Module):
 
     def forward(self, state):
         return self.policy(state)
+
+
+class TabularPolicy(nn.Module):
+    """u(x) = actions[idx(x)] on the 1-D state grid ``env.state_space_h``, with the index of
+    ``env.get_state_idx_truncate``: idx(x) = floor((clip(x, low, high) - low) / h_state), computed in float64 and clamped
+    to the table.  The GPU rollouts evaluate the same lookup on the state in state precision.
+
+    ``actions``: shape (n_states, 1) or (n_states,), e.g. ``env.action_space_h[greedy_action_idx]`` (DP) or ``sol.policy_opt_table(env)``
+    (HJB).  The table is a float32 buffer, not a parameter: a TabularPolicy cannot be trained."""
+
+    def __init__(self, env, actions):
+        super().__init__()
+        if int(env.d) != 1:
+            raise ValueError(f"a TabularPolicy is a control on the 1-D state grid; env.d = {env.d}")
+        a = torch.as_tensor(np.asarray(actions.detach().cpu() if torch.is_tensor(actions) else actions, dtype=np.float32))
+        n = int(env.n_states)
+        if tuple(a.shape) not in ((n, 1), (n,)):
+            raise ValueError(f"actions must have shape ({n}, 1) or ({n},) (env.state_space_h), got {tuple(a.shape)}")
+        self.register_buffer("table", a.reshape(n, 1).clone())
+        self.low, self.high, self.h = float(env.state_space_low), float(env.state_space_high), float(env.h_state)
+
+    @property
+    def grid(self):
+        """``(low, high, h)`` of the state grid the table lives on."""
+        return self.low, self.high, self.h
+
+    def index(self, state):
+        """idx(x) of every row of ``state`` (shape (..., 1)), int64, clamped to [0, n_states - 1]."""
+        x = torch.as_tensor(state).detach().to(device=self.table.device, dtype=torch.float64)[..., 0]
+        gi = torch.floor((x.clamp(self.low, self.high) - self.low) / self.h).long()
+        return gi.clamp(0, self.table.shape[0] - 1)
+
+    def forward(self, state):
+        return self.table[self.index(state)]

@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
+from .models import TabularPolicy
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -30,6 +31,9 @@ def policy_linears(model):
     The fused kernels evaluate exactly ``Linear -> Tanh -> Linear -> Tanh -> Linear [-> Identity]``; any other stack
     (another nonlinearity, an output activation, dropout, ...) would be computed wrongly without an error, so the
     structure is checked positively."""
+    if isinstance(model, TabularPolicy):
+        raise L.RlsdeError("a TabularPolicy has no parameters, so no gradient: train an MLP policy; tables are rolled out by "
+                           "test_policy_vectorized, estimate_fht_vectorized and is_estimate")
     seq = getattr(model, "policy", model)
     if not isinstance(seq, torch.nn.Sequential):
         raise L.RlsdeError("the policy must be an nn.Sequential (or expose one as .policy), as built by models.mlp")
@@ -183,6 +187,62 @@ def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, 
                                    _ptr(T), _ptr(l2), _ptr(logw), _ptr(path), _ptr(stats), _ptr(ws), ws.numel(), stream)
     L.check(rc, "rlsde_rollout_fwd")
     return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=path, stats_dev=stats, cfg=cfg)
+
+
+def rollout_forward_table(env_c, table, K, *, grid, seed=0, n_steps_lim=10**6, noise=None, traj_offset=0, K_global=None,
+                          stoch_int="reference", state_f64=False, policy_opt=None, want_logw=True, device=None, tuning=None):
+    """One launch of the d = 1 rollout under the control ``table[idx(x)]`` (``rlsde_rollout_fwd_table``).  ``table``:
+    float32 values on ``grid = (lo, hi, h)``; ``policy_opt`` (l2 error), if given, lives on the same grid."""
+    lib = L.load()
+    dev = _cuda_device(device)
+    K = int(K)
+    if env_c.d != 1:
+        raise L.RlsdeError(f"a tabulated control is a 1-D policy; env.d = {env_c.d}")
+
+    def on_dev(a):
+        t = a if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, dtype=np.float32))
+        return t.to(device=dev, dtype=torch.float32).reshape(-1).contiguous()
+
+    tab = on_dev(table)
+    cfg = L.RlsdeRolloutCfg()
+    cfg.K, cfg.traj_offset, cfg.K_global = K, int(traj_offset), int(K_global if K_global is not None else int(traj_offset) + K)
+    cfg.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    cfg.n_steps_lim = int(n_steps_lim)
+    lo, hi, h = grid
+    cfg.n_grid, cfg.grid_lo, cfg.grid_hi, cfg.grid_h = int(tab.numel()), float(lo), float(hi), float(h)
+    flags = 0
+    if noise is not None:
+        if noise.device != dev or noise.dtype != torch.float32 or not noise.is_contiguous() or noise.dim() != 3 \
+                or noise.shape[1] != cfg.K_global or noise.shape[2] != 1:
+            raise L.RlsdeError(f"noise must be a contiguous float32 CUDA tensor [n_steps, {cfg.K_global}, 1]")
+        flags |= L.F_NOISE_INJECTED
+        cfg.noise_steps = int(noise.shape[0])
+    flags |= {"reference": 0, "exact": L.F_STOCH_INT_EXACT}[stoch_int]
+    real = torch.float64 if state_f64 else torch.float32
+    if state_f64:
+        flags |= L.F_STATE_F64
+    pol = None
+    if policy_opt is not None:
+        pol = on_dev(policy_opt)
+        if pol.numel() != cfg.n_grid:
+            raise L.RlsdeError(f"policy_opt has {pol.numel()} entries, the control table {cfg.n_grid}: they share one grid")
+    cfg.flags = flags
+    L.apply_tuning(cfg, tuning)
+    G = torch.empty(K, dtype=real, device=dev)
+    S = torch.empty(K, dtype=real, device=dev)
+    T = torch.empty(K, dtype=torch.int32, device=dev)
+    l2 = torch.empty(K, dtype=real, device=dev) if pol is not None else None
+    logw = torch.empty(K, dtype=real, device=dev) if want_logw else None
+    stats = torch.zeros(L.RLSDE_NSTATS, dtype=torch.float64, device=dev)
+    if K == 0:
+        return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=None, stats_dev=stats, cfg=cfg)
+    ws = _workspace(dev, K)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib.rlsde_rollout_fwd_table(env_c, _ptr(tab), cfg, _ptr(noise), _ptr(pol), _ptr(G), _ptr(S), _ptr(T), _ptr(l2),
+                                         _ptr(logw), _ptr(stats), _ptr(ws), ws.numel(), stream)
+    L.check(rc, "rlsde_rollout_fwd_table")
+    return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=None, stats_dev=stats, cfg=cfg)
 
 
 @dataclass
