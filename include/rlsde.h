@@ -71,6 +71,22 @@ typedef enum rlsde_status {
 #define RLSDE_F_STATE_F64 (1u << 3)      /* numpy-path arithmetic: f64 state and accumulators, f32 policy
                                             (SURVEY App. A-5); G/S/l2/logw outputs are double* */
 #define RLSDE_F_STORE_PATH (1u << 4)     /* write X_k checkpoints (needed by rlsde_rollout_bwd) */
+#define RLSDE_F_HIT_BRIDGE (1u << 6)     /* d = 1, rlsde_rollout_fwd / rlsde_rollout_fwd_table only: also detect target hits
+                                            between passes with a Brownian-bridge crossing test.  After the Euler-Maruyama
+                                            update of a pass whose X_k was no hit, with a = X_k, b = X_{k+1} and the target
+                                            [lb, rb] (rb = +inf under RLSDE_HIT_ALL_GE_LB): a and b on opposite sides of it
+                                            crossed; both below lb (above rb) crossed if U < exp(-2 (c-a)(c-b) / (sigma^2 dt))
+                                            with c = lb (rb).  A crossing sets X_{k+1} to that barrier, which the next pass's
+                                            hit test detects: T, G, S, logw, l2 keep their definitions and the hit is
+                                            credited at t_{k+1}.  U = (r.x + 0.5) 2^-32, r = Philox4x32-10(counter (traj_lo,
+                                            traj_hi, k, 0x42524447), key seed) of the global trajectory id, also with
+                                            RLSDE_F_NOISE_INJECTED; the Brownian increments are those of the rollout without
+                                            the flag.  p is evaluated in double.  exp(G - S_exact) stays the exact likelihood
+                                            ratio of the process stopped this way, so every policy estimates the same Psi.
+                                            With RLSDE_F_STORE_PATH -> RLSDE_ERR_INVALID_ARG (the reverse pass knows nothing
+                                            of the projection); d >= 2 -> RLSDE_ERR_UNSUPPORTED (no closed form for the
+                                            orthant); rlsde_rollout_transitions, rlsde_env_step and the training entry points
+                                            refuse it (RLSDE_ERR_INVALID_ARG) */
 #define RLSDE_F_KERNEL_THREAD (1u << 8)   /* force the throughput kernels (one trajectory per thread) */
 #define RLSDE_F_KERNEL_WARP (1u << 9)     /* force the latency kernels (one trajectory per warp; hidden width 32, and for the
                                             reverse pass ckpt_every == 1).  Default: chosen from K (small batches -> warp) */

@@ -23,6 +23,7 @@ F_STOCH_INT_EXACT = 1 << 2
 F_STATE_F64 = 1 << 3
 F_STORE_PATH = 1 << 4
 F_GRAD_F32 = 1 << 5
+F_HIT_BRIDGE = 1 << 6
 F_KERNEL_THREAD = 1 << 8
 F_KERNEL_WARP = 1 << 9
 F_KERNEL_TENSOR = 1 << 10

@@ -22,9 +22,9 @@ from .reinforce_deterministic_core import _next_seed
 
 
 def _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, *, noise, seed, tanh, state_f64, device, dist, kernel="auto",
-                        stoch_int="reference", want_logw=False):
+                        stoch_int="reference", want_logw=False, bridge=False):
     """An MLP policy runs on the fused MLP kernels; a ``TabularPolicy`` on ``rlsde_rollout_fwd_table`` (``tanh`` and
-    ``kernel`` do not apply to it)."""
+    ``kernel`` do not apply to it).  ``bridge``: the Brownian-bridge hit test between passes (d = 1)."""
     table = isinstance(model, TabularPolicy)
     if table:
         if env.d != 1:
@@ -33,6 +33,8 @@ def _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, *, noise, see
         d, H = R.policy_shape(model)
         if d != env.d:
             raise L.RlsdeError(f"policy dimension {d} != env.d {env.d}")
+    if bridge:
+        R._check_bridge(env.d)
     rule = L.HIT_X0_IN_LB_RB if env.d == 1 else L.HIT_ALL_GE_LB      # environments.py:48-49 / environments_2d.py:56-57
     env_c = R.env_struct(env, rule)
     dev = R._cuda_device(device)
@@ -45,7 +47,7 @@ def _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, *, noise, see
             raise L.RlsdeError("the policy l2 error lookup is defined for the 1-D state grid only (environments.py:318-321)")
         grid = (env.state_space_low, env.state_space_high, env.h_state)
     opts = dict(seed=_next_seed(seed), n_steps_lim=int(k_max), noise=noise, state_f64=state_f64, policy_opt=policy_opt,
-                want_logw=want_logw, stoch_int=stoch_int, device=dev)
+                want_logw=want_logw, stoch_int=stoch_int, device=dev, bridge=bridge)
     if dist is not None:
         opts.update(traj_offset=dist.traj_offset, K_global=dist.K_global)
     if table:
@@ -63,14 +65,15 @@ def _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, *, noise, see
 
 
 def test_policy_vectorized(env, model, batch_size=10, k_max=10**7, policy_opt=None, *, noise=None, seed=None,
-                           tanh="precise", state_f64=True, device=None, dist=None, kernel="auto"):
+                           tanh="precise", state_f64=True, device=None, dist=None, kernel="auto", bridge=False):
     """``(mean return, var return (ddof=0), mean hit index[, mean policy l2 error])``; all-NaN if any
-    trajectory has not reached the target set within ``k_max`` passes (reference :640-643).
+    trajectory has not reached the target set within ``k_max`` passes (reference :640-643).  ``bridge=True`` also detects
+    hits between passes (Brownian-bridge crossing test, d = 1: ``rollout.rollout_forward``).
 
     Unlike the reference (which crashes at :610-611), ``policy_opt=None`` is accepted and returns the
     3-tuple its last branch (:647-648) intends."""
     _, st = _numpy_path_rollout(env, model, batch_size, k_max, policy_opt, noise=noise, seed=seed, tanh=tanh, kernel=kernel,
-                                state_f64=state_f64, device=device, dist=dist)
+                                state_f64=state_f64, device=device, dist=dist, bridge=bridge)
     n_out = 4 if policy_opt is not None else 3
     if st[L.ST_N_UNFINISHED] > 0:
         return (np.nan,) * n_out
@@ -87,11 +90,11 @@ test_policy_vectorized.__test__ = False     # not a pytest test, despite the ref
 
 
 def estimate_fht_vectorized(env, model, batch_size=int(1e5), k_max=10**7, *, noise=None, seed=None, tanh="precise", kernel="auto",
-                            state_f64=True, device=None, dist=None):
+                            state_f64=True, device=None, dist=None, bridge=False):
     """Mean first hitting time ``mean(dt * k*)`` (reference :650-695).  NaN if a trajectory is unfinished
-    (the reference would average uninitialised ``np.empty`` slots)."""
+    (the reference would average uninitialised ``np.empty`` slots).  ``bridge``: as in ``test_policy_vectorized``."""
     out, st = _numpy_path_rollout(env, model, batch_size, k_max, None, noise=noise, seed=seed, tanh=tanh, kernel=kernel,
-                                  state_f64=state_f64, device=device, dist=dist)
+                                  state_f64=state_f64, device=device, dist=dist, bridge=bridge)
     if st[L.ST_N_UNFINISHED] > 0:
         return np.nan
     if dist is None:
@@ -101,12 +104,15 @@ def estimate_fht_vectorized(env, model, batch_size=int(1e5), k_max=10**7, *, noi
 
 
 def is_estimate(env, model, batch_size, n_steps_lim=10**7, *, noise=None, seed=None, tanh="precise", state_f64=False, kernel="auto",
-                device=None, dist=None):
+                device=None, dist=None, bridge=False):
     """Importance-sampling estimate of Psi(x0) = E[exp(-tau)] under the policy's change of measure
     (SURVEY App. C): weights exp(G - S_exact).  Returns a dict with the estimator mean, its relative
-    error std/mean, return statistics, mean hitting index and the unfinished count."""
+    error std/mean, return statistics, mean hitting index and the unfinished count.  ``bridge=True`` also detects hits
+    between passes (Brownian-bridge crossing test, d = 1), which removes the O(sqrt(dt)) bias of a hit tested only on the
+    time grid; the weights stay exact, so every policy estimates the same Psi."""
     _, st = _numpy_path_rollout(env, model, batch_size, n_steps_lim, None, noise=noise, seed=seed, tanh=tanh, kernel=kernel,
-                                state_f64=state_f64, device=device, dist=dist, stoch_int="exact", want_logw=True)
+                                state_f64=state_f64, device=device, dist=dist, stoch_int="exact", want_logw=True,
+                                bridge=bridge)
     return R.summarize(st)
 
 

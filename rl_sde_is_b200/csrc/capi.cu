@@ -274,6 +274,12 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
   if ((A.flags & RLSDE_F_STORE_PATH) && !path_dev) return RLSDE_ERR_INVALID_ARG;
   if (policy_opt_dev && (cfg->n_grid < 1 || !(cfg->grid_h > 0) || env->d != 1)) return RLSDE_ERR_INVALID_ARG;
+  if (A.flags & RLSDE_F_HIT_BRIDGE) {
+    // the reverse pass recomputes states from checkpoints and knows nothing of the projection; the transition stream
+    // records the unprojected pass
+    if ((A.flags & RLSDE_F_STORE_PATH) || tr.base) return RLSDE_ERR_INVALID_ARG;
+    if (env->d != 1) return RLSDE_ERR_UNSUPPORTED;        // the target all_i x_i >= lb is an orthant: no closed form
+  }
   A.noise = noise_dev; A.policy_opt = policy_opt_dev;
   A.G = G_dev; A.S = S_dev; A.T = T_dev; A.l2 = l2_dev; A.logw = logw_dev; A.path = path_dev;
   A.tr_base = tr.base; A.tr_state = tr.state; A.tr_action = tr.action; A.tr_reward = tr.reward;
@@ -445,7 +451,8 @@ int rlsde_rollout_fwd_table(const rlsde_env* env, const float* u_table_dev, cons
   if (rc != RLSDE_OK) return rc;
   if (A.flags & RLSDE_F_STORE_PATH) return RLSDE_ERR_INVALID_ARG;                 // no reverse pass through a table
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
-  A.flags &= RLSDE_F_NOISE_INJECTED | RLSDE_F_STOCH_INT_EXACT | RLSDE_F_STATE_F64;   // kernel-family and tanh flags do not apply
+  // kernel-family and tanh flags do not apply
+  A.flags &= RLSDE_F_NOISE_INJECTED | RLSDE_F_STOCH_INT_EXACT | RLSDE_F_STATE_F64 | RLSDE_F_HIT_BRIDGE;
   A.noise = noise_dev; A.policy_opt = policy_opt_dev;
   A.G = G_dev; A.S = S_dev; A.T = T_dev; A.l2 = l2_dev; A.logw = logw_dev;
   A.counter = (unsigned long long*)workspace_dev;
@@ -491,6 +498,7 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
   memset(&A, 0, sizeof(A));
   fill_env(env, A);
   if ((rc = fill_cfg(cfg, A)) != RLSDE_OK) return rc;
+  if (A.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;   // no reverse pass through the projection
   if (A.flags & RLSDE_F_STATE_F64) return RLSDE_ERR_UNSUPPORTED;   // the reference differentiates the f32 torch path only
   if (!(A.flags & RLSDE_F_STORE_PATH)) return RLSDE_ERR_INVALID_ARG;
   if (A.ckpt_every > BWD_MAX_SEG) return RLSDE_ERR_INVALID_ARG;        // the reverse pass recomputes at most 32 passes per checkpoint
@@ -605,7 +613,8 @@ static int reinforce_rollout_impl(const rlsde_env* env, const rlsde_mlp* mlp, co
   memset(&A, 0, sizeof(A));
   fill_env(env, A);
   if ((rc = fill_cfg(cfg, A)) != RLSDE_OK) return rc;
-  if ((A.flags & RLSDE_F_STATE_F64) || !(A.flags & RLSDE_F_STORE_PATH) || A.ckpt_every != 1) return RLSDE_ERR_INVALID_ARG;
+  if ((A.flags & (RLSDE_F_STATE_F64 | RLSDE_F_HIT_BRIDGE)) || !(A.flags & RLSDE_F_STORE_PATH) || A.ckpt_every != 1)
+    return RLSDE_ERR_INVALID_ARG;
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
   if (A.K < 1) return RLSDE_ERR_INVALID_ARG;
   int sm = 0;
@@ -738,6 +747,7 @@ int rlsde_env_step(const rlsde_env* env, int64_t K, const void* state_dev, const
   if (!env || env->d < 1 || env->d > RLSDE_MAX_D || K < 0) return RLSDE_ERR_INVALID_ARG;
   if (!state_dev || !action_dev || !next_state_dev || !reward_dev || !done_dev) return RLSDE_ERR_INVALID_ARG;
   if (reward_type != RLSDE_REWARD_STATE_ACTION && reward_type != RLSDE_REWARD_STATE_ACTION_NEXT_STATE) return RLSDE_ERR_INVALID_ARG;
+  if (flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;      // a single pass has no next pass to detect a crossing
   StepArgs A;
   memset(&A, 0, sizeof(A));
   for (int i = 0; i < env->d; ++i) { A.c4a_d[i] = 4.0 * env->alpha[i]; A.c4a_f[i] = (float)(4.0 * env->alpha[i]); }

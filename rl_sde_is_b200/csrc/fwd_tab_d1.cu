@@ -10,7 +10,8 @@
 namespace rlsde {
 
 // SMEM: the block copies the table to shared memory first (n_grid <= FWD_TAB_SMEM_MAX); otherwise it reads it with __ldg
-template <bool F64, bool SMEM>
+// BRIDGE: the Brownian-bridge hit test between passes (TrajOwner::pass)
+template <bool F64, bool SMEM, bool BRIDGE = false>
 __global__ void __launch_bounds__(128, 8) rollout_fwd_tab_kernel(const __grid_constant__ FwdArgs A, const float* __restrict__ table) {
   constexpr unsigned FULL = 0xffffffffu;
   extern __shared__ float s_tab[];
@@ -21,7 +22,7 @@ __global__ void __launch_bounds__(128, 8) rollout_fwd_tab_kernel(const __grid_co
   const int lane = threadIdx.x & 31;
   const bool inject = (A.flags & RLSDE_F_NOISE_INJECTED) != 0;
   const long long lim = inject ? (A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim) : A.n_steps_lim;
-  TrajOwner<1, F64> o;
+  TrajOwner<1, F64, BRIDGE> o;
   o.init(A);
   for (;;) {
     const bool idle = !o.alive && !o.exhausted;
@@ -46,9 +47,9 @@ __global__ void __launch_bounds__(128, 8) rollout_fwd_tab_kernel(const __grid_co
   }
 }
 
-template <bool F64, bool SMEM>
+template <bool F64, bool SMEM, bool BRIDGE>
 static int launch_tab_variant(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  auto kern = rollout_fwd_tab_kernel<F64, SMEM>;
+  auto kern = rollout_fwd_tab_kernel<F64, SMEM, BRIDGE>;
   const size_t smem = SMEM ? (size_t)args.n_grid * sizeof(float) : 0;
   // as K1: one warp per block for small batches (spread over the SMs), a persistent grid of co-resident blocks otherwise
   int block = 128;
@@ -68,13 +69,19 @@ static int launch_tab_variant(const float* table, const FwdArgs& args, int sm_co
   return (int)cudaGetLastError();
 }
 
-int launch_rollout_fwd_table(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+template <bool BRIDGE>
+static int launch_tab_bridge(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0;
   const bool smem = args.n_grid <= FWD_TAB_SMEM_MAX;
-  if (f64) return smem ? launch_tab_variant<true, true>(table, args, sm_count, stream)
-                       : launch_tab_variant<true, false>(table, args, sm_count, stream);
-  return smem ? launch_tab_variant<false, true>(table, args, sm_count, stream)
-              : launch_tab_variant<false, false>(table, args, sm_count, stream);
+  if (f64) return smem ? launch_tab_variant<true, true, BRIDGE>(table, args, sm_count, stream)
+                       : launch_tab_variant<true, false, BRIDGE>(table, args, sm_count, stream);
+  return smem ? launch_tab_variant<false, true, BRIDGE>(table, args, sm_count, stream)
+              : launch_tab_variant<false, false, BRIDGE>(table, args, sm_count, stream);
+}
+
+int launch_rollout_fwd_table(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+  return (args.flags & RLSDE_F_HIT_BRIDGE) ? launch_tab_bridge<true>(table, args, sm_count, stream)
+                                           : launch_tab_bridge<false>(table, args, sm_count, stream);
 }
 
 }  // namespace rlsde

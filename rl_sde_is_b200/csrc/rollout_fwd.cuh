@@ -118,6 +118,42 @@ __device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(
 __device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
 __device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
 
+// ---- Brownian-bridge hit test between passes (RLSDE_F_HIT_BRIDGE, d = 1).  Every rollout kernel that carries out a pass
+// (K1 below, the warp / wide kernels and TrajOwner::pass) calls bridge_project after the Euler-Maruyama update of a pass
+// whose state a = X_k was not a hit, with b = X_{k+1}.  Within the pass the drift is frozen, so conditioned on its end
+// points the path is a Brownian bridge whatever the drift, and it reaches a barrier c that both end points lie beyond with
+// probability p = exp(-2 (c - a)(c - b) / (sigma^2 dt)).  Endpoints on opposite sides of [lb, rb] (rb = +inf under
+// RLSDE_HIT_ALL_GE_LB) crossed for certain; b inside the target is left to the next pass's hit test.  A crossing moves
+// X_{k+1} onto the barrier on a's side, where the next pass's ordinary hit test detects it, so no new per-trajectory state
+// exists and continuation records carry it unchanged.  U is drawn from its own Philox stream, counter (traj_lo, traj_hi,
+// pass k, "BRDG"), key seed: the Brownian increments are untouched.  A crossing needs U < p and U >= 2^-33, so p is only
+// evaluated (exp) and U only drawn where the exponent is at most 23 > 33 ln 2: whether a draw happens changes no result.
+// p is evaluated in double from the state values in either state precision; the comparisons with lb / rb are the hit
+// test's own (state precision), so an unprojected b outside the target is never detected by the next pass.
+#define RLSDE_BRIDGE_TAG 0x42524447u /* "BRDG" */
+constexpr double RLSDE_BRIDGE_ARG_MAX = 23.0;
+// 1 / (sigma^2 dt), correctly rounded: equal to the host's 1.0 / (sigma * sigma * dt) in double
+__device__ __forceinline__ double bridge_inv_s2dt(const FwdArgs& A) { return __drcp_rn(__dmul_rn(__dmul_rn(A.sigma_d, A.sigma_d), A.dt_d)); }
+template <typename real>
+__device__ __forceinline__ void bridge_project(const FwdArgs& A, double inv_s2dt, unsigned long long gt, int k, real a, real& b) {
+  constexpr bool F64 = sizeof(real) == 8;
+  const bool two = A.hit_rule == RLSDE_HIT_X0_IN_LB_RB;
+  const real lb = F64 ? (real)A.lb_d : (real)A.lb_f, rb = F64 ? (real)A.rb_d : (real)A.rb_f;
+  const bool a_lo = a < lb, b_lo = b < lb, b_hi = two && b > rb;
+  if (!b_lo && !b_hi) return;
+  bool cross = a_lo != b_lo;
+  if (!cross) {
+    const double c = a_lo ? A.lb_d : A.rb_d;
+    const double arg = __dmul_rn(__dmul_rn(__dmul_rn(2.0, __dsub_rn(c, (double)a)), __dsub_rn(c, (double)b)), inv_s2dt);
+    if (arg <= RLSDE_BRIDGE_ARG_MAX) {
+      const Philox4 r = philox4x32_10((uint32_t)gt, (uint32_t)(gt >> 32), (uint32_t)k, RLSDE_BRIDGE_TAG, (uint32_t)A.seed,
+                                      (uint32_t)(A.seed >> 32));
+      cross = __dmul_rn(__dadd_rn((double)r.x, 0.5), 2.3283064365386963e-10) < exp(-arg);
+    }
+  }
+  if (cross) b = a_lo ? lb : rb;
+}
+
 // Cold path of the FIFO: a producer found its slot still holding an unread record (the ring is larger than the number of
 // records in flight, so this needs a reader stalled for a whole lap).  Kept out of line: inlined, the spin loop costs the
 // rollout kernel ~15 registers.
@@ -167,7 +203,9 @@ template <int D, bool MMA>
 constexpr int fwd_min_blocks() { return MMA ? RLSDE_FWD_MMA_MIN_BLOCKS : (D == 1 ? 8 : (D <= 4 ? 5 : 4)); }
 // CLAMP2 = false (MMA, precise tanh): layer 2 of the policy without the clamp of rsig_group, launched where the host has
 // proven it cannot bind (fwd_mma_clamp_bounds)
-template <int D, int H, bool F64, bool FAST, bool MMA, bool CLAMP2 = true>
+// BRIDGE: the Brownian-bridge hit test between passes (bridge_project; instantiated at d = 1 only).  A compile-time choice,
+// so that the kernels without it keep their register allocation
+template <int D, int H, bool F64, bool FAST, bool MMA, bool CLAMP2 = true, bool BRIDGE = false>
 __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_kernel(const __grid_constant__ MlpConst<D, H> W,
                                                           const __grid_constant__ FwdArgs A,
                                                           const __grid_constant__ typename FwdMmaSel<D, MMA>::type M) {
@@ -192,6 +230,7 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
   const bool store_path = (A.flags & RLSDE_F_STORE_PATH) != 0 && A.path != nullptr;
   const bool want_l2 = (D == 1) && A.policy_opt != nullptr && A.l2 != nullptr;
   const long long lim = inject ? (A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim) : A.n_steps_lim;
+  const double inv_s2dt = BRIDGE ? bridge_inv_s2dt(A) : 0.0;
   typedef ContRec<D, F64> Rec;
   // tail strategy: 1 = time slices, 2 = hand-off to the latency kernel, 3 = none, 0 = adaptive launch, not decided yet
   const bool adaptive = A.q_ring != nullptr && A.q_adaptive != 0;
@@ -519,6 +558,7 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
         A.T[traj] = k;
         alive = false; fin = true;
       } else {
+        if constexpr (BRIDGE) bridge_project(A, inv_s2dt, (unsigned long long)(A.traj_offset + traj), k, x[0], xn[0]);
         G = add_rn(G, r);
 #pragma unroll
         for (int i = 0; i < D; ++i) x[i] = xn[i];

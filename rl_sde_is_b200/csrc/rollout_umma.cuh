@@ -124,7 +124,8 @@ __device__ __forceinline__ void ld32(uint32_t taddr, uint32_t (&r)[32]) {
 }
 }  // namespace umma
 
-template <int D, int H, bool F64, bool FAST>
+// BRIDGE: the Brownian-bridge hit test between passes (TrajOwner::pass; d = 1 only)
+template <int D, int H, bool F64, bool FAST, bool BRIDGE = false>
 __global__ void __launch_bounds__(umma_threads<H>(), umma_streams<H>() ? 2 : 4) rollout_fwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict__ Bimg,
                                                                            const __grid_constant__ FwdArgs A) {
   using namespace umma;
@@ -173,7 +174,7 @@ __global__ void __launch_bounds__(umma_threads<H>(), umma_streams<H>() ? 2 : 4) 
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = tmem_base_s;
 
-  TrajOwner<D, F64> T;
+  TrajOwner<D, F64, BRIDGE> T;
   T.init(A);
   const bool owner = warp < 4;
   float b3[D];

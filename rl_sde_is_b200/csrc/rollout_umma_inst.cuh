@@ -5,9 +5,9 @@
 
 namespace rlsde {
 
-template <int D, int H, bool F64, bool FAST>
+template <int D, int H, bool F64, bool FAST, bool BRIDGE>
 static int launch_fwd_umma_variant(const float* params_dev, const uint8_t* image_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  auto kern = rollout_fwd_umma_kernel<D, H, F64, FAST>;
+  auto kern = rollout_fwd_umma_kernel<D, H, F64, FAST, BRIDGE>;
   const size_t smem = umma_smem_bytes<D, H>();
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -45,10 +45,16 @@ int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t
   if (e != cudaSuccess) return (int)e;
   e = cudaMemcpyAsync(image_dev, wimg.data(), umma_image_bytes<H>(), cudaMemcpyHostToDevice, stream);
   if (e != cudaSuccess) return (int)e;
-  if (f64) return fast ? launch_fwd_umma_variant<D, H, true, true>(params_dev, image_dev, args, sm_count, stream)
-                       : launch_fwd_umma_variant<D, H, true, false>(params_dev, image_dev, args, sm_count, stream);
-  return fast ? launch_fwd_umma_variant<D, H, false, true>(params_dev, image_dev, args, sm_count, stream)
-              : launch_fwd_umma_variant<D, H, false, false>(params_dev, image_dev, args, sm_count, stream);
+#define RLSDE_UMMA_FWD(B_)                                                                                           \
+  (f64 ? (fast ? launch_fwd_umma_variant<D, H, true, true, B_>(params_dev, image_dev, args, sm_count, stream)         \
+               : launch_fwd_umma_variant<D, H, true, false, B_>(params_dev, image_dev, args, sm_count, stream))       \
+       : (fast ? launch_fwd_umma_variant<D, H, false, true, B_>(params_dev, image_dev, args, sm_count, stream)        \
+               : launch_fwd_umma_variant<D, H, false, false, B_>(params_dev, image_dev, args, sm_count, stream)))
+  if constexpr (D == 1) {      // RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
+    if (args.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_UMMA_FWD(true);
+  }
+  return RLSDE_UMMA_FWD(false);
+#undef RLSDE_UMMA_FWD
 }
 
 }  // namespace rlsde

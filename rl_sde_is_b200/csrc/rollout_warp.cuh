@@ -154,7 +154,8 @@ __device__ __forceinline__ void warp_policy_exact(const LaneParams<D>& P, const 
 // trajectories of its launch over (rollout_fwd.cuh); they are continued with K1's arithmetic: warp_policy_exact, or with
 // MMA (K1 evaluated its policy with mlp_forward_mma) the same tensor-core sequence with the trajectory's state in all
 // 32 rows of the tile.
-template <int D, bool F64, bool FAST, bool RESUME, bool MMA = false>
+// BRIDGE: the Brownian-bridge hit test between passes (bridge_project, rollout_fwd.cuh; d = 1 only)
+template <int D, bool F64, bool FAST, bool RESUME, bool MMA = false, bool BRIDGE = false>
 __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel(const __grid_constant__ MlpConst<D, WARP_H> W_param,
                                                                const MlpConst<D, WARP_H>* __restrict__ W_dev,
                                                                const __grid_constant__ FwdArgs A,
@@ -180,6 +181,7 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
   const bool store_path = (A.flags & RLSDE_F_STORE_PATH) != 0 && A.path != nullptr;
   const bool want_l2 = (D == 1) && A.policy_opt != nullptr && A.l2 != nullptr;
   const long long lim = inject ? (A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim) : A.n_steps_lim;
+  const double inv_s2dt = BRIDGE ? bridge_inv_s2dt(A) : 0.0;
   LaneParams<D> P;
   P.load(W, lane);
 
@@ -303,6 +305,7 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
       const float nn = (D == 1) ? n2 : __fmul_rn(sqrtf(n2), sqrtf(n2));
       if (F64) G = (real)__dadd_rn((double)G, -__dmul_rn(__dadd_rn(1.0, (double)__fmul_rn(0.5f, nn)), A.dt_d));
       else G = (real)__fadd_rn((float)G, -__fmul_rn(__fadd_rn(1.0f, __fmul_rn(0.5f, nn)), A.dt_f));
+      const real x_prev = x[0];
 #pragma unroll
       for (int i = 0; i < D; ++i) {
         if (F64) {
@@ -324,6 +327,7 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
           x[i] = (real)__fadd_rn(__fadd_rn(xi, drift), __fmul_rn(A.sigma_f, dB[i]));
         }
       }
+      if constexpr (BRIDGE) bridge_project(A, inv_s2dt, (unsigned long long)(A.traj_offset + traj), k, x_prev, x[0]);
     }
     if (lane == 0) {
       if (t_out < 0 && A.logw) {

@@ -41,27 +41,36 @@ int launch_pack_mlp_const_dev(const float* theta_dev, void* W_dev, bool fast_tan
   return (int)cudaGetLastError();
 }
 
-template <int D, bool F64, bool FAST>
+template <int D, bool F64, bool FAST, bool BRIDGE>
 static int launch_fwd_warp_variant(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, WARP_H> W;
   if (params_host != nullptr) pack_mlp_const<D, WARP_H>(params_host, FAST, W);
   else memset(&W, 0, sizeof(W));
-  rollout_fwd_warp_kernel<D, F64, FAST, false><<<(unsigned)warp_grid(args.K, sm_count), 128, 0, stream>>>(
+  rollout_fwd_warp_kernel<D, F64, FAST, false, false, BRIDGE><<<(unsigned)warp_grid(args.K, sm_count), 128, 0, stream>>>(
       W, params_host != nullptr ? nullptr : reinterpret_cast<const MlpConst<D, WARP_H>*>(W_dev), args, MlpMmaNone{0});
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
-template <int D>
-int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+template <int D, bool BRIDGE>
+static int launch_fwd_warp_bridge(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if (f64) return fast ? launch_fwd_warp_variant<D, true, true>(params_host, W_dev, args, sm_count, stream)
-                       : launch_fwd_warp_variant<D, true, false>(params_host, W_dev, args, sm_count, stream);
-  return fast ? launch_fwd_warp_variant<D, false, true>(params_host, W_dev, args, sm_count, stream)
-              : launch_fwd_warp_variant<D, false, false>(params_host, W_dev, args, sm_count, stream);
+  if (f64) return fast ? launch_fwd_warp_variant<D, true, true, BRIDGE>(params_host, W_dev, args, sm_count, stream)
+                       : launch_fwd_warp_variant<D, true, false, BRIDGE>(params_host, W_dev, args, sm_count, stream);
+  return fast ? launch_fwd_warp_variant<D, false, true, BRIDGE>(params_host, W_dev, args, sm_count, stream)
+              : launch_fwd_warp_variant<D, false, false, BRIDGE>(params_host, W_dev, args, sm_count, stream);
 }
 
-template <int D, bool F64, bool FAST, bool MMA>
+// RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
+template <int D>
+int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+  if constexpr (D == 1) {
+    if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_fwd_warp_bridge<D, true>(params_host, W_dev, args, sm_count, stream);
+  }
+  return launch_fwd_warp_bridge<D, false>(params_host, W_dev, args, sm_count, stream);
+}
+
+template <int D, bool F64, bool FAST, bool MMA, bool BRIDGE>
 static int launch_fwd_warp_resume_variant(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, WARP_H> W;
   if (!FAST && RLSDE_FWD_FOLDED) pack_mlp_const_folded<D, WARP_H>(params_host, W);      // the image K1 itself was launched with
@@ -70,18 +79,26 @@ static int launch_fwd_warp_resume_variant(const float* params_host, const FwdArg
   if constexpr (MMA) pack_mlp_mma<D>(W, M);
   else M.unused = 0;
   // the number of records is only known on the device: a full grid (16 warps per SM), warps without a record leave at once
-  rollout_fwd_warp_kernel<D, F64, FAST, true, MMA><<<(unsigned)(sm_count * 4), 128, 0, stream>>>(W, nullptr, args, M);
+  rollout_fwd_warp_kernel<D, F64, FAST, true, MMA, BRIDGE><<<(unsigned)(sm_count * 4), 128, 0, stream>>>(W, nullptr, args, M);
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
+template <int D, bool MMA, bool BRIDGE>
+static int launch_fwd_warp_resume_bridge(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
+  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
+  if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
+                       : launch_fwd_warp_resume_variant<D, true, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
+  return fast ? launch_fwd_warp_resume_variant<D, false, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
+              : launch_fwd_warp_resume_variant<D, false, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
+}
+
 template <int D, bool MMA>
 static int launch_fwd_warp_resume_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true, MMA>(params_host, args, sm_count, stream)
-                       : launch_fwd_warp_resume_variant<D, true, false, MMA>(params_host, args, sm_count, stream);
-  return fast ? launch_fwd_warp_resume_variant<D, false, true, MMA>(params_host, args, sm_count, stream)
-              : launch_fwd_warp_resume_variant<D, false, false, MMA>(params_host, args, sm_count, stream);
+  if constexpr (D == 1) {
+    if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_fwd_warp_resume_bridge<D, MMA, true>(params_host, args, sm_count, stream);
+  }
+  return launch_fwd_warp_resume_bridge<D, MMA, false>(params_host, args, sm_count, stream);
 }
 
 // continues with the policy arithmetic K1 was launched with (args.policy_mma)

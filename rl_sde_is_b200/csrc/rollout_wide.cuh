@@ -186,7 +186,8 @@ __device__ __forceinline__ void wide_head(const float* __restrict__ Wp, const fl
 }
 
 // ------------------------------------------------------------------------------------------------ forward
-template <int D, int H, int R, bool F64, bool FAST>
+// BRIDGE: the Brownian-bridge hit test between passes (bridge_project, rollout_fwd.cuh; d = 1 only)
+template <int D, int H, int R, bool F64, bool FAST, bool BRIDGE = false>
 __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const float* __restrict__ Wp, const __grid_constant__ FwdArgs A) {
   typedef typename RealT<F64>::type real;
   typedef WideParams<D, H> L;
@@ -208,6 +209,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const
   const bool store_path = (A.flags & RLSDE_F_STORE_PATH) != 0 && A.path != nullptr;
   const bool want_l2 = (D == 1) && A.policy_opt != nullptr && A.l2 != nullptr;
   const long long lim = inject ? (A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim) : A.n_steps_lim;
+  const double inv_s2dt = BRIDGE ? bridge_inv_s2dt(A) : 0.0;
 
   // owner state
   bool alive = false, exhausted = false;
@@ -351,6 +353,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const
         const float nn = (D == 1) ? n2 : __fmul_rn(sqrtf(n2), sqrtf(n2));
         if (F64) G = (real)__dadd_rn((double)G, -__dmul_rn(__dadd_rn(1.0, (double)__fmul_rn(0.5f, nn)), A.dt_d));
         else G = (real)__fadd_rn((float)G, -__fmul_rn(__fadd_rn(1.0f, __fmul_rn(0.5f, nn)), A.dt_f));
+        const real x_prev = x[0];
 #pragma unroll
         for (int i = 0; i < D; ++i) {
           if (F64) {
@@ -372,6 +375,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const
             x[i] = (real)__fadd_rn(__fadd_rn(xi, drift), __fmul_rn(A.sigma_f, dB[i]));
           }
         }
+        if constexpr (BRIDGE) bridge_project(A, inv_s2dt, (unsigned long long)(A.traj_offset + traj), k, x_prev, x[0]);
         ++k;
         if (k >= lim) {       // not detected within the pass budget: flagged, never garbage
           if (F64) {

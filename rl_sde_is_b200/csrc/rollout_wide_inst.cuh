@@ -17,9 +17,9 @@ static int wide_upload_params(const float* params_host, float* params_dev, bool 
 // rows per warp: 8 (tiles of 32 trajectories) when the batch fills the GPU with such tiles, else 4 (tiles of 16)
 static inline bool wide_small_tiles(long long K, int sm_count) { return K < (long long)sm_count * 32; }
 
-template <int D, int H, int R, bool F64, bool FAST>
+template <int D, int H, int R, bool F64, bool FAST, bool BRIDGE>
 static int launch_fwd_wide_variant(const float* params_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  auto kern = rollout_fwd_wide_kernel<D, H, R, F64, FAST>;
+  auto kern = rollout_fwd_wide_kernel<D, H, R, F64, FAST, BRIDGE>;
   const size_t smem = wide_fwd_smem_bytes<H>();
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -40,12 +40,15 @@ int launch_rollout_fwd_wide(const float* params_host, float* params_dev, const F
   int rc = wide_upload_params<D, H>(params_host, params_dev, fast, stream);
   if (rc != 0) return rc;
   const bool small = wide_small_tiles(args.K, sm_count);
-#define RLSDE_WIDE_FWD(R_) \
-  (f64 ? (fast ? launch_fwd_wide_variant<D, H, R_, true, true>(params_dev, args, sm_count, stream)    \
-               : launch_fwd_wide_variant<D, H, R_, true, false>(params_dev, args, sm_count, stream))  \
-       : (fast ? launch_fwd_wide_variant<D, H, R_, false, true>(params_dev, args, sm_count, stream)   \
-               : launch_fwd_wide_variant<D, H, R_, false, false>(params_dev, args, sm_count, stream)))
-  return small ? RLSDE_WIDE_FWD(4) : RLSDE_WIDE_FWD(8);
+#define RLSDE_WIDE_FWD(R_, B_) \
+  (f64 ? (fast ? launch_fwd_wide_variant<D, H, R_, true, true, B_>(params_dev, args, sm_count, stream)    \
+               : launch_fwd_wide_variant<D, H, R_, true, false, B_>(params_dev, args, sm_count, stream))  \
+       : (fast ? launch_fwd_wide_variant<D, H, R_, false, true, B_>(params_dev, args, sm_count, stream)   \
+               : launch_fwd_wide_variant<D, H, R_, false, false, B_>(params_dev, args, sm_count, stream)))
+  if constexpr (D == 1) {      // RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
+    if (args.flags & RLSDE_F_HIT_BRIDGE) return small ? RLSDE_WIDE_FWD(4, true) : RLSDE_WIDE_FWD(8, true);
+  }
+  return small ? RLSDE_WIDE_FWD(4, false) : RLSDE_WIDE_FWD(8, false);
 #undef RLSDE_WIDE_FWD
 }
 

@@ -19,7 +19,8 @@ __device__ __forceinline__ long long grid_index(const FwdArgs& A, double x) {
   return gi < 0 ? 0 : (gi >= A.n_grid ? A.n_grid - 1 : gi);
 }
 
-template <int D, bool F64>
+// BRIDGE: the Brownian-bridge hit test between passes (bridge_project, rollout_fwd.cuh; d = 1 only)
+template <int D, bool F64, bool BRIDGE = false>
 struct TrajOwner {
   typedef typename RealT<F64>::type real;
   static constexpr int SPB = NoisePlan<D>::SPB;
@@ -31,9 +32,11 @@ struct TrajOwner {
   real x[D];
   real G, S, L2;
   float z[NZ];
+  double inv_s2dt;
 
   __device__ __forceinline__ void init(const FwdArgs& A) {
     alive = false; exhausted = false; traj = 0; k = 0; ck = 0; G = 0; S = 0; L2 = 0;
+    inv_s2dt = BRIDGE ? bridge_inv_s2dt(A) : 0.0;
 #pragma unroll
     for (int i = 0; i < D; ++i) x[i] = F64 ? (real)A.x0_d[i] : (real)A.x0_f[i];
 #pragma unroll
@@ -128,6 +131,7 @@ struct TrajOwner {
     const float nn = (D == 1) ? n2 : __fmul_rn(sqrtf(n2), sqrtf(n2));
     if (F64) G = (real)__dadd_rn((double)G, -__dmul_rn(__dadd_rn(1.0, (double)__fmul_rn(0.5f, nn)), A.dt_d));
     else G = (real)__fadd_rn((float)G, -__fmul_rn(__fadd_rn(1.0f, __fmul_rn(0.5f, nn)), A.dt_f));
+    const real x_prev = x[0];
 #pragma unroll
     for (int i = 0; i < D; ++i) {
       if (F64) {
@@ -149,6 +153,7 @@ struct TrajOwner {
         x[i] = (real)__fadd_rn(__fadd_rn(xi, drift), __fmul_rn(A.sigma_f, dB[i]));
       }
     }
+    if constexpr (BRIDGE) bridge_project(A, inv_s2dt, (unsigned long long)(A.traj_offset + traj), k, x_prev, x[0]);
     ++k;
     if (k >= lim) {       // not detected within the pass budget: flagged, never garbage
       write_out(A, S, S, -1);

@@ -120,10 +120,22 @@ class RolloutOut:
         return self._stats
 
 
+def _check_bridge(d, store_path=False):
+    if d != 1:
+        raise L.RlsdeError(f"the Brownian-bridge hit test is defined at d = 1 only (the target of env.d = {d} is an orthant)")
+    if store_path:
+        raise L.RlsdeError("the Brownian-bridge hit test has no reverse pass: it cannot be combined with store_path")
+
+
 def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, noise=None, traj_offset=0,
                     K_global=None, tanh="precise", stoch_int="reference", state_f64=False, store_path=False,
-                    ckpt_every=1, policy_opt=None, grid=None, want_logw=True, device=None, out=None, kernel="auto", tuning=None):
-    """One launch of K1 for K trajectories.  ``params_host``: contiguous float32 numpy array (state_dict order)."""
+                    ckpt_every=1, policy_opt=None, grid=None, want_logw=True, device=None, out=None, kernel="auto", tuning=None,
+                    bridge=False):
+    """One launch of K1 for K trajectories.  ``params_host``: contiguous float32 numpy array (state_dict order).
+    ``bridge``: also detect target hits between passes with the Brownian-bridge crossing test (RLSDE_F_HIT_BRIDGE; d = 1,
+    not with ``store_path``)."""
+    if bridge:
+        _check_bridge(env_c.d, store_path)
     lib = L.load()
     dev = _cuda_device(device)
     K = int(K)
@@ -158,6 +170,8 @@ def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, 
     if state_f64:
         flags |= L.F_STATE_F64
     path = None
+    if bridge:
+        flags |= L.F_HIT_BRIDGE
     if store_path:
         flags |= L.F_STORE_PATH
         lim_eff = min(cfg.n_steps_lim, cfg.noise_steps) if noise is not None else cfg.n_steps_lim
@@ -190,9 +204,11 @@ def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, 
 
 
 def rollout_forward_table(env_c, table, K, *, grid, seed=0, n_steps_lim=10**6, noise=None, traj_offset=0, K_global=None,
-                          stoch_int="reference", state_f64=False, policy_opt=None, want_logw=True, device=None, tuning=None):
+                          stoch_int="reference", state_f64=False, policy_opt=None, want_logw=True, device=None, tuning=None,
+                          bridge=False):
     """One launch of the d = 1 rollout under the control ``table[idx(x)]`` (``rlsde_rollout_fwd_table``).  ``table``:
-    float32 values on ``grid = (lo, hi, h)``; ``policy_opt`` (l2 error), if given, lives on the same grid."""
+    float32 values on ``grid = (lo, hi, h)``; ``policy_opt`` (l2 error), if given, lives on the same grid.  ``bridge``: as
+    in ``rollout_forward``."""
     lib = L.load()
     dev = _cuda_device(device)
     K = int(K)
@@ -218,6 +234,8 @@ def rollout_forward_table(env_c, table, K, *, grid, seed=0, n_steps_lim=10**6, n
         flags |= L.F_NOISE_INJECTED
         cfg.noise_steps = int(noise.shape[0])
     flags |= {"reference": 0, "exact": L.F_STOCH_INT_EXACT}[stoch_int]
+    if bridge:
+        flags |= L.F_HIT_BRIDGE
     real = torch.float64 if state_f64 else torch.float32
     if state_f64:
         flags |= L.F_STATE_F64
