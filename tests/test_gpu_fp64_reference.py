@@ -46,11 +46,39 @@ def _policy(d, H, bias, seed):
     return m, params, ref.flatten_params(params)
 
 
-def _env_c(d, hit_rule):
+# The environment every case runs in unless it names another (tests/test_gpu_env_params.py): the reference's defaults.
+# ``alpha`` and ``x0`` may also be per-coordinate sequences.
+DEFAULT_ENV = dict(alpha=1.0, beta=1.0, dt=DT, x0=-1.0, lb=1.0, rb=2.0)
+
+
+def _spec(env):
+    return {**DEFAULT_ENV, **(env or {})}
+
+
+def _env_c(d, hit_rule, env=None):
+    """The environment object of the spec ``env`` (keys of DEFAULT_ENV; absent keys take their default) and its rlsde_env.
+    A per-coordinate alpha overwrites ``alpha`` / ``alpha_tensor`` of the d-D class, a per-coordinate x0 its float32
+    ``state_init``: the attributes rollout.env_struct reads."""
     from rl_sde_is_b200.environments import DoubleWellStoppingTime1D, DoubleWellStoppingTimeND
     L, R = _lib()
-    env = DoubleWellStoppingTime1D(beta=1.0, alpha=1.0, dt=DT) if d == 1 else DoubleWellStoppingTimeND(d, beta=1.0, alpha=1.0, dt=DT)
-    return env, R.env_struct(env, hit_rule)
+    s = _spec(env)
+    alpha = np.asarray(s["alpha"], dtype=np.float64)
+    a0 = float(alpha.reshape(-1)[0])
+    e = DoubleWellStoppingTime1D(beta=s["beta"], alpha=a0, dt=s["dt"]) if d == 1 else \
+        DoubleWellStoppingTimeND(d, beta=s["beta"], alpha=a0, dt=s["dt"])
+    if alpha.ndim:
+        assert d > 1 and alpha.shape == (d,)
+        e.alpha = alpha.copy()
+        e.alpha_tensor = torch.tensor(e.alpha, dtype=torch.float32)
+    e.state_init = np.broadcast_to(np.asarray(s["x0"], dtype=np.float32), (1, d)).copy()
+    e.lb, e.rb = float(s["lb"]), float(s["rb"])
+    return e, R.env_struct(e, hit_rule)
+
+
+def _reference(d, params, noise, env=None, **kw):
+    """oracle.reference_semantics.rollout_reference in the environment ``env`` (as _env_c)."""
+    s = _spec(env)
+    return ref.rollout_reference(d, s["alpha"], s["beta"], s["dt"], params, noise, lb=s["lb"], rb=s["rb"], x0=s["x0"], **kw)
 
 
 def _bound(n, value, c):
@@ -166,15 +194,31 @@ C_S = (2.0, 0.3)
 C_L2 = (12.0, 0.01)
 
 
-def _forward_case(family, d, H, f64, stoch_int, hit_rule, K=128, lim=2000, seed=None, extra=None, ref_out=None):
-    """One forced launch against the float64 reference on the same increments, teacher-forced on the kernel's hit passes.
-    Returns (kernel output, reference output, policy parameters) after asserting everything that does not need the other mode."""
+def _path_deviation(path, xr, n):
+    """Per trajectory, the largest |kernel state - reference state| over the passes 0..n it executed, and half an ulp of the
+    largest |reference state| there (the path is stored in float32 whatever the state's precision).  Slots past a
+    trajectory's last pass are never written: masked, not read."""
+    live = torch.as_tensor(np.arange(xr.shape[1])[None, :] <= n[:, None], device=xr.device)[..., None]
+    dev = _np(torch.where(live, (path[:, :xr.shape[1]].double() - xr).abs(), 0.0).amax(dim=(1, 2)))
+    store = EPS32 * _np(torch.where(live, xr.abs(), 0.0).amax(dim=(1, 2)))
+    return dev, store, live
+
+
+def _forward_case(family, d, H, f64, stoch_int, hit_rule, K=128, lim=2000, seed=None, extra=None, ref_out=None, env=None,
+                  ratios=None, tols=None):
+    """One forced launch against the float64 reference on the same increments, teacher-forced on the kernel's hit passes,
+    in the environment ``env`` (as _env_c).  Returns (kernel output, reference output, policy parameters) after asserting
+    everything that does not need the other mode.  ``ratios`` (a dict), if given, receives the largest |error| / bound(C = 1)
+    of each compared output; ``tols`` may replace any of the constants C_PATH, C_G, C_S, C_L2 (keys "path", "G", "S",
+    "l2")."""
     L, R = _lib()
+    s = _spec(env)
+    c = {"path": C_PATH, "G": C_G, "S": C_S, "l2": C_L2, **(tols or {})}
     seed = seed if seed is not None else 1000 * d + H
     model, params, flat = _policy(d, H, 1.0 if d == 1 else 2.5, seed)
-    env, env_c = _env_c(d, hit_rule)
+    _, env_c = _env_c(d, hit_rule, env)
     mlp_c = L.make_mlp(d, H)
-    noise = R.noise_fill(seed, K, d, lim, DT)
+    noise = R.noise_fill(seed, K, d, lim, s["dt"])
     pol = grid = None
     if d == 1:
         grid = (-2.0, 2.0, 0.05)
@@ -185,20 +229,18 @@ def _forward_case(family, d, H, f64, stoch_int, hit_rule, K=128, lim=2000, seed=
                             store_path=True, ckpt_every=1, want_logw=True, policy_opt=pol, grid=grid, **kw)
     T = out.T.cpu().numpy().astype(np.int64)
     if ref_out is None:
-        ref_out = ref.rollout_reference(d, 1.0, 1.0, DT, params, noise, hit_rule=ref.HIT_X0_IN_LB_RB if hit_rule else ref.HIT_ALL_GE_LB,
-                                        hit_index=T, f32_policy_input=f64, policy_opt=None if pol is None else pol[:, None],
-                                        grid=grid, keep_path=True, device="cuda")
+        ref_out = _reference(d, params, noise, env, hit_rule=ref.HIT_X0_IN_LB_RB if hit_rule else ref.HIT_ALL_GE_LB,
+                             hit_index=T, f32_policy_input=f64, policy_opt=None if pol is None else pol[:, None],
+                             grid=grid, keep_path=True, device="cuda")
     assert np.array_equal(ref_out["T"].cpu().numpy(), T)
     prec = 1 if f64 else 0
     n = np.where(T >= 0, T, lim - 1)                                           # last pass each trajectory executed
     # state path: the largest deviation along each path is itself bounded
     xr = ref_out["path"]
-    live = torch.as_tensor(np.arange(xr.shape[1])[None, :] <= n[:, None], device=xr.device)[..., None]
-    # (slots past a trajectory's last pass are never written: masked, not read)
-    dev = _np(torch.where(live, (out.path[:, :xr.shape[1]].double() - xr).abs(), 0.0).amax(dim=(1, 2)))
-    # the path is stored in float32 whatever the state's precision: half an ulp of |x| on top of the drift of the state
-    store = EPS32 * _np(torch.where(live, xr.abs(), 0.0).amax(dim=(1, 2)))
-    assert np.all(dev <= store + _bound(n, 1.0, C_PATH[prec])), (family, d, H, float(((dev - store) / _bound(n, 1.0, 1.0)).max()))
+    dev, store, live = _path_deviation(out.path, xr, n)
+    if ratios is not None:
+        ratios["path"] = float(((dev - store) / _bound(n, 1.0, 1.0)).max())
+    assert np.all(dev <= store + _bound(n, 1.0, c["path"][prec])), (family, d, H, float(((dev - store) / _bound(n, 1.0, 1.0)).max()))
     # own decisions: the kernel's hit pass is the reference's unless the reference's state lies within the path deviation
     # of the boundary at the first pass where they differ
     T_own = ref_out["T_own"].cpu().numpy()
@@ -209,21 +251,27 @@ def _forward_case(family, d, H, f64, stoch_int, hit_rule, K=128, lim=2000, seed=
     assert differ.mean() <= 0.05
     # per-trajectory outputs
     G = _np(out.G)
-    assert np.all(np.abs(G - _np(ref_out["G"])) <= _bound(n, G, C_G[prec]))
     S_want = _np(ref_out["S_exact" if stoch_int == "exact" else "S_ref"])
-    assert np.all(np.abs(_np(out.S) - S_want) <= _bound(n, S_want, C_S[prec]))
     logw = _np(out.logw)
-    assert np.all(np.abs(logw - _np(ref_out["logw"])) <= _bound(n, logw, C_S[prec]))
+    if ratios is not None:
+        for key, got, want, scale in (("G", G, _np(ref_out["G"]), G), ("S", _np(out.S), S_want, S_want),
+                                      ("logw", logw, _np(ref_out["logw"]), logw)):
+            ratios[key] = float((np.abs(got - want) / _bound(n, scale, 1.0)).max())
+    assert np.all(np.abs(G - _np(ref_out["G"])) <= _bound(n, G, c["G"][prec]))
+    assert np.all(np.abs(_np(out.S) - S_want) <= _bound(n, S_want, c["S"][prec]))
+    assert np.all(np.abs(logw - _np(ref_out["logw"])) <= _bound(n, logw, c["S"][prec]))
     if pol is not None:
         l2_want = _np(ref_out["l2"])
-        flips = _l2_cell_flips(params, xr[..., 0], out.path[:, :xr.shape[1], 0].double(), live[..., 0], pol, grid, f64)
-        assert np.all(np.abs(_np(out.l2) - l2_want) <= _bound(n, l2_want, C_L2[prec]) + flips), (family, d, H)
+        flips = _l2_cell_flips(params, xr[..., 0], out.path[:, :xr.shape[1], 0].double(), live[..., 0], pol, grid, f64, s["dt"])
+        if ratios is not None:
+            ratios["l2"] = float(((np.abs(_np(out.l2) - l2_want) - flips) / _bound(n, l2_want, 1.0)).max())
+        assert np.all(np.abs(_np(out.l2) - l2_want) <= _bound(n, l2_want, c["l2"][prec]) + flips), (family, d, H)
     # statistics record of this dispatch site = fsum reduction of the launch's own outputs
     _assert_stats(out.stats, out.G, out.S, out.T, out.l2, out.logw, lim)
     return out, ref_out, params
 
 
-def _l2_cell_flips(params, x, x_kernel, live, pol, grid, f64):
+def _l2_cell_flips(params, x, x_kernel, live, pol, grid, f64, dt=DT):
     """Per trajectory, the most the l2 error can move because the kernel's state and the reference's lie on either side
     of a grid-cell edge: over the passes (after the first, where both hold x0 exactly) whose reference state is within the
     two states' distance (plus the float32 storage rounding of the kernel's path) of an edge, the sum of
@@ -245,13 +293,14 @@ def _l2_cell_flips(params, x, x_kernel, live, pol, grid, f64):
         base = (u - pol_t[c]) ** 2
         alt = torch.maximum(((u - pol_t[(c - 1).clamp(min=0)]) ** 2 - base).abs(),
                             ((u - pol_t[(c + 1).clamp(max=pol_t.numel() - 1)]) ** 2 - base).abs())
-        out.index_add_(0, idx[:, 0], alt * DT)
+        out.index_add_(0, idx[:, 0], alt * dt)
     return _np(out)
 
 
-def _discriminates(family, d, H, f64, out_ref_mode, r_ref_mode, out_exact, r, params):
+def _discriminates(family, d, H, f64, out_ref_mode, r_ref_mode, out_exact, r, params, dt=DT):
     """The nearest wrong answers fail the same tolerances on a clear majority of the finished trajectories.  ``r`` /
-    ``r_ref_mode``: the float64 replays teacher-forced on the exact-mode / reference-mode launch's hit passes."""
+    ``r_ref_mode``: the float64 replays teacher-forced on the exact-mode / reference-mode launch's hit passes; ``dt`` their
+    time step."""
     prec = 1 if f64 else 0
     T = out_exact.T.cpu().numpy().astype(np.int64)
     fin = T >= 0
@@ -274,7 +323,7 @@ def _discriminates(family, d, H, f64, out_ref_mode, r_ref_mode, out_exact, r, pa
     p64 = {k: v.to(device="cuda", dtype=torch.float64) for k, v in params.items()}
     xin = x_hit.float().double() if f64 else x_hit
     u = ref.policy_torch(p64, xin)
-    wrong_G = _np(r["G"])[fin] + _np(-(1.0 + 0.5 * (u * u).sum(dim=1)) * DT)
+    wrong_G = _np(r["G"])[fin] + _np(-(1.0 + 0.5 * (u * u).sum(dim=1)) * dt)
     G = _np(out_exact.G)[fin]
     assert (np.abs(G - wrong_G) > _bound(n, G, C_G[prec])).mean() > 0.95, (family, d, H)
 
@@ -455,13 +504,18 @@ GRAD_TOL = {"K2": 2e-6,       # 4.1e-7 (d = 10), 4.9x
             "split": 5e-7}    # 1.1e-7, 4.5x
 
 
-def _grad_case(family, d, H, ckpt, K=192, lim=400, extra_cfg=None):
+def _grad_case(family, d, H, ckpt, K=192, lim=400, extra_cfg=None, env=None, wrong_envs=None):
+    """Kernel gradients in both integral modes against float64 autograd along the kernel's hit passes, in the environment
+    ``env`` (as _env_c).  Returns (relative error per mode, relative distance of the exact-mode gradient from the
+    reference-mode float64 one, {name: relative distance of the kernel's gradient from float64 autograd in the
+    environment ``wrong_envs[name]``, the smaller of the two modes})."""
     L, R = _lib()
+    s = _spec(env)
     seed = 77 + 100 * d + H
     _, params, flat = _policy(d, H, 2.0 if d == 1 else 3.0, seed)
-    env, env_c = _env_c(d, L.HIT_ALL_GE_LB)
+    _, env_c = _env_c(d, L.HIT_ALL_GE_LB, env)
     mlp_c = L.make_mlp(d, H)
-    noise = R.noise_fill(seed, K, d, lim, DT)
+    noise = R.noise_fill(seed, K, d, lim, s["dt"])
     fkw, cfg_set = BWD_FAMILIES[family]
     fwd = R.rollout_forward(env_c, mlp_c, flat, K, noise=noise, n_steps_lim=lim, stoch_int="exact", store_path=True,
                             ckpt_every=ckpt, want_logw=False, **fkw)
@@ -473,11 +527,23 @@ def _grad_case(family, d, H, ckpt, K=192, lim=400, extra_cfg=None):
     for mode in ("exact", "reference"):
         fwd.cfg.flags = (fwd.cfg.flags | L.F_STOCH_INT_EXACT) if mode == "exact" else (fwd.cfg.flags & ~L.F_STOCH_INT_EXACT)
         grads[mode] = R.rollout_backward(env_c, mlp_c, flat, fwd, 1.0 / K, noise=noise).cpu().numpy().astype(np.float64)
-    r = ref.rollout_reference(d, 1.0, 1.0, DT, params, noise, hit_index=T, grad_modes=("exact", "reference"), device="cuda")
-    want = {m: np.concatenate([r["grads"][m][k].reshape(-1) for k in ref.PARAM_KEYS]) for m in ("exact", "reference")}
-    errs = {m: np.abs(grads[m] - want[m]).max() / np.abs(want[m]).max() for m in want}
-    wrong = np.abs(grads["exact"] - want["reference"]).max() / np.abs(want["reference"]).max()
-    return errs, wrong
+    modes = ("exact", "reference")
+
+    def autograd(e):
+        r = _reference(d, params, noise, e, hit_index=T, grad_modes=modes, device="cuda")
+        return {m: np.concatenate([r["grads"][m][k].reshape(-1) for k in ref.PARAM_KEYS]) for m in modes}
+
+    def dist(a, b):
+        return np.abs(a - b).max() / np.abs(b).max()
+
+    want = autograd(env)
+    errs = {m: dist(grads[m], want[m]) for m in modes}
+    wrong = dist(grads["exact"], want["reference"])
+    wrong_env = {}
+    for name, e in (wrong_envs or {}).items():
+        w = autograd(e)
+        wrong_env[name] = min(dist(grads[m], w[m]) for m in modes)
+    return errs, wrong, wrong_env
 
 
 @pytest.mark.parametrize("family,d,H,ckpt", BWD_CASES)
@@ -485,7 +551,7 @@ def test_reverse_pass_matches_float64_autograd(family, d, H, ckpt):
     """Every reverse family in both stochastic-integral modes against float64 autograd of mean(-G - sg(G) S) along the
     kernel's hit passes; the exact-mode gradient is told apart from the reference-mode float64 gradient (short paths with a
     drift towards the target, where the detecting pass's u . dB is a visible share of the gradient)."""
-    errs, wrong = _grad_case(family, d, H, ckpt)
+    errs, wrong, _ = _grad_case(family, d, H, ckpt)
     tol = GRAD_TOL[family]
     assert errs["exact"] <= tol and errs["reference"] <= tol, (family, d, H, ckpt, errs)
     assert wrong > 10 * tol, (family, d, H, ckpt, wrong)
@@ -497,7 +563,7 @@ def test_reverse_pass_split_between_families_matches_float64_autograd(bulk):
     onto the warp kernel's gradient on the caller's stream) or to K2m (on a second stream, joined before its reduction);
     both integral modes, against float64 autograd."""
     n_sm = torch.cuda.get_device_properties(0).multi_processor_count
-    errs, wrong = _grad_case(bulk, 1, 32, 1, K=128 * n_sm + 200, lim=300, extra_cfg={"bwd_warp_share": 1000})
+    errs, wrong, _ = _grad_case(bulk, 1, 32, 1, K=128 * n_sm + 200, lim=300, extra_cfg={"bwd_warp_share": 1000})
     tol = GRAD_TOL["split"]
     assert errs["exact"] <= tol and errs["reference"] <= tol, errs
     assert wrong > 10 * tol, wrong

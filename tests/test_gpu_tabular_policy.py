@@ -143,14 +143,19 @@ C_OUT = (2.0, 0.3)
 FLIP_SHARE = (0.10, 0.01)
 
 
+def replay_env(env):
+    """rollout_reference_table's environment keywords from the attributes of a 1-D environment."""
+    return dict(alpha=env.alpha, beta=env.beta, dt=env.dt, lb=env.lb, rb=env.rb, x0=float(env.state_init.reshape(-1)[0]))
+
+
 def _fp64_case(table, env, f64, stoch_int, K=512, lim=4000, seed=5):
     L, R = _mods()
-    noise = R.noise_fill(seed, K, 1, lim, DT)
+    noise = R.noise_fill(seed, K, 1, lim, env.dt)
     pol_opt = np.asarray(table, dtype=np.float32).reshape(-1)[::-1].copy()       # a policy_opt that is not the table
     out = _table_rollout(env, table, K, noise=noise, n_steps_lim=lim, stoch_int=stoch_int, state_f64=f64, policy_opt=pol_opt)
     T = out.T.cpu().numpy().astype(np.int64)
     r = rollout_reference_table(table, _grid(env), noise, hit_index=T, policy_opt=pol_opt[:, None], grid=_grid(env),
-                                device="cuda")
+                                device="cuda", **replay_env(env))
     assert np.array_equal(r["T"].cpu().numpy(), T)
     prec = 1 if f64 else 0
     n = np.where(T >= 0, T, lim - 1).astype(np.float64)

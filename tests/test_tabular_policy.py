@@ -19,8 +19,8 @@ def _env(h=0.01, dt=DT):
     return env
 
 
-def rollout_reference_table(table, table_grid, noise, *, hit_rule=ref.HIT_X0_IN_LB_RB, **kw):
-    """oracle.reference_semantics.rollout_reference (d = 1, alpha = beta = 1, dt = 0.005) with the control
+def rollout_reference_table(table, table_grid, noise, *, hit_rule=ref.HIT_X0_IN_LB_RB, alpha=1.0, beta=1.0, dt=DT, **kw):
+    """oracle.reference_semantics.rollout_reference (d = 1, by default alpha = beta = 1, dt = 0.005) with the control
     u = table[idx(x)], idx(x) = floor((clip(x, lo, hi) - lo) / h) clamped to the table, in place of the MLP: the lookup
     sees the state in the replay's precision, everything else is the replay's arithmetic.  ``table_grid = (lo, hi, h)``;
     the ``grid=`` of rollout_reference belongs to its ``policy_opt``."""
@@ -34,7 +34,7 @@ def rollout_reference_table(table, table_grid, noise, *, hit_rule=ref.HIT_X0_IN_
         return tab[gi][:, None]
 
     with mock.patch.object(ref, "policy_torch", lookup):
-        return ref.rollout_reference(1, 1.0, 1.0, DT, {}, noise, hit_rule=hit_rule, **kw)
+        return ref.rollout_reference(1, alpha, beta, dt, {}, noise, hit_rule=hit_rule, **kw)
 
 
 def test_forward_is_the_environment_index():
