@@ -261,6 +261,24 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
                       float* grad_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /*
+ * Reverse pass of any loss over the returns and stochastic integrals: the gradient
+ *     grad = loss_scale * sum_k [T_k >= 0] ( cG_k dG_k/dtheta + cS_k dS_k/dtheta )
+ * with per-trajectory coefficients coef_G_dev / coef_S_dev (float[K], indexed by local trajectory id), S = S_ref, or
+ * S_exact under RLSDE_F_STOCH_INT_EXACT.  The derivative is the pathwise one along the sampled path with the hit passes
+ * held fixed, as in rlsde_rollout_bwd; only the adjoint input of pass j changes:
+ *     a_j = -cG_k [j<k*] u_j dt + cS_k [j<=k*, or j<k* with RLSDE_F_STOCH_INT_EXACT] dB_{j+1} + sigma dt lambda_{j+1}
+ * rlsde_rollout_bwd is the case cG = -1, cS = -G, and with those coefficients this call returns its gradient bit for bit.
+ * For a loss f(G, S) pass cG = df/dG, cS = df/dS (e.g. from autograd over G and S).  Kernel selection, order_dev,
+ * traj_offset / K_global, bwd_warp_share, the workspace (rlsde_workspace_bytes_bwd at hidden widths 64..256) and every
+ * refusal are those of rlsde_rollout_bwd; a NULL coefficient pointer is RLSDE_ERR_INVALID_ARG.
+ */
+int rlsde_rollout_bwd_weighted(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                               const rlsde_rollout_cfg* cfg, const float* noise_dev,
+                               const float* coef_G_dev, const float* coef_S_dev, const int32_t* T_dev,
+                               const float* path_dev, const int64_t* order_dev, double loss_scale,
+                               float* grad_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/*
  * One REINFORCE iteration with everything resident on the device (reinforce_deterministic_core.py:232-243:
  * zero_grad -> sample_loss_vectorized -> backward -> Adam step), for the latency-bound small-batch regime
  * (K <= 16 x SMs, hidden width 32; RLSDE_ERR_UNSUPPORTED otherwise): the policy is read from theta_dev (float[P],

@@ -4,7 +4,7 @@ Module names mirror the reference package ``rl_sde_is`` for the functions on the
 
     environments                  DoubleWellStoppingTime1D / 2D / ND  (env.step, env.step_torch, grids)
     models                        mlp, DeterministicPolicy
-    reinforce_deterministic_core  sample_loss_vectorized, reinforce
+    reinforce_deterministic_core  sample_loss_vectorized, sample_returns_vectorized, reinforce
     approximate_methods           test_policy_vectorized, estimate_fht_vectorized, is_estimate
     dynamic_programming           compute_r_table, compute_p_tensor_batch
     tabular_dp_tables             check_p_tensor, dynamic_programming_tables

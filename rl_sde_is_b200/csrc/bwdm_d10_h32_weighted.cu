@@ -1,0 +1,6 @@
+// weighted reverse-pass kernels (rlsde_rollout_bwd_weighted) for d = 10, hidden width = 32: the tensor-core
+// thread-per-trajectory family and the warp-per-trajectory kernel
+#include "rollout_bwd_mma_inst.cuh"
+#include "rollout_warp_inst.cuh"
+RLSDE_INSTANTIATE_BWD_MMA_WEIGHTED(10)
+RLSDE_INSTANTIATE_BWD_WARP_WEIGHTED(10)

@@ -485,14 +485,19 @@ int rlsde_rollout_transitions(const rlsde_env* env, const rlsde_mlp* mlp, const 
                           stats_dev, tr, workspace_dev, workspace_bytes, stream_);
 }
 
-int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
-                      const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* G_dev, const int32_t* T_dev,
-                      const float* path_dev, const int64_t* order_dev, double loss_scale, float* grad_dev,
-                      void* workspace_dev, size_t workspace_bytes, void* stream_) {
+// WEIGHTED = false: rlsde_rollout_bwd (cS_dev = G, cG_dev unused); true: rlsde_rollout_bwd_weighted.  The weighted kernels
+// read cS from FwdArgs::G and cG from FwdArgs::S (rollout_bwd.cuh, the comment above em_step_f32).
+extern "C++" {
+template <bool WEIGHTED>
+static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host, const rlsde_rollout_cfg* cfg,
+                            const float* noise_dev, const float* cS_dev, const float* cG_dev, const int32_t* T_dev,
+                            const float* path_dev, const int64_t* order_dev, double loss_scale, float* grad_dev,
+                            void* workspace_dev, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   int rc = check_env_mlp(env, mlp);
   if (rc != RLSDE_OK) return rc;
-  if (!params_host || !G_dev || !T_dev || !path_dev || !grad_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
+  if (!params_host || !cS_dev || !T_dev || !path_dev || !grad_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
+  if (WEIGHTED && !cG_dev) return RLSDE_ERR_INVALID_ARG;
   if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
   FwdArgs A;
   memset(&A, 0, sizeof(A));
@@ -504,7 +509,8 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
   if (A.ckpt_every > BWD_MAX_SEG) return RLSDE_ERR_INVALID_ARG;        // the reverse pass recomputes at most 32 passes per checkpoint
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
   A.noise = noise_dev;
-  A.G = (void*)G_dev; A.T = (int*)T_dev; A.path = (float*)path_dev;
+  A.G = (void*)cS_dev; A.T = (int*)T_dev; A.path = (float*)path_dev;
+  if (WEIGHTED) A.S = (void*)cG_dev;
   A.order = (const long long*)order_dev;
   A.counter = (unsigned long long*)workspace_dev;
   int sm = 0;
@@ -525,7 +531,7 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
       uint8_t* scratch = (uint8_t*)workspace_dev + ws_fixed_bytes();
 #define X(D_, H_)                                                                                                        \
   if (env->d == D_ && mlp->d_hidden == H_)                                                                               \
-    lrc = launch_rollout_bwd_umma<D_, H_>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A,   \
+    lrc = launch_rollout_bwd_umma<D_, H_, WEIGHTED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A,   \
                                           (float)loss_scale, grad_dev, scratch, workspace_bytes - ws_fixed_bytes(), sm, stream);
       RLSDE_UMMA_SHAPES(X)
 #undef X
@@ -534,7 +540,7 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
     }
 #define X(D_, H_)                                                                                                       \
   if (env->d == D_ && mlp->d_hidden == H_)                                                                              \
-    lrc = launch_rollout_bwd_wide<D_, H_>(params_host, ws_wide_params(workspace_dev), A, (float)loss_scale, grad_dev, partial, \
+    lrc = launch_rollout_bwd_wide<D_, H_, WEIGHTED>(params_host, ws_wide_params(workspace_dev), A, (float)loss_scale, grad_dev, partial, \
                                           bwd_partial_main_bytes(), sm, stream);
     RLSDE_WIDE_SHAPES(X)
 #undef X
@@ -578,7 +584,7 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
     }
 #define X(D_, H_)                                                                                                   \
   if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H)                                                          \
-    lrc = launch_rollout_bwd_warp<D_>(params_host, nullptr, Along, (float)loss_scale, grad_dev, partial_aux, sm, s_long);
+    lrc = launch_rollout_bwd_warp<D_, WEIGHTED>(params_host, nullptr, Along, (float)loss_scale, grad_dev, partial_aux, sm, s_long);
     RLSDE_SHAPES(X)
 #undef X
     if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd (long trajectories) launch");
@@ -590,13 +596,30 @@ int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* p
   }
 #define X(D_, H_)                                                                                                          \
   if (env->d == D_ && mlp->d_hidden == H_ && Abulk.K > 0)                                                                  \
-    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_bwd_warp<D_>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev, partial, sm, stream) \
-          : (use_mma && H_ == MMA_H)  ? launch_rollout_bwd_mma<D_>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream, join)      \
-                                      : launch_rollout_bwd<D_, H_>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream);
+    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_bwd_warp<D_, WEIGHTED>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev, partial, sm, stream) \
+          : (use_mma && H_ == MMA_H)  ? launch_rollout_bwd_mma<D_, WEIGHTED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream, join)      \
+                                      : launch_rollout_bwd<D_, H_, WEIGHTED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream);
   RLSDE_SHAPES(X)
 #undef X
   if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd launch");
   return RLSDE_OK;
+}
+}  // extern "C++"
+
+int rlsde_rollout_bwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                      const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* G_dev, const int32_t* T_dev,
+                      const float* path_dev, const int64_t* order_dev, double loss_scale, float* grad_dev,
+                      void* workspace_dev, size_t workspace_bytes, void* stream_) {
+  return rollout_bwd_impl<false>(env, mlp, params_host, cfg, noise_dev, G_dev, nullptr, T_dev, path_dev, order_dev, loss_scale,
+                                 grad_dev, workspace_dev, workspace_bytes, stream_);
+}
+
+int rlsde_rollout_bwd_weighted(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                               const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* coef_G_dev,
+                               const float* coef_S_dev, const int32_t* T_dev, const float* path_dev, const int64_t* order_dev,
+                               double loss_scale, float* grad_dev, void* workspace_dev, size_t workspace_bytes, void* stream_) {
+  return rollout_bwd_impl<true>(env, mlp, params_host, cfg, noise_dev, coef_S_dev, coef_G_dev, T_dev, path_dev, order_dev, loss_scale,
+                                grad_dev, workspace_dev, workspace_bytes, stream_);
 }
 
 // rollout + statistics + reverse pass of one device-resident REINFORCE iteration (everything but the parameter update)

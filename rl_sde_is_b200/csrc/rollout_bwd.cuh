@@ -8,6 +8,9 @@
 //     theta_bar += (d policy / d theta)(X_j)^T a_j
 //     lambda_j = (1 - dt 4 alpha (3 X_j^2 - 1)) * lambda_{j+1} + (d policy / d x)(X_j)^T a_j
 // (unscaled; `scale` is applied in the final reduction).
+// WEIGHTED (rlsde_rollout_bwd_weighted): L = scale * sum_k (cG_k G_k + cS_k S_k) for per-trajectory coefficients, i.e.
+//     a_j      = -cG [j<k*] u_j dt + cS dB_{j+1} [same condition as above] + sigma dt lambda_{j+1}
+// (the comment above em_step_f32); the unweighted kernels are the case cG = -1, cS = -G, folded at compile time.
 //
 // Mapping: one trajectory per thread, processed segment by segment from the last checkpoint
 // backwards.  A round = phase A (recompute the segment's states X_j from its checkpoint, identical
@@ -118,6 +121,12 @@ struct NoiseCache {
   }
 };
 
+// The weighted kernels (WEIGHTED = true) read the coefficients from FwdArgs fields no reverse pass reads otherwise: cS_k from
+// A.G (where the unweighted kernels read G_k, the negated coefficient of dB), cG_k from A.S.  They evaluate the unweighted
+// kernels' expression for a_j with G_k replaced by -cS_k and u_j by RN(-cG_k u_j), both negations and the product formed
+// with __fmul_rn (opaque to the compiler's rewriting).  With (cG, cS) = (-1, -G) they are exact and the expression keeps
+// its shape, so the compiler's choices (which products it contracts into FMAs differs between kernels and dimensions)
+// and hence every rounding are the unweighted kernels': the gradient is bit for bit that of rlsde_rollout_bwd.
 // f32 Euler-Maruyama pass, identical association to K1
 template <int D>
 __device__ __forceinline__ void em_step_f32(const FwdArgs& A, float (&x)[D], const float (&u)[D], const float (&dB)[D]) {
@@ -144,7 +153,7 @@ constexpr int kBwdUnroll = RLSDE_BWD_UNROLL;
 #endif
 
 // Per-warp partial gradient layout = state_dict order: W1 (H,D), b1 (H), W2 (H,H), b2 (H), W3 (D,H), b3 (D)
-template <int D, int H, bool FAST>
+template <int D, int H, bool FAST, bool WEIGHTED = false>
 __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kernel(const __grid_constant__ MlpConst<D, H> W,
                                                           const __grid_constant__ FwdArgs A, float* __restrict__ partial) {
   static_assert(H == 32 || H == 64, "column-per-lane accumulation needs H in {32, 64}");
@@ -184,7 +193,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
   long long slot = gl - n_lanes;   // next static assignment: slot += n_lanes, traj = order[slot]
   long long traj = 0;
   int kstar = 0, seg = 0;
-  float Gk = 0.f;
+  float Gk = 0.f, mG = 0.f;        // WEIGHTED: -cS, -cG
   float lam[D];
   float xs[BWD_MAX_SEG][D];
   NoiseCache<D> nc;
@@ -202,6 +211,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
       const int t = A.T[traj];
       if (t >= 0) {
         alive = true; kstar = t; seg = t / C; Gk = ((const float*)A.G)[traj];
+        if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
         nc.reset();
 #pragma unroll
         for (int i = 0; i < D; ++i) lam[i] = 0.f;
@@ -248,7 +258,8 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
           float v = 0.f;
           if (ok) {
             const bool incl = s_exact ? (j < kstar) : true;
-            v = (j < kstar ? u[i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+            if constexpr (WEIGHTED) v = (j < kstar ? __fmul_rn(mG, u[i]) * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+            else v = (j < kstar ? u[i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
           }
           a[i] = v;
         }
@@ -435,7 +446,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
   if (lane < D) ob3[lane] = (float)gb3;
 }
 
-template <int D, int H>
+template <int D, int H, bool WEIGHTED = false>
 int launch_rollout_bwd(const float* params_host, const FwdArgs& args, float scale, float* grad, float* partial,
                        int sm_count, cudaStream_t stream);
 

@@ -223,7 +223,9 @@ constexpr size_t bwd_mma_dyn_smem(int D, int block) {
 }
 
 // Per-warp partial gradient layout = state_dict order (W1 (H,D), b1, W2 (H,H), b2, W3 (D,H), b3), doubles.
-template <int D, bool FAST>
+// WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32); the per-pass scale window below adapts
+// to their magnitude as it does to G's
+template <int D, bool FAST, bool WEIGHTED = false>
 __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_mma_kernel(const __grid_constant__ MlpConst<D, MMA_H> W,
                                                                   const __grid_constant__ FwdArgs A,
                                                                   const __grid_constant__ BwdMmaWeights F,
@@ -413,7 +415,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_
   long long slot = gl - n_lanes;   // next static assignment: slot += n_lanes, traj = order[slot]
   long long traj = 0;
   int kstar = 0, seg = 0;
-  float Gk = 0.f;
+  float Gk = 0.f, mG = 0.f;        // WEIGHTED: -cS, -cG
   float lam[D];
   float xs[BWD_MAX_SEG][D];
   constexpr bool CACHE_DB = NoisePlan<D>::BPP > 1;
@@ -431,6 +433,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_
       const int t = A.T[traj];
       if (t >= 0) {
         alive = true; kstar = t; seg = t / C; Gk = ((const float*)A.G)[traj];
+        if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
         nc.reset();
 #pragma unroll
         for (int i = 0; i < D; ++i) { lam[i] = 0.f; xck[i] = A.path[((long long)traj * A.ckpt_stride + seg) * D + i]; }
@@ -585,7 +588,8 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_
           float v = 0.f;
           if (ok && my_half) {
             const bool incl = s_exact ? (j < kstar) : true;
-            v = (j < kstar ? u[i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+            if constexpr (WEIGHTED) v = (j < kstar ? __fmul_rn(mG, u[i]) * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+            else v = (j < kstar ? u[i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
           }
           a[i] = v;
           asum += fabsf(v);
@@ -900,7 +904,7 @@ static __global__ void bwd_reduce64_kernel(const double* __restrict__ partial, i
 
 // join: if non-null, the stream waits for this event between the rollout kernel and the reduction that adds into `grad`
 // (the warp-per-trajectory kernel working on the longest trajectories on a second stream writes `grad` first)
-template <int D>
+template <int D, bool WEIGHTED = false>
 int launch_rollout_bwd_mma(const float* params_host, const FwdArgs& args, float scale, float* grad, void* partial,
                            int sm_count, cudaStream_t stream, cudaEvent_t join);
 

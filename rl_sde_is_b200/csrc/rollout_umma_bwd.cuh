@@ -113,7 +113,8 @@ __device__ __forceinline__ float lane_transpose_sum(float (&v)[32], int lane) {
 }  // namespace umma
 
 // partial layout (float64): [n_cons][H * H] (dW2 in 2^esh units, row = out unit), then [n_prod][ub_small_count]
-template <int D, int H, bool FAST>
+// WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32); the launch's scale from ub_scale_weighted_kernel
+template <int D, int H, bool FAST, bool WEIGHTED = false>
 __global__ void __launch_bounds__(UB_THREADS, 1)
 rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict__ Bimg1, const uint8_t* __restrict__ Bimg2,
                         const __grid_constant__ FwdArgs A, uint8_t* __restrict__ xbuf, unsigned* __restrict__ ctl,
@@ -342,7 +343,7 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
     bool alive = false;
     long long traj = 0;
     int kstar = 0, j = -1;
-    float Gk = 0.f, lam[D], gb3[D], xn[D], xf[D];
+    float Gk = 0.f, mG = 0.f, lam[D], gb3[D], xn[D], xf[D];        // WEIGHTED: Gk = -cS, mG = -cG
     NoiseCache<D> nc;
     nc.reset();
 #pragma unroll
@@ -352,7 +353,10 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
       if (slot < A.K) {
         traj = A.order ? A.order[slot] : slot;
         const int t = A.T[traj];
-        if (t >= 0) { alive = true; kstar = t; j = t; Gk = ((const float*)A.G)[traj]; }
+        if (t >= 0) {
+          alive = true; kstar = t; j = t; Gk = ((const float*)A.G)[traj];
+          if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
+        }
       }
       const int np = __reduce_max_sync(0xffffffffu, alive ? j + 1 : 0);
       if (lane == 0 && half == 0) s_np[rgrp] = np;
@@ -490,7 +494,8 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
           if (live) {
             const bool incl = s_exact ? (j < kstar) : true;
             const float ui = (s_u[0][tr][i] + s_u[1][tr][i]) + b3[i];
-            v = (j < kstar ? ui * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+            if constexpr (WEIGHTED) v = (j < kstar ? __fmul_rn(mG, ui) * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+            else v = (j < kstar ? ui * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
           }
           a[i] = v;
           if (half == 0) gb3[i] += v;
@@ -708,6 +713,38 @@ static __global__ void ub_scale_kernel(const float* __restrict__ G, const int* _
   }
 }
 
+// The weighted reverse pass's scale exponent: a_j = -cG u_j dt + cS dB_j + sigma dt lambda_j, so the bound above becomes
+// |a|_1 <~ D (max |cS| 8 sqrt(dt) + max |cG|) over the finished trajectories; with (cG, cS) = (-1, -G) it is ub_scale_kernel's.
+static __global__ void ub_scale_weighted_kernel(const float* __restrict__ cG, const float* __restrict__ cS, const int* __restrict__ T,
+                                                long long K, float w3max, float sqrt_dt, int D, int n_prod, unsigned* __restrict__ ctl) {
+  __shared__ float s_max[2][32];
+  float mg = 0.f, ms = 0.f;
+  for (long long i = threadIdx.x; i < K; i += blockDim.x)
+    if (T[i] >= 0) { mg = fmaxf(mg, fabsf(cG[i])); ms = fmaxf(ms, fabsf(cS[i])); }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    mg = fmaxf(mg, __shfl_xor_sync(0xffffffffu, mg, o));
+    ms = fmaxf(ms, __shfl_xor_sync(0xffffffffu, ms, o));
+  }
+  if ((threadIdx.x & 31) == 0) { s_max[0][threadIdx.x >> 5] = mg; s_max[1][threadIdx.x >> 5] = ms; }
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    mg = threadIdx.x < (blockDim.x >> 5) ? s_max[0][threadIdx.x] : 0.f;
+    ms = threadIdx.x < (blockDim.x >> 5) ? s_max[1][threadIdx.x] : 0.f;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      mg = fmaxf(mg, __shfl_xor_sync(0xffffffffu, mg, o));
+      ms = fmaxf(ms, __shfl_xor_sync(0xffffffffu, ms, o));
+    }
+    const float bound = w3max * (float)D * fmaf(ms * 8.0f, sqrt_dt, mg);
+    int e = 0;
+    if (bound > 0.f && isfinite(bound)) frexpf(bound, &e);          // bound < 2^e
+    int esh = 15 - 3 - e;
+    esh = esh > 60 ? 60 : (esh < -60 ? -60 : esh);
+    for (int p = threadIdx.x; p < n_prod; p += 32) ctl[(size_t)p * UB_CTL_WORDS + 12] = (unsigned)esh;
+  }
+}
+
 // grad[...] (+)= scale * (partials in index order); the H x H block carries the 2^-esh unscale
 template <int D, int H>
 static __global__ void ub_reduce_kernel(const double* __restrict__ partial, int n_prod, int n_cons, float scale,
@@ -740,7 +777,7 @@ static __global__ void ub_reduce_kernel(const double* __restrict__ partial, int 
 // scratch the launcher needs behind the fixed workspace (exchange ring, control words, float64 partials, second image)
 template <int D, int H>
 size_t bwd_umma_scratch_bytes(int sm_count);
-template <int D, int H>
+template <int D, int H, bool WEIGHTED = false>
 int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, float scale,
                             float* grad, uint8_t* scratch, size_t scratch_bytes, int sm_count, cudaStream_t stream);
 

@@ -37,12 +37,12 @@ size_t bwd_umma_scratch_bytes(int sm_count) {
   return UbScratch<D, H>::total(n_prod, n_cons);
 }
 
-template <int D, int H, bool FAST>
+template <int D, int H, bool FAST, bool WEIGHTED>
 static int launch_bwd_umma_variant(const float* params_dev, const uint8_t* img1, const FwdArgs& args, float scale, float* grad,
                                    uint8_t* scratch, int n_prod, int n_cons, float w3max, cudaStream_t stream) {
   typedef UbScratch<D, H> S;
   constexpr int P = D * H + H + H * H + H + H * D + D;
-  auto kern = rollout_bwd_umma_kernel<D, H, FAST>;
+  auto kern = rollout_bwd_umma_kernel<D, H, FAST, WEIGHTED>;
   const size_t smem = ub_smem_bytes<D, H>();
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -56,7 +56,11 @@ static int launch_bwd_umma_variant(const float* params_dev, const uint8_t* img1,
   FwdArgs a = args;
   void* kargs[] = {(void*)&params_dev, (void*)&img1, (void*)&img2, (void*)&a, (void*)&xbuf, (void*)&ctl, (void*)&partial,
                    (void*)&n_prod, (void*)&n_cons};
-  ub_scale_kernel<<<1, 1024, 0, stream>>>((const float*)args.G, args.T, args.K, w3max, sqrtf(args.dt_f), D, n_prod, ctl);
+  if constexpr (WEIGHTED)
+    ub_scale_weighted_kernel<<<1, 1024, 0, stream>>>((const float*)args.S, (const float*)args.G, args.T, args.K, w3max, sqrtf(args.dt_f),
+                                                     D, n_prod, ctl);
+  else
+    ub_scale_kernel<<<1, 1024, 0, stream>>>((const float*)args.G, args.T, args.K, w3max, sqrtf(args.dt_f), D, n_prod, ctl);
   e = cudaLaunchCooperativeKernel((const void*)kern, dim3((unsigned)(n_prod + n_cons)), dim3(UB_THREADS), kargs, smem, stream);
   if (e != cudaSuccess) return (int)e;
   ub_reduce_kernel<D, H><<<(P + 127) / 128, 128, 0, stream>>>(partial, n_prod, n_cons, scale, ctl, grad, args.grad_accumulate);
@@ -77,7 +81,7 @@ static int launch_bwd_umma_variant(const float* params_dev, const uint8_t* img1,
   return (int)cudaGetLastError();
 }
 
-template <int D, int H>
+template <int D, int H, bool WEIGHTED>
 int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, float scale,
                             float* grad, uint8_t* scratch, size_t scratch_bytes, int sm_count, cudaStream_t stream) {
   typedef UbScratch<D, H> S;
@@ -91,7 +95,8 @@ int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t
   std::vector<uint16_t> w1(umma_image_bytes<H>() / 2), w2(umma_image_bytes<H>() / 2);
   pack_umma_weights<H>(img.data() + WideParams<D, H>::o_W2, w1.data());      // B[n = out][k = in]   (Z2 = H1 W2^T)
   pack_umma_weights<H>(img.data() + WideParams<D, H>::o_W2t, w2.data());     // B[n = in][k = out]   (dH1 = dZ2 W2)
-  // largest head weight: the device picks the launch's scale exponent from it and from max |G| (ub_scale_kernel)
+  // largest head weight: the device picks the launch's scale exponent from it and from max |G| (ub_scale_kernel) or the
+  // coefficients (ub_scale_weighted_kernel)
   double w3max = 0.0;
   for (int c = 0; c < H; ++c)
     for (int i = 0; i < D; ++i) w3max = fmax(w3max, fabs((double)img[WideParams<D, H>::o_W3 + (size_t)i * H + c]));
@@ -101,8 +106,8 @@ int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t
   if ((e = cudaMemcpyAsync(scratch + S::o_img2, w2.data(), umma_image_bytes<H>(), cudaMemcpyHostToDevice, stream)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(scratch + S::o_ctl, 0, S::o_img2, stream)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(scratch + S::o_partial, 0, S::partial_bytes(n_prod, n_cons), stream)) != cudaSuccess) return (int)e;
-  return fast ? launch_bwd_umma_variant<D, H, true>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream)
-              : launch_bwd_umma_variant<D, H, false>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream);
+  return fast ? launch_bwd_umma_variant<D, H, true, WEIGHTED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream)
+              : launch_bwd_umma_variant<D, H, false, WEIGHTED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream);
 }
 
 }  // namespace rlsde
@@ -111,3 +116,7 @@ int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t
   template size_t rlsde::bwd_umma_scratch_bytes<D, H>(int);                                                                       \
   template int rlsde::launch_rollout_bwd_umma<D, H>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, float*, uint8_t*, \
                                                     size_t, int, cudaStream_t);
+// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
+#define RLSDE_INSTANTIATE_UMMA_BWD_WEIGHTED(D, H)                                                                                 \
+  template int rlsde::launch_rollout_bwd_umma<D, H, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, float*,   \
+                                                          uint8_t*, size_t, int, cudaStream_t);

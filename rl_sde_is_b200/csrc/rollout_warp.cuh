@@ -348,7 +348,8 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
 
 // ------------------------------------------------------------------------------------------------ reverse
 // Needs every state (ckpt_every == 1).  Lane j accumulates row j of dW2 / dW1, column j of dW3, entry j of db1 / db2.
-template <int D, bool FAST>
+// WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32).
+template <int D, bool FAST, bool WEIGHTED = false>
 __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_constant__ MlpConst<D, WARP_H> W_param,
                                                                const MlpConst<D, WARP_H>* __restrict__ W_dev,
                                                                const __grid_constant__ FwdArgs A, float* __restrict__ partial) {
@@ -380,7 +381,9 @@ __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_cons
     const long long traj = A.order ? A.order[item] : item;
     const int kstar = A.T[traj];
     if (kstar < 0) continue;
-    const float Gk = ((const float*)A.G)[traj];
+    const float Gk = ((const float*)A.G)[traj];                       // WEIGHTED: cS
+    const float nS = WEIGHTED ? __fmul_rn(-1.0f, Gk) : 0.f;
+    const float mG = WEIGHTED ? __fmul_rn(-1.0f, ((const float*)A.S)[traj]) : 0.f;
     float lam[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) lam[i] = 0.f;
@@ -405,7 +408,8 @@ __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_cons
 #pragma unroll
       for (int i = 0; i < D; ++i) {
         const bool incl = s_exact ? (j < kstar) : true;
-        a[i] = (j < kstar ? u[i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+        if constexpr (WEIGHTED) a[i] = (j < kstar ? __fmul_rn(mG, u[i]) * A.dt_f : 0.f) - (incl ? nS * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+        else a[i] = (j < kstar ? u[i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
         gW3[i] = fmaf(a[i], h2, gW3[i]);
         gb3[i] += a[i];
         dh2 = fmaf(P.w3[i], a[i], dh2);
@@ -460,7 +464,7 @@ inline long long warp_path_max_k(int sm_count) { return (long long)sm_count * 16
 // params_host == nullptr: the policy is read from W_dev (an MlpConst<D, WARP_H> in device memory, see pack_mlp_const_dev)
 template <int D>
 int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream);
-template <int D>
+template <int D, bool WEIGHTED = false>
 int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                             float* partial, int sm_count, cudaStream_t stream);
 // continues the trajectories the thread-per-trajectory kernel left in args.q_ring (args.q_ctrl[1] records)

@@ -110,7 +110,7 @@ int launch_rollout_fwd_warp_resume(const float* params_host, const FwdArgs& args
   return launch_fwd_warp_resume_policy<D, false>(params_host, args, sm_count, stream);
 }
 
-template <int D, bool FAST>
+template <int D, bool FAST, bool WEIGHTED>
 static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                                    float* partial, int sm_count, cudaStream_t stream) {
   constexpr int P = D * WARP_H + WARP_H + WARP_H * WARP_H + WARP_H + WARP_H * D + D;
@@ -118,7 +118,7 @@ static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, 
   if (params_host != nullptr) pack_mlp_const<D, WARP_H>(params_host, FAST, W);
   else memset(&W, 0, sizeof(W));
   const long long grid = warp_grid(args.K, sm_count);
-  rollout_bwd_warp_kernel<D, FAST><<<(unsigned)grid, 128, 0, stream>>>(
+  rollout_bwd_warp_kernel<D, FAST, WEIGHTED><<<(unsigned)grid, 128, 0, stream>>>(
       W, params_host != nullptr ? nullptr : reinterpret_cast<const MlpConst<D, WARP_H>*>(W_dev), args, partial);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;
@@ -127,12 +127,12 @@ static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, 
   return (int)cudaGetLastError();
 }
 
-template <int D>
+template <int D, bool WEIGHTED>
 int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                             float* partial, int sm_count, cudaStream_t stream) {
   return (args.flags & RLSDE_F_TANH_FAST)
-             ? launch_bwd_warp_variant<D, true>(params_host, W_dev, args, scale, grad, partial, sm_count, stream)
-             : launch_bwd_warp_variant<D, false>(params_host, W_dev, args, scale, grad, partial, sm_count, stream);
+             ? launch_bwd_warp_variant<D, true, WEIGHTED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream)
+             : launch_bwd_warp_variant<D, false, WEIGHTED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream);
 }
 
 }  // namespace rlsde
@@ -143,3 +143,7 @@ int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const F
                                                  int, cudaStream_t);                                                       \
   template int rlsde::launch_pack_mlp_const_dev<D>(const float*, void*, bool, cudaStream_t);                              \
   template int rlsde::launch_rollout_fwd_warp_resume<D>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
+// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
+#define RLSDE_INSTANTIATE_BWD_WARP_WEIGHTED(D)                                                                             \
+  template int rlsde::launch_rollout_bwd_warp<D, true>(const float*, const void*, const rlsde::FwdArgs&, float, float*,   \
+                                                       float*, int, cudaStream_t);

@@ -399,7 +399,8 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const
 // Block-private partial gradient in global memory: state_dict order, float32 [P].  The H x H block is updated in place
 // every pass (read-modify-write by the thread that owns the element); the small blocks are kept in registers / shared
 // memory and written at the end.
-template <int D, int H, int R, bool FAST>
+// WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32)
+template <int D, int H, int R, bool FAST, bool WEIGHTED = false>
 __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const float* __restrict__ Wp, const __grid_constant__ FwdArgs A,
                                                                            float* __restrict__ partial) {
   typedef WideParams<D, H> L;
@@ -445,7 +446,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const
   bool alive = false;
   long long traj = 0;
   int kstar = 0, j = 0;
-  float Gk = 0.f;
+  float Gk = 0.f, mG = 0.f;        // WEIGHTED: -cS, -cG
   float lam[D];
   NoiseCache<D> nc;
   nc.reset();
@@ -466,6 +467,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const
           const int t = A.T[traj];
           if (t >= 0) {
             alive = true; kstar = t; j = t; Gk = ((const float*)A.G)[traj];
+            if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
             nc.reset();
 #pragma unroll
             for (int i = 0; i < D; ++i) lam[i] = 0.f;
@@ -509,7 +511,9 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const
         float v = 0.f;
         if (alive) {
           const bool incl = s_exact ? (j < kstar) : true;
-          v = (j < kstar ? uS[lane * RLSDE_MAX_D + i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+          if constexpr (WEIGHTED)
+            v = (j < kstar ? __fmul_rn(mG, uS[lane * RLSDE_MAX_D + i]) * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
+          else v = (j < kstar ? uS[lane * RLSDE_MAX_D + i] * A.dt_f : 0.f) - (incl ? Gk * dB[i] : 0.f) + A.sigma_f * A.dt_f * lam[i];
         }
         aS[lane * RLSDE_MAX_D + i] = v;
         gb3[i] += v;
@@ -688,7 +692,7 @@ static __global__ void wide_reduce_kernel(const float* __restrict__ partial, int
 // params_dev: WideParams<D, H> buffer in the caller's workspace (filled from params_host by the launcher)
 template <int D, int H>
 int launch_rollout_fwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, int sm_count, cudaStream_t stream);
-template <int D, int H>
+template <int D, int H, bool WEIGHTED = false>
 int launch_rollout_bwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, float scale, float* grad, float* partial,
                             size_t partial_bytes, int sm_count, cudaStream_t stream);
 

@@ -52,11 +52,11 @@ int launch_rollout_fwd_wide(const float* params_host, float* params_dev, const F
 #undef RLSDE_WIDE_FWD
 }
 
-template <int D, int H, int R, bool FAST>
+template <int D, int H, int R, bool FAST, bool WEIGHTED>
 static int launch_bwd_wide_variant(const float* params_dev, const FwdArgs& args, float scale, float* grad, float* partial,
                                    size_t partial_bytes, int sm_count, cudaStream_t stream) {
   constexpr int P = D * H + H + H * H + H + H * D + D;
-  auto kern = rollout_bwd_wide_kernel<D, H, R, FAST>;
+  auto kern = rollout_bwd_wide_kernel<D, H, R, FAST, WEIGHTED>;
   const size_t smem = wide_bwd_smem_bytes<H>();
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -76,7 +76,7 @@ static int launch_bwd_wide_variant(const float* params_dev, const FwdArgs& args,
   return (int)cudaGetLastError();
 }
 
-template <int D, int H>
+template <int D, int H, bool WEIGHTED>
 int launch_rollout_bwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, float scale, float* grad, float* partial,
                             size_t partial_bytes, int sm_count, cudaStream_t stream) {
   if (args.ckpt_every != 1) return (int)cudaErrorInvalidValue;
@@ -84,10 +84,10 @@ int launch_rollout_bwd_wide(const float* params_host, float* params_dev, const F
   int rc = wide_upload_params<D, H>(params_host, params_dev, fast, stream);
   if (rc != 0) return rc;
   const bool small = wide_small_tiles(args.K, sm_count);
-  if (small) return fast ? launch_bwd_wide_variant<D, H, 4, true>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream)
-                         : launch_bwd_wide_variant<D, H, 4, false>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream);
-  return fast ? launch_bwd_wide_variant<D, H, 8, true>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream)
-              : launch_bwd_wide_variant<D, H, 8, false>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream);
+  if (small) return fast ? launch_bwd_wide_variant<D, H, 4, true, WEIGHTED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream)
+                         : launch_bwd_wide_variant<D, H, 4, false, WEIGHTED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream);
+  return fast ? launch_bwd_wide_variant<D, H, 8, true, WEIGHTED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream)
+              : launch_bwd_wide_variant<D, H, 8, false, WEIGHTED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream);
 }
 
 }  // namespace rlsde
@@ -96,3 +96,7 @@ int launch_rollout_bwd_wide(const float* params_host, float* params_dev, const F
   template int rlsde::launch_rollout_fwd_wide<D, H>(const float*, float*, const rlsde::FwdArgs&, int, cudaStream_t);       \
   template int rlsde::launch_rollout_bwd_wide<D, H>(const float*, float*, const rlsde::FwdArgs&, float, float*, float*,   \
                                                     size_t, int, cudaStream_t);
+// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
+#define RLSDE_INSTANTIATE_WIDE_BWD_WEIGHTED(D, H)                                                                           \
+  template int rlsde::launch_rollout_bwd_wide<D, H, true>(const float*, float*, const rlsde::FwdArgs&, float, float*, float*, \
+                                                          size_t, int, cudaStream_t);

@@ -1,0 +1,6 @@
+// weighted reverse-pass kernels (rlsde_rollout_bwd_weighted) for d = 1, hidden width = 128: the wide-policy tile kernel
+// and the tcgen05 producer / consumer kernel
+#include "rollout_wide_inst.cuh"
+#include "rollout_umma_bwd_inst.cuh"
+RLSDE_INSTANTIATE_WIDE_BWD_WEIGHTED(1, 128)
+RLSDE_INSTANTIATE_UMMA_BWD_WEIGHTED(1, 128)

@@ -3,12 +3,14 @@
 Reference: rl_sde_is/reinforce_deterministic_core.py
   * ``sample_loss_vectorized(env, model, K)`` (:30-93)  -> one K1 launch (+ K2 when ``.backward()`` runs)
   * ``reinforce(env, ...)`` (:102-336)                  -> same arguments, same keys in the returned dict
+  * ``sample_returns_vectorized(env, model, K)``        -> (G, S) with a ``grad_fn``: train any loss over them
 
 Keyword-only extras (defaults = reference behaviour): ``noise`` (injected increments
 ``[n_steps, K, d]``), ``seed`` (Philox key), ``n_steps_lim``, ``tanh`` ('precise' | 'fast'),
 ``stoch_int`` ('reference' | 'exact'), ``ckpt_every``, ``device``, ``dist`` (shard the batch over a
 torch.distributed process group and all-reduce the packed gradient + statistics).
 """
+import dataclasses
 import time
 
 import numpy as np
@@ -65,6 +67,47 @@ def sample_loss_vectorized(env, model, K, *, noise=None, seed=None, n_steps_lim=
         raise L.RlsdeError(f"{int((T < 0).sum())} of {K} trajectories did not reach the target set within "
                            f"{lim} passes; raise n_steps_lim")
     return loss, out.G.cpu().numpy(), (T + 1).astype(np.float64)
+
+
+def sample_returns_vectorized(env, model, K, *, noise=None, seed=None, n_steps_lim=10**6, tanh="precise",
+                              stoch_int="reference", ckpt_every=None, device=None, kernel="auto"):
+    """Sample K trajectories under the policy and return ``(return_fht, stoch_int_fht, time_steps)``, so that any loss
+    over the returns G and the stochastic integrals S can be trained, as the reference allows by editing its surrogate
+    (:91).  ``return_fht`` and ``stoch_int_fht`` are float32 CUDA tensors [K] with a ``grad_fn``: a loss formed from them
+    on the GPU and ``.backward()``-ed fills ``p.grad`` of ``model.parameters()`` (accumulating, as autograd does) through
+    one weighted reverse pass (``rlsde_rollout_bwd_weighted``).  The derivative is the pathwise one along the sampled paths
+    with the hit passes held fixed, the derivative the reference's autograd graph takes.  S is S_ref, or S_exact with
+    ``stoch_int="exact"``; ``time_steps`` is ``np.float64[K]`` (= k*+1) as in ``sample_loss_vectorized``.
+
+    The log-variance loss, zero under the optimal control u* (where G - S_exact = log Psi(x0)):
+
+        G, S, _ = sample_returns_vectorized(env, model, K, stoch_int="exact")
+        torch.var(G - S, unbiased=False).backward()
+
+    ``sample_loss_vectorized``'s ``eff_loss`` is ``torch.mean(-G - G.detach() * S)`` over the reference S.
+    """
+    d, H = R.policy_shape(model)
+    if d != env.d:
+        raise L.RlsdeError(f"policy dimension {d} != env.d {env.d}")
+    env_c = R.env_struct(env, L.HIT_ALL_GE_LB)
+    mlp_c = L.make_mlp(d, H)
+    dev = R._cuda_device(device)
+    if noise is not None and not torch.is_tensor(noise):
+        noise = torch.as_tensor(np.ascontiguousarray(noise, dtype=np.float32))
+    if noise is not None:
+        noise = noise.to(device=dev, dtype=torch.float32).contiguous()
+    lim = int(n_steps_lim) if noise is None else min(int(n_steps_lim), int(noise.shape[0]))
+    if ckpt_every is None:
+        ckpt_every = R.choose_ckpt_every(int(K), d, lim, hidden=H)
+    opts = dict(seed=_next_seed(seed), n_steps_lim=n_steps_lim, noise=noise, tanh=tanh, stoch_int=stoch_int,
+                ckpt_every=ckpt_every, device=dev, kernel=kernel)
+    holder = {}
+    G, S = _ReturnsWithAux.apply(R.flat_parameters(model), env_c, mlp_c, int(K), opts, holder)
+    T = holder["out"].T.cpu().numpy()
+    if (T < 0).any():
+        raise L.RlsdeError(f"{int((T < 0).sum())} of {K} trajectories did not reach the target set within "
+                           f"{lim} passes; raise n_steps_lim")
+    return G, S, (T + 1).astype(np.float64)
 
 
 def _loss_and_grads_fused(env, model, K, *, noise=None, seed=None, n_steps_lim=10**6, tanh="precise", stoch_int="reference",
@@ -245,6 +288,33 @@ class _LossWithAux(torch.autograd.Function):
             g = ctx.dist.all_reduce_sum(g)
         g = g.to(grad_out.device) * grad_out.to(torch.float32)
         return g, None, None, None, None, None, None
+
+
+class _ReturnsWithAux(torch.autograd.Function):
+    """(G, S) [K] as differentiable functions of the flat policy parameters: forward launches the rollout kernel (with
+    state checkpoints), backward the weighted reverse kernel with the incoming gradients as per-trajectory coefficients,
+    grad = sum_k (dL/dG_k dG_k/dtheta + dL/dS_k dS_k/dtheta)."""
+
+    @staticmethod
+    def forward(ctx, flat_params, env_c, mlp_c, K, opts, holder):
+        params_host = flat_params.detach().to("cpu", torch.float32).contiguous().numpy()
+        out = R.rollout_forward(env_c, mlp_c, params_host, K, store_path=True, want_logw=False, **opts)
+        holder["out"] = out
+        # ctx keeps what the reverse pass reads (T, path, cfg), not the returned G and S: outputs reachable from their own
+        # grad_fn through ctx form a cycle that the garbage collector cannot see, and every rollout would stay allocated
+        ctx.fwd = dataclasses.replace(out, G=None, S=None, l2=None, logw=None)
+        ctx.env_c, ctx.mlp_c, ctx.params_host, ctx.opts = env_c, mlp_c, params_host, opts
+        ctx.param_device = flat_params.device
+        return out.G, out.S
+
+    @staticmethod
+    def backward(ctx, gG, gS):
+        fwd = ctx.fwd
+        coef = tuple(torch.zeros(fwd.T.shape, dtype=torch.float32, device=fwd.T.device) if g is None
+                     else g.to(fwd.T.device, torch.float32).contiguous() for g in (gG, gS))
+        g = R.rollout_backward(ctx.env_c, ctx.mlp_c, ctx.params_host, fwd, 1.0, noise=ctx.opts.get("noise"),
+                               device=ctx.opts.get("device"), coef=coef)
+        return g.to(ctx.param_device), None, None, None, None, None
 
 
 def reinforce(env, gamma=1., d_hidden_layer=256, n_layers=3, batch_size=1000, lr=1e-3, n_iterations=100, seed=None,

@@ -331,12 +331,23 @@ def rollout_transitions(env_c, mlp_c, params_host, K, *, seed=0, n_max=10**6, no
                        counts=counts, rollout=out)
 
 
-def rollout_backward(env_c, mlp_c, params_host, fwd: RolloutOut, loss_scale, *, noise=None, device=None, balance=True):
-    """K2: gradient of loss_scale * sum_k(-G_k - sg(G_k) S_k) w.r.t. the flat parameters (float32 CUDA tensor)."""
+def rollout_backward(env_c, mlp_c, params_host, fwd: RolloutOut, loss_scale, *, noise=None, device=None, balance=True,
+                     coef=None):
+    """K2: gradient of loss_scale * sum_k(-G_k - sg(G_k) S_k) w.r.t. the flat parameters (float32 CUDA tensor).
+
+    With ``coef=(coef_G, coef_S)`` (float32 CUDA tensors [K] on the rollout's device) the gradient is that of
+    loss_scale * sum_k (coef_G[k] G_k + coef_S[k] S_k) instead (rlsde_rollout_bwd_weighted; unfinished trajectories
+    contribute 0)."""
     lib = L.load()
     dev = _cuda_device(device)
     if fwd.path is None:
         raise L.RlsdeError("the forward rollout must be run with store_path=True")
+    if coef is not None:
+        coef = tuple(coef)
+        K = fwd.T.numel()
+        if len(coef) != 2 or any(not isinstance(c, torch.Tensor) or c.device != dev or c.dtype != torch.float32
+                                 or not c.is_contiguous() or c.shape != (K,) for c in coef):
+            raise L.RlsdeError(f"coef must be (coef_G, coef_S), contiguous float32 tensors [{K}] on {dev}")
     params_host = np.ascontiguousarray(params_host, dtype=np.float32)
     grad = torch.empty(int(lib.rlsde_param_count(mlp_c)), dtype=torch.float32, device=dev)
     ws = _workspace(dev, 0, mlp_c)
@@ -347,9 +358,14 @@ def rollout_backward(env_c, mlp_c, params_host, fwd: RolloutOut, loss_scale, *, 
         thread_path = (fwd.cfg.flags & L.F_KERNEL_THREAD) or not ((fwd.cfg.flags & L.F_KERNEL_WARP) or fwd.T.numel() <= 16 * n_sm)
         order = torch.argsort(fwd.T, descending=True, stable=True) if balance and thread_path and fwd.T.numel() > 32 else None
         stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib.rlsde_rollout_bwd(env_c, mlp_c, params_host.ctypes.data, fwd.cfg, _ptr(noise), _ptr(fwd.G), _ptr(fwd.T),
-                                   _ptr(fwd.path), _ptr(order), float(loss_scale), _ptr(grad), _ptr(ws), ws.numel(), stream)
-    L.check(rc, "rlsde_rollout_bwd")
+        if coef is None:
+            rc = lib.rlsde_rollout_bwd(env_c, mlp_c, params_host.ctypes.data, fwd.cfg, _ptr(noise), _ptr(fwd.G), _ptr(fwd.T),
+                                       _ptr(fwd.path), _ptr(order), float(loss_scale), _ptr(grad), _ptr(ws), ws.numel(), stream)
+        else:
+            rc = lib.rlsde_rollout_bwd_weighted(env_c, mlp_c, params_host.ctypes.data, fwd.cfg, _ptr(noise), _ptr(coef[0]),
+                                                _ptr(coef[1]), _ptr(fwd.T), _ptr(fwd.path), _ptr(order), float(loss_scale),
+                                                _ptr(grad), _ptr(ws), ws.numel(), stream)
+    L.check(rc, "rlsde_rollout_bwd_weighted" if coef is not None else "rlsde_rollout_bwd")
     return grad
 
 
