@@ -279,6 +279,33 @@ int rlsde_rollout_bwd_weighted(const rlsde_env* env, const rlsde_mlp* mlp, const
                                float* grad_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /*
+ * The ragged checkpoint store: memory in proportion to the passes the trajectories run, not to the pass budget.  With
+ * C = cfg->ckpt_every (1 .. 32), the checkpoints of trajectory t are X_{cC} for c = 0 .. floor(T_t / C), stored as
+ * float[d] rows path_dev[(path_base_dev[t] + c) * d ...]; path_base_dev is int64[K + 1], nondecreasing, and trajectory t
+ * owns rows [path_base_dev[t], path_base_dev[t + 1]).  A trajectory with T = -1 is given 0 rows.  The lengths are only
+ * known after a rollout: run one first with the same cfg (the counter-based noise makes the second rollout identical;
+ * the same entry point with a base of K + 1 zeros stores nothing and runs the same kernels), form the base as the
+ * exclusive prefix sum of (T >= 0 ? T / C + 1 : 0) with the total in entry K, then call rlsde_rollout_fwd_ragged.
+ *
+ * rlsde_rollout_fwd_ragged: rlsde_rollout_fwd with RLSDE_F_STORE_PATH implied and cfg->ckpt_stride not read; flags,
+ * kernel selection, outputs and the statistics record are rlsde_rollout_fwd's.  A checkpoint outside a trajectory's rows
+ * is not written.  rlsde_rollout_bwd_ragged: rlsde_rollout_bwd_weighted over the ragged store (same semantics, kernel
+ * selection, workspace and refusals; with coefficients (-1, -G) it returns rlsde_rollout_bwd's gradient); a trajectory
+ * whose rows do not hold checkpoints 0 .. floor(T_t / C) contributes 0, so nothing outside its rows is read.
+ * Refusals, before any device work: RLSDE_F_HIT_BRIDGE, ckpt_every outside 1 .. 32 (rlsde_rollout_fwd_ragged), a NULL
+ * path_base_dev or path_dev -> RLSDE_ERR_INVALID_ARG; RLSDE_F_STATE_F64 -> RLSDE_ERR_UNSUPPORTED.
+ */
+int rlsde_rollout_fwd_ragged(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                             const rlsde_rollout_cfg* cfg, const float* noise_dev, const int64_t* path_base_dev,
+                             void* G_dev, void* S_dev, int32_t* T_dev, float* path_dev, double* stats_dev,
+                             void* workspace_dev, size_t workspace_bytes, void* stream);
+int rlsde_rollout_bwd_ragged(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                             const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* coef_G_dev,
+                             const float* coef_S_dev, const int32_t* T_dev, const int64_t* path_base_dev,
+                             const float* path_dev, const int64_t* order_dev, double loss_scale, float* grad_dev,
+                             void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/*
  * One REINFORCE iteration with everything resident on the device (reinforce_deterministic_core.py:232-243:
  * zero_grad -> sample_loss_vectorized -> backward -> Adam step), for the latency-bound small-batch regime
  * (K <= 16 x SMs, hidden width 32; RLSDE_ERR_UNSUPPORTED otherwise): the policy is read from theta_dev (float[P],

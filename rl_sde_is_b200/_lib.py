@@ -41,7 +41,7 @@ EXPORTED_SYMBOLS = [
     "rlsde_tables", "rlsde_tables_colsum", "rlsde_env_step", "rlsde_noise_fill",
     "rlsde_dp_scratch_bytes", "rlsde_dp_sweep", "rlsde_dp_rowmax", "rlsde_rollout_transitions", "rlsde_launch_count", "rlsde_reinforce_step",
     "rlsde_reinforce_rollout", "rlsde_reinforce_apply", "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table",
-    "rlsde_rollout_bwd_weighted",
+    "rlsde_rollout_bwd_weighted", "rlsde_rollout_fwd_ragged", "rlsde_rollout_bwd_ragged",
 ]
 
 
@@ -116,6 +116,10 @@ def load():
                                       vp, vp, vp, vp, vp, dbl, vp, vp, C.c_size_t, vp]
     lib.rlsde_rollout_bwd_weighted.argtypes = [C.POINTER(RlsdeEnv), C.POINTER(RlsdeMlp), vp, C.POINTER(RlsdeRolloutCfg),
                                                vp, vp, vp, vp, vp, vp, dbl, vp, vp, C.c_size_t, vp]
+    lib.rlsde_rollout_fwd_ragged.argtypes = [C.POINTER(RlsdeEnv), C.POINTER(RlsdeMlp), vp, C.POINTER(RlsdeRolloutCfg),
+                                             vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
+    lib.rlsde_rollout_bwd_ragged.argtypes = [C.POINTER(RlsdeEnv), C.POINTER(RlsdeMlp), vp, C.POINTER(RlsdeRolloutCfg),
+                                             vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp, C.c_size_t, vp]
     lib.rlsde_reduce_stats.argtypes = [i64, i64, u32, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]
     lib.rlsde_tables.argtypes = [vp, i64, vp, i64, vp, i64, dbl, dbl, dbl, dbl, dbl, dbl, i64, i64, vp, vp, i32, dbl, vp]
     lib.rlsde_tables_colsum.argtypes = [vp, i64, i64, i64, vp, vp]
@@ -129,7 +133,8 @@ def load():
     for name in ("rlsde_device_info", "rlsde_supported", "rlsde_rollout_fwd", "rlsde_rollout_bwd", "rlsde_reduce_stats",
                  "rlsde_tables", "rlsde_tables_colsum", "rlsde_env_step", "rlsde_noise_fill", "rlsde_dp_sweep", "rlsde_dp_rowmax",
                  "rlsde_rollout_transitions", "rlsde_reinforce_step", "rlsde_reinforce_rollout", "rlsde_reinforce_apply",
-                 "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table", "rlsde_rollout_bwd_weighted"):
+                 "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table", "rlsde_rollout_bwd_weighted",
+                 "rlsde_rollout_fwd_ragged", "rlsde_rollout_bwd_ragged"):
         getattr(lib, name).restype = C.c_int
     _lib = lib
     return lib

@@ -125,7 +125,9 @@ static void fill_env(const rlsde_env* env, FwdArgs& A) {
   A.hit_rule = env->hit_rule;
 }
 
-static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A) {
+// ragged: the checkpoints go to the ragged store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged), whose size the
+// caller has fitted to the trajectories: cfg->ckpt_stride is not read
+static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A, bool ragged = false) {
   if (!cfg || cfg->K < 0 || cfg->n_steps_lim < 1 || cfg->n_steps_lim > 2000000000LL) return RLSDE_ERR_INVALID_ARG;
   if (cfg->traj_offset < 0) return RLSDE_ERR_INVALID_ARG;
   if ((cfg->flags & RLSDE_F_NOISE_INJECTED) && cfg->noise_steps < 1) return RLSDE_ERR_INVALID_ARG;
@@ -136,7 +138,7 @@ static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A) {
   A.K_global = cfg->K_global > 0 ? cfg->K_global : cfg->K;
   A.seed = cfg->seed; A.n_steps_lim = cfg->n_steps_lim; A.noise_steps = cfg->noise_steps;
   A.flags = cfg->flags; A.ckpt_every = cfg->ckpt_every > 0 ? cfg->ckpt_every : 1; A.ckpt_stride = cfg->ckpt_stride;
-  if (cfg->flags & RLSDE_F_STORE_PATH) {
+  if ((cfg->flags & RLSDE_F_STORE_PATH) && !ragged) {
     // the kernels write path[(traj * ckpt_stride + k / ckpt_every) * d] for every pass k they execute
     const long long lim_eff = (cfg->flags & RLSDE_F_NOISE_INJECTED) && cfg->noise_steps < cfg->n_steps_lim ? cfg->noise_steps
                                                                                                              : cfg->n_steps_lim;
@@ -257,11 +259,14 @@ struct TransitionOut {
   unsigned char* done;
 };
 
+// RAGGED: rlsde_rollout_fwd_ragged (checkpoints into the ragged store at path_base; no transition stream)
+extern "C++" {
+template <bool RAGGED>
 static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
                             const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* policy_opt_dev,
                             void* G_dev, void* S_dev, int32_t* T_dev, void* l2_dev, void* logw_dev, float* path_dev,
-                            double* stats_dev, const TransitionOut& tr, void* workspace_dev, size_t workspace_bytes,
-                            void* stream_) {
+                            double* stats_dev, const TransitionOut& tr, const long long* path_base, void* workspace_dev,
+                            size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   int rc = check_env_mlp(env, mlp);
   if (rc != RLSDE_OK) return rc;
@@ -270,7 +275,16 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   FwdArgs A;
   memset(&A, 0, sizeof(A));
   fill_env(env, A);
-  if ((rc = fill_cfg(cfg, A)) != RLSDE_OK) return rc;
+  if ((rc = fill_cfg(cfg, A, RAGGED)) != RLSDE_OK) return rc;
+  if (RAGGED) {
+    // the store exists for the reverse pass, so it takes that pass's conditions: a float32 state, no projection (below)
+    // and at most BWD_MAX_SEG passes per checkpoint
+    if (!path_base || !path_dev || tr.base) return RLSDE_ERR_INVALID_ARG;
+    if (cfg->ckpt_every < 1 || cfg->ckpt_every > BWD_MAX_SEG) return RLSDE_ERR_INVALID_ARG;
+    A.flags |= RLSDE_F_STORE_PATH;
+    if (A.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;
+    if (A.flags & RLSDE_F_STATE_F64) return RLSDE_ERR_UNSUPPORTED;
+  }
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
   if ((A.flags & RLSDE_F_STORE_PATH) && !path_dev) return RLSDE_ERR_INVALID_ARG;
   if (policy_opt_dev && (cfg->n_grid < 1 || !(cfg->grid_h > 0) || env->d != 1)) return RLSDE_ERR_INVALID_ARG;
@@ -284,6 +298,7 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   A.G = G_dev; A.S = S_dev; A.T = T_dev; A.l2 = l2_dev; A.logw = logw_dev; A.path = path_dev;
   A.tr_base = tr.base; A.tr_state = tr.state; A.tr_action = tr.action; A.tr_reward = tr.reward;
   A.tr_next = tr.next_state; A.tr_done = tr.done;
+  if (RAGGED) A.path_base = path_base;                  // shares tr_base's field: the ragged kernels have no stream
   if (tr.base) A.flags = (A.flags & ~RLSDE_F_KERNEL_WARP) | RLSDE_F_KERNEL_THREAD;   // the stream lives in the throughput kernel
   A.counter = (unsigned long long*)workspace_dev;
   A.q_ctrl = (unsigned long long*)workspace_dev;
@@ -309,12 +324,12 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
     if (use_umma) {
 #define X(D_, H_)                                                                                                          \
   if (env->d == D_ && mlp->d_hidden == H_)                                                                                 \
-    lrc = launch_rollout_fwd_umma<D_, H_>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A, sm, stream);
+    lrc = launch_rollout_fwd_umma<D_, H_, RAGGED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A, sm, stream);
       RLSDE_UMMA_FWD_SHAPES(X)
 #undef X
     } else {
 #define X(D_, H_) \
-  if (env->d == D_ && mlp->d_hidden == H_) lrc = launch_rollout_fwd_wide<D_, H_>(params_host, ws_wide_params(workspace_dev), A, sm, stream);
+  if (env->d == D_ && mlp->d_hidden == H_) lrc = launch_rollout_fwd_wide<D_, H_, RAGGED>(params_host, ws_wide_params(workspace_dev), A, sm, stream);
       RLSDE_WIDE_SHAPES(X)
 #undef X
     }
@@ -354,7 +369,7 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
       if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
 #define X(D_, H_)                                                                                                          \
   if (env->d == D_ && mlp->d_hidden == H_)                                                                                 \
-    lrc = launch_rollout_fwd_umma<D_, H_>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A, sm, stream);
+    lrc = launch_rollout_fwd_umma<D_, H_, RAGGED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A, sm, stream);
       RLSDE_UMMA_NARROW_SHAPES(X)
 #undef X
       if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd (tensor) launch");
@@ -398,8 +413,8 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   }
 #define X(D_, H_)                                                                              \
   if (env->d == D_ && mlp->d_hidden == H_)                                                     \
-    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_fwd_warp<D_>(params_host, nullptr, A, sm, stream) \
-                                      : launch_rollout_fwd<D_, H_>(params_host, A, sm, stream);
+    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_fwd_warp<D_, RAGGED>(params_host, nullptr, A, sm, stream) \
+                                      : launch_rollout_fwd<D_, H_, RAGGED>(params_host, A, sm, stream);
   RLSDE_SHAPES(X)
 #undef X
   if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd launch");
@@ -407,7 +422,7 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
     // the trajectories K1 left in the ring (none if it ran without one): one warp each, K1's arithmetic
     lrc = -1;
 #define X(D_, H_) \
-  if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H) lrc = launch_rollout_fwd_warp_resume<D_>(params_host, A, sm, stream);
+  if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H) lrc = launch_rollout_fwd_warp_resume<D_, RAGGED>(params_host, A, sm, stream);
     RLSDE_SHAPES(X)
 #undef X
     if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd resume launch");
@@ -422,14 +437,24 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   }
   return RLSDE_OK;
 }
+}  // extern "C++"
 
 int rlsde_rollout_fwd(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
                       const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* policy_opt_dev,
                       void* G_dev, void* S_dev, int32_t* T_dev, void* l2_dev, void* logw_dev, float* path_dev,
                       double* stats_dev, void* workspace_dev, size_t workspace_bytes, void* stream_) {
   const TransitionOut none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  return rollout_fwd_impl(env, mlp, params_host, cfg, noise_dev, policy_opt_dev, G_dev, S_dev, T_dev, l2_dev, logw_dev,
-                          path_dev, stats_dev, none, workspace_dev, workspace_bytes, stream_);
+  return rollout_fwd_impl<false>(env, mlp, params_host, cfg, noise_dev, policy_opt_dev, G_dev, S_dev, T_dev, l2_dev, logw_dev,
+                                 path_dev, stats_dev, none, nullptr, workspace_dev, workspace_bytes, stream_);
+}
+
+int rlsde_rollout_fwd_ragged(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                             const rlsde_rollout_cfg* cfg, const float* noise_dev, const int64_t* path_base_dev,
+                             void* G_dev, void* S_dev, int32_t* T_dev, float* path_dev, double* stats_dev,
+                             void* workspace_dev, size_t workspace_bytes, void* stream_) {
+  const TransitionOut none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  return rollout_fwd_impl<true>(env, mlp, params_host, cfg, noise_dev, nullptr, G_dev, S_dev, T_dev, nullptr, nullptr, path_dev,
+                                stats_dev, none, (const long long*)path_base_dev, workspace_dev, workspace_bytes, stream_);
 }
 
 int rlsde_rollout_fwd_table(const rlsde_env* env, const float* u_table_dev, const rlsde_rollout_cfg* cfg,
@@ -481,18 +506,20 @@ int rlsde_rollout_transitions(const rlsde_env* env, const rlsde_mlp* mlp, const 
   if (!slot_base_dev || !states_dev || !actions_dev || !rewards_dev || !next_states_dev || !done_dev) return RLSDE_ERR_INVALID_ARG;
   if (cfg && (cfg->flags & RLSDE_F_STORE_PATH)) return RLSDE_ERR_INVALID_ARG;
   const TransitionOut tr = {(const long long*)slot_base_dev, states_dev, actions_dev, rewards_dev, next_states_dev, done_dev};
-  return rollout_fwd_impl(env, mlp, params_host, cfg, noise_dev, nullptr, G_dev, S_dev, T_dev, nullptr, nullptr, nullptr,
-                          stats_dev, tr, workspace_dev, workspace_bytes, stream_);
+  return rollout_fwd_impl<false>(env, mlp, params_host, cfg, noise_dev, nullptr, G_dev, S_dev, T_dev, nullptr, nullptr, nullptr,
+                                 stats_dev, tr, nullptr, workspace_dev, workspace_bytes, stream_);
 }
 
 // WEIGHTED = false: rlsde_rollout_bwd (cS_dev = G, cG_dev unused); true: rlsde_rollout_bwd_weighted.  The weighted kernels
 // read cS from FwdArgs::G and cG from FwdArgs::S (rollout_bwd.cuh, the comment above em_step_f32).
+// RAGGED (with WEIGHTED only): rlsde_rollout_bwd_ragged, the checkpoints come from the ragged store at path_base.
 extern "C++" {
-template <bool WEIGHTED>
+template <bool WEIGHTED, bool RAGGED = false>
 static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host, const rlsde_rollout_cfg* cfg,
                             const float* noise_dev, const float* cS_dev, const float* cG_dev, const int32_t* T_dev,
                             const float* path_dev, const int64_t* order_dev, double loss_scale, float* grad_dev,
-                            void* workspace_dev, size_t workspace_bytes, void* stream_) {
+                            void* workspace_dev, size_t workspace_bytes, void* stream_, const long long* path_base = nullptr) {
+  static_assert(WEIGHTED || !RAGGED, "the ragged reverse pass is the weighted one");
   cudaStream_t stream = (cudaStream_t)stream_;
   int rc = check_env_mlp(env, mlp);
   if (rc != RLSDE_OK) return rc;
@@ -502,7 +529,11 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   FwdArgs A;
   memset(&A, 0, sizeof(A));
   fill_env(env, A);
-  if ((rc = fill_cfg(cfg, A)) != RLSDE_OK) return rc;
+  if ((rc = fill_cfg(cfg, A, RAGGED)) != RLSDE_OK) return rc;
+  if (RAGGED) {
+    if (!path_base) return RLSDE_ERR_INVALID_ARG;
+    A.flags |= RLSDE_F_STORE_PATH;                                   // implied, as in rlsde_rollout_fwd_ragged
+  }
   if (A.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;   // no reverse pass through the projection
   if (A.flags & RLSDE_F_STATE_F64) return RLSDE_ERR_UNSUPPORTED;   // the reference differentiates the f32 torch path only
   if (!(A.flags & RLSDE_F_STORE_PATH)) return RLSDE_ERR_INVALID_ARG;
@@ -512,6 +543,7 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   A.G = (void*)cS_dev; A.T = (int*)T_dev; A.path = (float*)path_dev;
   if (WEIGHTED) A.S = (void*)cG_dev;
   A.order = (const long long*)order_dev;
+  if (RAGGED) A.path_base = path_base;
   A.counter = (unsigned long long*)workspace_dev;
   int sm = 0;
   if ((rc = device_sm_count(&sm)) != RLSDE_OK) return rc;
@@ -531,7 +563,7 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
       uint8_t* scratch = (uint8_t*)workspace_dev + ws_fixed_bytes();
 #define X(D_, H_)                                                                                                        \
   if (env->d == D_ && mlp->d_hidden == H_)                                                                               \
-    lrc = launch_rollout_bwd_umma<D_, H_, WEIGHTED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A,   \
+    lrc = launch_rollout_bwd_umma<D_, H_, WEIGHTED, RAGGED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A,   \
                                           (float)loss_scale, grad_dev, scratch, workspace_bytes - ws_fixed_bytes(), sm, stream);
       RLSDE_UMMA_SHAPES(X)
 #undef X
@@ -540,7 +572,7 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
     }
 #define X(D_, H_)                                                                                                       \
   if (env->d == D_ && mlp->d_hidden == H_)                                                                              \
-    lrc = launch_rollout_bwd_wide<D_, H_, WEIGHTED>(params_host, ws_wide_params(workspace_dev), A, (float)loss_scale, grad_dev, partial, \
+    lrc = launch_rollout_bwd_wide<D_, H_, WEIGHTED, RAGGED>(params_host, ws_wide_params(workspace_dev), A, (float)loss_scale, grad_dev, partial, \
                                           bwd_partial_main_bytes(), sm, stream);
     RLSDE_WIDE_SHAPES(X)
 #undef X
@@ -584,7 +616,7 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
     }
 #define X(D_, H_)                                                                                                   \
   if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H)                                                          \
-    lrc = launch_rollout_bwd_warp<D_, WEIGHTED>(params_host, nullptr, Along, (float)loss_scale, grad_dev, partial_aux, sm, s_long);
+    lrc = launch_rollout_bwd_warp<D_, WEIGHTED, RAGGED>(params_host, nullptr, Along, (float)loss_scale, grad_dev, partial_aux, sm, s_long);
     RLSDE_SHAPES(X)
 #undef X
     if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd (long trajectories) launch");
@@ -596,9 +628,9 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   }
 #define X(D_, H_)                                                                                                          \
   if (env->d == D_ && mlp->d_hidden == H_ && Abulk.K > 0)                                                                  \
-    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_bwd_warp<D_, WEIGHTED>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev, partial, sm, stream) \
-          : (use_mma && H_ == MMA_H)  ? launch_rollout_bwd_mma<D_, WEIGHTED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream, join)      \
-                                      : launch_rollout_bwd<D_, H_, WEIGHTED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream);
+    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_bwd_warp<D_, WEIGHTED, RAGGED>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev, partial, sm, stream) \
+          : (use_mma && H_ == MMA_H)  ? launch_rollout_bwd_mma<D_, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream, join)      \
+                                      : launch_rollout_bwd<D_, H_, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream);
   RLSDE_SHAPES(X)
 #undef X
   if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd launch");
@@ -620,6 +652,16 @@ int rlsde_rollout_bwd_weighted(const rlsde_env* env, const rlsde_mlp* mlp, const
                                double loss_scale, float* grad_dev, void* workspace_dev, size_t workspace_bytes, void* stream_) {
   return rollout_bwd_impl<true>(env, mlp, params_host, cfg, noise_dev, coef_S_dev, coef_G_dev, T_dev, path_dev, order_dev, loss_scale,
                                 grad_dev, workspace_dev, workspace_bytes, stream_);
+}
+
+int rlsde_rollout_bwd_ragged(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
+                             const rlsde_rollout_cfg* cfg, const float* noise_dev, const float* coef_G_dev,
+                             const float* coef_S_dev, const int32_t* T_dev, const int64_t* path_base_dev, const float* path_dev,
+                             const int64_t* order_dev, double loss_scale, float* grad_dev, void* workspace_dev,
+                             size_t workspace_bytes, void* stream_) {
+  return rollout_bwd_impl<true, true>(env, mlp, params_host, cfg, noise_dev, coef_S_dev, coef_G_dev, T_dev, path_dev, order_dev,
+                                      loss_scale, grad_dev, workspace_dev, workspace_bytes, stream_,
+                                      (const long long*)path_base_dev);
 }
 
 // rollout + statistics + reverse pass of one device-resident REINFORCE iteration (everything but the parameter update)

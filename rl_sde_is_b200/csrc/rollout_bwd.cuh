@@ -153,7 +153,8 @@ constexpr int kBwdUnroll = RLSDE_BWD_UNROLL;
 #endif
 
 // Per-warp partial gradient layout = state_dict order: W1 (H,D), b1 (H), W2 (H,H), b2 (H), W3 (D,H), b3 (D)
-template <int D, int H, bool FAST, bool WEIGHTED = false>
+// RAGGED: the checkpoints come from the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, int H, bool FAST, bool WEIGHTED = false, bool RAGGED = false>
 __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kernel(const __grid_constant__ MlpConst<D, H> W,
                                                           const __grid_constant__ FwdArgs A, float* __restrict__ partial) {
   static_assert(H == 32 || H == 64, "column-per-lane accumulation needs H in {32, 64}");
@@ -209,7 +210,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
       slot += n_lanes;
       traj = A.order ? A.order[slot] : slot;
       const int t = A.T[traj];
-      if (t >= 0) {
+      if (t >= 0 && ckpt_covered<RAGGED>(A, traj, t)) {
         alive = true; kstar = t; seg = t / C; Gk = ((const float*)A.G)[traj];
         if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
         nc.reset();
@@ -226,7 +227,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
     // share one copy of the policy-forward code; the branch on the phase is warp-uniform.
     {
 #pragma unroll
-      for (int i = 0; i < D; ++i) xs[0][i] = alive ? A.path[((long long)traj * A.ckpt_stride + seg) * D + i] : A.x0_f[i];
+      for (int i = 0; i < D; ++i) xs[0][i] = alive ? A.path[ckpt_slot<RAGGED>(A, traj, seg) * D + i] : A.x0_f[i];
     }
     for (int t = 0; t < 2 * C - 1; ++t) {
       const bool phase_a = t < C - 1;
@@ -446,7 +447,7 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MIN_BLOCKS(D)) rollout_bwd_kern
   if (lane < D) ob3[lane] = (float)gb3;
 }
 
-template <int D, int H, bool WEIGHTED = false>
+template <int D, int H, bool WEIGHTED = false, bool RAGGED = false>
 int launch_rollout_bwd(const float* params_host, const FwdArgs& args, float scale, float* grad, float* partial,
                        int sm_count, cudaStream_t stream);
 

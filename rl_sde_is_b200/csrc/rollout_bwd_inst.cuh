@@ -15,7 +15,7 @@ static __global__ void bwd_reduce_kernel(const float* __restrict__ partial, int 
   grad[p] = accumulate ? grad[p] + g : g;
 }
 
-template <int D, int H, bool FAST, bool WEIGHTED>
+template <int D, int H, bool FAST, bool WEIGHTED, bool RAGGED>
 static int launch_bwd_variant(const float* params_host, const FwdArgs& args, float scale, float* grad, float* partial,
                               int sm_count, cudaStream_t stream) {
   constexpr int P = D * H + H + H * H + H + H * D + D;
@@ -23,7 +23,7 @@ static int launch_bwd_variant(const float* params_host, const FwdArgs& args, flo
   if (args.ckpt_every > BWD_MAX_SEG) return (int)cudaErrorInvalidValue;
   MlpConst<D, H> W;
   pack_mlp_const<D, H>(params_host, FAST, W);
-  auto kern = rollout_bwd_kernel<D, H, FAST, WEIGHTED>;
+  auto kern = rollout_bwd_kernel<D, H, FAST, WEIGHTED, RAGGED>;
   int block = 128;
   long long grid;
   const size_t smem_per_warp = (size_t)(2 * tile_floats<H, bwd_tiles_padded(D)>() + 64 * D) * sizeof(float);
@@ -52,11 +52,11 @@ static int launch_bwd_variant(const float* params_host, const FwdArgs& args, flo
   return (int)cudaGetLastError();
 }
 
-template <int D, int H, bool WEIGHTED>
+template <int D, int H, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd(const float* params_host, const FwdArgs& args, float scale, float* grad, float* partial,
                        int sm_count, cudaStream_t stream) {
-  return (args.flags & RLSDE_F_TANH_FAST) ? launch_bwd_variant<D, H, true, WEIGHTED>(params_host, args, scale, grad, partial, sm_count, stream)
-                                          : launch_bwd_variant<D, H, false, WEIGHTED>(params_host, args, scale, grad, partial, sm_count, stream);
+  return (args.flags & RLSDE_F_TANH_FAST) ? launch_bwd_variant<D, H, true, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream)
+                                          : launch_bwd_variant<D, H, false, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream);
 }
 
 }  // namespace rlsde
@@ -66,3 +66,6 @@ int launch_rollout_bwd(const float* params_host, const FwdArgs& args, float scal
 // the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
 #define RLSDE_INSTANTIATE_BWD_WEIGHTED(D, H) \
   template int rlsde::launch_rollout_bwd<D, H, true>(const float*, const rlsde::FwdArgs&, float, float*, float*, int, cudaStream_t);
+// the weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged), in translation units of its own
+#define RLSDE_INSTANTIATE_BWD_RAGGED(D, H) \
+  template int rlsde::launch_rollout_bwd<D, H, true, true>(const float*, const rlsde::FwdArgs&, float, float*, float*, int, cudaStream_t);

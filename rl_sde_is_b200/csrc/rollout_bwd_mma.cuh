@@ -225,7 +225,8 @@ constexpr size_t bwd_mma_dyn_smem(int D, int block) {
 // Per-warp partial gradient layout = state_dict order (W1 (H,D), b1, W2 (H,H), b2, W3 (D,H), b3), doubles.
 // WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32); the per-pass scale window below adapts
 // to their magnitude as it does to G's
-template <int D, bool FAST, bool WEIGHTED = false>
+// RAGGED: the checkpoints come from the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, bool FAST, bool WEIGHTED = false, bool RAGGED = false>
 __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_mma_kernel(const __grid_constant__ MlpConst<D, MMA_H> W,
                                                                   const __grid_constant__ FwdArgs A,
                                                                   const __grid_constant__ BwdMmaWeights F,
@@ -431,12 +432,12 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_
       slot += n_lanes;
       traj = A.order ? A.order[slot] : slot;
       const int t = A.T[traj];
-      if (t >= 0) {
+      if (t >= 0 && ckpt_covered<RAGGED>(A, traj, t)) {
         alive = true; kstar = t; seg = t / C; Gk = ((const float*)A.G)[traj];
         if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
         nc.reset();
 #pragma unroll
-        for (int i = 0; i < D; ++i) { lam[i] = 0.f; xck[i] = A.path[((long long)traj * A.ckpt_stride + seg) * D + i]; }
+        for (int i = 0; i < D; ++i) { lam[i] = 0.f; xck[i] = A.path[ckpt_slot<RAGGED>(A, traj, seg) * D + i]; }
       }
     }
     if (!__any_sync(FULL, alive)) break;
@@ -446,7 +447,9 @@ __global__ void __launch_bounds__(128, RLSDE_BWD_MMA_MIN_BLOCKS(D)) rollout_bwd_
     for (int i = 0; i < D; ++i) xs[0][i] = xck[i];
     if (alive && seg > 0) {
 #pragma unroll
-      for (int i = 0; i < D; ++i) xck[i] = A.path[((long long)traj * A.ckpt_stride + seg - 1) * D + i];
+      for (int i = 0; i < D; ++i)
+        xck[i] = RAGGED ? A.path[ckpt_slot<RAGGED>(A, traj, seg - 1) * D + i]
+                        : A.path[((long long)traj * A.ckpt_stride + seg - 1) * D + i];     // (the dense kernels' code as it was)
     }
 
     for (int t = 0; t < 2 * C - 1; ++t) {
@@ -904,7 +907,7 @@ static __global__ void bwd_reduce64_kernel(const double* __restrict__ partial, i
 
 // join: if non-null, the stream waits for this event between the rollout kernel and the reduction that adds into `grad`
 // (the warp-per-trajectory kernel working on the longest trajectories on a second stream writes `grad` first)
-template <int D, bool WEIGHTED = false>
+template <int D, bool WEIGHTED = false, bool RAGGED = false>
 int launch_rollout_bwd_mma(const float* params_host, const FwdArgs& args, float scale, float* grad, void* partial,
                            int sm_count, cudaStream_t stream, cudaEvent_t join);
 

@@ -6,7 +6,7 @@
 
 namespace rlsde {
 
-template <int D, bool FAST, bool WEIGHTED>
+template <int D, bool FAST, bool WEIGHTED, bool RAGGED>
 static int launch_bwd_mma_variant(const float* params_host, const FwdArgs& args, float scale, float* grad, void* partial,
                                   int sm_count, cudaStream_t stream, cudaEvent_t join) {
   constexpr int P = D * MMA_H + MMA_H + MMA_H * MMA_H + MMA_H + MMA_H * D + D;
@@ -18,7 +18,7 @@ static int launch_bwd_mma_variant(const float* params_host, const FwdArgs& args,
   pack_bwd_mma_weights<D>(W, F);
   typename BwdMmaSmallSel<D>::type FS;
   pack_bwd_mma_small<D>(W, FAST, FS);
-  auto kern = rollout_bwd_mma_kernel<D, FAST, WEIGHTED>;
+  auto kern = rollout_bwd_mma_kernel<D, FAST, WEIGHTED, RAGGED>;
   int block = 128;
   long long grid;
   // d > 4: fragment table of the d-sized products + per-warp staging rows; accumulator tiles (rollout_bwd_mma.cuh)
@@ -47,11 +47,11 @@ static int launch_bwd_mma_variant(const float* params_host, const FwdArgs& args,
   return (int)cudaGetLastError();
 }
 
-template <int D, bool WEIGHTED>
+template <int D, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd_mma(const float* params_host, const FwdArgs& args, float scale, float* grad, void* partial,
                            int sm_count, cudaStream_t stream, cudaEvent_t join) {
-  return (args.flags & RLSDE_F_TANH_FAST) ? launch_bwd_mma_variant<D, true, WEIGHTED>(params_host, args, scale, grad, partial, sm_count, stream, join)
-                                          : launch_bwd_mma_variant<D, false, WEIGHTED>(params_host, args, scale, grad, partial, sm_count, stream, join);
+  return (args.flags & RLSDE_F_TANH_FAST) ? launch_bwd_mma_variant<D, true, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream, join)
+                                          : launch_bwd_mma_variant<D, false, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream, join);
 }
 
 }  // namespace rlsde
@@ -60,3 +60,6 @@ int launch_rollout_bwd_mma(const float* params_host, const FwdArgs& args, float 
   template int rlsde::launch_rollout_bwd_mma<D>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, cudaStream_t, cudaEvent_t);
 #define RLSDE_INSTANTIATE_BWD_MMA_WEIGHTED(D) \
   template int rlsde::launch_rollout_bwd_mma<D, true>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, cudaStream_t, cudaEvent_t);
+// the weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged), in translation units of its own
+#define RLSDE_INSTANTIATE_BWD_MMA_RAGGED(D) \
+  template int rlsde::launch_rollout_bwd_mma<D, true, true>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, cudaStream_t, cudaEvent_t);

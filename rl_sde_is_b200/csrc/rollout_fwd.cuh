@@ -81,7 +81,13 @@ struct FwdArgs {
                                  // have max_i |x_i| <= this (fwd_mma_clamp_bounds)
   // ---- transition stream (replay-buffer sampler, approximate_methods.py:513-545): trajectory `t` writes the tuple of
   //      its pass k at slot tr_base[t] + k of the five arrays below.  nullptr = no stream.
-  const long long* tr_base;
+  //      path_base (kernels instantiated with RAGGED only, which never carry the stream): the ragged checkpoint store,
+  //      trajectory t owns rows [path_base[t], path_base[t + 1]) of `path` (ckpt_slot).  One field for both keeps the
+  //      struct, and so the code of every kernel compiled without RAGGED, unchanged.
+  union {
+    const long long* tr_base;
+    const long long* path_base;
+  };
   float* tr_state;               // [n][d]  state the pass starts from
   float* tr_action;              // [n][d]
   float* tr_reward;              // [n]
@@ -112,6 +118,26 @@ struct alignas(8) ContRec {
   typename RealT<F64>::type x[D];
   typename RealT<F64>::type G, S, L2;
 };
+
+// Row of `path` that holds checkpoint ci (the state X_{ci * ckpt_every}) of trajectory traj: the dense store
+// path[K][ckpt_stride][d], or (RAGGED, rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged) the ragged one, in which the
+// trajectory owns rows [path_base[traj], path_base[traj + 1]).  A ragged writer drops a checkpoint that falls outside
+// them (ckpt_writable); a ragged reverse pass takes a trajectory only if they hold all its checkpoints (ckpt_covered).
+template <bool RAGGED>
+__device__ __forceinline__ long long ckpt_slot(const FwdArgs& A, long long traj, int ci) {
+  if constexpr (RAGGED) return A.path_base[traj] + ci;
+  else return traj * A.ckpt_stride + ci;
+}
+template <bool RAGGED>
+__device__ __forceinline__ bool ckpt_writable(const FwdArgs& A, long long traj, long long slot) {
+  if constexpr (RAGGED) return slot < A.path_base[traj + 1];
+  else return true;
+}
+template <bool RAGGED>
+__device__ __forceinline__ bool ckpt_covered(const FwdArgs& A, long long traj, int kstar) {
+  if constexpr (RAGGED) return A.path_base[traj] + kstar / A.ckpt_every < A.path_base[traj + 1];
+  else return true;
+}
 
 __device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
 __device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
@@ -205,7 +231,8 @@ constexpr int fwd_min_blocks() { return MMA ? RLSDE_FWD_MMA_MIN_BLOCKS : (D == 1
 // proven it cannot bind (fwd_mma_clamp_bounds)
 // BRIDGE: the Brownian-bridge hit test between passes (bridge_project; instantiated at d = 1 only).  A compile-time choice,
 // so that the kernels without it keep their register allocation
-template <int D, int H, bool F64, bool FAST, bool MMA, bool CLAMP2 = true, bool BRIDGE = false>
+// RAGGED: checkpoints go to the ragged store (ckpt_slot); no transition stream (path_base shares its field)
+template <int D, int H, bool F64, bool FAST, bool MMA, bool CLAMP2 = true, bool BRIDGE = false, bool RAGGED = false>
 __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_kernel(const __grid_constant__ MlpConst<D, H> W,
                                                           const __grid_constant__ FwdArgs A,
                                                           const __grid_constant__ typename FwdMmaSel<D, MMA>::type M) {
@@ -484,9 +511,12 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
       if (store_path) {
         if (ck == 0) {
           const int ci = A.ckpt_log2 >= 0 ? (k >> A.ckpt_log2) : (k / A.ckpt_every);      // no integer division per pass
-          float* dst = A.path + ((long long)traj * A.ckpt_stride + ci) * D;
+          const long long row = ckpt_slot<RAGGED>(A, traj, ci);
+          if (ckpt_writable<RAGGED>(A, traj, row)) {
+            float* dst = A.path + row * D;
 #pragma unroll
-          for (int i = 0; i < D; ++i) dst[i] = (float)x[i];
+            for (int i = 0; i < D; ++i) dst[i] = (float)x[i];
+          }
           ck = A.ckpt_every;
         }
         --ck;
@@ -529,7 +559,7 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
           xn[i] = (real)__fadd_rn(__fadd_rn(xi, drift), __fmul_rn(A.sigma_f, dB[i]));
         }
       }
-      if (A.tr_base != nullptr) {
+      if (!RAGGED && A.tr_base != nullptr) {
         // (state, action, reward, next_state, done) of this pass, cast to the replay buffer's float32 arrays
         // (replay_buffers.py:23-33,56-68); on the detecting pass the reward is -g(x) = -0 (environments.py:104-110)
         const long long slot = A.tr_base[traj] + k;
@@ -584,8 +614,9 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
   }
 }
 
-// host-side launcher for one (D, H) shape; defined in rollout_fwd_inst.cuh
-template <int D, int H>
+// host-side launcher for one (D, H) shape; defined in rollout_fwd_inst.cuh.  RAGGED: the ragged checkpoint store (float32
+// state only, no Brownian-bridge test: the caller refuses both)
+template <int D, int H, bool RAGGED = false>
 int launch_rollout_fwd(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream);
 
 // d = 1 rollout under the control table_dev[grid_index(x)] (fwd_tab_d1.cu).  Tables of up to FWD_TAB_SMEM_MAX entries

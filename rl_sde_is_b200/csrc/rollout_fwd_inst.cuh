@@ -4,7 +4,7 @@
 
 namespace rlsde {
 
-template <int D, int H, bool F64, bool FAST, bool MMA, bool BRIDGE>
+template <int D, int H, bool F64, bool FAST, bool MMA, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, H> W;
   if (!FAST && RLSDE_FWD_FOLDED) pack_mlp_const_folded<D, H>(params_host, W);
@@ -13,14 +13,14 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
   if constexpr (MMA) pack_mlp_mma<D>(W, M);
   else M.unused = 0;
   FwdArgs a = args;
-  auto kern = rollout_fwd_kernel<D, H, F64, FAST, MMA, true, BRIDGE>;
+  auto kern = rollout_fwd_kernel<D, H, F64, FAST, MMA, true, BRIDGE, RAGGED>;
   a.mma_x1_max = -1.0f;
   if constexpr (MMA && !FAST) {
     // leave the clamp of the grouped reciprocal out where it provably cannot bind (same bits, fewer instructions)
     double z2_max, x1_max;
     fwd_mma_clamp_bounds<D, H>(W, z2_max, x1_max);
     a.mma_x1_max = (float)x1_max;
-    if (z2_max <= RCP_GROUP_SAFE_Z) kern = rollout_fwd_kernel<D, H, F64, FAST, MMA, false, BRIDGE>;
+    if (z2_max <= RCP_GROUP_SAFE_Z) kern = rollout_fwd_kernel<D, H, F64, FAST, MMA, false, BRIDGE, RAGGED>;
   }
   // Small batches: one warp per block so the warps spread over SMs (latency-bound regime);
   // large batches: persistent grid of 128-thread blocks, as many as are co-resident.
@@ -62,42 +62,48 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
   return (int)cudaGetLastError();
 }
 
-template <int D, int H, bool MMA, bool BRIDGE>
+template <int D, int H, bool MMA, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_prec(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0;
   const bool fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if (f64) {
-    return fast ? launch_fwd_variant<D, H, true, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
-                : launch_fwd_variant<D, H, true, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
+  if constexpr (!RAGGED) {     // the ragged store is refused with the float64 state
+    if (f64) {
+      return fast ? launch_fwd_variant<D, H, true, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
+                  : launch_fwd_variant<D, H, true, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
+    }
   }
-  return fast ? launch_fwd_variant<D, H, false, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
-              : launch_fwd_variant<D, H, false, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
+  return fast ? launch_fwd_variant<D, H, false, true, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream)
+              : launch_fwd_variant<D, H, false, false, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
 }
 
 // args.policy_mma selects the policy arithmetic; the caller checks fwd_mma_shape(D, H) before it sets it
-template <int D, int H, bool BRIDGE>
+template <int D, int H, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   if constexpr (fwd_mma_shape(D, H)) {
-    if (args.policy_mma) return launch_fwd_prec<D, H, true, BRIDGE>(params_host, args, sm_count, stream);
+    if (args.policy_mma) return launch_fwd_prec<D, H, true, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
   }
-  return launch_fwd_prec<D, H, false, BRIDGE>(params_host, args, sm_count, stream);
+  return launch_fwd_prec<D, H, false, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
 }
 
 // The kernels with the Brownian-bridge hit test (RLSDE_F_HIT_BRIDGE, d = 1) live in a translation unit of their own
 // (fwd_d1_h32_bridge.cu): compiled next to the others, they changed how ptxas allocated an existing kernel's registers.
+// So do the ragged-store kernels (fwd_d*_h32_ragged.cu).
 template <int D, int H>
 int launch_rollout_fwd_bridge(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream);
 
-template <int D, int H>
+template <int D, int H, bool RAGGED>
 int launch_rollout_fwd(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (D == 1) {      // the caller accepts RLSDE_F_HIT_BRIDGE at d = 1 only
+  if constexpr (D == 1 && !RAGGED) {      // the caller accepts RLSDE_F_HIT_BRIDGE at d = 1 only, and not with RAGGED
     if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_rollout_fwd_bridge<D, H>(params_host, args, sm_count, stream);
   }
-  return launch_fwd_policy<D, H, false>(params_host, args, sm_count, stream);
+  return launch_fwd_policy<D, H, false, RAGGED>(params_host, args, sm_count, stream);
 }
 
 }  // namespace rlsde
 
 #define RLSDE_INSTANTIATE_FWD(D, H) \
   template int rlsde::launch_rollout_fwd<D, H>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
+// the ragged checkpoint store (rlsde_rollout_fwd_ragged), in translation units of its own
+#define RLSDE_INSTANTIATE_FWD_RAGGED(D, H) \
+  template int rlsde::launch_rollout_fwd<D, H, true>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
 

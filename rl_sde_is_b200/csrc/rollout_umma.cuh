@@ -125,7 +125,8 @@ __device__ __forceinline__ void ld32(uint32_t taddr, uint32_t (&r)[32]) {
 }  // namespace umma
 
 // BRIDGE: the Brownian-bridge hit test between passes (TrajOwner::pass; d = 1 only)
-template <int D, int H, bool F64, bool FAST, bool BRIDGE = false>
+// RAGGED: checkpoints go to the ragged store (TrajOwner::pass)
+template <int D, int H, bool F64, bool FAST, bool BRIDGE = false, bool RAGGED = false>
 __global__ void __launch_bounds__(umma_threads<H>(), umma_streams<H>() ? 2 : 4) rollout_fwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict__ Bimg,
                                                                            const __grid_constant__ FwdArgs A) {
   using namespace umma;
@@ -174,7 +175,7 @@ __global__ void __launch_bounds__(umma_threads<H>(), umma_streams<H>() ? 2 : 4) 
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = tmem_base_s;
 
-  TrajOwner<D, F64, BRIDGE> T;
+  TrajOwner<D, F64, BRIDGE, RAGGED> T;
   T.init(A);
   const bool owner = warp < 4;
   float b3[D];
@@ -311,8 +312,9 @@ __global__ void __launch_bounds__(umma_threads<H>(), umma_streams<H>() ? 2 : 4) 
   if (warp == 4) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(umma_tmem_cols<H>()) : "memory");
 }
 
-// params_dev: WideParams<D, H> image; image_dev: umma_image_bytes<H>() bytes (both in the caller's workspace)
-template <int D, int H>
+// params_dev: WideParams<D, H> image; image_dev: umma_image_bytes<H>() bytes (both in the caller's workspace).
+// RAGGED: the ragged checkpoint store (float32 state only, no Brownian-bridge test: the caller refuses both)
+template <int D, int H, bool RAGGED = false>
 int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, int sm_count,
                             cudaStream_t stream);
 

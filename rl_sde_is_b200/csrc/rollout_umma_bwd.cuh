@@ -114,7 +114,8 @@ __device__ __forceinline__ float lane_transpose_sum(float (&v)[32], int lane) {
 
 // partial layout (float64): [n_cons][H * H] (dW2 in 2^esh units, row = out unit), then [n_prod][ub_small_count]
 // WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32); the launch's scale from ub_scale_weighted_kernel
-template <int D, int H, bool FAST, bool WEIGHTED = false>
+// RAGGED: the states come from the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, int H, bool FAST, bool WEIGHTED = false, bool RAGGED = false>
 __global__ void __launch_bounds__(UB_THREADS, 1)
 rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict__ Bimg1, const uint8_t* __restrict__ Bimg2,
                         const __grid_constant__ FwdArgs A, uint8_t* __restrict__ xbuf, unsigned* __restrict__ ctl,
@@ -353,7 +354,7 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
       if (slot < A.K) {
         traj = A.order ? A.order[slot] : slot;
         const int t = A.T[traj];
-        if (t >= 0) {
+        if (t >= 0 && ckpt_covered<RAGGED>(A, traj, t)) {
           alive = true; kstar = t; j = t; Gk = ((const float*)A.G)[traj];
           if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
         }
@@ -362,7 +363,7 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
       if (lane == 0 && half == 0) s_np[rgrp] = np;
       if (alive) {
 #pragma unroll
-        for (int i = 0; i < D; ++i) xn[i] = A.path[((long long)traj * A.ckpt_stride + j) * D + i];
+        for (int i = 0; i < D; ++i) xn[i] = A.path[ckpt_slot<RAGGED>(A, traj, j) * D + i];
       }
     }
     __syncthreads();
@@ -402,7 +403,7 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
         for (int i = 0; i < D; ++i) xf[i] = xn[i];
         if (live && j >= 1) {                      // next pass's state: issued now, used in a pass's time
 #pragma unroll
-          for (int i = 0; i < D; ++i) xn[i] = A.path[((long long)traj * A.ckpt_stride + (j - 1)) * D + i];
+          for (int i = 0; i < D; ++i) xn[i] = A.path[ckpt_slot<RAGGED>(A, traj, j - 1) * D + i];
         }
 
         // ---- layer 1 -> A ring (K-major, MMA 1) and exchange B planes (MN-major operand of dW2); this half's chunks
@@ -777,7 +778,7 @@ static __global__ void ub_reduce_kernel(const double* __restrict__ partial, int 
 // scratch the launcher needs behind the fixed workspace (exchange ring, control words, float64 partials, second image)
 template <int D, int H>
 size_t bwd_umma_scratch_bytes(int sm_count);
-template <int D, int H, bool WEIGHTED = false>
+template <int D, int H, bool WEIGHTED = false, bool RAGGED = false>
 int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, float scale,
                             float* grad, uint8_t* scratch, size_t scratch_bytes, int sm_count, cudaStream_t stream);
 

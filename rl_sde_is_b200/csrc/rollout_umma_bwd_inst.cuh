@@ -37,12 +37,12 @@ size_t bwd_umma_scratch_bytes(int sm_count) {
   return UbScratch<D, H>::total(n_prod, n_cons);
 }
 
-template <int D, int H, bool FAST, bool WEIGHTED>
+template <int D, int H, bool FAST, bool WEIGHTED, bool RAGGED>
 static int launch_bwd_umma_variant(const float* params_dev, const uint8_t* img1, const FwdArgs& args, float scale, float* grad,
                                    uint8_t* scratch, int n_prod, int n_cons, float w3max, cudaStream_t stream) {
   typedef UbScratch<D, H> S;
   constexpr int P = D * H + H + H * H + H + H * D + D;
-  auto kern = rollout_bwd_umma_kernel<D, H, FAST, WEIGHTED>;
+  auto kern = rollout_bwd_umma_kernel<D, H, FAST, WEIGHTED, RAGGED>;
   const size_t smem = ub_smem_bytes<D, H>();
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -81,7 +81,7 @@ static int launch_bwd_umma_variant(const float* params_dev, const uint8_t* img1,
   return (int)cudaGetLastError();
 }
 
-template <int D, int H, bool WEIGHTED>
+template <int D, int H, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, float scale,
                             float* grad, uint8_t* scratch, size_t scratch_bytes, int sm_count, cudaStream_t stream) {
   typedef UbScratch<D, H> S;
@@ -106,8 +106,8 @@ int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t
   if ((e = cudaMemcpyAsync(scratch + S::o_img2, w2.data(), umma_image_bytes<H>(), cudaMemcpyHostToDevice, stream)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(scratch + S::o_ctl, 0, S::o_img2, stream)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(scratch + S::o_partial, 0, S::partial_bytes(n_prod, n_cons), stream)) != cudaSuccess) return (int)e;
-  return fast ? launch_bwd_umma_variant<D, H, true, WEIGHTED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream)
-              : launch_bwd_umma_variant<D, H, false, WEIGHTED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream);
+  return fast ? launch_bwd_umma_variant<D, H, true, WEIGHTED, RAGGED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream)
+              : launch_bwd_umma_variant<D, H, false, WEIGHTED, RAGGED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream);
 }
 
 }  // namespace rlsde
@@ -120,3 +120,7 @@ int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t
 #define RLSDE_INSTANTIATE_UMMA_BWD_WEIGHTED(D, H)                                                                                 \
   template int rlsde::launch_rollout_bwd_umma<D, H, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, float*,   \
                                                           uint8_t*, size_t, int, cudaStream_t);
+// the weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged), in translation units of its own
+#define RLSDE_INSTANTIATE_UMMA_BWD_RAGGED(D, H)                                                                             \
+  template int rlsde::launch_rollout_bwd_umma<D, H, true, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, \
+                                                                float*, uint8_t*, size_t, int, cudaStream_t);

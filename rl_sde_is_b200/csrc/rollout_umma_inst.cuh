@@ -5,9 +5,9 @@
 
 namespace rlsde {
 
-template <int D, int H, bool F64, bool FAST, bool BRIDGE>
+template <int D, int H, bool F64, bool FAST, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_umma_variant(const float* params_dev, const uint8_t* image_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  auto kern = rollout_fwd_umma_kernel<D, H, F64, FAST, BRIDGE>;
+  auto kern = rollout_fwd_umma_kernel<D, H, F64, FAST, BRIDGE, RAGGED>;
   const size_t smem = umma_smem_bytes<D, H>();
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -33,7 +33,7 @@ static int launch_fwd_umma_variant(const float* params_dev, const uint8_t* image
   return (int)cudaGetLastError();
 }
 
-template <int D, int H>
+template <int D, int H, bool RAGGED>
 int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, int sm_count,
                             cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
@@ -50,10 +50,15 @@ int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t
                : launch_fwd_umma_variant<D, H, true, false, B_>(params_dev, image_dev, args, sm_count, stream))       \
        : (fast ? launch_fwd_umma_variant<D, H, false, true, B_>(params_dev, image_dev, args, sm_count, stream)        \
                : launch_fwd_umma_variant<D, H, false, false, B_>(params_dev, image_dev, args, sm_count, stream)))
-  if constexpr (D == 1) {      // RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
-    if (args.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_UMMA_FWD(true);
+  if constexpr (RAGGED) {      // float32 state, no Brownian-bridge test: the caller refuses both
+    return fast ? launch_fwd_umma_variant<D, H, false, true, false, true>(params_dev, image_dev, args, sm_count, stream)
+                : launch_fwd_umma_variant<D, H, false, false, false, true>(params_dev, image_dev, args, sm_count, stream);
+  } else {
+    if constexpr (D == 1) {      // RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
+      if (args.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_UMMA_FWD(true);
+    }
+    return RLSDE_UMMA_FWD(false);
   }
-  return RLSDE_UMMA_FWD(false);
 #undef RLSDE_UMMA_FWD
 }
 
@@ -61,3 +66,6 @@ int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t
 
 #define RLSDE_INSTANTIATE_UMMA(D, H) \
   template int rlsde::launch_rollout_fwd_umma<D, H>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, int, cudaStream_t);
+// the ragged checkpoint store (rlsde_rollout_fwd_ragged), in translation units of its own
+#define RLSDE_INSTANTIATE_UMMA_RAGGED(D, H) \
+  template int rlsde::launch_rollout_fwd_umma<D, H, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, int, cudaStream_t);

@@ -155,7 +155,8 @@ __device__ __forceinline__ void warp_policy_exact(const LaneParams<D>& P, const 
 // MMA (K1 evaluated its policy with mlp_forward_mma) the same tensor-core sequence with the trajectory's state in all
 // 32 rows of the tile.
 // BRIDGE: the Brownian-bridge hit test between passes (bridge_project, rollout_fwd.cuh; d = 1 only)
-template <int D, bool F64, bool FAST, bool RESUME, bool MMA = false, bool BRIDGE = false>
+// RAGGED: checkpoints go to the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, bool F64, bool FAST, bool RESUME, bool MMA = false, bool BRIDGE = false, bool RAGGED = false>
 __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel(const __grid_constant__ MlpConst<D, WARP_H> W_param,
                                                                const MlpConst<D, WARP_H>* __restrict__ W_dev,
                                                                const __grid_constant__ FwdArgs A,
@@ -286,9 +287,12 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
       if (store_path) {
         if (ck == 0) {
           const int ci = A.ckpt_log2 >= 0 ? (k >> A.ckpt_log2) : (k / A.ckpt_every);      // no integer division per pass
+          const long long row = ckpt_slot<RAGGED>(A, traj, ci);
+          if (ckpt_writable<RAGGED>(A, traj, row)) {
 #pragma unroll
-          for (int i = 0; i < D; ++i)
-            if (lane == i) A.path[((long long)traj * A.ckpt_stride + ci) * D + i] = (float)x[i];
+            for (int i = 0; i < D; ++i)
+              if (lane == i) A.path[row * D + i] = (float)x[i];
+          }
           ck = A.ckpt_every;
         }
         --ck;
@@ -349,7 +353,8 @@ __global__ void __launch_bounds__(128, (D <= 2 ? 4 : 1)) rollout_fwd_warp_kernel
 // ------------------------------------------------------------------------------------------------ reverse
 // Needs every state (ckpt_every == 1).  Lane j accumulates row j of dW2 / dW1, column j of dW3, entry j of db1 / db2.
 // WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32).
-template <int D, bool FAST, bool WEIGHTED = false>
+// RAGGED: the states come from the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, bool FAST, bool WEIGHTED = false, bool RAGGED = false>
 __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_constant__ MlpConst<D, WARP_H> W_param,
                                                                const MlpConst<D, WARP_H>* __restrict__ W_dev,
                                                                const __grid_constant__ FwdArgs A, float* __restrict__ partial) {
@@ -380,7 +385,7 @@ __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_cons
   for (long long item = gw; item < A.K; item += n_warps) {
     const long long traj = A.order ? A.order[item] : item;
     const int kstar = A.T[traj];
-    if (kstar < 0) continue;
+    if (kstar < 0 || !ckpt_covered<RAGGED>(A, traj, kstar)) continue;
     const float Gk = ((const float*)A.G)[traj];                       // WEIGHTED: cS
     const float nS = WEIGHTED ? __fmul_rn(-1.0f, Gk) : 0.f;
     const float mG = WEIGHTED ? __fmul_rn(-1.0f, ((const float*)A.S)[traj]) : 0.f;
@@ -390,7 +395,7 @@ __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_cons
     nc.reset();
     // X_j is loaded one pass ahead: the load's latency (~500 cycles) overlaps the previous pass's arithmetic instead
     // of heading the dependency chain of its own pass
-    const float* xp = A.path + (long long)traj * A.ckpt_stride * D;
+    const float* xp = A.path + ckpt_slot<RAGGED>(A, traj, 0) * D;
     float x_next[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) x_next[i] = xp[(long long)kstar * D + i];
@@ -462,13 +467,14 @@ __global__ void __launch_bounds__(128) rollout_bwd_warp_kernel(const __grid_cons
 inline long long warp_path_max_k(int sm_count) { return (long long)sm_count * 16; }
 
 // params_host == nullptr: the policy is read from W_dev (an MlpConst<D, WARP_H> in device memory, see pack_mlp_const_dev)
-template <int D>
+// RAGGED: the ragged checkpoint store (float32 state only, no Brownian-bridge test: the caller refuses both)
+template <int D, bool RAGGED = false>
 int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream);
-template <int D, bool WEIGHTED = false>
+template <int D, bool WEIGHTED = false, bool RAGGED = false>
 int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                             float* partial, int sm_count, cudaStream_t stream);
 // continues the trajectories the thread-per-trajectory kernel left in args.q_ring (args.q_ctrl[1] records)
-template <int D>
+template <int D, bool RAGGED = false>
 int launch_rollout_fwd_warp_resume(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream);
 // theta_dev (flat float32, state_dict order) -> MlpConst<D, WARP_H> in device memory, same rounding as the host packer
 template <int D>

@@ -41,36 +41,38 @@ int launch_pack_mlp_const_dev(const float* theta_dev, void* W_dev, bool fast_tan
   return (int)cudaGetLastError();
 }
 
-template <int D, bool F64, bool FAST, bool BRIDGE>
+template <int D, bool F64, bool FAST, bool BRIDGE, bool RAGGED>
 static int launch_fwd_warp_variant(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, WARP_H> W;
   if (params_host != nullptr) pack_mlp_const<D, WARP_H>(params_host, FAST, W);
   else memset(&W, 0, sizeof(W));
-  rollout_fwd_warp_kernel<D, F64, FAST, false, false, BRIDGE><<<(unsigned)warp_grid(args.K, sm_count), 128, 0, stream>>>(
+  rollout_fwd_warp_kernel<D, F64, FAST, false, false, BRIDGE, RAGGED><<<(unsigned)warp_grid(args.K, sm_count), 128, 0, stream>>>(
       W, params_host != nullptr ? nullptr : reinterpret_cast<const MlpConst<D, WARP_H>*>(W_dev), args, MlpMmaNone{0});
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
-template <int D, bool BRIDGE>
+template <int D, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_warp_bridge(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if (f64) return fast ? launch_fwd_warp_variant<D, true, true, BRIDGE>(params_host, W_dev, args, sm_count, stream)
-                       : launch_fwd_warp_variant<D, true, false, BRIDGE>(params_host, W_dev, args, sm_count, stream);
-  return fast ? launch_fwd_warp_variant<D, false, true, BRIDGE>(params_host, W_dev, args, sm_count, stream)
-              : launch_fwd_warp_variant<D, false, false, BRIDGE>(params_host, W_dev, args, sm_count, stream);
+  if constexpr (!RAGGED) {     // the ragged store is refused with the float64 state
+    if (f64) return fast ? launch_fwd_warp_variant<D, true, true, BRIDGE, false>(params_host, W_dev, args, sm_count, stream)
+                         : launch_fwd_warp_variant<D, true, false, BRIDGE, false>(params_host, W_dev, args, sm_count, stream);
+  }
+  return fast ? launch_fwd_warp_variant<D, false, true, BRIDGE, RAGGED>(params_host, W_dev, args, sm_count, stream)
+              : launch_fwd_warp_variant<D, false, false, BRIDGE, RAGGED>(params_host, W_dev, args, sm_count, stream);
 }
 
-// RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
-template <int D>
+// RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only, and not with RAGGED
+template <int D, bool RAGGED>
 int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (D == 1) {
+  if constexpr (D == 1 && !RAGGED) {
     if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_fwd_warp_bridge<D, true>(params_host, W_dev, args, sm_count, stream);
   }
-  return launch_fwd_warp_bridge<D, false>(params_host, W_dev, args, sm_count, stream);
+  return launch_fwd_warp_bridge<D, false, RAGGED>(params_host, W_dev, args, sm_count, stream);
 }
 
-template <int D, bool F64, bool FAST, bool MMA, bool BRIDGE>
+template <int D, bool F64, bool FAST, bool MMA, bool BRIDGE, bool RAGGED>
 static int launch_fwd_warp_resume_variant(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   MlpConst<D, WARP_H> W;
   if (!FAST && RLSDE_FWD_FOLDED) pack_mlp_const_folded<D, WARP_H>(params_host, W);      // the image K1 itself was launched with
@@ -79,38 +81,40 @@ static int launch_fwd_warp_resume_variant(const float* params_host, const FwdArg
   if constexpr (MMA) pack_mlp_mma<D>(W, M);
   else M.unused = 0;
   // the number of records is only known on the device: a full grid (16 warps per SM), warps without a record leave at once
-  rollout_fwd_warp_kernel<D, F64, FAST, true, MMA, BRIDGE><<<(unsigned)(sm_count * 4), 128, 0, stream>>>(W, nullptr, args, M);
+  rollout_fwd_warp_kernel<D, F64, FAST, true, MMA, BRIDGE, RAGGED><<<(unsigned)(sm_count * 4), 128, 0, stream>>>(W, nullptr, args, M);
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
-template <int D, bool MMA, bool BRIDGE>
+template <int D, bool MMA, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_warp_resume_bridge(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
-                       : launch_fwd_warp_resume_variant<D, true, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
-  return fast ? launch_fwd_warp_resume_variant<D, false, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
-              : launch_fwd_warp_resume_variant<D, false, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
+  if constexpr (!RAGGED) {     // the ragged store is refused with the float64 state
+    if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true, MMA, BRIDGE, false>(params_host, args, sm_count, stream)
+                         : launch_fwd_warp_resume_variant<D, true, false, MMA, BRIDGE, false>(params_host, args, sm_count, stream);
+  }
+  return fast ? launch_fwd_warp_resume_variant<D, false, true, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream)
+              : launch_fwd_warp_resume_variant<D, false, false, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
 }
 
-template <int D, bool MMA>
+template <int D, bool MMA, bool RAGGED>
 static int launch_fwd_warp_resume_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (D == 1) {
+  if constexpr (D == 1 && !RAGGED) {
     if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_fwd_warp_resume_bridge<D, MMA, true>(params_host, args, sm_count, stream);
   }
-  return launch_fwd_warp_resume_bridge<D, MMA, false>(params_host, args, sm_count, stream);
+  return launch_fwd_warp_resume_bridge<D, MMA, false, RAGGED>(params_host, args, sm_count, stream);
 }
 
 // continues with the policy arithmetic K1 was launched with (args.policy_mma)
-template <int D>
+template <int D, bool RAGGED>
 int launch_rollout_fwd_warp_resume(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   if constexpr (fwd_mma_shape(D, WARP_H)) {
-    if (args.policy_mma) return launch_fwd_warp_resume_policy<D, true>(params_host, args, sm_count, stream);
+    if (args.policy_mma) return launch_fwd_warp_resume_policy<D, true, RAGGED>(params_host, args, sm_count, stream);
   }
-  return launch_fwd_warp_resume_policy<D, false>(params_host, args, sm_count, stream);
+  return launch_fwd_warp_resume_policy<D, false, RAGGED>(params_host, args, sm_count, stream);
 }
 
-template <int D, bool FAST, bool WEIGHTED>
+template <int D, bool FAST, bool WEIGHTED, bool RAGGED>
 static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                                    float* partial, int sm_count, cudaStream_t stream) {
   constexpr int P = D * WARP_H + WARP_H + WARP_H * WARP_H + WARP_H + WARP_H * D + D;
@@ -118,7 +122,7 @@ static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, 
   if (params_host != nullptr) pack_mlp_const<D, WARP_H>(params_host, FAST, W);
   else memset(&W, 0, sizeof(W));
   const long long grid = warp_grid(args.K, sm_count);
-  rollout_bwd_warp_kernel<D, FAST, WEIGHTED><<<(unsigned)grid, 128, 0, stream>>>(
+  rollout_bwd_warp_kernel<D, FAST, WEIGHTED, RAGGED><<<(unsigned)grid, 128, 0, stream>>>(
       W, params_host != nullptr ? nullptr : reinterpret_cast<const MlpConst<D, WARP_H>*>(W_dev), args, partial);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;
@@ -127,12 +131,12 @@ static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, 
   return (int)cudaGetLastError();
 }
 
-template <int D, bool WEIGHTED>
+template <int D, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                             float* partial, int sm_count, cudaStream_t stream) {
   return (args.flags & RLSDE_F_TANH_FAST)
-             ? launch_bwd_warp_variant<D, true, WEIGHTED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream)
-             : launch_bwd_warp_variant<D, false, WEIGHTED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream);
+             ? launch_bwd_warp_variant<D, true, WEIGHTED, RAGGED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream)
+             : launch_bwd_warp_variant<D, false, WEIGHTED, RAGGED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream);
 }
 
 }  // namespace rlsde
@@ -147,3 +151,10 @@ int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const F
 #define RLSDE_INSTANTIATE_BWD_WARP_WEIGHTED(D)                                                                             \
   template int rlsde::launch_rollout_bwd_warp<D, true>(const float*, const void*, const rlsde::FwdArgs&, float, float*,   \
                                                        float*, int, cudaStream_t);
+// the ragged checkpoint store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged), in translation units of its own
+#define RLSDE_INSTANTIATE_FWD_WARP_RAGGED(D)                                                                               \
+  template int rlsde::launch_rollout_fwd_warp<D, true>(const float*, const void*, const rlsde::FwdArgs&, int, cudaStream_t); \
+  template int rlsde::launch_rollout_fwd_warp_resume<D, true>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_BWD_WARP_RAGGED(D)                                                                               \
+  template int rlsde::launch_rollout_bwd_warp<D, true, true>(const float*, const void*, const rlsde::FwdArgs&, float, float*, \
+                                                             float*, int, cudaStream_t);

@@ -187,7 +187,7 @@ __device__ __forceinline__ void wide_head(const float* __restrict__ Wp, const fl
 
 // ------------------------------------------------------------------------------------------------ forward
 // BRIDGE: the Brownian-bridge hit test between passes (bridge_project, rollout_fwd.cuh; d = 1 only)
-template <int D, int H, int R, bool F64, bool FAST, bool BRIDGE = false>
+template <int D, int H, int R, bool F64, bool FAST, bool BRIDGE = false, bool RAGGED = false>
 __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const float* __restrict__ Wp, const __grid_constant__ FwdArgs A) {
   typedef typename RealT<F64>::type real;
   typedef WideParams<D, H> L;
@@ -329,9 +329,12 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const
       if (store_path) {
         if (ck == 0) {
           const int ci = A.ckpt_log2 >= 0 ? (k >> A.ckpt_log2) : (k / A.ckpt_every);
-          float* dst = A.path + ((long long)traj * A.ckpt_stride + ci) * D;
+          const long long row = ckpt_slot<RAGGED>(A, traj, ci);
+          if (ckpt_writable<RAGGED>(A, traj, row)) {
+            float* dst = A.path + row * D;
 #pragma unroll
-          for (int i = 0; i < D; ++i) dst[i] = (float)x[i];
+            for (int i = 0; i < D; ++i) dst[i] = (float)x[i];
+          }
           ck = A.ckpt_every;
         }
         --ck;
@@ -400,7 +403,8 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_fwd_wide_kernel(const
 // every pass (read-modify-write by the thread that owns the element); the small blocks are kept in registers / shared
 // memory and written at the end.
 // WEIGHTED: per-trajectory coefficients (rollout_bwd.cuh, the comment above em_step_f32)
-template <int D, int H, int R, bool FAST, bool WEIGHTED = false>
+// RAGGED: the states come from the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, int H, int R, bool FAST, bool WEIGHTED = false, bool RAGGED = false>
 __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const float* __restrict__ Wp, const __grid_constant__ FwdArgs A,
                                                                            float* __restrict__ partial) {
   typedef WideParams<D, H> L;
@@ -465,7 +469,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const
         if (owner && slot < A.K) {
           traj = A.order ? A.order[slot] : slot;
           const int t = A.T[traj];
-          if (t >= 0) {
+          if (t >= 0 && ckpt_covered<RAGGED>(A, traj, t)) {
             alive = true; kstar = t; j = t; Gk = ((const float*)A.G)[traj];
             if constexpr (WEIGHTED) { Gk = __fmul_rn(-1.0f, Gk); mG = __fmul_rn(-1.0f, ((const float*)A.S)[traj]); }
             nc.reset();
@@ -478,7 +482,7 @@ __global__ void __launch_bounds__(WIDE_THREADS, 1) rollout_bwd_wide_kernel(const
       if (lane == 0) s_live = live != 0u;
       if (owner) {
 #pragma unroll
-        for (int i = 0; i < D; ++i) xS[lane * RLSDE_MAX_D + i] = alive ? A.path[((long long)traj * A.ckpt_stride + j) * D + i] : A.x0_f[i];
+        for (int i = 0; i < D; ++i) xS[lane * RLSDE_MAX_D + i] = alive ? A.path[ckpt_slot<RAGGED>(A, traj, j) * D + i] : A.x0_f[i];
       }
     }
     __syncthreads();
@@ -689,10 +693,11 @@ static __global__ void wide_reduce_kernel(const float* __restrict__ partial, int
   grad[p] = accumulate ? grad[p] + g : g;
 }
 
-// params_dev: WideParams<D, H> buffer in the caller's workspace (filled from params_host by the launcher)
-template <int D, int H>
+// params_dev: WideParams<D, H> buffer in the caller's workspace (filled from params_host by the launcher).
+// RAGGED: the ragged checkpoint store (float32 state only, no Brownian-bridge test: the caller refuses both)
+template <int D, int H, bool RAGGED = false>
 int launch_rollout_fwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, int sm_count, cudaStream_t stream);
-template <int D, int H, bool WEIGHTED = false>
+template <int D, int H, bool WEIGHTED = false, bool RAGGED = false>
 int launch_rollout_bwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, float scale, float* grad, float* partial,
                             size_t partial_bytes, int sm_count, cudaStream_t stream);
 

@@ -20,7 +20,8 @@ __device__ __forceinline__ long long grid_index(const FwdArgs& A, double x) {
 }
 
 // BRIDGE: the Brownian-bridge hit test between passes (bridge_project, rollout_fwd.cuh; d = 1 only)
-template <int D, bool F64, bool BRIDGE = false>
+// RAGGED: checkpoints go to the ragged store (ckpt_slot, rollout_fwd.cuh)
+template <int D, bool F64, bool BRIDGE = false, bool RAGGED = false>
 struct TrajOwner {
   typedef typename RealT<F64>::type real;
   static constexpr int SPB = NoisePlan<D>::SPB;
@@ -116,9 +117,12 @@ struct TrajOwner {
     if (store_path) {
       if (ck == 0) {
         const int ci = A.ckpt_log2 >= 0 ? (k >> A.ckpt_log2) : (k / A.ckpt_every);
-        float* dst = A.path + ((long long)traj * A.ckpt_stride + ci) * D;
+        const long long row = ckpt_slot<RAGGED>(A, traj, ci);
+        if (ckpt_writable<RAGGED>(A, traj, row)) {
+          float* dst = A.path + row * D;
 #pragma unroll
-        for (int i = 0; i < D; ++i) dst[i] = (float)x[i];
+          for (int i = 0; i < D; ++i) dst[i] = (float)x[i];
+        }
         ck = A.ckpt_every;
       }
       --ck;

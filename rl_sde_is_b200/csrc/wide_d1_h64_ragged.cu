@@ -1,0 +1,6 @@
+// the ragged checkpoint store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged) for d = 1, hidden width = 64: the
+// CUDA-core tile kernels and the tcgen05 forward kernel
+#include "rollout_wide_inst.cuh"
+#include "rollout_umma_inst.cuh"
+RLSDE_INSTANTIATE_WIDE_RAGGED(1, 64)
+RLSDE_INSTANTIATE_UMMA_RAGGED(1, 64)

@@ -1,0 +1,8 @@
+// the ragged checkpoint store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged) for d = 2, hidden width = 128: the
+// CUDA-core tile kernels and the tcgen05 kernels
+#include "rollout_wide_inst.cuh"
+#include "rollout_umma_inst.cuh"
+#include "rollout_umma_bwd_inst.cuh"
+RLSDE_INSTANTIATE_WIDE_RAGGED(2, 128)
+RLSDE_INSTANTIATE_UMMA_RAGGED(2, 128)
+RLSDE_INSTANTIATE_UMMA_BWD_RAGGED(2, 128)

@@ -9,6 +9,10 @@ Keyword-only extras (defaults = reference behaviour): ``noise`` (injected increm
 ``[n_steps, K, d]``), ``seed`` (Philox key), ``n_steps_lim``, ``tanh`` ('precise' | 'fast'),
 ``stoch_int`` ('reference' | 'exact'), ``ckpt_every``, ``device``, ``dist`` (shard the batch over a
 torch.distributed process group and all-reduce the packed gradient + statistics).
+
+Without ``ckpt_every`` the reverse pass's checkpoints go to the dense store (every trajectory reserves the whole pass
+budget) where it fits ``rollout.PATH_BUDGET_BYTES``, and to the ragged store (memory for the passes run, one more
+rollout and host synchronisation) where it does not (``rollout.choose_path_store``).
 """
 import dataclasses
 import time
@@ -52,7 +56,7 @@ def sample_loss_vectorized(env, model, K, *, noise=None, seed=None, n_steps_lim=
         noise = noise.to(device=dev, dtype=torch.float32).contiguous()
     lim = int(n_steps_lim) if noise is None else min(int(n_steps_lim), int(noise.shape[0]))
     if ckpt_every is None:
-        ckpt_every = R.choose_ckpt_every(int(K), d, lim, hidden=H)
+        ckpt_every = R.choose_path_store(int(K), d, lim, hidden=H)      # None: the ragged store
     opts = dict(seed=_next_seed(seed), n_steps_lim=n_steps_lim, noise=noise, tanh=tanh, stoch_int=stoch_int,
                 ckpt_every=ckpt_every, device=dev, kernel=kernel)
     if dist is not None:
@@ -98,7 +102,7 @@ def sample_returns_vectorized(env, model, K, *, noise=None, seed=None, n_steps_l
         noise = noise.to(device=dev, dtype=torch.float32).contiguous()
     lim = int(n_steps_lim) if noise is None else min(int(n_steps_lim), int(noise.shape[0]))
     if ckpt_every is None:
-        ckpt_every = R.choose_ckpt_every(int(K), d, lim, hidden=H)
+        ckpt_every = R.choose_path_store(int(K), d, lim, hidden=H)      # None: the ragged store
     opts = dict(seed=_next_seed(seed), n_steps_lim=n_steps_lim, noise=noise, tanh=tanh, stoch_int=stoch_int,
                 ckpt_every=ckpt_every, device=dev, kernel=kernel)
     holder = {}
@@ -126,7 +130,7 @@ def _loss_and_grads_fused(env, model, K, *, noise=None, seed=None, n_steps_lim=1
         noise = noise.to(device=dev, dtype=torch.float32).contiguous()
     lim = int(n_steps_lim) if noise is None else min(int(n_steps_lim), int(noise.shape[0]))
     if ckpt_every is None:
-        ckpt_every = R.choose_ckpt_every(int(K), d, lim, hidden=H)
+        ckpt_every = R.choose_path_store(int(K), d, lim, hidden=H)      # None: the ragged store
     linears = R.policy_linears(model)
     with torch.no_grad():
         params_host = torch.cat([t.reshape(-1) for lin in linears for t in (lin.weight, lin.bias)]).to(torch.float32).numpy()
@@ -267,7 +271,7 @@ class _LossWithAux(torch.autograd.Function):
     @staticmethod
     def forward(ctx, flat_params, env_c, mlp_c, K, opts, holder, dist):
         params_host = flat_params.detach().to("cpu", torch.float32).contiguous().numpy()
-        out = R.rollout_forward(env_c, mlp_c, params_host, K, store_path=True, want_logw=False, **opts)
+        out = R.rollout_forward_stored(env_c, mlp_c, params_host, K, **opts)
         holder["out"] = out
         K_global = out.cfg.K_global
         if dist is not None:
@@ -298,7 +302,7 @@ class _ReturnsWithAux(torch.autograd.Function):
     @staticmethod
     def forward(ctx, flat_params, env_c, mlp_c, K, opts, holder):
         params_host = flat_params.detach().to("cpu", torch.float32).contiguous().numpy()
-        out = R.rollout_forward(env_c, mlp_c, params_host, K, store_path=True, want_logw=False, **opts)
+        out = R.rollout_forward_stored(env_c, mlp_c, params_host, K, **opts)
         holder["out"] = out
         # ctx keeps what the reverse pass reads (T, path, cfg), not the returned G and S: outputs reachable from their own
         # grad_fn through ctx form a cycle that the garbage collector cannot see, and every rollout would stay allocated

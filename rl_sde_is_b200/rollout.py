@@ -110,6 +110,7 @@ class RolloutOut:
     path: Optional[torch.Tensor]
     stats_dev: torch.Tensor             # float64[RLSDE_NSTATS] on the device
     cfg: object = None
+    path_base: Optional[torch.Tensor] = None    # int64[K + 1]: path is the ragged store (rlsde_rollout_fwd_ragged); None: dense
     _stats: Optional[np.ndarray] = None
 
     @property
@@ -130,10 +131,13 @@ def _check_bridge(d, store_path=False):
 def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, noise=None, traj_offset=0,
                     K_global=None, tanh="precise", stoch_int="reference", state_f64=False, store_path=False,
                     ckpt_every=1, policy_opt=None, grid=None, want_logw=True, device=None, out=None, kernel="auto", tuning=None,
-                    bridge=False):
+                    bridge=False, path_base=None, n_slots=0):
     """One launch of K1 for K trajectories.  ``params_host``: contiguous float32 numpy array (state_dict order).
     ``bridge``: also detect target hits between passes with the Brownian-bridge crossing test (RLSDE_F_HIT_BRIDGE; d = 1,
-    not with ``store_path``)."""
+    not with ``store_path``).  ``path_base`` (int64 CUDA tensor [K + 1], with ``store_path``): checkpoints go to a ragged
+    store of ``n_slots`` rows laid out by it (``rlsde_rollout_fwd_ragged``; see ``rollout_forward_ragged``)."""
+    if path_base is not None and not store_path:
+        raise L.RlsdeError("path_base lays out the checkpoint store: it needs store_path=True")
     if bridge:
         _check_bridge(env_c.d, store_path)
     lib = L.load()
@@ -176,8 +180,14 @@ def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, 
         flags |= L.F_STORE_PATH
         lim_eff = min(cfg.n_steps_lim, cfg.noise_steps) if noise is not None else cfg.n_steps_lim
         cfg.ckpt_every = int(ckpt_every)
-        cfg.ckpt_stride = (lim_eff + cfg.ckpt_every - 1) // cfg.ckpt_every
-        path = torch.empty((K, cfg.ckpt_stride, d), dtype=torch.float32, device=dev)
+        if path_base is None:
+            cfg.ckpt_stride = (lim_eff + cfg.ckpt_every - 1) // cfg.ckpt_every
+            path = torch.empty((K, cfg.ckpt_stride, d), dtype=torch.float32, device=dev)
+        else:
+            if path_base.device != dev or path_base.dtype != torch.int64 or not path_base.is_contiguous() \
+                    or path_base.shape != (K + 1,):
+                raise L.RlsdeError(f"path_base must be a contiguous int64 tensor [{K + 1}] on {dev}")
+            path = torch.empty((max(int(n_slots), 1), d), dtype=torch.float32, device=dev)    # never empty: a pointer
     pol = None
     if policy_opt is not None:
         pol = torch.as_tensor(np.ascontiguousarray(np.asarray(policy_opt, dtype=np.float32).reshape(-1)), device=dev) \
@@ -193,14 +203,20 @@ def rollout_forward(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=10**6, 
     logw = torch.empty(K, dtype=real, device=dev) if want_logw else None
     stats = torch.zeros(L.RLSDE_NSTATS, dtype=torch.float64, device=dev)
     if K == 0:          # nothing to launch (and empty tensors have no device pointer to hand over)
-        return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=path, stats_dev=stats, cfg=cfg)
+        return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=path, stats_dev=stats, cfg=cfg, path_base=path_base)
     ws = _workspace(dev, K)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib.rlsde_rollout_fwd(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), _ptr(pol), _ptr(G), _ptr(S),
-                                   _ptr(T), _ptr(l2), _ptr(logw), _ptr(path), _ptr(stats), _ptr(ws), ws.numel(), stream)
-    L.check(rc, "rlsde_rollout_fwd")
-    return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=path, stats_dev=stats, cfg=cfg)
+        if path_base is None:
+            rc = lib.rlsde_rollout_fwd(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), _ptr(pol), _ptr(G), _ptr(S),
+                                       _ptr(T), _ptr(l2), _ptr(logw), _ptr(path), _ptr(stats), _ptr(ws), ws.numel(), stream)
+        else:
+            if pol is not None or logw is not None:
+                raise L.RlsdeError("the ragged store's rollout has no l2 or logw output")
+            rc = lib.rlsde_rollout_fwd_ragged(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), _ptr(path_base), _ptr(G),
+                                              _ptr(S), _ptr(T), _ptr(path), _ptr(stats), _ptr(ws), ws.numel(), stream)
+    L.check(rc, "rlsde_rollout_fwd" if path_base is None else "rlsde_rollout_fwd_ragged")
+    return RolloutOut(G=G, S=S, T=T, l2=l2, logw=logw, path=path, stats_dev=stats, cfg=cfg, path_base=path_base)
 
 
 def rollout_forward_table(env_c, table, K, *, grid, seed=0, n_steps_lim=10**6, noise=None, traj_offset=0, K_global=None,
@@ -298,9 +314,9 @@ def rollout_transitions(env_c, mlp_c, params_host, K, *, seed=0, n_max=10**6, no
     lim = int(n_max) if noise is None else min(int(n_max), int(noise.shape[0]))
     T = first.T.to(torch.int64)
     counts = torch.where(T >= 0, T + 1, torch.full_like(T, lim))
-    ends = torch.cumsum(counts, 0)
-    base = (ends - counts).contiguous()
-    n = int(ends[-1].item()) if K > 0 else 0
+    offsets, total = slot_offsets(counts)
+    base = offsets[:-1]
+    n = int(total.item()) if K > 0 else 0
     states = torch.empty((n, d), dtype=torch.float32, device=dev)
     actions = torch.empty((n, d), dtype=torch.float32, device=dev)
     next_states = torch.empty((n, d), dtype=torch.float32, device=dev)
@@ -331,17 +347,98 @@ def rollout_transitions(env_c, mlp_c, params_host, K, *, seed=0, n_max=10**6, no
                        counts=counts, rollout=out)
 
 
+def slot_offsets(counts):
+    """Offsets of per-trajectory slot ranges, on the device: ``counts`` int64 [K] -> ``(base int64 [K + 1], total)``, where
+    trajectory t owns slots [base[t], base[t + 1]) and ``total`` = base[K] is a 0-d device tensor (reading it synchronises).
+    The transition stream (``rollout_transitions``) and the ragged checkpoint store (``rollout_forward_ragged``) lay out
+    their buffers with it."""
+    base = torch.zeros(counts.numel() + 1, dtype=torch.int64, device=counts.device)
+    torch.cumsum(counts, 0, out=base[1:])
+    return base, base[-1]
+
+
+def ragged_ckpt_counts(T, ckpt_every):
+    """Checkpoints of each trajectory in the ragged store: floor(T / C) + 1 if it finished, 0 if not (T = -1)."""
+    T = T.to(torch.int64)
+    return torch.where(T >= 0, T // int(ckpt_every) + 1, torch.zeros_like(T))
+
+
+# Device memory a training rollout's checkpoint store may take, dense (choose_ckpt_every) or ragged
+# (choose_ragged_ckpt_every).  Module-level, so that a test can lower it.
+PATH_BUDGET_BYTES = 8 << 30
+RAGGED_SPACINGS = (1, 2, 4, 8, 16, 32)
+
+
+def choose_path_store(K, d, n_steps_lim, hidden=32):
+    """Checkpoint spacing of the dense store where it fits (``choose_ckpt_every`` at PATH_BUDGET_BYTES), else None: the
+    ragged store, whose spacing ``rollout_forward_ragged`` picks once the trajectories' lengths are known."""
+    try:
+        return choose_ckpt_every(K, d, n_steps_lim, budget_bytes=PATH_BUDGET_BYTES, hidden=hidden)
+    except L.RlsdeError:
+        return None
+
+
+def choose_ragged_ckpt_every(slot_totals, d, hidden=32):
+    """Smallest spacing C of RAGGED_SPACINGS (hidden width 32; C = 1 above, where the reverse pass reads every state) whose
+    ragged store fits the budget of ``choose_ckpt_every``.  ``slot_totals[i]``: sum_k (floor(T_k / C) + 1) over the
+    finished trajectories at C = RAGGED_SPACINGS[i]."""
+    budget = PATH_BUDGET_BYTES if hidden == 32 else max(PATH_BUDGET_BYTES, 32 << 30)
+    for c, n in zip(RAGGED_SPACINGS if hidden == 32 else RAGGED_SPACINGS[:1], slot_totals):
+        if int(n) * d * 4 <= budget:
+            return c
+    raise L.RlsdeError(f"the checkpoints of the passes the trajectories ran ({int(slot_totals[0])} states of d={d}) do not fit "
+                       f"{budget / 2**30:.1f} GiB even at spacing {32 if hidden == 32 else 1}; pass a smaller batch")
+
+
+def rollout_forward_ragged(env_c, mlp_c, params_host, K, *, kernel="auto", device=None, **opts):
+    """``rollout_forward(store_path=True)`` into the ragged checkpoint store: memory for the passes the trajectories run,
+    not for the pass budget.  Two rollouts with the same counter-based noise: the first stores nothing (a base of zeros,
+    so it runs the kernels of the second) and yields the hit indices; their checkpoint counts size the store (one host
+    synchronisation, which also picks the spacing, ``choose_ragged_ckpt_every``); the second fills it.  Raises if the
+    two rollouts' hit indices differ.  The returned ``path_base`` marks the store as ragged for ``rollout_backward``."""
+    dev = _cuda_device(device)
+    K = int(K)
+    d, H = env_c.d, int(mlp_c.d_hidden)
+    if kernel == "auto" and H == 32 and K <= 16 * torch.cuda.get_device_properties(dev).multi_processor_count:
+        # the warp-per-trajectory kernels store every state or nothing (ckpt_every = 1): the spacing is known only after
+        # the first rollout, so both run the thread-per-trajectory kernel
+        kernel = "thread"
+    common = dict(opts, store_path=True, want_logw=False, device=dev, kernel=kernel)
+    first = rollout_forward(env_c, mlp_c, params_host, K, ckpt_every=1, path_base=torch.zeros(K + 1, dtype=torch.int64, device=dev),
+                            **common)
+    spacings = RAGGED_SPACINGS if H == 32 else RAGGED_SPACINGS[:1]
+    totals = torch.stack([ragged_ckpt_counts(first.T, c).sum() for c in spacings]).cpu().numpy() if K > 0 else [0] * len(spacings)
+    c = choose_ragged_ckpt_every(totals, d, hidden=H)
+    base, _ = slot_offsets(ragged_ckpt_counts(first.T, c))
+    out = rollout_forward(env_c, mlp_c, params_host, K, ckpt_every=c, path_base=base, n_slots=int(totals[spacings.index(c)]),
+                          **common)
+    if K > 0 and not torch.equal(out.T, first.T):
+        raise L.RlsdeError("the two rollouts of the ragged checkpoint store disagree on the hit indices")
+    return out
+
+
+def rollout_forward_stored(env_c, mlp_c, params_host, K, *, ckpt_every=1, **opts):
+    """The training rollout: checkpoints in the dense store at spacing ``ckpt_every``, or in the ragged store when
+    ``ckpt_every`` is None (``choose_path_store``)."""
+    if ckpt_every is None:
+        return rollout_forward_ragged(env_c, mlp_c, params_host, K, **opts)
+    return rollout_forward(env_c, mlp_c, params_host, K, store_path=True, want_logw=False, ckpt_every=ckpt_every, **opts)
+
+
 def rollout_backward(env_c, mlp_c, params_host, fwd: RolloutOut, loss_scale, *, noise=None, device=None, balance=True,
                      coef=None):
     """K2: gradient of loss_scale * sum_k(-G_k - sg(G_k) S_k) w.r.t. the flat parameters (float32 CUDA tensor).
 
     With ``coef=(coef_G, coef_S)`` (float32 CUDA tensors [K] on the rollout's device) the gradient is that of
     loss_scale * sum_k (coef_G[k] G_k + coef_S[k] S_k) instead (rlsde_rollout_bwd_weighted; unfinished trajectories
-    contribute 0)."""
+    contribute 0).  A rollout with the ragged store (``fwd.path_base``) takes the weighted pass over it
+    (rlsde_rollout_bwd_ragged), with coefficients (-1, -G) for the plain surrogate."""
     lib = L.load()
     dev = _cuda_device(device)
     if fwd.path is None:
         raise L.RlsdeError("the forward rollout must be run with store_path=True")
+    if fwd.path_base is not None and coef is None:
+        coef = (torch.full_like(fwd.G, -1.0), torch.neg(fwd.G))
     if coef is not None:
         coef = tuple(coef)
         K = fwd.T.numel()
@@ -358,14 +455,19 @@ def rollout_backward(env_c, mlp_c, params_host, fwd: RolloutOut, loss_scale, *, 
         thread_path = (fwd.cfg.flags & L.F_KERNEL_THREAD) or not ((fwd.cfg.flags & L.F_KERNEL_WARP) or fwd.T.numel() <= 16 * n_sm)
         order = torch.argsort(fwd.T, descending=True, stable=True) if balance and thread_path and fwd.T.numel() > 32 else None
         stream = torch.cuda.current_stream(dev).cuda_stream
-        if coef is None:
+        if fwd.path_base is not None:
+            rc = lib.rlsde_rollout_bwd_ragged(env_c, mlp_c, params_host.ctypes.data, fwd.cfg, _ptr(noise), _ptr(coef[0]),
+                                              _ptr(coef[1]), _ptr(fwd.T), _ptr(fwd.path_base), _ptr(fwd.path), _ptr(order),
+                                              float(loss_scale), _ptr(grad), _ptr(ws), ws.numel(), stream)
+        elif coef is None:
             rc = lib.rlsde_rollout_bwd(env_c, mlp_c, params_host.ctypes.data, fwd.cfg, _ptr(noise), _ptr(fwd.G), _ptr(fwd.T),
                                        _ptr(fwd.path), _ptr(order), float(loss_scale), _ptr(grad), _ptr(ws), ws.numel(), stream)
         else:
             rc = lib.rlsde_rollout_bwd_weighted(env_c, mlp_c, params_host.ctypes.data, fwd.cfg, _ptr(noise), _ptr(coef[0]),
                                                 _ptr(coef[1]), _ptr(fwd.T), _ptr(fwd.path), _ptr(order), float(loss_scale),
                                                 _ptr(grad), _ptr(ws), ws.numel(), stream)
-    L.check(rc, "rlsde_rollout_bwd_weighted" if coef is not None else "rlsde_rollout_bwd")
+    L.check(rc, "rlsde_rollout_bwd_ragged" if fwd.path_base is not None else
+            "rlsde_rollout_bwd_weighted" if coef is not None else "rlsde_rollout_bwd")
     return grad
 
 
@@ -379,7 +481,8 @@ def rollout_loss_and_grad(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=1
 
     Returns ``(stats float64[RLSDE_NSTATS], grad float32[P] of mean_k(-G_k - sg(G_k) S_k), G float32[K], T int32[K])``
     as NumPy arrays.  With ``dist`` (a ``distributed.Shard``) the K trajectories are this rank's shard: statistics and
-    gradient are those of the global batch (one all-gather of the packed rows), G and T stay local."""
+    gradient are those of the global batch (one all-gather of the packed rows), G and T stay local.  ``ckpt_every=None``:
+    the ragged checkpoint store (``rollout_forward_ragged``), at the cost of one more rollout and synchronisation."""
     lib = L.load()
     dev = _cuda_device(device)
     K = int(K)
@@ -411,23 +514,34 @@ def rollout_loss_and_grad(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=1
     flags |= {"reference": 0, "exact": L.F_STOCH_INT_EXACT}[stoch_int]
     flags |= {"auto": 0, "thread": L.F_KERNEL_THREAD, "warp": L.F_KERNEL_WARP, "tensor": L.F_KERNEL_TENSOR}[kernel]
     lim_eff = min(cfg.n_steps_lim, cfg.noise_steps) if noise is not None else cfg.n_steps_lim
-    cfg.ckpt_every = int(ckpt_every)
-    cfg.ckpt_stride = (lim_eff + cfg.ckpt_every - 1) // cfg.ckpt_every
-    cfg.flags = flags
-    L.apply_tuning(cfg, tuning)
-    path = torch.empty((K, cfg.ckpt_stride, env_c.d), dtype=torch.float32, device=dev)
     ws = _workspace(dev, K, mlp_c)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib.rlsde_rollout_fwd(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), 0, _ptr(G), _ptr(S), _ptr(T), 0, 0,
-                                   _ptr(path), _ptr(stats), _ptr(ws), ws.numel(), stream)
-        L.check(rc, "rlsde_rollout_fwd")
-        n_sm = torch.cuda.get_device_properties(dev).multi_processor_count
-        thread_path = (flags & L.F_KERNEL_THREAD) or not ((flags & L.F_KERNEL_WARP) or K <= 16 * n_sm)
-        order = torch.argsort(T, descending=True, stable=True) if balance and thread_path and K > 32 else None
-        rc = lib.rlsde_rollout_bwd(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), _ptr(G), _ptr(T), _ptr(path),
-                                   _ptr(order), 1.0 / cfg.K_global, _ptr(grad), _ptr(ws), ws.numel(), stream)
-        L.check(rc, "rlsde_rollout_bwd")
+        if ckpt_every is None:
+            # the ragged checkpoint store (choose_path_store): one more rollout and one more synchronisation
+            out = rollout_forward_ragged(env_c, mlp_c, params_host, K, seed=seed, n_steps_lim=n_steps_lim, noise=noise, tanh=tanh,
+                                         stoch_int=stoch_int, traj_offset=cfg.traj_offset, K_global=cfg.K_global, kernel=kernel,
+                                         tuning=tuning, device=dev)
+            grad.copy_(rollout_backward(env_c, mlp_c, params_host, out, 1.0 / cfg.K_global, noise=noise, device=dev,
+                                        balance=balance))
+            stats.copy_(out.stats_dev)
+            G.copy_(out.G)
+            T.copy_(out.T)
+        else:
+            cfg.ckpt_every = int(ckpt_every)
+            cfg.ckpt_stride = (lim_eff + cfg.ckpt_every - 1) // cfg.ckpt_every
+            cfg.flags = flags
+            L.apply_tuning(cfg, tuning)
+            path = torch.empty((K, cfg.ckpt_stride, env_c.d), dtype=torch.float32, device=dev)
+            rc = lib.rlsde_rollout_fwd(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), 0, _ptr(G), _ptr(S), _ptr(T), 0, 0,
+                                       _ptr(path), _ptr(stats), _ptr(ws), ws.numel(), stream)
+            L.check(rc, "rlsde_rollout_fwd")
+            n_sm = torch.cuda.get_device_properties(dev).multi_processor_count
+            thread_path = (flags & L.F_KERNEL_THREAD) or not ((flags & L.F_KERNEL_WARP) or K <= 16 * n_sm)
+            order = torch.argsort(T, descending=True, stable=True) if balance and thread_path and K > 32 else None
+            rc = lib.rlsde_rollout_bwd(env_c, mlp_c, params_host.ctypes.data, cfg, _ptr(noise), _ptr(G), _ptr(T), _ptr(path),
+                                       _ptr(order), 1.0 / cfg.K_global, _ptr(grad), _ptr(ws), ws.numel(), stream)
+            L.check(rc, "rlsde_rollout_bwd")
         if dist is not None and dist.world_size > 1:
             # the iteration's ONE exchange (SURVEY 8e): every rank's [gradient | statistics] row, added in rank order
             from .distributed import pack_grad_and_stats, reduce_gathered
