@@ -1,4 +1,4 @@
 // weighted reverse-pass kernels (rlsde_rollout_bwd_weighted) for d = 1, hidden width = 32: the thread-per-trajectory
 // CUDA-core family (a translation unit of its own, like every weighted instantiation: the unweighted kernels keep their code)
 #include "rollout_bwd_inst.cuh"
-RLSDE_INSTANTIATE_BWD_WEIGHTED(1, 32)
+RLSDE_INSTANTIATE_BWD(1, 32, true, false)

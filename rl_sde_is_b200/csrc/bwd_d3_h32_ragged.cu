@@ -1,4 +1,4 @@
 // weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged) for d = 3, hidden width = 32: the
 // thread-per-trajectory CUDA-core family
 #include "rollout_bwd_inst.cuh"
-RLSDE_INSTANTIATE_BWD_RAGGED(3, 32)
+RLSDE_INSTANTIATE_BWD(3, 32, true, true)

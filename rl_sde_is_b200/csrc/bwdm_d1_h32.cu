@@ -1,3 +1,3 @@
 // tensor-core (mma.sync, float16 x 3 split) reverse-pass kernels for d = 1, hidden width = 32
 #include "rollout_bwd_mma_inst.cuh"
-RLSDE_INSTANTIATE_BWD_MMA(1)
+RLSDE_INSTANTIATE_BWD_MMA(1, false, false)

@@ -2,5 +2,5 @@
 // thread-per-trajectory family and the warp-per-trajectory kernel
 #include "rollout_bwd_mma_inst.cuh"
 #include "rollout_warp_inst.cuh"
-RLSDE_INSTANTIATE_BWD_MMA_WEIGHTED(2)
-RLSDE_INSTANTIATE_BWD_WARP_WEIGHTED(2)
+RLSDE_INSTANTIATE_BWD_MMA(2, true, false)
+RLSDE_INSTANTIATE_BWD_WARP(2, true, false)

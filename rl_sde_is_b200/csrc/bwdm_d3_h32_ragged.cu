@@ -2,5 +2,5 @@
 // tensor-core thread-per-trajectory family and the warp-per-trajectory kernel
 #include "rollout_bwd_mma_inst.cuh"
 #include "rollout_warp_inst.cuh"
-RLSDE_INSTANTIATE_BWD_MMA_RAGGED(3)
-RLSDE_INSTANTIATE_BWD_WARP_RAGGED(3)
+RLSDE_INSTANTIATE_BWD_MMA(3, true, true)
+RLSDE_INSTANTIATE_BWD_WARP(3, true, true)

@@ -50,20 +50,28 @@ static int cuda_fail(cudaError_t e, const char* where) {
   return RLSDE_ERR_CUDA;
 }
 
-// shapes with compiled fused kernels: X(d, H).  Hidden width 32: the fully unrolled register / constant-bank kernels
+// The policy shapes (d, H) with compiled fused kernels, the one list: with_shape calls f(Shape<D, H>{}) for a compiled shape
+// and returns RLSDE_ERR_UNSUPPORTED for any other.  Hidden width 32: the fully unrolled register / constant-bank kernels
 // (rollout_fwd.cuh, rollout_bwd*.cuh, rollout_warp.cuh).  Hidden widths 64 / 128 / 256 (the reference's reinforce()
 // default is 256): the tile kernels of rollout_wide.cuh, for the state dimensions the reference has environments for.
-#define RLSDE_SHAPES(X) X(1, 32) X(2, 32) X(3, 32) X(4, 32) X(10, 32)
-#define RLSDE_WIDE_SHAPES(X) X(1, 64) X(1, 128) X(1, 256) X(2, 64) X(2, 128) X(2, 256)
-#define RLSDE_UMMA_SHAPES(X) X(1, 128) X(1, 256) X(2, 128) X(2, 256)
-#define RLSDE_UMMA_FWD_SHAPES(X) X(1, 64) X(2, 64) RLSDE_UMMA_SHAPES(X)      /* forward only: width 64 with resident weights */
-#define RLSDE_UMMA_NARROW_SHAPES(X) X(1, 32) X(2, 32) X(3, 32) X(4, 32) X(10, 32)
+// The predicates say which kernel families a shape has; the callers test them with if constexpr, so that no launcher is
+// referenced for a shape that has none.
+template <int D_, int H_>
+struct Shape {
+  static constexpr int D = D_, H = H_;
+  static constexpr bool narrow = H == 32;          // K1, K1w, K2, K2m, K2w and the H = 32 tcgen05 forward (K1u)
+  static constexpr bool wide = H >= 64;            // K1x, K2x
+  static constexpr bool umma_fwd_wide = H >= 64;   // the tcgen05 forward at H >= 64 (K1u)
+  static constexpr bool umma_bwd = H >= 128;       // the tcgen05 reverse pass (K2u)
+};
 
-static bool shape_is_wide(int d, int H) {
-#define X(D_, H_) if (d == D_ && H == H_) return true;
-  RLSDE_WIDE_SHAPES(X)
+template <class F>
+static int with_shape(int d, int H, F&& f) {
+#define X(D_, H_) \
+  if (d == D_ && H == H_) return f(Shape<D_, H_>{});
+  X(1, 32) X(2, 32) X(3, 32) X(4, 32) X(10, 32) X(1, 64) X(1, 128) X(1, 256) X(2, 64) X(2, 128) X(2, 256)
 #undef X
-  return false;
+  return RLSDE_ERR_UNSUPPORTED;
 }
 
 // smallest batch the tcgen05 tile kernels take automatically.  They advance 128-trajectory tiles at ~13 us (forward) /
@@ -73,11 +81,7 @@ static bool shape_is_wide(int d, int H) {
 static long long umma_min_k(int H, int sm) { return H >= 256 ? 4 * UMMA_M : (long long)sm * UMMA_M / 2; }
 
 static bool shape_supported(int d, int H, int n_hidden) {
-  if (n_hidden != 2) return false;
-#define X(D_, H_) if (d == D_ && H == H_) return true;
-  RLSDE_SHAPES(X)
-#undef X
-  return shape_is_wide(d, H);
+  return n_hidden == 2 && with_shape(d, H, [](auto) { return RLSDE_OK; }) == RLSDE_OK;
 }
 
 // kernel family for a call: latency kernels (warp per trajectory) for small batches, throughput kernels otherwise
@@ -110,24 +114,27 @@ static int check_env_mlp(const rlsde_env* env, const rlsde_mlp* mlp) {
   return RLSDE_OK;
 }
 
-static void fill_env(const rlsde_env* env, FwdArgs& A) {
-  for (int i = 0; i < RLSDE_MAX_D; ++i) {
-    const double al = i < env->d ? env->alpha[i] : 0.0;
-    A.c4a_d[i] = 4.0 * al;
-    A.c4a_f[i] = (float)(4.0 * al);   // torch multiplies the f32 state by the python scalar 4*alpha cast to f32
-    A.x0_d[i] = i < env->d ? (double)(float)env->x0[i] : 0.0;   // state_init is float32 (environments.py:30)
-    A.x0_f[i] = i < env->d ? (float)env->x0[i] : 0.f;
-  }
-  A.sigma_d = env->sigma; A.sigma_f = (float)env->sigma;   // sigma_tensor / dt_tensor are float32 (environments.py:19,23)
+// the environment constants FwdArgs and StepArgs share, rounded the way the reference rounds them: torch multiplies the
+// f32 state by the python scalar 4*alpha cast to f32; sigma_tensor / dt_tensor are float32 (environments.py:19,23).  The
+// caller has zeroed A.
+template <class Args>
+static void fill_env_consts(const rlsde_env* env, Args& A) {
+  for (int i = 0; i < env->d; ++i) { A.c4a_d[i] = 4.0 * env->alpha[i]; A.c4a_f[i] = (float)(4.0 * env->alpha[i]); }
+  A.sigma_d = env->sigma; A.sigma_f = (float)env->sigma;
   A.dt_d = env->dt; A.dt_f = (float)env->dt;
   A.lb_d = env->lb; A.rb_d = env->rb; A.lb_f = (float)env->lb; A.rb_f = (float)env->rb;
   A.noise_scale2 = (float)(-2.0 * env->dt * 0.6931471805599453);
   A.hit_rule = env->hit_rule;
 }
 
+// passes an undetected trajectory executes: the budget, or the injected noise if that is shorter
+static long long passes_run(const FwdArgs& A) {
+  return (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
+}
+
 // ragged: the checkpoints go to the ragged store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged), whose size the
 // caller has fitted to the trajectories: cfg->ckpt_stride is not read
-static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A, bool ragged = false) {
+static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A, bool ragged) {
   if (!cfg || cfg->K < 0 || cfg->n_steps_lim < 1 || cfg->n_steps_lim > 2000000000LL) return RLSDE_ERR_INVALID_ARG;
   if (cfg->traj_offset < 0) return RLSDE_ERR_INVALID_ARG;
   if ((cfg->flags & RLSDE_F_NOISE_INJECTED) && cfg->noise_steps < 1) return RLSDE_ERR_INVALID_ARG;
@@ -140,9 +147,7 @@ static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A, bool ragged = fals
   A.flags = cfg->flags; A.ckpt_every = cfg->ckpt_every > 0 ? cfg->ckpt_every : 1; A.ckpt_stride = cfg->ckpt_stride;
   if ((cfg->flags & RLSDE_F_STORE_PATH) && !ragged) {
     // the kernels write path[(traj * ckpt_stride + k / ckpt_every) * d] for every pass k they execute
-    const long long lim_eff = (cfg->flags & RLSDE_F_NOISE_INJECTED) && cfg->noise_steps < cfg->n_steps_lim ? cfg->noise_steps
-                                                                                                             : cfg->n_steps_lim;
-    if (cfg->ckpt_every < 1 || cfg->ckpt_stride < (lim_eff + cfg->ckpt_every - 1) / cfg->ckpt_every) return RLSDE_ERR_INVALID_ARG;
+    if (cfg->ckpt_every < 1 || cfg->ckpt_stride < (passes_run(A) + cfg->ckpt_every - 1) / cfg->ckpt_every) return RLSDE_ERR_INVALID_ARG;
   }
   A.ckpt_log2 = -1;
   for (int b = 0; b < 31; ++b)
@@ -153,13 +158,69 @@ static int fill_cfg(const rlsde_rollout_cfg* cfg, FwdArgs& A, bool ragged = fals
   return RLSDE_OK;
 }
 
-// workspace layout: [0, 1024) counters (u64: items claimed, records queued, trajectories completed); statistics partials;
-// reverse-pass partials; then, to the end of the buffer, the ring of continuation records of the time-sliced forward
-// rollout (one record per trajectory + one per lane: rlsde_workspace_bytes(K) sizes it for the largest record)
+// the arguments every rollout and reverse pass starts from: the environment and the cfg; the ragged store implies
+// RLSDE_F_STORE_PATH
+static int make_args(const rlsde_env* env, const rlsde_rollout_cfg* cfg, FwdArgs& A, bool ragged = false) {
+  memset(&A, 0, sizeof(A));
+  fill_env_consts(env, A);
+  for (int i = 0; i < env->d; ++i) {
+    A.x0_d[i] = (double)(float)env->x0[i];     // state_init is float32 (environments.py:30)
+    A.x0_f[i] = (float)env->x0[i];
+  }
+  const int rc = fill_cfg(cfg, A, ragged);
+  if (rc == RLSDE_OK && ragged) A.flags |= RLSDE_F_STORE_PATH;
+  return rc;
+}
+
+// Workspace layout, in order: counters (u64: items claimed, records queued, trajectories completed); statistics partials;
+// device copy of the packed policy (device-resident training step); reverse-pass partials; device image of a wide policy
+// (rollout_wide.cuh); float16 hi / lo image of W2 for the tcgen05 kernels (H = 256).  Then, to the end of the buffer, the
+// ring of continuation records of the time-sliced forward rollout (one record per trajectory + one per lane:
+// rlsde_workspace_bytes(K) sizes it for the largest record), or the tcgen05 reverse pass's exchange ring and float64
+// partials (rlsde_workspace_bytes_bwd).
 constexpr size_t WS_COUNTER_BYTES = 1024;
 constexpr size_t WS_STATS_BYTES = (size_t)STATS_BLOCKS * RLSDE_NSTATS * sizeof(double);
+constexpr size_t WS_POLICY_BYTES = 16384;
+constexpr size_t WS_WIDE_BYTES = (WIDE_PARAM_BYTES_MAX + 255) & ~(size_t)255;
+constexpr size_t WS_UMMA_BYTES = 256 * 256 * 4;
 constexpr long long WS_MAX_LANES = 148LL * 16 * 128;                          // lanes of the largest forward grid
 constexpr size_t WS_CONT_REC_BYTES = 16 + 8 * (RLSDE_MAX_D + 3);              // >= sizeof(ContRec<D, F64>) for every D
+static_assert(sizeof(MlpConst<RLSDE_MAX_D, WARP_H>) <= WS_POLICY_BYTES, "raise WS_POLICY_BYTES");
+
+struct Workspace {
+  static constexpr size_t o_stats = WS_COUNTER_BYTES;
+  static constexpr size_t o_policy = o_stats + WS_STATS_BYTES;     // also the least a forward rollout takes
+  static constexpr size_t o_bwd = o_policy + WS_POLICY_BYTES;
+  static size_t o_wide() { return o_bwd + bwd_workspace_bytes(); }
+  static size_t o_umma() { return o_wide() + WS_WIDE_BYTES; }
+  static size_t fixed_bytes() { return o_umma() + WS_UMMA_BYTES; }
+
+  char* base;
+  unsigned long long* counters() const { return (unsigned long long*)base; }
+  double* stats() const { return (double*)(base + o_stats); }
+  void* policy() const { return base + o_policy; }
+  float* bwd_partial() const { return (float*)(base + o_bwd); }
+  float* wide_params() const { return (float*)(base + o_wide()); }
+  uint8_t* umma_image() const { return (uint8_t*)base + o_umma(); }
+  uint8_t* tail() const { return (uint8_t*)base + fixed_bytes(); }
+};
+
+static int launch_status(int lrc, const char* what) { return lrc != 0 ? cuda_fail((cudaError_t)lrc, what) : RLSDE_OK; }
+
+// the device's SM count, and the work counters cleared on the stream
+static int begin_launch(const Workspace& ws, cudaStream_t stream, int& sm) {
+  const int rc = device_sm_count(&sm);
+  if (rc != RLSDE_OK) return rc;
+  const cudaError_t e = cudaMemsetAsync(ws.base, 0, WS_COUNTER_BYTES, stream);
+  return e != cudaSuccess ? cuda_fail(e, "cudaMemsetAsync(workspace)") : RLSDE_OK;
+}
+
+// the statistics record of a rollout (stats_dev may be null: none)
+static int reduce_stats(const FwdArgs& A, double* stats_dev, const Workspace& ws, cudaStream_t stream) {
+  if (!stats_dev) return RLSDE_OK;
+  return launch_status(launch_reduce_stats(A.K, passes_run(A), (A.flags & RLSDE_F_STATE_F64) != 0, A.G, A.S, A.T, A.l2, A.logw,
+                                           stats_dev, ws.stats(), stream), "reduce_stats launch");
+}
 
 }  // namespace rlsde
 
@@ -210,42 +271,27 @@ int64_t rlsde_param_count(const rlsde_mlp* mlp) {
   return d * H + H + (int64_t)(mlp->n_hidden - 1) * (H * H + H) + H * o + o;
 }
 
-constexpr size_t WS_POLICY_BYTES = 16384;          // device copy of the packed policy (device-resident training step)
-constexpr size_t WS_WIDE_BYTES = (WIDE_PARAM_BYTES_MAX + 255) & ~(size_t)255;   // device image of a wide policy (rollout_wide.cuh)
-constexpr size_t WS_UMMA_BYTES = 256 * 256 * 4;     // float16 hi / lo image of W2 streamed by the tcgen05 forward kernel (H = 256)
-static size_t ws_fixed_bytes() {
-  return WS_COUNTER_BYTES + WS_STATS_BYTES + WS_POLICY_BYTES + bwd_workspace_bytes() + WS_WIDE_BYTES + WS_UMMA_BYTES;
-}
-static uint8_t* ws_umma_image(void* workspace_dev) {
-  return (uint8_t*)workspace_dev + WS_COUNTER_BYTES + WS_STATS_BYTES + WS_POLICY_BYTES + bwd_workspace_bytes() + WS_WIDE_BYTES;
-}
-static float* ws_wide_params(void* workspace_dev) {
-  return (float*)((char*)workspace_dev + WS_COUNTER_BYTES + WS_STATS_BYTES + WS_POLICY_BYTES + bwd_workspace_bytes());
-}
-
 size_t rlsde_workspace_bytes(int64_t K) {
   const long long k = K > 0 ? K : 0;
   long long cap = 1;
   while (cap < k + WS_MAX_LANES) cap <<= 1;             // the ring's capacity is a power of two
-  return ws_fixed_bytes() + (size_t)cap * WS_CONT_REC_BYTES;
+  return Workspace::fixed_bytes() + (size_t)cap * WS_CONT_REC_BYTES;
 }
 
-// Reverse pass of a wide policy on the tensor cores (rollout_umma_bwd.cuh): its exchange ring and float64 partials live
-// behind the fixed part of the workspace, where the forward rollout keeps its continuation records.
-static size_t bwd_umma_scratch(int d, int H, int sm) {
-#define X(D_, H_) if (d == D_ && H == H_) return bwd_umma_scratch_bytes<D_, H_>(sm);
-  RLSDE_UMMA_SHAPES(X)
-#undef X
-  return 0;
-}
-
+// the reverse pass of a wide policy on the tensor cores (rollout_umma_bwd.cuh) keeps its scratch behind the fixed part
 size_t rlsde_workspace_bytes_bwd(int64_t K, int32_t d, int32_t d_hidden) {
   size_t n = rlsde_workspace_bytes(K);
-  int sm = 0;
-  if ((d_hidden == 128 || d_hidden == 256) && device_sm_count(&sm) == RLSDE_OK) {
-    const size_t need = ws_fixed_bytes() + bwd_umma_scratch(d, d_hidden, sm);
-    if (need > n) n = need;
-  }
+  with_shape(d, d_hidden, [&](auto s) {
+    using S = decltype(s);
+    int sm = 0;
+    if constexpr (S::umma_bwd) {
+      if (device_sm_count(&sm) == RLSDE_OK) {
+        const size_t need = Workspace::fixed_bytes() + bwd_umma_scratch_bytes<S::D, S::H>(sm);
+        if (need > n) n = need;
+      }
+    }
+    return RLSDE_OK;
+  });
   return n;
 }
 
@@ -271,17 +317,14 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   int rc = check_env_mlp(env, mlp);
   if (rc != RLSDE_OK) return rc;
   if (!params_host || !G_dev || !S_dev || !T_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
-  if (workspace_bytes < WS_COUNTER_BYTES + WS_STATS_BYTES) return RLSDE_ERR_WORKSPACE;
+  if (workspace_bytes < Workspace::o_policy) return RLSDE_ERR_WORKSPACE;
   FwdArgs A;
-  memset(&A, 0, sizeof(A));
-  fill_env(env, A);
-  if ((rc = fill_cfg(cfg, A, RAGGED)) != RLSDE_OK) return rc;
+  if ((rc = make_args(env, cfg, A, RAGGED)) != RLSDE_OK) return rc;
   if (RAGGED) {
     // the store exists for the reverse pass, so it takes that pass's conditions: a float32 state, no projection (below)
     // and at most BWD_MAX_SEG passes per checkpoint
     if (!path_base || !path_dev || tr.base) return RLSDE_ERR_INVALID_ARG;
     if (cfg->ckpt_every < 1 || cfg->ckpt_every > BWD_MAX_SEG) return RLSDE_ERR_INVALID_ARG;
-    A.flags |= RLSDE_F_STORE_PATH;
     if (A.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;
     if (A.flags & RLSDE_F_STATE_F64) return RLSDE_ERR_UNSUPPORTED;
   }
@@ -300,142 +343,97 @@ static int rollout_fwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   A.tr_next = tr.next_state; A.tr_done = tr.done;
   if (RAGGED) A.path_base = path_base;                  // shares tr_base's field: the ragged kernels have no stream
   if (tr.base) A.flags = (A.flags & ~RLSDE_F_KERNEL_WARP) | RLSDE_F_KERNEL_THREAD;   // the stream lives in the throughput kernel
-  A.counter = (unsigned long long*)workspace_dev;
-  A.q_ctrl = (unsigned long long*)workspace_dev;
-  if (workspace_bytes > ws_fixed_bytes()) {             // ring of continuation records: whatever lies behind the fixed part
-    A.q_ring = (unsigned char*)workspace_dev + ws_fixed_bytes();
-    A.q_cap = (long long)(workspace_bytes - ws_fixed_bytes());      // bytes; the launcher turns it into a record count
+  const Workspace ws{(char*)workspace_dev};
+  A.counter = ws.counters();
+  A.q_ctrl = ws.counters();
+  if (workspace_bytes > Workspace::fixed_bytes()) {     // ring of continuation records: whatever lies behind the fixed part
+    A.q_ring = ws.tail();
+    A.q_cap = (long long)(workspace_bytes - Workspace::fixed_bytes());   // bytes; the launcher turns it into a record count
   }
   if (A.K == 0) return RLSDE_OK;
   int sm = 0;
-  if ((rc = device_sm_count(&sm)) != RLSDE_OK) return rc;
-  cudaError_t e = cudaMemsetAsync(workspace_dev, 0, WS_COUNTER_BYTES, stream);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-  int lrc = -1;
-  if (shape_is_wide(env->d, mlp->d_hidden)) {
-    // wide policies: one kernel family (tiles of trajectories per block), no transition stream, no time slices
-    if (tr.base) return RLSDE_ERR_UNSUPPORTED;
-    if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
-    // hidden width 64 / 128 / 256 with enough trajectories (umma_min_k: four 128-row tiles at H = 256, half the SMs below): the tcgen05 kernel
-    // (rollout_umma.cuh; weights resident at width 64, streamed above); otherwise the CUDA-core tile kernel (rollout_wide.cuh).
-    // cfg.wide_kernel: 1 forces tcgen05, 2 forces the CUDA-core kernel.
-    const bool umma_shape = mlp->d_hidden == 64 || mlp->d_hidden == 128 || mlp->d_hidden == 256;
-    const bool use_umma = umma_shape && (cfg->wide_kernel == 1 || (cfg->wide_kernel == 0 && A.K >= umma_min_k(mlp->d_hidden, sm)));
-    if (use_umma) {
-#define X(D_, H_)                                                                                                          \
-  if (env->d == D_ && mlp->d_hidden == H_)                                                                                 \
-    lrc = launch_rollout_fwd_umma<D_, H_, RAGGED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A, sm, stream);
-      RLSDE_UMMA_FWD_SHAPES(X)
-#undef X
-    } else {
-#define X(D_, H_) \
-  if (env->d == D_ && mlp->d_hidden == H_) lrc = launch_rollout_fwd_wide<D_, H_, RAGGED>(params_host, ws_wide_params(workspace_dev), A, sm, stream);
-      RLSDE_WIDE_SHAPES(X)
-#undef X
-    }
-    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd (wide) launch");
-    if (stats_dev) {
-      double* partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
-      const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
-      lrc = launch_reduce_stats(A.K, lim_eff, (A.flags & RLSDE_F_STATE_F64) != 0, G_dev, S_dev, T_dev, l2_dev, logw_dev,
-                                stats_dev, partial, stream);
-      if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reduce_stats launch");
-    }
-    return RLSDE_OK;
-  }
-  const bool warp_path = use_warp_kernels(A, mlp->d_hidden, sm, (A.flags & RLSDE_F_STORE_PATH) != 0);
-  // ---- policy arithmetic of the thread-per-trajectory kernel and of the kernel that continues its tail (mlp_mma.cuh or
-  // FFMA2).  A function of (d, H, cfg.fwd_policy) only: the replay sampler launches it twice, with and without the
-  // transition stream, and needs the same hit passes from both launches.
-  if (cfg->fwd_policy == 1 && !fwd_mma_shape(env->d, mlp->d_hidden)) return RLSDE_ERR_UNSUPPORTED;
-  A.policy_mma = fwd_mma_shape(env->d, mlp->d_hidden) && cfg->fwd_policy != 2 ? 1 : 0;
-  // ---- hidden width 32 on the tensor cores (rollout_umma.cuh with resident weights: tiles of 128 trajectories, one thread
-  // per trajectory, lane refill).  The per-pass work of a warp drops from ~1 290 to ~860 instructions; like K1 it ends up
-  // bound by the MUFU pipe (71 % busy with the two-MUFU tanh: profiles/r02/ncu_rollout_fwd_umma_h32_v1.txt).  Measured at
-  // 1e6 trajectories, budget 1 000 passes (tools/bench_fwd_kernels.py): d = 1 precise tanh 27.5 ms against K1's 25.1 ms,
-  // fast tanh 20.6 against 21.5; d = 2: 54.5 % of the FP32 roofline against 52 %; d = 4: 58.1 % against 53.4 %; d = 10:
-  // 50.9 % against 44.9 %.  It has no breadth-first schedule, so its launch ends with a tail of (longest trajectory) x
-  // (~1 us per pass).  At d = 1 the thread-per-trajectory kernel with its 32 x 32 layer on mma.sync (mlp_mma.cuh) beats it
-  // in both tanh modes: 21.1 / 15.4 ms against 27.4 / 20.6 ms (profiles/r03).  Automatic where it wins: d >= 2, large
-  // batches, a bounded pass budget -- and never when the caller pins a kernel family, a schedule or the policy arithmetic
-  // of the thread-per-trajectory kernel.
-  {
-    const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
-    const bool forced = (A.flags & RLSDE_F_KERNEL_TENSOR) != 0;
-    const bool pinned = (A.flags & (RLSDE_F_KERNEL_THREAD | RLSDE_F_KERNEL_WARP)) != 0 || cfg->fwd_quantum != 0 ||
-                        cfg->fwd_handoff != 0 || cfg->fwd_policy != 0;
-    const bool automatic = !pinned && !warp_path && A.K >= (long long)sm * UMMA_M * 2 && lim_eff <= 4096 && env->d >= 2;
-    if (mlp->d_hidden == 32 && !tr.base && (forced || automatic)) {
-      if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
-#define X(D_, H_)                                                                                                          \
-  if (env->d == D_ && mlp->d_hidden == H_)                                                                                 \
-    lrc = launch_rollout_fwd_umma<D_, H_, RAGGED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A, sm, stream);
-      RLSDE_UMMA_NARROW_SHAPES(X)
-#undef X
-      if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd (tensor) launch");
-      if (stats_dev) {
-        double* partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
-        lrc = launch_reduce_stats(A.K, lim_eff, (A.flags & RLSDE_F_STATE_F64) != 0, G_dev, S_dev, T_dev, l2_dev, logw_dev,
-                                  stats_dev, partial, stream);
-        if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reduce_stats launch");
+  if ((rc = begin_launch(ws, stream, sm)) != RLSDE_OK) return rc;
+  rc = with_shape(env->d, mlp->d_hidden, [&](auto shape) -> int {
+    using S = decltype(shape);
+    if constexpr (S::wide) {
+      // wide policies: one kernel family (tiles of trajectories per block), no transition stream, no time slices
+      if (tr.base) return RLSDE_ERR_UNSUPPORTED;
+      if (workspace_bytes < Workspace::fixed_bytes()) return RLSDE_ERR_WORKSPACE;
+      // hidden width 64 / 128 / 256 with enough trajectories (umma_min_k: four 128-row tiles at H = 256, half the SMs
+      // below): the tcgen05 kernel (rollout_umma.cuh; weights resident at width 64, streamed above); otherwise the
+      // CUDA-core tile kernel (rollout_wide.cuh).  cfg.wide_kernel: 1 forces tcgen05, 2 forces the CUDA-core kernel.
+      if constexpr (S::umma_fwd_wide) {
+        if (cfg->wide_kernel == 1 || (cfg->wide_kernel == 0 && A.K >= umma_min_k(S::H, sm)))
+          return launch_status(launch_rollout_fwd_umma<S::D, S::H, RAGGED>(params_host, ws.wide_params(), ws.umma_image(), A, sm,
+                                                                           stream), "rollout_fwd (wide) launch");
       }
+      return launch_status(launch_rollout_fwd_wide<S::D, S::H, RAGGED>(params_host, ws.wide_params(), A, sm, stream),
+                           "rollout_fwd (wide) launch");
+    } else {
+      const bool warp_path = use_warp_kernels(A, S::H, sm, (A.flags & RLSDE_F_STORE_PATH) != 0);
+      // ---- policy arithmetic of the thread-per-trajectory kernel and of the kernel that continues its tail (mlp_mma.cuh
+      // or FFMA2).  A function of (d, H, cfg.fwd_policy) only: the replay sampler launches it twice, with and without the
+      // transition stream, and needs the same hit passes from both launches.
+      if (cfg->fwd_policy == 1 && !fwd_mma_shape(S::D, S::H)) return RLSDE_ERR_UNSUPPORTED;
+      A.policy_mma = fwd_mma_shape(S::D, S::H) && cfg->fwd_policy != 2 ? 1 : 0;
+      // ---- hidden width 32 on the tensor cores (rollout_umma.cuh with resident weights: tiles of 128 trajectories, one
+      // thread per trajectory, lane refill).  The per-pass work of a warp drops from ~1 290 to ~860 instructions; like K1
+      // it ends up bound by the MUFU pipe (71 % busy with the two-MUFU tanh: profiles/r02/ncu_rollout_fwd_umma_h32_v1.txt).
+      // Measured at 1e6 trajectories, budget 1 000 passes (tools/bench_fwd_kernels.py): d = 1 precise tanh 27.5 ms against
+      // K1's 25.1 ms, fast tanh 20.6 against 21.5; d = 2: 54.5 % of the FP32 roofline against 52 %; d = 4: 58.1 % against
+      // 53.4 %; d = 10: 50.9 % against 44.9 %.  It has no breadth-first schedule, so its launch ends with a tail of
+      // (longest trajectory) x (~1 us per pass).  At d = 1 the thread-per-trajectory kernel with its 32 x 32 layer on
+      // mma.sync (mlp_mma.cuh) beats it in both tanh modes: 21.1 / 15.4 ms against 27.4 / 20.6 ms (profiles/r03).
+      // Automatic where it wins: d >= 2, large batches, a bounded pass budget -- and never when the caller pins a kernel
+      // family, a schedule or the policy arithmetic of the thread-per-trajectory kernel.
+      const long long passes = passes_run(A);
+      const bool forced = (A.flags & RLSDE_F_KERNEL_TENSOR) != 0;
+      const bool pinned = (A.flags & (RLSDE_F_KERNEL_THREAD | RLSDE_F_KERNEL_WARP)) != 0 || cfg->fwd_quantum != 0 ||
+                          cfg->fwd_handoff != 0 || cfg->fwd_policy != 0;
+      const bool automatic = !pinned && !warp_path && A.K >= (long long)sm * UMMA_M * 2 && passes <= 4096 && S::D >= 2;
+      if (!tr.base && (forced || automatic)) {
+        if (workspace_bytes < Workspace::fixed_bytes()) return RLSDE_ERR_WORKSPACE;
+        return launch_status(launch_rollout_fwd_umma<S::D, S::H, RAGGED>(params_host, ws.wide_params(), ws.umma_image(), A, sm,
+                                                                         stream), "rollout_fwd (tensor) launch");
+      }
+      // ---- schedule of the thread-per-trajectory kernel (rollout_fwd.cuh).  Two ways to deal with the tail of a launch:
+      //  * time slices (FIFO of continuation records, breadth-first): right when many trajectories run into the pass
+      //    budget -- the bench workload, 24 % of them: 24.5 ms against 27.8 ms; passes per slice = 1/128 of the budget,
+      //    between 8 and 128 (24.3 / 24.5 / 24.9 / 25.4 / 27.8 ms at 4 / 8 / 16 / 32 / 128) -- but 3-13 % slower in
+      //    steady state;
+      //  * run to completion and hand the last live trajectories to the warp-per-trajectory kernel (RESUME mode, K1's
+      //    arithmetic, ~5x faster on a lone trajectory): right when the tail is a few very long trajectories (metastable
+      //    configuration 5.68 -> 4.14 s, training forward 21.5 -> 13.9 ms, d = 2 test rollouts 16.6 -> 14.5 ms).
+      // Which one applies depends on the length distribution, which the launch only learns as it goes: it starts running
+      // to completion and switches to time slices as soon as 5 % of the completed trajectories have run into the budget
+      // (q_adaptive).  RLSDE_FWD_QUANTUM forces one or the other (0 = run to completion + hand-off, n = n-pass slices).
+      long long quantum = passes / 128 > 128 ? 128 : (passes / 128 < 8 ? 8 : passes / 128);
+      const bool can_hand_off = !tr.base;                   // the latency kernel has no transition stream
+      A.q_adaptive = can_hand_off ? 1 : 0;
+      if (!can_hand_off && passes > 4096) quantum = 0;
+      if (cfg->fwd_quantum != 0) { quantum = cfg->fwd_quantum > 0 ? cfg->fwd_quantum : 0; A.q_adaptive = 0; }
+      if (quantum > 0) {                                    // a power of two, at least one noise block (4 passes)
+        long long q2 = 4;
+        while (q2 < quantum && q2 < (1LL << 30)) q2 <<= 1;
+        quantum = q2;
+      }
+      A.q_quantum = (int)quantum;
+      A.q_handoff = (can_hand_off && (quantum == 0 || A.q_adaptive)) ? 4LL * warp_path_max_k(sm) : 0;
+      if (cfg->fwd_handoff != 0) {
+        if (A.q_handoff > 0) A.q_handoff = cfg->fwd_handoff;
+        if (A.q_handoff <= 0) { A.q_handoff = 0; A.q_adaptive = 0; }
+      }
+      const int lrc = warp_path ? launch_rollout_fwd_warp<S::D, RAGGED>(params_host, nullptr, A, sm, stream)
+                                : launch_rollout_fwd<S::D, S::H, RAGGED>(params_host, A, sm, stream);
+      if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd launch");
+      // the trajectories K1 left in the ring (none if it ran without one): one warp each, K1's arithmetic
+      if (!warp_path && A.q_handoff > 0 && (A.q_quantum == 0 || A.q_adaptive) && A.q_ring != nullptr)
+        return launch_status(launch_rollout_fwd_warp_resume<S::D, RAGGED>(params_host, A, sm, stream), "rollout_fwd resume launch");
       return RLSDE_OK;
     }
-  }
-  // ---- schedule of the thread-per-trajectory kernel (rollout_fwd.cuh).  Two ways to deal with the tail of a launch:
-  //  * time slices (FIFO of continuation records, breadth-first): right when many trajectories run into the pass budget
-  //    -- the bench workload, 24 % of them: 24.5 ms against 27.8 ms; passes per slice = 1/128 of the budget, between 8 and
-  //    128 (24.3 / 24.5 / 24.9 / 25.4 / 27.8 ms at 4 / 8 / 16 / 32 / 128) -- but 3-13 % slower in steady state;
-  //  * run to completion and hand the last live trajectories to the warp-per-trajectory kernel (RESUME mode, K1's
-  //    arithmetic, ~5x faster on a lone trajectory): right when the tail is a few very long trajectories (metastable
-  //    configuration 5.68 -> 4.14 s, training forward 21.5 -> 13.9 ms, d = 2 test rollouts 16.6 -> 14.5 ms).
-  // Which one applies depends on the length distribution, which the launch only learns as it goes: it starts running to
-  // completion and switches to time slices as soon as 5 % of the completed trajectories have run into the budget
-  // (q_adaptive).  RLSDE_FWD_QUANTUM forces one or the other (0 = run to completion + hand-off, n = n-pass slices).
-  {
-    const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
-    long long quantum = lim_eff / 128 > 128 ? 128 : (lim_eff / 128 < 8 ? 8 : lim_eff / 128);
-    const bool can_hand_off = mlp->d_hidden == WARP_H && !tr.base;     // the latency kernel has no transition stream
-    A.q_adaptive = can_hand_off ? 1 : 0;
-    if (!can_hand_off && lim_eff > 4096) quantum = 0;
-    if (cfg->fwd_quantum != 0) { quantum = cfg->fwd_quantum > 0 ? cfg->fwd_quantum : 0; A.q_adaptive = 0; }
-    if (quantum > 0) {                                    // a power of two, at least one noise block (4 passes)
-      long long q2 = 4;
-      while (q2 < quantum && q2 < (1LL << 30)) q2 <<= 1;
-      quantum = q2;
-    }
-    A.q_quantum = (int)quantum;
-    A.q_handoff = (can_hand_off && (quantum == 0 || A.q_adaptive)) ? 4LL * warp_path_max_k(sm) : 0;
-    if (cfg->fwd_handoff != 0) {
-      if (A.q_handoff > 0) A.q_handoff = cfg->fwd_handoff;
-      if (A.q_handoff <= 0) { A.q_handoff = 0; A.q_adaptive = 0; }
-    }
-  }
-#define X(D_, H_)                                                                              \
-  if (env->d == D_ && mlp->d_hidden == H_)                                                     \
-    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_fwd_warp<D_, RAGGED>(params_host, nullptr, A, sm, stream) \
-                                      : launch_rollout_fwd<D_, H_, RAGGED>(params_host, A, sm, stream);
-  RLSDE_SHAPES(X)
-#undef X
-  if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd launch");
-  if (!warp_path && A.q_handoff > 0 && (A.q_quantum == 0 || A.q_adaptive) && A.q_ring != nullptr) {
-    // the trajectories K1 left in the ring (none if it ran without one): one warp each, K1's arithmetic
-    lrc = -1;
-#define X(D_, H_) \
-  if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H) lrc = launch_rollout_fwd_warp_resume<D_, RAGGED>(params_host, A, sm, stream);
-    RLSDE_SHAPES(X)
-#undef X
-    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd resume launch");
-  }
-  if (stats_dev) {
-    double* partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
-    // passes an undetected trajectory has executed: the budget, or the injected noise if that is shorter
-    const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
-    lrc = launch_reduce_stats(A.K, lim_eff, (A.flags & RLSDE_F_STATE_F64) != 0, G_dev, S_dev, T_dev, l2_dev, logw_dev,
-                              stats_dev, partial, stream);
-    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reduce_stats launch");
-  }
-  return RLSDE_OK;
+  });
+  if (rc != RLSDE_OK) return rc;
+  return reduce_stats(A, stats_dev, ws, stream);
 }
 }  // extern "C++"
 
@@ -468,11 +466,9 @@ int rlsde_rollout_fwd_table(const rlsde_env* env, const float* u_table_dev, cons
   if (env->hit_rule != RLSDE_HIT_ALL_GE_LB && env->hit_rule != RLSDE_HIT_X0_IN_LB_RB) return RLSDE_ERR_INVALID_ARG;
   if (!u_table_dev || cfg->n_grid < 1 || !(cfg->grid_h > 0)) return RLSDE_ERR_INVALID_ARG;
   if (!G_dev || !S_dev || !T_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
-  if (workspace_bytes < WS_COUNTER_BYTES + WS_STATS_BYTES) return RLSDE_ERR_WORKSPACE;
+  if (workspace_bytes < Workspace::o_policy) return RLSDE_ERR_WORKSPACE;
   FwdArgs A;
-  memset(&A, 0, sizeof(A));
-  fill_env(env, A);
-  int rc = fill_cfg(cfg, A);
+  int rc = make_args(env, cfg, A);
   if (rc != RLSDE_OK) return rc;
   if (A.flags & RLSDE_F_STORE_PATH) return RLSDE_ERR_INVALID_ARG;                 // no reverse pass through a table
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
@@ -480,22 +476,13 @@ int rlsde_rollout_fwd_table(const rlsde_env* env, const float* u_table_dev, cons
   A.flags &= RLSDE_F_NOISE_INJECTED | RLSDE_F_STOCH_INT_EXACT | RLSDE_F_STATE_F64 | RLSDE_F_HIT_BRIDGE;
   A.noise = noise_dev; A.policy_opt = policy_opt_dev;
   A.G = G_dev; A.S = S_dev; A.T = T_dev; A.l2 = l2_dev; A.logw = logw_dev;
-  A.counter = (unsigned long long*)workspace_dev;
+  const Workspace ws{(char*)workspace_dev};
+  A.counter = ws.counters();
   if (A.K == 0) return RLSDE_OK;
   int sm = 0;
-  if ((rc = device_sm_count(&sm)) != RLSDE_OK) return rc;
-  cudaError_t e = cudaMemsetAsync(workspace_dev, 0, WS_COUNTER_BYTES, stream);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-  int lrc = launch_rollout_fwd_table(u_table_dev, A, sm, stream);
-  if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_fwd_table launch");
-  if (stats_dev) {
-    double* partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
-    const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
-    lrc = launch_reduce_stats(A.K, lim_eff, (A.flags & RLSDE_F_STATE_F64) != 0, G_dev, S_dev, T_dev, l2_dev, logw_dev,
-                              stats_dev, partial, stream);
-    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reduce_stats launch");
-  }
-  return RLSDE_OK;
+  if ((rc = begin_launch(ws, stream, sm)) != RLSDE_OK) return rc;
+  if ((rc = launch_status(launch_rollout_fwd_table(u_table_dev, A, sm, stream), "rollout_fwd_table launch")) != RLSDE_OK) return rc;
+  return reduce_stats(A, stats_dev, ws, stream);
 }
 
 int rlsde_rollout_transitions(const rlsde_env* env, const rlsde_mlp* mlp, const float* params_host,
@@ -525,15 +512,10 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   if (rc != RLSDE_OK) return rc;
   if (!params_host || !cS_dev || !T_dev || !path_dev || !grad_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
   if (WEIGHTED && !cG_dev) return RLSDE_ERR_INVALID_ARG;
-  if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
+  if (workspace_bytes < Workspace::fixed_bytes()) return RLSDE_ERR_WORKSPACE;
   FwdArgs A;
-  memset(&A, 0, sizeof(A));
-  fill_env(env, A);
-  if ((rc = fill_cfg(cfg, A, RAGGED)) != RLSDE_OK) return rc;
-  if (RAGGED) {
-    if (!path_base) return RLSDE_ERR_INVALID_ARG;
-    A.flags |= RLSDE_F_STORE_PATH;                                   // implied, as in rlsde_rollout_fwd_ragged
-  }
+  if ((rc = make_args(env, cfg, A, RAGGED)) != RLSDE_OK) return rc;
+  if (RAGGED && !path_base) return RLSDE_ERR_INVALID_ARG;
   if (A.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;   // no reverse pass through the projection
   if (A.flags & RLSDE_F_STATE_F64) return RLSDE_ERR_UNSUPPORTED;   // the reference differentiates the f32 torch path only
   if (!(A.flags & RLSDE_F_STORE_PATH)) return RLSDE_ERR_INVALID_ARG;
@@ -544,97 +526,85 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   if (WEIGHTED) A.S = (void*)cG_dev;
   A.order = (const long long*)order_dev;
   if (RAGGED) A.path_base = path_base;
-  A.counter = (unsigned long long*)workspace_dev;
+  const Workspace ws{(char*)workspace_dev};
+  A.counter = ws.counters();
   int sm = 0;
-  if ((rc = device_sm_count(&sm)) != RLSDE_OK) return rc;
-  cudaError_t e = cudaMemsetAsync(workspace_dev, 0, WS_COUNTER_BYTES, stream);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-  float* partial = (float*)((char*)workspace_dev + WS_COUNTER_BYTES + WS_STATS_BYTES + WS_POLICY_BYTES);
-  int lrc = -1;
-  if (shape_is_wide(env->d, mlp->d_hidden)) {
-    if (A.ckpt_every != 1) return RLSDE_ERR_UNSUPPORTED;        // the wide reverse kernel reads every state from the path
-    // hidden width 128 / 256 with enough trajectories (umma_min_k): the tcgen05 kernel
-    // (rollout_umma_bwd.cuh), given a workspace from rlsde_workspace_bytes_bwd; cfg.wide_kernel as in the forward rollout
-    const bool umma_shape = mlp->d_hidden == 128 || mlp->d_hidden == 256;
-    const size_t umma_need = umma_shape ? ws_fixed_bytes() + bwd_umma_scratch(env->d, mlp->d_hidden, sm) : 0;
-    if (umma_shape && cfg->wide_kernel == 1 && workspace_bytes < umma_need) return RLSDE_ERR_WORKSPACE;
-    if (umma_shape && workspace_bytes >= umma_need &&
-        (cfg->wide_kernel == 1 || (cfg->wide_kernel == 0 && A.K >= umma_min_k(mlp->d_hidden, sm)))) {
-      uint8_t* scratch = (uint8_t*)workspace_dev + ws_fixed_bytes();
-#define X(D_, H_)                                                                                                        \
-  if (env->d == D_ && mlp->d_hidden == H_)                                                                               \
-    lrc = launch_rollout_bwd_umma<D_, H_, WEIGHTED, RAGGED>(params_host, ws_wide_params(workspace_dev), ws_umma_image(workspace_dev), A,   \
-                                          (float)loss_scale, grad_dev, scratch, workspace_bytes - ws_fixed_bytes(), sm, stream);
-      RLSDE_UMMA_SHAPES(X)
-#undef X
-      if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd (tcgen05) launch");
-      return RLSDE_OK;
+  if ((rc = begin_launch(ws, stream, sm)) != RLSDE_OK) return rc;
+  float* partial = ws.bwd_partial();
+  return with_shape(env->d, mlp->d_hidden, [&](auto shape) -> int {
+    using S = decltype(shape);
+    if constexpr (S::wide) {
+      if (A.ckpt_every != 1) return RLSDE_ERR_UNSUPPORTED;        // the wide reverse kernel reads every state from the path
+      // hidden width 128 / 256 with enough trajectories (umma_min_k): the tcgen05 kernel (rollout_umma_bwd.cuh), given a
+      // workspace from rlsde_workspace_bytes_bwd; cfg.wide_kernel as in the forward rollout
+      if constexpr (S::umma_bwd) {
+        const size_t umma_need = Workspace::fixed_bytes() + bwd_umma_scratch_bytes<S::D, S::H>(sm);
+        if (cfg->wide_kernel == 1 && workspace_bytes < umma_need) return RLSDE_ERR_WORKSPACE;
+        if (workspace_bytes >= umma_need && (cfg->wide_kernel == 1 || (cfg->wide_kernel == 0 && A.K >= umma_min_k(S::H, sm))))
+          return launch_status(launch_rollout_bwd_umma<S::D, S::H, WEIGHTED, RAGGED>(
+                                   params_host, ws.wide_params(), ws.umma_image(), A, (float)loss_scale, grad_dev, ws.tail(),
+                                   workspace_bytes - Workspace::fixed_bytes(), sm, stream),
+                               "rollout_bwd (tcgen05) launch");
+      }
+      return launch_status(launch_rollout_bwd_wide<S::D, S::H, WEIGHTED, RAGGED>(params_host, ws.wide_params(), A, (float)loss_scale,
+                                                                                  grad_dev, partial, bwd_partial_main_bytes(), sm, stream),
+                           "rollout_bwd (wide) launch");
+    } else {
+      const bool warp_path = use_warp_kernels(A, S::H, sm, true);
+      // Large batches with a length-sorted order: the reverse pass of a trajectory is sequential, and K2 walks a lone
+      // trajectory at ~12 us per pass -- the longest few thousand trajectories, not the total work, set its run time
+      // (K = 4e5, longest 3 900 passes: 47 ms for ~28 ms of throughput work).  They go to the warp-per-trajectory kernel
+      // instead (~0.5 us per pass), the bulk stays in K2; the two gradients are added in a fixed order.  The split depends
+      // on the sorted lengths only, so the result is deterministic.
+      long long n_long = 0;
+      if (!warp_path && order_dev && A.ckpt_every == 1 && A.K > (long long)sm * 128) {
+        // measured (K = 4e5, d = 1): 46.2 / 36.7 / 36.7 / 37.5 / 41.9 ms at 0 / 2 368 / 4 736 / 9 472 / 25 000 long trajectories
+        n_long = A.K / 16 < warp_path_max_k(sm) ? A.K / 16 : warp_path_max_k(sm);
+        if (cfg->bwd_warp_share != 0) n_long = cfg->bwd_warp_share < A.K ? cfg->bwd_warp_share : A.K;
+        if (n_long < 0) n_long = 0;
+      }
+      FwdArgs Abulk = A;
+      float* partial_aux = (float*)((char*)partial + bwd_partial_main_bytes());
+      // thread-per-trajectory family, hidden width 32: the tensor-core kernel (rollout_bwd_mma.cuh) unless the caller asks
+      // for the CUDA-core one (cfg.bwd_kernel == 2; kept for A/B measurements and as a second implementation in the tests)
+      // (state dimensions above 4: the d-sized products -- layer 1, head, dW1, dW3, dX -- run as padded 16-wide tiles on
+      // the tensor cores as well; d = 10: 16.3 ms against 26.1 ms at K = 2e5, 61 against 109 ms at K = 1e6)
+      const bool use_mma = cfg->bwd_kernel != 2;
+      cudaEvent_t join = nullptr;
+      int lrc = -1;                                         // an empty batch without long trajectories fails as a launch
+      if (n_long > 0) {
+        FwdArgs Along = A;
+        Along.K = n_long;
+        Abulk.order = A.order + n_long;
+        Abulk.K = A.K - n_long;
+        Abulk.grad_accumulate = 1;
+        // the long trajectories run concurrently with the bulk on the second stream when the bulk's reduction can wait
+        // for them (tensor-core kernel); otherwise first, on the caller's stream
+        cudaStream_t s_long = stream;
+        cudaError_t e;
+        if (use_mma && Abulk.K > 0 && g_aux.get()) {
+          if ((e = cudaEventRecord(g_aux.fork, stream)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(fork)");
+          if ((e = cudaStreamWaitEvent(g_aux.stream, g_aux.fork, 0)) != cudaSuccess) return cuda_fail(e, "cudaStreamWaitEvent(fork)");
+          s_long = g_aux.stream;
+        }
+        lrc = launch_rollout_bwd_warp<S::D, WEIGHTED, RAGGED>(params_host, nullptr, Along, (float)loss_scale, grad_dev, partial_aux,
+                                                              sm, s_long);
+        if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd (long trajectories) launch");
+        if (s_long != stream) {
+          if ((e = cudaEventRecord(g_aux.join, s_long)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(join)");
+          join = g_aux.join;
+        }
+      }
+      if (Abulk.K > 0)
+        lrc = warp_path ? launch_rollout_bwd_warp<S::D, WEIGHTED, RAGGED>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev,
+                                                                           partial, sm, stream)
+              : use_mma ? launch_rollout_bwd_mma<S::D, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial,
+                                                                          sm, stream, join)
+                        : launch_rollout_bwd<S::D, S::H, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial,
+                                                                            sm, stream);
+      return launch_status(lrc, "rollout_bwd launch");
     }
-#define X(D_, H_)                                                                                                       \
-  if (env->d == D_ && mlp->d_hidden == H_)                                                                              \
-    lrc = launch_rollout_bwd_wide<D_, H_, WEIGHTED, RAGGED>(params_host, ws_wide_params(workspace_dev), A, (float)loss_scale, grad_dev, partial, \
-                                          bwd_partial_main_bytes(), sm, stream);
-    RLSDE_WIDE_SHAPES(X)
-#undef X
-    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd (wide) launch");
-    return RLSDE_OK;
-  }
-  const bool warp_path = use_warp_kernels(A, mlp->d_hidden, sm, true);
-  // Large batches with a length-sorted order: the reverse pass of a trajectory is sequential, and K2 walks a lone
-  // trajectory at ~12 us per pass -- the longest few thousand trajectories, not the total work, set its run time (K = 4e5,
-  // longest 3 900 passes: 47 ms for ~28 ms of throughput work).  They go to the warp-per-trajectory kernel instead
-  // (~0.5 us per pass), the bulk stays in K2; the two gradients are added in a fixed order.  The split depends on the
-  // sorted lengths only, so the result is deterministic.
-  long long n_long = 0;
-  if (!warp_path && order_dev && A.ckpt_every == 1 && mlp->d_hidden == WARP_H && A.K > (long long)sm * 128) {
-    // measured (K = 4e5, d = 1): 46.2 / 36.7 / 36.7 / 37.5 / 41.9 ms at 0 / 2 368 / 4 736 / 9 472 / 25 000 long trajectories
-    n_long = A.K / 16 < warp_path_max_k(sm) ? A.K / 16 : warp_path_max_k(sm);
-    if (cfg->bwd_warp_share != 0) n_long = cfg->bwd_warp_share < A.K ? cfg->bwd_warp_share : A.K;
-    if (n_long < 0) n_long = 0;
-  }
-  FwdArgs Abulk = A;
-  float* partial_aux = (float*)((char*)partial + bwd_partial_main_bytes());
-  // thread-per-trajectory family, hidden width 32: the tensor-core kernel (rollout_bwd_mma.cuh) unless the caller asks for
-  // the CUDA-core one (cfg.bwd_kernel == 2; kept for A/B measurements and as a second implementation in the tests)
-  // (state dimensions above 4: the d-sized products -- layer 1, head, dW1, dW3, dX -- run as padded 16-wide tiles on the
-  // tensor cores as well; d = 10: 16.3 ms against 26.1 ms at K = 2e5, 61 against 109 ms at K = 1e6)
-  const bool use_mma = mlp->d_hidden == MMA_H && cfg->bwd_kernel != 2;
-  cudaEvent_t join = nullptr;
-  if (n_long > 0) {
-    FwdArgs Along = A;
-    Along.K = n_long;
-    Abulk.order = A.order + n_long;
-    Abulk.K = A.K - n_long;
-    Abulk.grad_accumulate = 1;
-    // the long trajectories run concurrently with the bulk on the second stream when the bulk's reduction can wait for
-    // them (tensor-core kernel); otherwise first, on the caller's stream
-    cudaStream_t s_long = stream;
-    if (use_mma && Abulk.K > 0 && g_aux.get()) {
-      if ((e = cudaEventRecord(g_aux.fork, stream)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(fork)");
-      if ((e = cudaStreamWaitEvent(g_aux.stream, g_aux.fork, 0)) != cudaSuccess) return cuda_fail(e, "cudaStreamWaitEvent(fork)");
-      s_long = g_aux.stream;
-    }
-#define X(D_, H_)                                                                                                   \
-  if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H)                                                          \
-    lrc = launch_rollout_bwd_warp<D_, WEIGHTED, RAGGED>(params_host, nullptr, Along, (float)loss_scale, grad_dev, partial_aux, sm, s_long);
-    RLSDE_SHAPES(X)
-#undef X
-    if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd (long trajectories) launch");
-    if (s_long != stream) {
-      if ((e = cudaEventRecord(g_aux.join, s_long)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(join)");
-      join = g_aux.join;
-    }
-    lrc = Abulk.K > 0 ? -1 : 0;
-  }
-#define X(D_, H_)                                                                                                          \
-  if (env->d == D_ && mlp->d_hidden == H_ && Abulk.K > 0)                                                                  \
-    lrc = (warp_path && H_ == WARP_H) ? launch_rollout_bwd_warp<D_, WEIGHTED, RAGGED>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev, partial, sm, stream) \
-          : (use_mma && H_ == MMA_H)  ? launch_rollout_bwd_mma<D_, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream, join)      \
-                                      : launch_rollout_bwd<D_, H_, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial, sm, stream);
-  RLSDE_SHAPES(X)
-#undef X
-  if (lrc != 0) return cuda_fail((cudaError_t)lrc, "rollout_bwd launch");
-  return RLSDE_OK;
+  });
 }
 }  // extern "C++"
 
@@ -672,12 +642,9 @@ static int reinforce_rollout_impl(const rlsde_env* env, const rlsde_mlp* mlp, co
   int rc = check_env_mlp(env, mlp);
   if (rc != RLSDE_OK) return rc;
   if (!theta_dev || !G_dev || !S_dev || !T_dev || !path_dev || !stats_dev || !grad_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
-  if (workspace_bytes < ws_fixed_bytes()) return RLSDE_ERR_WORKSPACE;
-  static_assert(sizeof(MlpConst<RLSDE_MAX_D, WARP_H>) <= WS_POLICY_BYTES, "raise WS_POLICY_BYTES");
+  if (workspace_bytes < Workspace::fixed_bytes()) return RLSDE_ERR_WORKSPACE;
   FwdArgs A;
-  memset(&A, 0, sizeof(A));
-  fill_env(env, A);
-  if ((rc = fill_cfg(cfg, A)) != RLSDE_OK) return rc;
+  if ((rc = make_args(env, cfg, A)) != RLSDE_OK) return rc;
   if ((A.flags & (RLSDE_F_STATE_F64 | RLSDE_F_HIT_BRIDGE)) || !(A.flags & RLSDE_F_STORE_PATH) || A.ckpt_every != 1)
     return RLSDE_ERR_INVALID_ARG;
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
@@ -688,27 +655,23 @@ static int reinforce_rollout_impl(const rlsde_env* env, const rlsde_mlp* mlp, co
   if (mlp->d_hidden != WARP_H || A.K > warp_path_max_k(sm) || (A.flags & RLSDE_F_KERNEL_THREAD)) return RLSDE_ERR_UNSUPPORTED;
   A.noise = noise_dev;
   A.G = G_dev; A.S = S_dev; A.T = T_dev; A.path = path_dev;
-  A.counter = (unsigned long long*)workspace_dev;
-  A.q_ctrl = (unsigned long long*)workspace_dev;
-  void* W_dev = (char*)workspace_dev + WS_COUNTER_BYTES + WS_STATS_BYTES;
-  double* stats_partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
-  float* partial = (float*)((char*)workspace_dev + WS_COUNTER_BYTES + WS_STATS_BYTES + WS_POLICY_BYTES);
+  const Workspace ws{(char*)workspace_dev};
+  A.counter = ws.counters();
+  A.q_ctrl = ws.counters();
   const bool fast = (A.flags & RLSDE_F_TANH_FAST) != 0;
-  const long long lim_eff = (A.flags & RLSDE_F_NOISE_INJECTED) && A.noise_steps < A.n_steps_lim ? A.noise_steps : A.n_steps_lim;
   const float scale = (float)(1.0 / (double)A.K_global);       // the loss is the mean over ALL shards' trajectories
-  int lrc = -1;
-#define X(D_, H_)                                                                                                        \
-  if (env->d == D_ && mlp->d_hidden == H_ && H_ == WARP_H) {                                                             \
-    lrc = launch_pack_mlp_const_dev<D_>(theta_dev, W_dev, fast, stream);                                                 \
-    if (lrc == 0) lrc = launch_rollout_fwd_warp<D_>(nullptr, W_dev, A, sm, stream);                                      \
-    if (lrc == 0) lrc = launch_reduce_stats(A.K, lim_eff, false, G_dev, S_dev, T_dev, nullptr, nullptr, stats_dev,       \
-                                            stats_partial, stream);                                                     \
-    if (lrc == 0) lrc = launch_rollout_bwd_warp<D_>(nullptr, W_dev, A, scale, grad_dev, partial, sm, stream);            \
-  }
-  RLSDE_SHAPES(X)
-#undef X
-  if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reinforce rollout launch");
-  return RLSDE_OK;
+  return with_shape(env->d, mlp->d_hidden, [&](auto shape) -> int {
+    using S = decltype(shape);
+    int lrc = -1;
+    if constexpr (S::narrow) {
+      lrc = launch_pack_mlp_const_dev<S::D>(theta_dev, ws.policy(), fast, stream);
+      if (lrc == 0) lrc = launch_rollout_fwd_warp<S::D>(nullptr, ws.policy(), A, sm, stream);
+      if (lrc == 0) lrc = launch_reduce_stats(A.K, passes_run(A), false, G_dev, S_dev, T_dev, nullptr, nullptr, stats_dev, ws.stats(),
+                                              stream);
+      if (lrc == 0) lrc = launch_rollout_bwd_warp<S::D>(nullptr, ws.policy(), A, scale, grad_dev, ws.bwd_partial(), sm, stream);
+    }
+    return launch_status(lrc, "reinforce rollout launch");
+  });
 }
 
 int rlsde_reinforce_step(const rlsde_env* env, const rlsde_mlp* mlp, float* theta_dev, float* adam_m_dev, float* adam_v_dev,
@@ -757,10 +720,10 @@ int rlsde_reduce_stats(int64_t K, int64_t n_steps_lim, uint32_t flags, const voi
                        const int32_t* T_dev, const void* l2_dev, const void* logw_dev, double* stats_dev,
                        void* workspace_dev, size_t workspace_bytes, void* stream_) {
   if (K < 0 || !G_dev || !S_dev || !T_dev || !stats_dev || !workspace_dev) return RLSDE_ERR_INVALID_ARG;
-  if (workspace_bytes < WS_COUNTER_BYTES + WS_STATS_BYTES) return RLSDE_ERR_WORKSPACE;
-  double* partial = (double*)((char*)workspace_dev + WS_COUNTER_BYTES);
+  if (workspace_bytes < Workspace::o_policy) return RLSDE_ERR_WORKSPACE;
+  const Workspace ws{(char*)workspace_dev};
   const int lrc = launch_reduce_stats(K, n_steps_lim, (flags & RLSDE_F_STATE_F64) != 0, G_dev, S_dev, T_dev, l2_dev, logw_dev,
-                                      stats_dev, partial, (cudaStream_t)stream_);
+                                      stats_dev, ws.stats(), (cudaStream_t)stream_);
   if (lrc != 0) return cuda_fail((cudaError_t)lrc, "reduce_stats launch");
   return RLSDE_OK;
 }
@@ -815,12 +778,9 @@ int rlsde_env_step(const rlsde_env* env, int64_t K, const void* state_dev, const
   if (flags & RLSDE_F_HIT_BRIDGE) return RLSDE_ERR_INVALID_ARG;      // a single pass has no next pass to detect a crossing
   StepArgs A;
   memset(&A, 0, sizeof(A));
-  for (int i = 0; i < env->d; ++i) { A.c4a_d[i] = 4.0 * env->alpha[i]; A.c4a_f[i] = (float)(4.0 * env->alpha[i]); }
-  A.sigma_d = env->sigma; A.sigma_f = (float)env->sigma; A.dt_d = env->dt; A.dt_f = (float)env->dt;
-  A.lb_d = env->lb; A.rb_d = env->rb; A.lb_f = (float)env->lb; A.rb_f = (float)env->rb;
+  fill_env_consts(env, A);
   A.grad_f32 = (flags & RLSDE_F_GRAD_F32) ? 1 : 0;
-  A.noise_scale2 = (float)(-2.0 * env->dt * 0.6931471805599453);
-  A.d = env->d; A.hit_rule = env->hit_rule; A.reward_type = reward_type;
+  A.d = env->d; A.reward_type = reward_type;
   A.K = K; A.traj_offset = traj_offset; A.pass_index = pass_index; A.seed = seed;
   A.state = state_dev; A.action = action_dev; A.dbt_in = dbt_in_dev;
   A.next_state = next_state_dev; A.reward = reward_dev; A.done = done_dev; A.dbt_out = dbt_out_dev;

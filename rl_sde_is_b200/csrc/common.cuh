@@ -11,6 +11,7 @@
 //    "fast" = tanh.approx (MUFU.TANH, 2^-11 rel. error).
 #pragma once
 #include <cstdint>
+#include <type_traits>
 #include <cuda_runtime.h>
 
 namespace rlsde {
@@ -404,6 +405,39 @@ __device__ __forceinline__ void mlp_forward_folded(const MlpConst<D, H>& W, cons
   dense_tanh<D, H, false, true>(W.W1t, W.b1, x, r1);
   dense_tanh<H, H, false, true>(W.W2t, W.b2, r1, r2);
   mlp_head<D, H>(W, r2, u);
+}
+
+// ------------------------------------------------------------------ host-side launch helpers
+// A runtime flag as a compile-time one: f(std::true_type{}) if b holds and ALLOWED, else f(std::false_type{}).  Where
+// ALLOWED is false the true branch is never instantiated, so a pruned kernel variant is never compiled; the C ABI refuses
+// such flags before it launches.
+template <bool ALLOWED = true, class F>
+static inline int with_flag(bool b, F&& f) {
+  if constexpr (ALLOWED) {
+    if (b) return f(std::true_type{});
+  }
+  return f(std::false_type{});
+}
+
+// Grid of a kernel that runs one trajectory per thread: one warp per block for small batches, so that the warps spread
+// over the SMs (latency-bound regime); otherwise a persistent grid of 128-thread blocks, as many as are co-resident with
+// smem bytes of dynamic shared memory each (at most cap per SM when cap >= 1).  Sets block; returns the grid.
+template <class Kern>
+static long long persistent_grid(Kern kern, long long K, int sm_count, size_t smem, int cap, int& block) {
+  long long grid;
+  block = 128;
+  if (K <= (long long)sm_count * 128) {
+    block = 32;
+    grid = (K + 31) / 32;
+  } else {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+    if (cap >= 1 && cap < per_sm) per_sm = cap;
+    grid = (long long)sm_count * per_sm;
+    const long long need = (K + block - 1) / block;
+    if (grid > need) grid = need;
+  }
+  return grid < 1 ? 1 : grid;
 }
 
 }  // namespace rlsde

@@ -3,5 +3,5 @@
 // of its own, like every ragged instantiation: the dense-store kernels keep their code)
 #include "rollout_fwd_inst.cuh"
 #include "rollout_warp_inst.cuh"
-RLSDE_INSTANTIATE_FWD_RAGGED(1, 32)
-RLSDE_INSTANTIATE_FWD_WARP_RAGGED(1)
+RLSDE_INSTANTIATE_FWD(1, 32, true)
+RLSDE_INSTANTIATE_FWD_WARP(1, true)

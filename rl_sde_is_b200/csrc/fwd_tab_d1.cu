@@ -51,37 +51,19 @@ template <bool F64, bool SMEM, bool BRIDGE>
 static int launch_tab_variant(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
   auto kern = rollout_fwd_tab_kernel<F64, SMEM, BRIDGE>;
   const size_t smem = SMEM ? (size_t)args.n_grid * sizeof(float) : 0;
-  // as K1: one warp per block for small batches (spread over the SMs), a persistent grid of co-resident blocks otherwise
-  int block = 128;
-  long long grid;
-  if (args.K <= (long long)sm_count * 128) {
-    block = 32;
-    grid = (args.K + 31) / 32;
-  } else {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-    grid = (long long)sm_count * per_sm;
-    const long long need = (args.K + block - 1) / block;
-    if (grid > need) grid = need;
-  }
+  int block;
+  const long long grid = persistent_grid(kern, args.K, sm_count, smem, 0, block);
   kern<<<(unsigned)grid, block, smem, stream>>>(args, table);
   note_kernel_launches(1);
   return (int)cudaGetLastError();
 }
 
-template <bool BRIDGE>
-static int launch_tab_bridge(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0;
-  const bool smem = args.n_grid <= FWD_TAB_SMEM_MAX;
-  if (f64) return smem ? launch_tab_variant<true, true, BRIDGE>(table, args, sm_count, stream)
-                       : launch_tab_variant<true, false, BRIDGE>(table, args, sm_count, stream);
-  return smem ? launch_tab_variant<false, true, BRIDGE>(table, args, sm_count, stream)
-              : launch_tab_variant<false, false, BRIDGE>(table, args, sm_count, stream);
-}
-
 int launch_rollout_fwd_table(const float* table, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  return (args.flags & RLSDE_F_HIT_BRIDGE) ? launch_tab_bridge<true>(table, args, sm_count, stream)
-                                           : launch_tab_bridge<false>(table, args, sm_count, stream);
+  return with_fwd_variant<1, false>(args.flags, [&](auto f64, auto, auto bridge) {
+    return with_flag(args.n_grid <= FWD_TAB_SMEM_MAX, [&](auto smem) {
+      return launch_tab_variant<f64, smem, bridge>(table, args, sm_count, stream);
+    });
+  });
 }
 
 }  // namespace rlsde

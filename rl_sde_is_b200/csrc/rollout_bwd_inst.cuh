@@ -24,22 +24,10 @@ static int launch_bwd_variant(const float* params_host, const FwdArgs& args, flo
   MlpConst<D, H> W;
   pack_mlp_const<D, H>(params_host, FAST, W);
   auto kern = rollout_bwd_kernel<D, H, FAST, WEIGHTED, RAGGED>;
-  int block = 128;
-  long long grid;
   const size_t smem_per_warp = (size_t)(2 * tile_floats<H, bwd_tiles_padded(D)>() + 64 * D) * sizeof(float);
-  if (args.K <= (long long)sm_count * 128) {
-    block = 32;
-    grid = (args.K + 31) / 32;
-  } else {
-    const size_t smem = smem_per_warp * 4;
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-    grid = (long long)sm_count * per_sm;
-    const long long need = (args.K + block - 1) / block;
-    if (grid > need) grid = need;
-  }
-  if (grid < 1) grid = 1;
+  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem_per_warp * 4));
+  int block;
+  long long grid = persistent_grid(kern, args.K, sm_count, smem_per_warp * 4, 0, block);
   long long n_warps = grid * (block / 32);
   if (n_warps > BWD_MAX_WARPS) { grid = BWD_MAX_WARPS / (block / 32); n_warps = grid * (block / 32); }
   const size_t smem = smem_per_warp * (block / 32);
@@ -55,17 +43,12 @@ static int launch_bwd_variant(const float* params_host, const FwdArgs& args, flo
 template <int D, int H, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd(const float* params_host, const FwdArgs& args, float scale, float* grad, float* partial,
                        int sm_count, cudaStream_t stream) {
-  return (args.flags & RLSDE_F_TANH_FAST) ? launch_bwd_variant<D, H, true, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream)
-                                          : launch_bwd_variant<D, H, false, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream);
+  return with_flag((args.flags & RLSDE_F_TANH_FAST) != 0, [&](auto fast) {
+    return launch_bwd_variant<D, H, fast, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream);
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_BWD(D, H) \
-  template int rlsde::launch_rollout_bwd<D, H>(const float*, const rlsde::FwdArgs&, float, float*, float*, int, cudaStream_t);
-// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
-#define RLSDE_INSTANTIATE_BWD_WEIGHTED(D, H) \
-  template int rlsde::launch_rollout_bwd<D, H, true>(const float*, const rlsde::FwdArgs&, float, float*, float*, int, cudaStream_t);
-// the weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_BWD_RAGGED(D, H) \
-  template int rlsde::launch_rollout_bwd<D, H, true, true>(const float*, const rlsde::FwdArgs&, float, float*, float*, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_BWD(D, H, WEIGHTED, RAGGED) \
+  template int rlsde::launch_rollout_bwd<D, H, WEIGHTED, RAGGED>(const float*, const rlsde::FwdArgs&, float, float*, float*, int, cudaStream_t);

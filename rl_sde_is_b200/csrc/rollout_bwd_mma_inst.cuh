@@ -19,22 +19,11 @@ static int launch_bwd_mma_variant(const float* params_host, const FwdArgs& args,
   typename BwdMmaSmallSel<D>::type FS;
   pack_bwd_mma_small<D>(W, FAST, FS);
   auto kern = rollout_bwd_mma_kernel<D, FAST, WEIGHTED, RAGGED>;
-  int block = 128;
-  long long grid;
   // d > 4: fragment table of the d-sized products + per-warp staging rows; accumulator tiles (rollout_bwd_mma.cuh)
   auto dyn_smem = [](int blk) { return bwd_mma_dyn_smem(D, blk); };
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem(128));
-  if (args.K <= (long long)sm_count * 128) {
-    block = 32;
-    grid = (args.K + 31) / 32;
-  } else {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, dyn_smem(block)) != cudaSuccess || per_sm < 1) per_sm = 1;
-    grid = (long long)sm_count * per_sm;
-    const long long need = (args.K + block - 1) / block;
-    if (grid > need) grid = need;
-  }
-  if (grid < 1) grid = 1;
+  int block;
+  long long grid = persistent_grid(kern, args.K, sm_count, dyn_smem(128), 0, block);
   long long n_warps = grid * (block / 32);
   if (n_warps > BWD_MAX_WARPS) { grid = BWD_MAX_WARPS / (block / 32); n_warps = grid * (block / 32); }
   kern<<<(unsigned)grid, block, dyn_smem(block), stream>>>(W, args, F, FS, reinterpret_cast<double*>(partial));
@@ -50,16 +39,13 @@ static int launch_bwd_mma_variant(const float* params_host, const FwdArgs& args,
 template <int D, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd_mma(const float* params_host, const FwdArgs& args, float scale, float* grad, void* partial,
                            int sm_count, cudaStream_t stream, cudaEvent_t join) {
-  return (args.flags & RLSDE_F_TANH_FAST) ? launch_bwd_mma_variant<D, true, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream, join)
-                                          : launch_bwd_mma_variant<D, false, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream, join);
+  return with_flag((args.flags & RLSDE_F_TANH_FAST) != 0, [&](auto fast) {
+    return launch_bwd_mma_variant<D, fast, WEIGHTED, RAGGED>(params_host, args, scale, grad, partial, sm_count, stream, join);
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_BWD_MMA(D) \
-  template int rlsde::launch_rollout_bwd_mma<D>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, cudaStream_t, cudaEvent_t);
-#define RLSDE_INSTANTIATE_BWD_MMA_WEIGHTED(D) \
-  template int rlsde::launch_rollout_bwd_mma<D, true>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, cudaStream_t, cudaEvent_t);
-// the weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_BWD_MMA_RAGGED(D) \
-  template int rlsde::launch_rollout_bwd_mma<D, true, true>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, cudaStream_t, cudaEvent_t);
+#define RLSDE_INSTANTIATE_BWD_MMA(D, WEIGHTED, RAGGED)                                                                  \
+  template int rlsde::launch_rollout_bwd_mma<D, WEIGHTED, RAGGED>(const float*, const rlsde::FwdArgs&, float, float*, void*, int, \
+                                                                  cudaStream_t, cudaEvent_t);

@@ -614,6 +614,27 @@ __global__ void __launch_bounds__(128, fwd_min_blocks<D, MMA>()) rollout_fwd_ker
   }
 }
 
+// Kernel variant of a forward launch from its flags, for every forward family, as std::bool_constant arguments.  Two
+// rules prune what is compiled, and the C ABI refuses the flags they exclude: the Brownian-bridge test is compiled at
+// d = 1 only and never with the ragged checkpoint store (with_fwd_bridge: f(BRIDGE)); the ragged store takes the float32
+// state only (with_fwd_state: f(F64, FAST)).  with_fwd_variant: f(F64, FAST, BRIDGE).
+template <int D, bool RAGGED, class F>
+static inline int with_fwd_bridge(unsigned flags, F&& f) {
+  return with_flag<D == 1 && !RAGGED>((flags & RLSDE_F_HIT_BRIDGE) != 0, f);
+}
+template <bool RAGGED, class F>
+static inline int with_fwd_state(unsigned flags, F&& f) {
+  return with_flag<!RAGGED>((flags & RLSDE_F_STATE_F64) != 0, [&](auto f64) {
+    return with_flag((flags & RLSDE_F_TANH_FAST) != 0, [&](auto fast) { return f(f64, fast); });
+  });
+}
+template <int D, bool RAGGED, class F>
+static inline int with_fwd_variant(unsigned flags, F&& f) {
+  return with_fwd_bridge<D, RAGGED>(flags, [&](auto bridge) {
+    return with_fwd_state<RAGGED>(flags, [&](auto f64, auto fast) { return f(f64, fast, bridge); });
+  });
+}
+
 // host-side launcher for one (D, H) shape; defined in rollout_fwd_inst.cuh.  RAGGED: the ragged checkpoint store (float32
 // state only, no Brownian-bridge test: the caller refuses both)
 template <int D, int H, bool RAGGED = false>

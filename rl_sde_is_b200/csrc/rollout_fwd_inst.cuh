@@ -22,22 +22,8 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
     a.mma_x1_max = (float)x1_max;
     if (z2_max <= RCP_GROUP_SAFE_Z) kern = rollout_fwd_kernel<D, H, F64, FAST, MMA, false, BRIDGE, RAGGED>;
   }
-  // Small batches: one warp per block so the warps spread over SMs (latency-bound regime);
-  // large batches: persistent grid of 128-thread blocks, as many as are co-resident.
-  int block = 128;
-  long long grid;
-  if (args.K <= (long long)sm_count * 128) {
-    block = 32;
-    grid = (args.K + 31) / 32;
-  } else {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-    if (args.blocks_per_sm_cap >= 1 && args.blocks_per_sm_cap < per_sm) per_sm = args.blocks_per_sm_cap;   // tuning knob
-    grid = (long long)sm_count * per_sm;
-    const long long need = (args.K + block - 1) / block;
-    if (grid > need) grid = need;
-  }
-  if (grid < 1) grid = 1;
+  int block;
+  const long long grid = persistent_grid(kern, args.K, sm_count, 0, args.blocks_per_sm_cap, block);
   // Schedule (rollout_fwd.cuh; chosen by the C ABI layer: args.q_quantum passes per slice, or run to completion with
   // the tail handed over to the warp-per-trajectory kernel at args.q_handoff live trajectories): large batches only, and
   // only if the caller's workspace holds a ring with one record per trajectory plus one per lane.
@@ -62,27 +48,14 @@ static int launch_fwd_variant(const float* params_host, const FwdArgs& args, int
   return (int)cudaGetLastError();
 }
 
-template <int D, int H, bool MMA, bool BRIDGE, bool RAGGED = false>
-static int launch_fwd_prec(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0;
-  const bool fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if constexpr (!RAGGED) {     // the ragged store is refused with the float64 state
-    if (f64) {
-      return fast ? launch_fwd_variant<D, H, true, true, MMA, BRIDGE>(params_host, args, sm_count, stream)
-                  : launch_fwd_variant<D, H, true, false, MMA, BRIDGE>(params_host, args, sm_count, stream);
-    }
-  }
-  return fast ? launch_fwd_variant<D, H, false, true, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream)
-              : launch_fwd_variant<D, H, false, false, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
-}
-
 // args.policy_mma selects the policy arithmetic; the caller checks fwd_mma_shape(D, H) before it sets it
 template <int D, int H, bool BRIDGE, bool RAGGED = false>
 static int launch_fwd_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (fwd_mma_shape(D, H)) {
-    if (args.policy_mma) return launch_fwd_prec<D, H, true, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
-  }
-  return launch_fwd_prec<D, H, false, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
+  return with_flag<fwd_mma_shape(D, H)>(args.policy_mma != 0, [&](auto mma) {
+    return with_fwd_state<RAGGED>(args.flags, [&](auto f64, auto fast) {
+      return launch_fwd_variant<D, H, f64, fast, mma, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
+    });
+  });
 }
 
 // The kernels with the Brownian-bridge hit test (RLSDE_F_HIT_BRIDGE, d = 1) live in a translation unit of their own
@@ -93,17 +66,13 @@ int launch_rollout_fwd_bridge(const float* params_host, const FwdArgs& args, int
 
 template <int D, int H, bool RAGGED>
 int launch_rollout_fwd(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (D == 1 && !RAGGED) {      // the caller accepts RLSDE_F_HIT_BRIDGE at d = 1 only, and not with RAGGED
-    if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_rollout_fwd_bridge<D, H>(params_host, args, sm_count, stream);
-  }
-  return launch_fwd_policy<D, H, false, RAGGED>(params_host, args, sm_count, stream);
+  return with_fwd_bridge<D, RAGGED>(args.flags, [&](auto bridge) {
+    if constexpr (bridge) return launch_rollout_fwd_bridge<D, H>(params_host, args, sm_count, stream);
+    else return launch_fwd_policy<D, H, false, RAGGED>(params_host, args, sm_count, stream);
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_FWD(D, H) \
-  template int rlsde::launch_rollout_fwd<D, H>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
-// the ragged checkpoint store (rlsde_rollout_fwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_FWD_RAGGED(D, H) \
-  template int rlsde::launch_rollout_fwd<D, H, true>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
-
+#define RLSDE_INSTANTIATE_FWD(D, H, RAGGED) \
+  template int rlsde::launch_rollout_fwd<D, H, RAGGED>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);

@@ -106,21 +106,15 @@ int launch_rollout_bwd_umma(const float* params_host, float* params_dev, uint8_t
   if ((e = cudaMemcpyAsync(scratch + S::o_img2, w2.data(), umma_image_bytes<H>(), cudaMemcpyHostToDevice, stream)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(scratch + S::o_ctl, 0, S::o_img2, stream)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(scratch + S::o_partial, 0, S::partial_bytes(n_prod, n_cons), stream)) != cudaSuccess) return (int)e;
-  return fast ? launch_bwd_umma_variant<D, H, true, WEIGHTED, RAGGED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream)
-              : launch_bwd_umma_variant<D, H, false, WEIGHTED, RAGGED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons, (float)w3max, stream);
+  return with_flag(fast, [&](auto fast_c) {
+    return launch_bwd_umma_variant<D, H, fast_c, WEIGHTED, RAGGED>(params_dev, image_dev, args, scale, grad, scratch, n_prod, n_cons,
+                                                                   (float)w3max, stream);
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_UMMA_BWD(D, H)                                                                                          \
-  template size_t rlsde::bwd_umma_scratch_bytes<D, H>(int);                                                                       \
-  template int rlsde::launch_rollout_bwd_umma<D, H>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, float*, uint8_t*, \
-                                                    size_t, int, cudaStream_t);
-// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
-#define RLSDE_INSTANTIATE_UMMA_BWD_WEIGHTED(D, H)                                                                                 \
-  template int rlsde::launch_rollout_bwd_umma<D, H, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, float*,   \
-                                                          uint8_t*, size_t, int, cudaStream_t);
-// the weighted reverse pass over the ragged checkpoint store (rlsde_rollout_bwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_UMMA_BWD_RAGGED(D, H)                                                                             \
-  template int rlsde::launch_rollout_bwd_umma<D, H, true, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, \
-                                                                float*, uint8_t*, size_t, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_UMMA_BWD(D, H, WEIGHTED, RAGGED)                                                                  \
+  template int rlsde::launch_rollout_bwd_umma<D, H, WEIGHTED, RAGGED>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, float, \
+                                                                      float*, uint8_t*, size_t, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_UMMA_BWD_SCRATCH(D, H) template size_t rlsde::bwd_umma_scratch_bytes<D, H>(int);

@@ -36,7 +36,7 @@ static int launch_fwd_umma_variant(const float* params_dev, const uint8_t* image
 template <int D, int H, bool RAGGED>
 int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t* image_dev, const FwdArgs& args, int sm_count,
                             cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
+  const bool fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
   std::vector<float> img(WideParams<D, H>::count);
   pack_wide_params<D, H>(params_host, fast, img.data());
   std::vector<uint16_t> wimg(umma_image_bytes<H>() / 2);
@@ -45,27 +45,12 @@ int launch_rollout_fwd_umma(const float* params_host, float* params_dev, uint8_t
   if (e != cudaSuccess) return (int)e;
   e = cudaMemcpyAsync(image_dev, wimg.data(), umma_image_bytes<H>(), cudaMemcpyHostToDevice, stream);
   if (e != cudaSuccess) return (int)e;
-#define RLSDE_UMMA_FWD(B_)                                                                                           \
-  (f64 ? (fast ? launch_fwd_umma_variant<D, H, true, true, B_>(params_dev, image_dev, args, sm_count, stream)         \
-               : launch_fwd_umma_variant<D, H, true, false, B_>(params_dev, image_dev, args, sm_count, stream))       \
-       : (fast ? launch_fwd_umma_variant<D, H, false, true, B_>(params_dev, image_dev, args, sm_count, stream)        \
-               : launch_fwd_umma_variant<D, H, false, false, B_>(params_dev, image_dev, args, sm_count, stream)))
-  if constexpr (RAGGED) {      // float32 state, no Brownian-bridge test: the caller refuses both
-    return fast ? launch_fwd_umma_variant<D, H, false, true, false, true>(params_dev, image_dev, args, sm_count, stream)
-                : launch_fwd_umma_variant<D, H, false, false, false, true>(params_dev, image_dev, args, sm_count, stream);
-  } else {
-    if constexpr (D == 1) {      // RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
-      if (args.flags & RLSDE_F_HIT_BRIDGE) return RLSDE_UMMA_FWD(true);
-    }
-    return RLSDE_UMMA_FWD(false);
-  }
-#undef RLSDE_UMMA_FWD
+  return with_fwd_variant<D, RAGGED>(args.flags, [&](auto f64, auto fast, auto bridge) {
+    return launch_fwd_umma_variant<D, H, f64, fast, bridge, RAGGED>(params_dev, image_dev, args, sm_count, stream);
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_UMMA(D, H) \
-  template int rlsde::launch_rollout_fwd_umma<D, H>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, int, cudaStream_t);
-// the ragged checkpoint store (rlsde_rollout_fwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_UMMA_RAGGED(D, H) \
-  template int rlsde::launch_rollout_fwd_umma<D, H, true>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_UMMA(D, H, RAGGED) \
+  template int rlsde::launch_rollout_fwd_umma<D, H, RAGGED>(const float*, float*, uint8_t*, const rlsde::FwdArgs&, int, cudaStream_t);

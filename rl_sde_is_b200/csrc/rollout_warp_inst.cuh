@@ -52,24 +52,11 @@ static int launch_fwd_warp_variant(const float* params_host, const void* W_dev, 
   return (int)cudaGetLastError();
 }
 
-template <int D, bool BRIDGE, bool RAGGED = false>
-static int launch_fwd_warp_bridge(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if constexpr (!RAGGED) {     // the ragged store is refused with the float64 state
-    if (f64) return fast ? launch_fwd_warp_variant<D, true, true, BRIDGE, false>(params_host, W_dev, args, sm_count, stream)
-                         : launch_fwd_warp_variant<D, true, false, BRIDGE, false>(params_host, W_dev, args, sm_count, stream);
-  }
-  return fast ? launch_fwd_warp_variant<D, false, true, BRIDGE, RAGGED>(params_host, W_dev, args, sm_count, stream)
-              : launch_fwd_warp_variant<D, false, false, BRIDGE, RAGGED>(params_host, W_dev, args, sm_count, stream);
-}
-
-// RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only, and not with RAGGED
 template <int D, bool RAGGED>
 int launch_rollout_fwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (D == 1 && !RAGGED) {
-    if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_fwd_warp_bridge<D, true>(params_host, W_dev, args, sm_count, stream);
-  }
-  return launch_fwd_warp_bridge<D, false, RAGGED>(params_host, W_dev, args, sm_count, stream);
+  return with_fwd_variant<D, RAGGED>(args.flags, [&](auto f64, auto fast, auto bridge) {
+    return launch_fwd_warp_variant<D, f64, fast, bridge, RAGGED>(params_host, W_dev, args, sm_count, stream);
+  });
 }
 
 template <int D, bool F64, bool FAST, bool MMA, bool BRIDGE, bool RAGGED>
@@ -86,32 +73,14 @@ static int launch_fwd_warp_resume_variant(const float* params_host, const FwdArg
   return (int)cudaGetLastError();
 }
 
-template <int D, bool MMA, bool BRIDGE, bool RAGGED = false>
-static int launch_fwd_warp_resume_bridge(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  if constexpr (!RAGGED) {     // the ragged store is refused with the float64 state
-    if (f64) return fast ? launch_fwd_warp_resume_variant<D, true, true, MMA, BRIDGE, false>(params_host, args, sm_count, stream)
-                         : launch_fwd_warp_resume_variant<D, true, false, MMA, BRIDGE, false>(params_host, args, sm_count, stream);
-  }
-  return fast ? launch_fwd_warp_resume_variant<D, false, true, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream)
-              : launch_fwd_warp_resume_variant<D, false, false, MMA, BRIDGE, RAGGED>(params_host, args, sm_count, stream);
-}
-
-template <int D, bool MMA, bool RAGGED>
-static int launch_fwd_warp_resume_policy(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (D == 1 && !RAGGED) {
-    if (args.flags & RLSDE_F_HIT_BRIDGE) return launch_fwd_warp_resume_bridge<D, MMA, true>(params_host, args, sm_count, stream);
-  }
-  return launch_fwd_warp_resume_bridge<D, MMA, false, RAGGED>(params_host, args, sm_count, stream);
-}
-
 // continues with the policy arithmetic K1 was launched with (args.policy_mma)
 template <int D, bool RAGGED>
 int launch_rollout_fwd_warp_resume(const float* params_host, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  if constexpr (fwd_mma_shape(D, WARP_H)) {
-    if (args.policy_mma) return launch_fwd_warp_resume_policy<D, true, RAGGED>(params_host, args, sm_count, stream);
-  }
-  return launch_fwd_warp_resume_policy<D, false, RAGGED>(params_host, args, sm_count, stream);
+  return with_flag<fwd_mma_shape(D, WARP_H)>(args.policy_mma != 0, [&](auto mma) {
+    return with_fwd_variant<D, RAGGED>(args.flags, [&](auto f64, auto fast, auto bridge) {
+      return launch_fwd_warp_resume_variant<D, f64, fast, mma, bridge, RAGGED>(params_host, args, sm_count, stream);
+    });
+  });
 }
 
 template <int D, bool FAST, bool WEIGHTED, bool RAGGED>
@@ -134,27 +103,19 @@ static int launch_bwd_warp_variant(const float* params_host, const void* W_dev, 
 template <int D, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd_warp(const float* params_host, const void* W_dev, const FwdArgs& args, float scale, float* grad,
                             float* partial, int sm_count, cudaStream_t stream) {
-  return (args.flags & RLSDE_F_TANH_FAST)
-             ? launch_bwd_warp_variant<D, true, WEIGHTED, RAGGED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream)
-             : launch_bwd_warp_variant<D, false, WEIGHTED, RAGGED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream);
+  return with_flag((args.flags & RLSDE_F_TANH_FAST) != 0, [&](auto fast) {
+    return launch_bwd_warp_variant<D, fast, WEIGHTED, RAGGED>(params_host, W_dev, args, scale, grad, partial, sm_count, stream);
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_WARP(D)                                                                                          \
-  template int rlsde::launch_rollout_fwd_warp<D>(const float*, const void*, const rlsde::FwdArgs&, int, cudaStream_t);     \
-  template int rlsde::launch_rollout_bwd_warp<D>(const float*, const void*, const rlsde::FwdArgs&, float, float*, float*, \
-                                                 int, cudaStream_t);                                                       \
-  template int rlsde::launch_pack_mlp_const_dev<D>(const float*, void*, bool, cudaStream_t);                              \
-  template int rlsde::launch_rollout_fwd_warp_resume<D>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
-// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
-#define RLSDE_INSTANTIATE_BWD_WARP_WEIGHTED(D)                                                                             \
-  template int rlsde::launch_rollout_bwd_warp<D, true>(const float*, const void*, const rlsde::FwdArgs&, float, float*,   \
-                                                       float*, int, cudaStream_t);
-// the ragged checkpoint store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_FWD_WARP_RAGGED(D)                                                                               \
-  template int rlsde::launch_rollout_fwd_warp<D, true>(const float*, const void*, const rlsde::FwdArgs&, int, cudaStream_t); \
-  template int rlsde::launch_rollout_fwd_warp_resume<D, true>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
-#define RLSDE_INSTANTIATE_BWD_WARP_RAGGED(D)                                                                               \
-  template int rlsde::launch_rollout_bwd_warp<D, true, true>(const float*, const void*, const rlsde::FwdArgs&, float, float*, \
-                                                             float*, int, cudaStream_t);
+// the forward launchers of the warp-per-trajectory kernel: fresh trajectories and the ones K1 handed over
+#define RLSDE_INSTANTIATE_FWD_WARP(D, RAGGED)                                                                              \
+  template int rlsde::launch_rollout_fwd_warp<D, RAGGED>(const float*, const void*, const rlsde::FwdArgs&, int, cudaStream_t); \
+  template int rlsde::launch_rollout_fwd_warp_resume<D, RAGGED>(const float*, const rlsde::FwdArgs&, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_BWD_WARP(D, WEIGHTED, RAGGED)                                                                    \
+  template int rlsde::launch_rollout_bwd_warp<D, WEIGHTED, RAGGED>(const float*, const void*, const rlsde::FwdArgs&, float, \
+                                                                   float*, float*, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_PACK_DEV(D) \
+  template int rlsde::launch_pack_mlp_const_dev<D>(const float*, void*, bool, cudaStream_t);

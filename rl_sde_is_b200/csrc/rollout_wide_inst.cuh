@@ -36,27 +36,13 @@ static int launch_fwd_wide_variant(const float* params_dev, const FwdArgs& args,
 
 template <int D, int H, bool RAGGED>
 int launch_rollout_fwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, int sm_count, cudaStream_t stream) {
-  const bool f64 = (args.flags & RLSDE_F_STATE_F64) != 0, fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  int rc = wide_upload_params<D, H>(params_host, params_dev, fast, stream);
+  int rc = wide_upload_params<D, H>(params_host, params_dev, (args.flags & RLSDE_F_TANH_FAST) != 0, stream);
   if (rc != 0) return rc;
-  const bool small = wide_small_tiles(args.K, sm_count);
-#define RLSDE_WIDE_FWD(R_, B_) \
-  (f64 ? (fast ? launch_fwd_wide_variant<D, H, R_, true, true, B_>(params_dev, args, sm_count, stream)    \
-               : launch_fwd_wide_variant<D, H, R_, true, false, B_>(params_dev, args, sm_count, stream))  \
-       : (fast ? launch_fwd_wide_variant<D, H, R_, false, true, B_>(params_dev, args, sm_count, stream)   \
-               : launch_fwd_wide_variant<D, H, R_, false, false, B_>(params_dev, args, sm_count, stream)))
-  if constexpr (RAGGED) {      // float32 state, no Brownian-bridge test: the caller refuses both
-    if (small) return fast ? launch_fwd_wide_variant<D, H, 4, false, true, false, true>(params_dev, args, sm_count, stream)
-                           : launch_fwd_wide_variant<D, H, 4, false, false, false, true>(params_dev, args, sm_count, stream);
-    return fast ? launch_fwd_wide_variant<D, H, 8, false, true, false, true>(params_dev, args, sm_count, stream)
-                : launch_fwd_wide_variant<D, H, 8, false, false, false, true>(params_dev, args, sm_count, stream);
-  } else {
-    if constexpr (D == 1) {      // RLSDE_F_HIT_BRIDGE: the caller accepts it at d = 1 only
-      if (args.flags & RLSDE_F_HIT_BRIDGE) return small ? RLSDE_WIDE_FWD(4, true) : RLSDE_WIDE_FWD(8, true);
-    }
-    return small ? RLSDE_WIDE_FWD(4, false) : RLSDE_WIDE_FWD(8, false);
-  }
-#undef RLSDE_WIDE_FWD
+  return with_flag(wide_small_tiles(args.K, sm_count), [&](auto small) {
+    return with_fwd_variant<D, RAGGED>(args.flags, [&](auto f64, auto fast, auto bridge) {
+      return launch_fwd_wide_variant<D, H, small ? 4 : 8, f64, fast, bridge, RAGGED>(params_dev, args, sm_count, stream);
+    });
+  });
 }
 
 template <int D, int H, int R, bool FAST, bool WEIGHTED, bool RAGGED>
@@ -87,28 +73,20 @@ template <int D, int H, bool WEIGHTED, bool RAGGED>
 int launch_rollout_bwd_wide(const float* params_host, float* params_dev, const FwdArgs& args, float scale, float* grad, float* partial,
                             size_t partial_bytes, int sm_count, cudaStream_t stream) {
   if (args.ckpt_every != 1) return (int)cudaErrorInvalidValue;
-  const bool fast = (args.flags & RLSDE_F_TANH_FAST) != 0;
-  int rc = wide_upload_params<D, H>(params_host, params_dev, fast, stream);
+  int rc = wide_upload_params<D, H>(params_host, params_dev, (args.flags & RLSDE_F_TANH_FAST) != 0, stream);
   if (rc != 0) return rc;
-  const bool small = wide_small_tiles(args.K, sm_count);
-  if (small) return fast ? launch_bwd_wide_variant<D, H, 4, true, WEIGHTED, RAGGED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream)
-                         : launch_bwd_wide_variant<D, H, 4, false, WEIGHTED, RAGGED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream);
-  return fast ? launch_bwd_wide_variant<D, H, 8, true, WEIGHTED, RAGGED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream)
-              : launch_bwd_wide_variant<D, H, 8, false, WEIGHTED, RAGGED>(params_dev, args, scale, grad, partial, partial_bytes, sm_count, stream);
+  return with_flag(wide_small_tiles(args.K, sm_count), [&](auto small) {
+    return with_flag((args.flags & RLSDE_F_TANH_FAST) != 0, [&](auto fast) {
+      return launch_bwd_wide_variant<D, H, small ? 4 : 8, fast, WEIGHTED, RAGGED>(params_dev, args, scale, grad, partial,
+                                                                                 partial_bytes, sm_count, stream);
+    });
+  });
 }
 
 }  // namespace rlsde
 
-#define RLSDE_INSTANTIATE_WIDE(D, H)                                                                                        \
-  template int rlsde::launch_rollout_fwd_wide<D, H>(const float*, float*, const rlsde::FwdArgs&, int, cudaStream_t);       \
-  template int rlsde::launch_rollout_bwd_wide<D, H>(const float*, float*, const rlsde::FwdArgs&, float, float*, float*,   \
-                                                    size_t, int, cudaStream_t);
-// the weighted reverse pass (rlsde_rollout_bwd_weighted), in translation units of its own
-#define RLSDE_INSTANTIATE_WIDE_BWD_WEIGHTED(D, H)                                                                           \
-  template int rlsde::launch_rollout_bwd_wide<D, H, true>(const float*, float*, const rlsde::FwdArgs&, float, float*, float*, \
-                                                          size_t, int, cudaStream_t);
-// the ragged checkpoint store (rlsde_rollout_fwd_ragged / rlsde_rollout_bwd_ragged), in translation units of its own
-#define RLSDE_INSTANTIATE_WIDE_RAGGED(D, H)                                                                                 \
-  template int rlsde::launch_rollout_fwd_wide<D, H, true>(const float*, float*, const rlsde::FwdArgs&, int, cudaStream_t); \
-  template int rlsde::launch_rollout_bwd_wide<D, H, true, true>(const float*, float*, const rlsde::FwdArgs&, float, float*,  \
-                                                                float*, size_t, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_FWD_WIDE(D, H, RAGGED) \
+  template int rlsde::launch_rollout_fwd_wide<D, H, RAGGED>(const float*, float*, const rlsde::FwdArgs&, int, cudaStream_t);
+#define RLSDE_INSTANTIATE_BWD_WIDE(D, H, WEIGHTED, RAGGED)                                                                  \
+  template int rlsde::launch_rollout_bwd_wide<D, H, WEIGHTED, RAGGED>(const float*, float*, const rlsde::FwdArgs&, float,   \
+                                                                      float*, float*, size_t, int, cudaStream_t);

@@ -1,4 +1,4 @@
 // forward rollout into the ragged checkpoint store (rlsde_rollout_fwd_ragged) for d = 3, hidden width = 32: the
 // tcgen05 kernel
 #include "rollout_umma_inst.cuh"
-RLSDE_INSTANTIATE_UMMA_RAGGED(3, 32)
+RLSDE_INSTANTIATE_UMMA(3, 32, true)

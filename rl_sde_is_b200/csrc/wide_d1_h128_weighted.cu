@@ -2,5 +2,5 @@
 // and the tcgen05 producer / consumer kernel
 #include "rollout_wide_inst.cuh"
 #include "rollout_umma_bwd_inst.cuh"
-RLSDE_INSTANTIATE_WIDE_BWD_WEIGHTED(1, 128)
-RLSDE_INSTANTIATE_UMMA_BWD_WEIGHTED(1, 128)
+RLSDE_INSTANTIATE_BWD_WIDE(1, 128, true, false)
+RLSDE_INSTANTIATE_UMMA_BWD(1, 128, true, false)

@@ -2,5 +2,6 @@
 // CUDA-core tile kernels and the tcgen05 forward kernel
 #include "rollout_wide_inst.cuh"
 #include "rollout_umma_inst.cuh"
-RLSDE_INSTANTIATE_WIDE_RAGGED(1, 64)
-RLSDE_INSTANTIATE_UMMA_RAGGED(1, 64)
+RLSDE_INSTANTIATE_FWD_WIDE(1, 64, true)
+RLSDE_INSTANTIATE_BWD_WIDE(1, 64, true, true)
+RLSDE_INSTANTIATE_UMMA(1, 64, true)

@@ -1,3 +1,4 @@
 // wide-policy rollout kernels (tile contraction through shared memory) for d = 2, hidden width = 128
 #include "rollout_wide_inst.cuh"
-RLSDE_INSTANTIATE_WIDE(2, 128)
+RLSDE_INSTANTIATE_FWD_WIDE(2, 128, false)
+RLSDE_INSTANTIATE_BWD_WIDE(2, 128, false, false)

@@ -3,6 +3,7 @@
 #include "rollout_wide_inst.cuh"
 #include "rollout_umma_inst.cuh"
 #include "rollout_umma_bwd_inst.cuh"
-RLSDE_INSTANTIATE_WIDE_RAGGED(2, 256)
-RLSDE_INSTANTIATE_UMMA_RAGGED(2, 256)
-RLSDE_INSTANTIATE_UMMA_BWD_RAGGED(2, 256)
+RLSDE_INSTANTIATE_FWD_WIDE(2, 256, true)
+RLSDE_INSTANTIATE_BWD_WIDE(2, 256, true, true)
+RLSDE_INSTANTIATE_UMMA(2, 256, true)
+RLSDE_INSTANTIATE_UMMA_BWD(2, 256, true, true)
