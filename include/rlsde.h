@@ -18,6 +18,9 @@
  *                       (BPTT through every pass; states are never detached, :88)
  *   rlsde_tables        compute_r_table / compute_p_tensor_batch   dynamic_programming.py:3-36
  *                       + state_action_transition_function          environments.py:87-102
+ *   rlsde_dp_sweep      the Bellman sweeps of q_table_update_vect / v_table_update_vect / policy_update_vect
+ *                       over a device-resident tensor; rlsde_dp_sweep_implicit the same sweep with the
+ *                       tensor generated inside it, for grids whose tensor does not fit
  *   rlsde_env_step      env.step / env.step_torch (single pass, API completeness)
  *   rlsde_noise_fill    the Brownian increments env.step* draws (environments.py:145,208),
  *                       from the same counter-based generator the rollout kernels use
@@ -380,6 +383,21 @@ size_t rlsde_dp_scratch_bytes(int64_t Ns, int64_t Na);
 int rlsde_dp_sweep(const double* P_dev, int64_t Ns, int64_t Na, const double* R_dev, const uint8_t* in_ts_dev,
                    const double* v_dev, double gamma, double* values_dev, void* scratch_dev, size_t scratch_bytes,
                    void* stream);
+/*
+ * The same sweep without the tensor: P[s', s, a] is generated inside the sweep, exactly as rlsde_tables defines it
+ * (same arguments, same choice between the erf/erfc and the quadrature path), and contracted at once.  Memory is
+ * O(Ns Na) whatever the grid, so grids whose tensor (8 Ns^2 Na bytes) does not fit on the device can be swept.  Cells
+ * lying entirely beyond 9 sd of a column's mean are skipped: at most 2^-60 of each column's mass.  Deterministic and
+ * bitwise repeatable; bound by the FP64 pipe, not by memory.  Columns of target-set states are R[s, a].
+ * state_grid_dev: double[Ns], increasing; action_grid_dev: double[Na]; in_ts_dev: uint8[Ns]; R_dev, values_dev:
+ * double[Ns][Na]; v_dev: double[Ns].
+ * Refused before any device work (RLSDE_ERR_INVALID_ARG): a NULL pointer, Ns < 1 or Na < 1, sigma, dt or h_half not
+ * positive, state_grid_uniform != 0 with state_grid_step not positive.
+ */
+int rlsde_dp_sweep_implicit(const double* state_grid_dev, int64_t Ns, const double* action_grid_dev, int64_t Na,
+                            const uint8_t* in_ts_dev, double alpha, double sigma, double dt, double h_half,
+                            int32_t state_grid_uniform, double state_grid_step, const double* R_dev, const double* v_dev,
+                            double gamma, double* values_dev, void* stream);
 /* vmax[s] = max_a values[s, a] and argmax[s] = first maximiser (np.max / np.argmax, axis 1); either output may be NULL */
 int rlsde_dp_rowmax(const double* values_dev, int64_t Ns, int64_t Na, double* vmax_dev, int64_t* argmax_dev, void* stream);
 

@@ -41,7 +41,7 @@ EXPORTED_SYMBOLS = [
     "rlsde_tables", "rlsde_tables_colsum", "rlsde_env_step", "rlsde_noise_fill",
     "rlsde_dp_scratch_bytes", "rlsde_dp_sweep", "rlsde_dp_rowmax", "rlsde_rollout_transitions", "rlsde_launch_count", "rlsde_reinforce_step",
     "rlsde_reinforce_rollout", "rlsde_reinforce_apply", "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table",
-    "rlsde_rollout_bwd_weighted", "rlsde_rollout_fwd_ragged", "rlsde_rollout_bwd_ragged",
+    "rlsde_rollout_bwd_weighted", "rlsde_rollout_fwd_ragged", "rlsde_rollout_bwd_ragged", "rlsde_dp_sweep_implicit",
 ]
 
 
@@ -128,13 +128,14 @@ def load():
     lib.rlsde_dp_scratch_bytes.restype = C.c_size_t
     lib.rlsde_dp_scratch_bytes.argtypes = [i64, i64]
     lib.rlsde_dp_sweep.argtypes = [vp, i64, i64, vp, vp, vp, dbl, vp, vp, C.c_size_t, vp]
+    lib.rlsde_dp_sweep_implicit.argtypes = [vp, i64, vp, i64, vp, dbl, dbl, dbl, dbl, i32, dbl, vp, vp, dbl, vp, vp]
     lib.rlsde_dp_rowmax.argtypes = [vp, i64, i64, vp, vp, vp]
     lib.rlsde_fwd_mma_clamp_bounds.argtypes = [vp, vp]
     for name in ("rlsde_device_info", "rlsde_supported", "rlsde_rollout_fwd", "rlsde_rollout_bwd", "rlsde_reduce_stats",
                  "rlsde_tables", "rlsde_tables_colsum", "rlsde_env_step", "rlsde_noise_fill", "rlsde_dp_sweep", "rlsde_dp_rowmax",
                  "rlsde_rollout_transitions", "rlsde_reinforce_step", "rlsde_reinforce_rollout", "rlsde_reinforce_apply",
                  "rlsde_fwd_mma_clamp_bounds", "rlsde_rollout_fwd_table", "rlsde_rollout_bwd_weighted",
-                 "rlsde_rollout_fwd_ragged", "rlsde_rollout_bwd_ragged"):
+                 "rlsde_rollout_fwd_ragged", "rlsde_rollout_bwd_ragged", "rlsde_dp_sweep_implicit"):
         getattr(lib, name).restype = C.c_int
     _lib = lib
     return lib

@@ -45,6 +45,11 @@ int launch_tables_colsum(const double* P, long long n_sprime, long long Ns, long
 int launch_dp_sweep(const double* P, long long Ns, long long Na, const double* R, const unsigned char* in_ts,
                     const double* v, double gamma, double* values, double* scratch, cudaStream_t stream);
 size_t dp_sweep_scratch_bytes(long long Ns, long long Na);
+int launch_dp_sweep_implicit(const double* sgrid, long long Ns, const double* agrid, long long Na,
+                             const unsigned char* in_ts, double alpha, double sigma, double dt, double h_half,
+                             int uniform_grid, double grid_step, const double* R, const double* v, double gamma,
+                             double* values, cudaStream_t stream);
+constexpr int IMPLICIT_THREADS = 128;            // actions per block of the tensor-free sweep
 int launch_dp_rowmax(const double* values, long long Ns, long long Na, double* vmax, long long* arg, cudaStream_t stream);
 
 }  // namespace rlsde

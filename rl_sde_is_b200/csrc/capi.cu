@@ -761,6 +761,22 @@ int rlsde_dp_sweep(const double* P_dev, int64_t Ns, int64_t Na, const double* R_
   return RLSDE_OK;
 }
 
+int rlsde_dp_sweep_implicit(const double* state_grid_dev, int64_t Ns, const double* action_grid_dev, int64_t Na,
+                            const uint8_t* in_ts_dev, double alpha, double sigma, double dt, double h_half,
+                            int32_t state_grid_uniform, double state_grid_step, const double* R_dev, const double* v_dev,
+                            double gamma, double* values_dev, void* stream_) {
+  if (!state_grid_dev || !action_grid_dev || !in_ts_dev || !R_dev || !v_dev || !values_dev) return RLSDE_ERR_INVALID_ARG;
+  if (Ns < 1 || Na < 1) return RLSDE_ERR_INVALID_ARG;
+  if (Na > INT32_MAX || Ns > INT32_MAX / ((Na + IMPLICIT_THREADS - 1) / IMPLICIT_THREADS)) return RLSDE_ERR_INVALID_ARG;  // one block per (s, action tile)
+  if (!(sigma > 0) || !(dt > 0) || !(h_half > 0)) return RLSDE_ERR_INVALID_ARG;
+  if (state_grid_uniform && !(state_grid_step > 0)) return RLSDE_ERR_INVALID_ARG;
+  const int lrc = launch_dp_sweep_implicit(state_grid_dev, Ns, action_grid_dev, Na, in_ts_dev, alpha, sigma, dt, h_half,
+                                           state_grid_uniform, state_grid_step, R_dev, v_dev, gamma, values_dev,
+                                           (cudaStream_t)stream_);
+  if (lrc != 0) return cuda_fail((cudaError_t)lrc, "dp_sweep_implicit launch");
+  return RLSDE_OK;
+}
+
 int rlsde_dp_rowmax(const double* values_dev, int64_t Ns, int64_t Na, double* vmax_dev, int64_t* argmax_dev, void* stream_) {
   if (!values_dev || Ns < 1 || Na < 1 || (!vmax_dev && !argmax_dev)) return RLSDE_ERR_INVALID_ARG;
   const int lrc = launch_dp_rowmax(values_dev, Ns, Na, vmax_dev, (long long*)argmax_dev, (cudaStream_t)stream_);

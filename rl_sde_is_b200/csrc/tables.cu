@@ -14,23 +14,9 @@
 // next (TILE+1 CDF evaluations per TILE entries instead of 2 TILE).  The kernel is bound by the FP64
 // pipe (erf/erfc), not by HBM: see DESIGN.md.
 #include "aux_kernels.cuh"
+#include "transition.cuh"
 
 namespace rlsde {
-
-// scipy.special.ndtr (cephes ndtr.c) branch structure, with CUDA's erf / erfc
-__device__ __forceinline__ double ndtr(double a) {
-  const double kSqrtH = 0.70710678118654752440;
-  const double x = a * kSqrtH;
-  const double z = fabs(x);
-  double y;
-  if (z < kSqrtH) {
-    y = 0.5 + 0.5 * erf(x);
-  } else {
-    y = 0.5 * erfc(z);
-    if (x > 0) y = 1.0 - y;
-  }
-  return y;
-}
 
 constexpr int TABLE_TILE = 8;
 
@@ -70,54 +56,10 @@ __global__ void __launch_bounds__(128) tables_kernel(const double* __restrict__ 
   }
 }
 
-// ---- fast path: uniform state grid with fine cells (cell width <= 0.2 sd) -------------------------------
-// P_cell = integral of the N(0,1) density over the cell [m - D/2, m + D/2] by 4-point Gauss-Legendre (truncation error
-// 9e-14 at D = 0.25, 1e-14 at D = 0.2: the path is taken up to D = 0.2).  The nodes sit symmetrically at m +- a, m +- b,
-// and phi(m +- o) = phi(m) exp(-o^2/2) exp(-+ m o), so
-//     P = phi(m) * (Ya + Yb),   Ya = 2 D w_a exp(-a^2/2) cosh(m a),   Yb likewise with (w_b, b).
-// Walking s' moves m by the constant step ds, and all three factors follow cheap recurrences:
-//     phi(m + ds) = phi(m) r,   r <- r exp(-ds^2)                                (2 DMUL)
-//     Y(m + ds)   = Y + dY,     dY <- dY + 4 sinh^2(o ds / 2) Y(m + ds)          (DADD + DFMA each; the second-difference
-//                                                                                 form of cosh's three-term recurrence,
-//                                                                                 stable because the small quantity is kept)
-// 8 FP64 operations and one 8-byte store per entry, re-anchored with exact exp() every GL_ANCHOR cells (measured
-// |P - reference formula| <= 5e-15 at config 3; tests hold 1e-13).  One thread owns one (s, a) column of one chunk of
-// at most GL_ANCHOR rows of one row class (see the kernel); columns are the flat index s * Na + a, so every lane of every
-// warp is busy and a block stores 1 KB of contiguous bytes per row.
-constexpr int GL_ANCHOR = 64;
-constexpr double GL_SPAN_SD = 21.0;
-
-struct GlConst {
-  double inv_sd, dcell, dstep, rho;        // 1/sd, D, ds, exp(-ds^2)
-  double off_a, off_b;                     // node offsets a, b
-  double coef_a, coef_b;                   // 2 D w exp(-o^2/2)
-  double mu_a, mu_b;                       // 4 sinh^2(o ds / 2)
-  double sh_a, sh_b;                       // sinh(o ds / 2)
-  double eh_a, eh_b;                       // exp(o ds / 2)
-  double half_ds2;                         // ds^2 / 2
-};
-
-// host side: the constants of the recurrences are the same for every column; they travel as a kernel parameter (round 1
-// formed them once per block behind a barrier: 4.1 warps per issue slot stalled there, profiles/r01/ncu_tables_gl_v2.txt)
-static GlConst make_gl_const(double grid_step, double sigma, double dt, double h) {
-  GlConst C;
-  C.inv_sd = 1.0 / (sigma * sqrt(dt));
-  C.dcell = 2.0 * h * C.inv_sd;
-  C.dstep = grid_step * C.inv_sd;
-  C.rho = exp(-C.dstep * C.dstep);
-  C.half_ds2 = 0.5 * C.dstep * C.dstep;
-  C.off_a = 0.4305681557970263 * C.dcell;
-  C.off_b = 0.1699905217924281 * C.dcell;
-  C.coef_a = 2.0 * C.dcell * 0.1739274225687269 * exp(-0.5 * C.off_a * C.off_a);
-  C.coef_b = 2.0 * C.dcell * 0.3260725774312731 * exp(-0.5 * C.off_b * C.off_b);
-  C.sh_a = sinh(0.5 * C.off_a * C.dstep);
-  C.sh_b = sinh(0.5 * C.off_b * C.dstep);
-  C.mu_a = 4.0 * C.sh_a * C.sh_a;
-  C.mu_b = 4.0 * C.sh_b * C.sh_b;
-  C.eh_a = exp(0.5 * C.off_a * C.dstep);
-  C.eh_b = exp(0.5 * C.off_b * C.dstep);
-  return C;
-}
+// ---- fast path: uniform state grid with fine cells (cell width <= 0.2 sd): the Gauss-Legendre density recurrences of
+// transition.cuh, one 8-byte store per entry.  One thread owns one (s, a) column of one chunk of at most GL_ANCHOR rows of
+// one row class (see the kernel); columns are the flat index s * Na + a, so every lane of every warp is busy and a block
+// stores 1 KB of contiguous bytes per row.
 
 // Stores.  A row of P has Ns Na entries and Ns Na is odd at config 3 (401 x 601), so consecutive rows start 72 bytes
 // apart modulo 128.  With one thread per column walking consecutive rows, a warp's 256-byte store sits at 8-byte alignment
@@ -211,19 +153,13 @@ int launch_tables(const double* state_grid, long long Ns, const double* action_g
                   double lb, double rb, long long sprime_begin, long long sprime_end, double* P, double* R,
                   int uniform_grid, double grid_step, cudaStream_t stream) {
   (void)lb; (void)rb;
-  const double dcell = 2.0 * h_half / (sigma * sqrt(dt));
-  if (P && sprime_end > sprime_begin && uniform_grid && grid_step > 0.0 && Ns >= 2 && dcell <= 0.2 ) {
+  if (P && sprime_end > sprime_begin && gl_path(Ns, uniform_grid, grid_step, sigma, dt, h_half)) {
     // row classes (see tables_gl_kernel) and chunks of `steps` rows per class, both defined on the full grid so that a
     // slab reproduces the full tensor's entries bit for bit
     const long long cols = Ns * Na;
     const int Q = (cols & 3) == 0 ? 1 : ((cols & 1) == 0 ? 2 : 4);
     const long long rows_per_class = (Ns + Q - 1) / Q;
-    // a chunk spans at most GL_ANCHOR steps and at most GL_SPAN_SD standard deviations: phi at the anchor must not
-    // underflow (|m| < 37) while cells that matter (|m| < 9) are still ahead of it, and the relative error of r grows
-    // with |m ds|
-    const double step_sd = Q * grid_step / (sigma * sqrt(dt));
-    long long steps_cap = (long long)(GL_SPAN_SD / step_sd);
-    steps_cap = steps_cap < 1 ? 1 : (steps_cap > GL_ANCHOR ? GL_ANCHOR : steps_cap);
+    const long long steps_cap = gl_anchor_steps(Q * grid_step / (sigma * sqrt(dt)));
     const long long n_chunks_full = (rows_per_class + steps_cap - 1) / steps_cap;
     const int steps = (int)((rows_per_class + n_chunks_full - 1) / n_chunks_full);
     const long long kc_lo = (sprime_begin >= Q ? (sprime_begin - (Q - 1)) / Q : 0) / steps;

@@ -34,6 +34,17 @@ def _device_grids(env, dev):
     return grids
 
 
+def _state_grid_spacing(env):
+    """(uniform, step): whether the state grid is equally spaced to 1e-14, which lets the kernels take the quadrature
+    path, and its mean spacing (x_{Ns-1} - x_0) / (Ns - 1)."""
+    grid = np.asarray(env.state_space_h, dtype=np.float64)
+    Ns = grid.size
+    if Ns < 2:
+        return 0, 0.0
+    uniform = int(np.abs(grid - (grid[0] + np.arange(Ns) * (grid[-1] - grid[0]) / (Ns - 1))).max() <= 1e-14)
+    return uniform, float((grid[-1] - grid[0]) / (Ns - 1))
+
+
 def _tables(env, want_p, want_r, device, sprime_range=None, exact_cdf=False, out=None):
     if env.d != 1:
         raise L.RlsdeError("the tabular builder covers the 1-D environment (as the reference's does)")
@@ -42,8 +53,8 @@ def _tables(env, want_p, want_r, device, sprime_range=None, exact_cdf=False, out
     sg, ag, ts = _device_grids(env, dev)
     Ns, Na = int(sg.numel()), int(ag.numel())
     lo, hi = (0, Ns) if sprime_range is None else (int(sprime_range[0]), int(sprime_range[1]))
-    grid = np.asarray(env.state_space_h, dtype=np.float64)
-    uniform = int(Ns >= 2 and np.abs(grid - (grid[0] + np.arange(Ns) * (grid[-1] - grid[0]) / (Ns - 1))).max() <= 1e-14 and not exact_cdf)
+    uniform, step = _state_grid_spacing(env)
+    uniform = int(uniform and not exact_cdf)
     P = None
     if want_p:
         P = out if out is not None else torch.empty((hi - lo, Ns, Na), dtype=torch.float64, device=dev)
@@ -53,7 +64,7 @@ def _tables(env, want_p, want_r, device, sprime_range=None, exact_cdf=False, out
     with torch.cuda.device(dev):
         rc = lib.rlsde_tables(_ptr(sg), Ns, _ptr(ag), Na, _ptr(ts), int(env.is_in_ts.sum()), float(env.alpha),
                               float(env.sigma), float(env.dt), float(env.h_state) / 2.0, float(env.lb), float(env.rb),
-                              lo, hi, _ptr(P), _ptr(Rt), uniform, float((grid[-1] - grid[0]) / (Ns - 1)) if Ns >= 2 else 0.0,
+                              lo, hi, _ptr(P), _ptr(Rt), uniform, step,
                               torch.cuda.current_stream(dev).cuda_stream)
     L.check(rc, "rlsde_tables")
     return P, Rt

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from .dynamic_programming import compute_p_tensor_batch, compute_r_table, p_tensor_column_sums
-from .tabular_dp_sweeps import DeviceTables, _like
+from .tabular_dp_sweeps import _like, _tables
 from .utils_path import get_dynamic_programming_tables_dir_path, load_data, save_data
 
 
@@ -25,10 +25,11 @@ def check_p_tensor(env, p_tensor):
 
 
 def compute_optimal_q_table(env, r_table, p_tensor, value_function_opt, policy_opt=None):
-    """``(1 - d) P^T v_opt + r`` for every (state, action)  (:32-42)."""
-    T = p_tensor if isinstance(p_tensor, DeviceTables) else DeviceTables(env, r_table, p_tensor)
+    """``(1 - d) P^T v_opt + r`` for every (state, action)  (:32-42).  ``p_tensor`` may also be a ``DeviceTables`` or an
+    ``ImplicitTables``; the result is then a CUDA tensor."""
+    T = _tables(env, r_table, p_tensor)
     v = np.asarray(value_function_opt, dtype=np.float64).reshape(-1)
-    return _like(p_tensor.P if isinstance(p_tensor, DeviceTables) else p_tensor, T.sweep(v, 1.0))
+    return _like(T.R if T is p_tensor else p_tensor, T.sweep(v, 1.0))
 
 
 def compute_optimal_v_table(env, r_table, p_tensor, value_function_opt, policy_opt):
