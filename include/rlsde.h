@@ -144,8 +144,8 @@ typedef struct rlsde_rollout_cfg {
                                    (-1 = never, 0 = automatic) */
   int64_t bwd_warp_share;       /* longest trajectories the reverse pass gives to the warp-per-trajectory kernel
                                    (-1 = none, 0 = automatic) */
-  int32_t bwd_kernel;           /* thread-per-trajectory reverse pass, hidden width 32: 0 = automatic (tensor-core kernel),
-                                   1 = tensor-core kernel (mma.sync, float16 x 3 split), 2 = CUDA-core kernel (FFMA2) */
+  int32_t bwd_kernel;           /* thread-per-trajectory reverse pass, hidden width 32: 0 or 1 = tensor-core kernel
+                                   (mma.sync, float16 x 3 split); any other value is refused (RLSDE_ERR_UNSUPPORTED) */
   int32_t wide_kernel;          /* forward rollout (hidden width 64 / 128 / 256) and reverse pass (128 / 256): 0 = automatic (tcgen05
                                    kernels for batches of at least 512 trajectories at width 256, 64 x SMs below; the reverse pass also needs a
                                    workspace of rlsde_workspace_bytes_bwd), 1 = tcgen05 kernels, 2 = CUDA-core tile kernels */

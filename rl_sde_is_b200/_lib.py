@@ -144,7 +144,7 @@ def load():
 def apply_tuning(cfg, tuning=None):
     """Scheduling knobs of a rollout cfg (include/rlsde.h: they change the schedule, never a result).  ``tuning`` is a dict
     with any of ``fwd_quantum`` (passes per time slice, 0 = run to completion), ``fwd_handoff``, ``bwd_warp_share``,
-    ``fwd_blocks_per_sm``, ``bwd_kernel`` ('mma' | 'ffma'), ``wide_kernel`` ('umma' | 'ffma'), ``fwd_policy`` ('mma' | 'ffma');
+    ``fwd_blocks_per_sm``, ``bwd_kernel`` ('mma'), ``wide_kernel`` ('umma' | 'ffma'), ``fwd_policy`` ('mma' | 'ffma');
     keys that are absent fall back to the environment variables RLSDE_FWD_QUANTUM, RLSDE_FWD_HANDOFF, RLSDE_BWD_WARP_SHARE,
     RLSDE_FWD_BLOCKS_PER_SM, RLSDE_BWD_KERNEL, RLSDE_WIDE_KERNEL, RLSDE_FWD_POLICY (read HERE, in
     Python -- the library reads none), and to "automatic" if those are unset too."""
@@ -165,7 +165,7 @@ def apply_tuning(cfg, tuning=None):
     b = knob("fwd_blocks_per_sm")
     cfg.fwd_blocks_per_sm = 0 if b is None or b < 1 else b
     bk = tuning.get("bwd_kernel") or os.environ.get("RLSDE_BWD_KERNEL") or "auto"
-    cfg.bwd_kernel = {"auto": 0, "mma": 1, "ffma": 2}[str(bk).lower()]
+    cfg.bwd_kernel = {"auto": 0, "mma": 1}[str(bk).lower()]
     wk = tuning.get("wide_kernel") or os.environ.get("RLSDE_WIDE_KERNEL") or "auto"
     cfg.wide_kernel = {"auto": 0, "umma": 1, "tcgen05": 1, "ffma": 2}[str(wk).lower()]
     fp = tuning.get("fwd_policy") or os.environ.get("RLSDE_FWD_POLICY") or "auto"

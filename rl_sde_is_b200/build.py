@@ -34,9 +34,6 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "--expt-relaxed-constexpr",
 ] + os.environ.get("RLSDE_NVCC_EXTRA", "").split()
-# ptxas' default register-usage heuristic (level >= 4) degenerates on the fully unrolled reverse-pass
-# kernels (32 registers + everything spilled to local memory); level 3 allocates normally.
-EXTRA_FLAGS = {"bwd_": ["-Xptxas", "-regUsageLevel=3"]}
 
 
 def _nvcc():
@@ -60,11 +57,7 @@ def _headers_digest():
 
 def _compile_one(args):
     src, obj, stamp, digest, verbose = args
-    flags = list(NVCC_FLAGS)
-    for prefix, extra in EXTRA_FLAGS.items():
-        if os.path.basename(src).startswith(prefix):
-            flags += extra
-    cmd = [_nvcc()] + flags + ["-I", CSRC, "-c", src, "-o", obj]
+    cmd = [_nvcc()] + NVCC_FLAGS + ["-I", CSRC, "-c", src, "-o", obj]
     if verbose:
         cmd.insert(1, "-Xptxas")
         cmd.insert(2, "-v")

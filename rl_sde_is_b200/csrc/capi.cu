@@ -59,7 +59,7 @@ static int cuda_fail(cudaError_t e, const char* where) {
 template <int D_, int H_>
 struct Shape {
   static constexpr int D = D_, H = H_;
-  static constexpr bool narrow = H == 32;          // K1, K1w, K2, K2m, K2w and the H = 32 tcgen05 forward (K1u)
+  static constexpr bool narrow = H == 32;          // K1, K1w, K2m, K2w and the H = 32 tcgen05 forward (K1u)
   static constexpr bool wide = H >= 64;            // K1x, K2x
   static constexpr bool umma_fwd_wide = H >= 64;   // the tcgen05 forward at H >= 64 (K1u)
   static constexpr bool umma_bwd = H >= 128;       // the tcgen05 reverse pass (K2u)
@@ -520,6 +520,7 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
   if (A.flags & RLSDE_F_STATE_F64) return RLSDE_ERR_UNSUPPORTED;   // the reference differentiates the f32 torch path only
   if (!(A.flags & RLSDE_F_STORE_PATH)) return RLSDE_ERR_INVALID_ARG;
   if (A.ckpt_every > BWD_MAX_SEG) return RLSDE_ERR_INVALID_ARG;        // the reverse pass recomputes at most 32 passes per checkpoint
+  if (cfg->bwd_kernel != 0 && cfg->bwd_kernel != 1) return RLSDE_ERR_UNSUPPORTED;   // the tensor-core kernel is the only one
   if ((A.flags & RLSDE_F_NOISE_INJECTED) && !noise_dev) return RLSDE_ERR_INVALID_ARG;
   A.noise = noise_dev;
   A.G = (void*)cS_dev; A.T = (int*)T_dev; A.path = (float*)path_dev;
@@ -551,11 +552,12 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
                            "rollout_bwd (wide) launch");
     } else {
       const bool warp_path = use_warp_kernels(A, S::H, sm, true);
-      // Large batches with a length-sorted order: the reverse pass of a trajectory is sequential, and K2 walks a lone
-      // trajectory at ~12 us per pass -- the longest few thousand trajectories, not the total work, set its run time
-      // (K = 4e5, longest 3 900 passes: 47 ms for ~28 ms of throughput work).  They go to the warp-per-trajectory kernel
-      // instead (~0.5 us per pass), the bulk stays in K2; the two gradients are added in a fixed order.  The split depends
-      // on the sorted lengths only, so the result is deterministic.
+      // Large batches with a length-sorted order: the reverse pass of a trajectory is sequential, and a thread-per-
+      // trajectory kernel walks a lone trajectory slowly (~12 us per pass for the CUDA-core kernel K2 this split was made
+      // for) -- the longest few thousand trajectories, not the total work, set its run time (K = 4e5, longest 3 900 passes:
+      // 47 ms for ~28 ms of throughput work).  They go to the warp-per-trajectory kernel instead (~0.5 us per pass), the bulk
+      // to the tensor-core kernel; the two gradients are added in a fixed order.  The split depends on the sorted lengths
+      // only, so the result is deterministic.
       long long n_long = 0;
       if (!warp_path && order_dev && A.ckpt_every == 1 && A.K > (long long)sm * 128) {
         // measured (K = 4e5, d = 1): 46.2 / 36.7 / 36.7 / 37.5 / 41.9 ms at 0 / 2 368 / 4 736 / 9 472 / 25 000 long trajectories
@@ -565,11 +567,6 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
       }
       FwdArgs Abulk = A;
       float* partial_aux = (float*)((char*)partial + bwd_partial_main_bytes());
-      // thread-per-trajectory family, hidden width 32: the tensor-core kernel (rollout_bwd_mma.cuh) unless the caller asks
-      // for the CUDA-core one (cfg.bwd_kernel == 2; kept for A/B measurements and as a second implementation in the tests)
-      // (state dimensions above 4: the d-sized products -- layer 1, head, dW1, dW3, dX -- run as padded 16-wide tiles on
-      // the tensor cores as well; d = 10: 16.3 ms against 26.1 ms at K = 2e5, 61 against 109 ms at K = 1e6)
-      const bool use_mma = cfg->bwd_kernel != 2;
       cudaEvent_t join = nullptr;
       int lrc = -1;                                         // an empty batch without long trajectories fails as a launch
       if (n_long > 0) {
@@ -578,11 +575,11 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
         Abulk.order = A.order + n_long;
         Abulk.K = A.K - n_long;
         Abulk.grad_accumulate = 1;
-        // the long trajectories run concurrently with the bulk on the second stream when the bulk's reduction can wait
-        // for them (tensor-core kernel); otherwise first, on the caller's stream
+        // the long trajectories run concurrently with the bulk on the second stream, and the bulk's reduction waits for
+        // them; without a second stream they run first, on the caller's stream
         cudaStream_t s_long = stream;
         cudaError_t e;
-        if (use_mma && Abulk.K > 0 && g_aux.get()) {
+        if (Abulk.K > 0 && g_aux.get()) {
           if ((e = cudaEventRecord(g_aux.fork, stream)) != cudaSuccess) return cuda_fail(e, "cudaEventRecord(fork)");
           if ((e = cudaStreamWaitEvent(g_aux.stream, g_aux.fork, 0)) != cudaSuccess) return cuda_fail(e, "cudaStreamWaitEvent(fork)");
           s_long = g_aux.stream;
@@ -595,13 +592,13 @@ static int rollout_bwd_impl(const rlsde_env* env, const rlsde_mlp* mlp, const fl
           join = g_aux.join;
         }
       }
+      // thread-per-trajectory family, hidden width 32: the tensor-core kernel (rollout_bwd_mma.cuh; state dimensions above
+      // 4: the d-sized products -- layer 1, head, dW1, dW3, dX -- run as padded 16-wide tiles on the tensor cores as well)
       if (Abulk.K > 0)
         lrc = warp_path ? launch_rollout_bwd_warp<S::D, WEIGHTED, RAGGED>(params_host, nullptr, Abulk, (float)loss_scale, grad_dev,
                                                                            partial, sm, stream)
-              : use_mma ? launch_rollout_bwd_mma<S::D, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial,
-                                                                          sm, stream, join)
-                        : launch_rollout_bwd<S::D, S::H, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial,
-                                                                            sm, stream);
+                        : launch_rollout_bwd_mma<S::D, WEIGHTED, RAGGED>(params_host, Abulk, (float)loss_scale, grad_dev, partial,
+                                                                         sm, stream, join);
       return launch_status(lrc, "rollout_bwd launch");
     }
   });

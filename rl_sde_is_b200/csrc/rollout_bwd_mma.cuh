@@ -1,11 +1,16 @@
 // K2m: reverse (adjoint) pass of the REINFORCE surrogate loss with the three 32 x 32 x 32 products of a warp-pass on the
 // tensor cores (hidden width 32).
 //
-// Same recursion, work assignment and checkpoint segments as K2 (rollout_bwd.cuh; SURVEY.md Appendix C; replaces
-// eff_loss.backward(), reinforce_deterministic_core.py:240).  What changes is where a warp's 32 trajectories live.  K2
-// keeps one trajectory per lane and stages (delta, activation) tiles in shared memory for an FFMA2 outer product: 3 717
-// instructions per warp-pass, 1 564 of them FFMA2, at 62 % issue utilisation (profiles/r01/ncu_rollout_bwd_v4.txt).
-// Here the activations of the 32 trajectories are held in mma.sync FRAGMENT layout across the warp (row = trajectory,
+// The recursion is rollout_bwd.cuh's (SURVEY.md Appendix C; replaces eff_loss.backward(), reinforce_deterministic_core.py:240).
+// Work assignment: one trajectory per lane, processed segment by segment from the last checkpoint backwards.  A round =
+// phase A (recompute the segment's states X_j from its checkpoint, identical arithmetic to K1) + phase B (walk the segment
+// in reverse: recompute the activations, backpropagate).  All lanes of a warp are in the same phase at the same time, so
+// the 32 trajectories stay in lock step although their lengths differ.  dB is regenerated from Philox, never stored.
+// Trajectories go to lanes statically, round robin over the length-sorted order, so the gradients are deterministic.
+//
+// The CUDA-core kernel this one replaced (K2, DESIGN.md) had the same assignment and staged (delta, activation) tiles in
+// shared memory for an FFMA2 outer product: 3 717 instructions per warp-pass, 1 564 of them FFMA2, at 62 % issue
+// utilisation (profiles/r01/ncu_rollout_bwd_v4.txt).  Here the activations of the 32 trajectories are held in mma.sync FRAGMENT layout across the warp (row = trajectory,
 // column = hidden unit), so that
 //     Z2  = H1  W2^T      (recomputed forward, layer 2)        M = trajectory, K = in,  N = out
 //     dH1 = dZ2 W2                                              M = trajectory, K = out, N = in

@@ -12,7 +12,7 @@
 //   * PRODUCER CTAs (about four fifths of the SMs) run the recursion.  Threads 0-127 own one trajectory each (= one TMEM
 //     lane), exactly as in K1u: layer 1 into the A-operand ring (float16 hi / lo), accumulator read back row by row.
 //     Sweep 1 reads Z2, applies bias + tanh, sums the head and parks h2 in the same tensor-memory columns; the owner then
-//     forms its a_j (K2's formula) and sweep 2 turns h2 into dz2 = (W3^T a)(1 - h2^2), which goes -- scaled by a power of
+//     forms its a_j (rollout_bwd.cuh's formula) and sweep 2 turns h2 into dz2 = (W3^T a)(1 - h2^2), which goes -- scaled by a power of
 //     two 2^esh chosen per launch from max |G| (ub_scale_kernel) so that float16 holds it, hi / lo -- into the A ring again; sweep 3 reads
 //     dH1, forms dz1 and dX and updates the adjoint.  Warp 4 issues the MMAs, warp 5 streams both weight images
 //     (W2 as [out][in] and as [in][out]) through the mbarrier ring, as in K1u.
@@ -486,7 +486,7 @@ rollout_bwd_umma_kernel(const float* __restrict__ Wp, const uint8_t* __restrict_
         bar_owners();
         UB_T(3);
 
-        // ---- a_j (K2's formula; zero for rows that are not on a trajectory this pass)
+        // ---- a_j (rollout_bwd.cuh's formula; zero for rows that are not on a trajectory this pass)
         float a[D], dB[D];
         nc.get(A, inject, live, traj, j, dB);
 #pragma unroll

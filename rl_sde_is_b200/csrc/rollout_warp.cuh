@@ -8,7 +8,7 @@
 // ~400 cycles (forward) instead of the ~5 500 cycles a lone warp of the thread-per-trajectory kernel needs
 // (there, every FFMA2 pair waits for an LDCU.128: profiles/r01/README.md).
 //
-// Semantics are those of K1 / K2 (rollout_fwd.cuh, rollout_bwd.cuh): same per-pass arithmetic with the
+// Semantics are those of K1 and of the reverse pass (rollout_fwd.cuh, rollout_bwd.cuh): same per-pass arithmetic with the
 // reference's association for the environment step, same Philox stream, same outputs.  The dot products are
 // summed in a different order than in K1, so per-trajectory values agree with K1 to rounding (~1e-6 relative),
 // not bit for bit; the reverse kernel recomputes the forward pass with THIS kernel's arithmetic.

@@ -1,10 +1,21 @@
 // Launchers + explicit instantiation helper for the warp-per-trajectory kernels of one state dimension D (H = 32).
 #pragma once
 #include <cstring>
-#include "rollout_bwd_inst.cuh"
+#include "rollout_bwd.cuh"
 #include "rollout_warp.cuh"
 
 namespace rlsde {
+
+// grad[p] (+)= scale * sum_w partial[w][p], warps in index order
+static __global__ void bwd_reduce_kernel(const float* __restrict__ partial, int n_warps, int P, float scale, float* __restrict__ grad,
+                                         int accumulate) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= P) return;
+  double acc = 0.0;
+  for (int w = 0; w < n_warps; ++w) acc += (double)partial[(long long)w * P + p];
+  const float g = (float)(acc * (double)scale);
+  grad[p] = accumulate ? grad[p] + g : g;
+}
 
 static inline long long warp_grid(long long K, int sm_count) {
   long long g = (K + 3) / 4;

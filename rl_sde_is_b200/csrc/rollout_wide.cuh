@@ -2,7 +2,7 @@
 // reinforce_deterministic_core.py:102), where the hidden-hidden layer no longer fits a thread's registers or the
 // constant bank and a pass becomes a small dense contraction per TILE of trajectories.
 //
-// Same semantics, Philox stream and outputs as K1 / K2 (rollout_fwd.cuh, rollout_bwd.cuh); what changes is the mapping:
+// Same semantics, Philox stream and outputs as K1 and the reverse pass (rollout_fwd.cuh, rollout_bwd.cuh); what changes is the mapping:
 //   * a block of 128 threads advances a tile of M = 32 (or 16) trajectories in lock step; warp w owns rows
 //     R w .. R w + R - 1 of the tile (R = 8 or 4), lane l owns the hidden units l, l + 32, l + 64, ...;
 //   * activations of the tile live in shared memory unit-major ([unit][trajectory], rows padded to 36 floats: row

@@ -1,7 +1,7 @@
 """Deterministic-policy REINFORCE on the fused rollout kernels (drop-in for the reference module).
 
 Reference: rl_sde_is/reinforce_deterministic_core.py
-  * ``sample_loss_vectorized(env, model, K)`` (:30-93)  -> one K1 launch (+ K2 when ``.backward()`` runs)
+  * ``sample_loss_vectorized(env, model, K)`` (:30-93)  -> one K1 launch (+ the reverse pass when ``.backward()`` runs)
   * ``reinforce(env, ...)`` (:102-336)                  -> same arguments, same keys in the returned dict
   * ``sample_returns_vectorized(env, model, K)``        -> (G, S) with a ``grad_fn``: train any loss over them
 

@@ -427,7 +427,7 @@ def rollout_forward_stored(env_c, mlp_c, params_host, K, *, ckpt_every=1, **opts
 
 def rollout_backward(env_c, mlp_c, params_host, fwd: RolloutOut, loss_scale, *, noise=None, device=None, balance=True,
                      coef=None):
-    """K2: gradient of loss_scale * sum_k(-G_k - sg(G_k) S_k) w.r.t. the flat parameters (float32 CUDA tensor).
+    """The reverse pass: gradient of loss_scale * sum_k(-G_k - sg(G_k) S_k) w.r.t. the flat parameters (float32 CUDA tensor).
 
     With ``coef=(coef_G, coef_S)`` (float32 CUDA tensors [K] on the rollout's device) the gradient is that of
     loss_scale * sum_k (coef_G[k] G_k + coef_S[k] S_k) instead (rlsde_rollout_bwd_weighted; unfinished trajectories
@@ -475,7 +475,7 @@ def rollout_loss_and_grad(env_c, mlp_c, params_host, K, *, seed=0, n_steps_lim=1
                           stoch_int="reference", ckpt_every=1, device=None, kernel="auto", balance=True, tuning=None,
                           dist=None):
     """One REINFORCE evaluation with a single host synchronisation: K1 (with checkpoints), the statistics reduction and
-    K2 are enqueued back to back, and loss numerator, gradient, returns and hit indices come back in ONE device-to-host
+    the reverse pass are enqueued back to back, and loss numerator, gradient, returns and hit indices come back in ONE device-to-host
     copy.  (The autograd route -- sample_loss_vectorized + .backward() -- synchronises after each kernel; at the
     reference's K = 100 those round trips cost as much as the kernels.)
 

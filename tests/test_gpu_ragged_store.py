@@ -166,11 +166,11 @@ def test_reverse_matches_dense_store(family, d, H, ckpt):
     _bwd_bitwise(env_c, mlp_c, flat, noise, dense, rag, seed=d + H + ckpt)
 
 
-@pytest.mark.parametrize("bulk", ["K2", "K2m"])
-def test_reverse_split_between_families(bulk):
-    """The longest trajectories on the warp kernel, the rest on K2 / K2m."""
+@pytest.mark.parametrize("bulk,d", [("K2m", 1), ("K2m", 2)])
+def test_reverse_split_between_families(bulk, d):
+    """The longest trajectories on the warp kernel, the rest on K2m."""
     n_sm = torch.cuda.get_device_properties(0).multi_processor_count
-    pair = _bwd_pair(bulk, 1, 32, 1, K=128 * n_sm + 200, lim=300, extra_cfg={"bwd_warp_share": 1000})
+    pair = _bwd_pair(bulk, d, 32, 1, K=128 * n_sm + 200, lim=300, extra_cfg={"bwd_warp_share": 1000})
     _bwd_bitwise(*pair, seed=3)
 
 

@@ -32,7 +32,7 @@ OPTIONAL = {"noise", "policy_opt", "l2", "logw", "stats", "order"}
 
 def call(entry, d=1, H=32, n_hidden=2, d_in=None, env=True, dt=DT, sigma=np.sqrt(2.0), hit_rule=L.HIT_ALL_GE_LB,
          flags=None, C=1, stride=100, K=64, K_global=None, traj_offset=0, noise_steps=0, n_steps_lim=100, fwd_policy=0,
-         n_grid=401, grid_h=0.01, ws=None, null=(), set_=(), step_t=1):
+         bwd_kernel=0, n_grid=401, grid_h=0.01, ws=None, null=(), set_=(), step_t=1):
     lib = L.load()
     if flags is None:              # the reverse passes and the device-resident step need the checkpoint store
         flags = P if entry.startswith("bwd") or entry.startswith("reinforce") else 0
@@ -47,7 +47,7 @@ def call(entry, d=1, H=32, n_hidden=2, d_in=None, env=True, dt=DT, sigma=np.sqrt
     if "cfg" not in null:
         c = L.RlsdeRolloutCfg()
         c.K, c.K_global, c.traj_offset, c.n_steps_lim, c.flags = K, K if K_global is None else K_global, traj_offset, n_steps_lim, flags
-        c.noise_steps, c.ckpt_every, c.ckpt_stride, c.fwd_policy = noise_steps, C, stride, fwd_policy
+        c.noise_steps, c.ckpt_every, c.ckpt_stride, c.fwd_policy, c.bwd_kernel = noise_steps, C, stride, fwd_policy, bwd_kernel
         c.n_grid, c.grid_lo, c.grid_hi, c.grid_h = n_grid, -2.0, 2.0, grid_h
     optional = OPTIONAL - {"stats"} if entry.startswith("reinforce") else OPTIONAL
     p = {name: (0 if name in null or (name in optional and name not in set_) else FAKE) for name in PTRS[entry]}
@@ -133,6 +133,7 @@ TABLE = [
     (MLP_ENTRIES + ("fwd_table",), "noise_steps_zero", dict(flags=NOISE, noise_steps=0), INVALID),
     (MLP_ENTRIES + ("fwd_table",), "shard_outside_batch", dict(flags=NOISE, noise_steps=100, traj_offset=8, K_global=64), INVALID),
     (MLP_ENTRIES + ("fwd_table",), "fwd_policy_3", dict(fwd_policy=3), INVALID),
+    (REVERSE, "bwd_kernel_2", dict(bwd_kernel=2), UNSUPPORTED),
     (("fwd", "fwd_ragged", "transitions", "fwd_table"), "noise_null", dict(flags=NOISE, noise_steps=100), INVALID),
     (REVERSE + REINFORCE, "noise_null", dict(flags=NOISE | P, noise_steps=100), INVALID),
     (("fwd", "bwd", "bwd_weighted", "reinforce_step", "reinforce_rollout"), "stride_below_budget",
